@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — ORB front-end throughput on B200 (contract: one JSON line on stdout from rank 0).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--no-knn2]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--no-knn2] [--dump-outputs DIR]
 
 Workload (BASELINE.json metric "ORB extract frames/s (752x480, 1000kp) & 2-NN Hamming compares/s"):
   * main line: batched ORBextractor::operator() on synthetic 752x480 frames, nFeatures=1000, 8 levels, scale 1.2,
@@ -13,6 +13,9 @@ Workload (BASELINE.json metric "ORB extract frames/s (752x480, 1000kp) & 2-NN Ha
   * "cfg4" block: BASELINE.json configs[3] as written — 8192 synthetic 1280x720 frames, 2000 features each, frame range
     [r*F/G, (r+1)*F/G) on rank r (strong scaling, no collective on the data path), resident and host-fed, with a checksum of
     all keypoints / descriptors reduced over the ranks and compared with the value a single GPU produced.
+  * --dump-outputs DIR: after the timed steps, what the last resident extraction step and the 2-NN pass returned, as
+    DIR/<name>.npy in float32 / float64 (a fixed sample of the frames; about 25 MB), so that two builds can be compared output
+    for output.  The inputs are synthetic and seeded: the same arguments give the same inputs on every run.
   * --impl reference: the CPU oracle (a restatement of the reference's CPU path; the reference itself cannot be
     compiled here, see DESIGN.md) on all host threads, same metric / config.  That arm never loads the CUDA library.
 """
@@ -27,10 +30,45 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # a benchmark run writes nothing into the tree (which may be read-only)
 
 COLS, ROWS, NFEAT, NLEVELS, SCALE, INI_TH, MIN_TH = 752, 480, 1000, 8, 1.2, 20, 7
 NQ, NDB = 100_000, 10_000_000
 METRIC = "orb_extract_frames_per_s_752x480_1000kp"
+DUMP_FRAMES, DUMP_QUERIES = 128, 100_000       # --dump-outputs sample sizes: ~21 MB of extraction + ~4 MB of 2-NN results
+
+
+def dump_sample(n, k, seed):
+    """Ascending indices of a fixed, seeded sample of k of n rows (all rows when n <= k)."""
+    import numpy as np
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def extraction_outputs(d_kps, d_desc, d_n, d_nm):
+    """What one resident extraction step hands its caller, as float arrays: keypoint and monocular counts of every frame and,
+    for a sample of the frames, the keypoint rows (x, y, size, angle, response | octave, class_id) and the descriptor bytes,
+    zero past each frame's count."""
+    import numpy as np
+    import torch
+    n = d_n.cpu().numpy()
+    frames = dump_sample(len(n), DUMP_FRAMES, seed=0)
+    sel = torch.as_tensor(frames, device=d_kps.device)
+    kps, desc = d_kps[sel].cpu().numpy(), d_desc[sel].cpu().numpy()
+    valid = (np.arange(kps.shape[1])[None, :] < n[frames, None])[..., None]
+    return {"extract_n_keypoints": n.astype(np.float64), "extract_n_mono": d_nm.cpu().numpy().astype(np.float64),
+            "extract_sample_frames": frames.astype(np.float64),
+            "extract_keypoints": np.where(valid, kps[..., :5], 0).astype(np.float32),
+            "extract_keypoint_octave_class_id": np.where(valid, kps[..., 5:].view(np.int32), 0).astype(np.float32),
+            "extract_descriptors": np.where(valid, desc, 0).astype(np.float32)}
+
+
+def write_outputs(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def level_sizes():
@@ -275,6 +313,7 @@ def run_ours(args, rank, world, local_rank):
     torch.cuda.synchronize()
     ms = ev0.elapsed_time(ev1)
     launches = lib().orbx_launch_count() - launches0
+    outputs = extraction_outputs(d_kps, d_desc, d_n, d_nm) if args.dump_outputs and rank == 0 else None
     # per-stage device times: the same K steps again with CUDA events between the stages (kept out of the timed region above)
     ex.profile_begin()
     for _ in range(args.steps):
@@ -406,7 +445,7 @@ def run_ours(args, rank, world, local_rank):
     # ---- 2-NN Hamming: 100k x 10M, database sharded over the ranks, NCCL all-gather + merge -------------------------------
     knn = None
     if not args.no_knn2:
-        knn = run_knn2(args, rank, world, local_rank, dev, barrier, max_over_ranks)
+        knn = run_knn2(args, rank, world, local_rank, dev, barrier, max_over_ranks, outputs)
 
     # ---- CPU baseline (rank 0, N=1 only): the oracle on all host threads, bounded sample -----------------------------------
     cpu = None
@@ -422,6 +461,9 @@ def run_ours(args, rank, world, local_rank):
         if hyb is not None:
             hyb["frames_per_s_all_threads_if_it_scaled_perfectly"] = hyb["frames_per_s_one_thread"] * threads
             cpu["cv2_simd_hybrid"] = hyb
+
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
 
     if rank == 0:
         line = {
@@ -684,7 +726,7 @@ def knn2_roofline(per_gpu, popc_peak):
                     "peak = orbx_measure_popc_peak microbenchmark on this GPU"}
 
 
-def run_knn2(args, rank, world, local_rank, dev, barrier, max_over_ranks):
+def run_knn2(args, rank, world, local_rank, dev, barrier, max_over_ranks, outputs=None):
     """BASELINE.json configs[4]: 100k queries x 10M database rows, database sharded over the ranks.  The whole exchange is inside
     the C ABI: orbx_knn2_sharded = local scan + ONE ncclAllGather of the packed candidates + merge (csrc/api_shard.cu); torch
     only carries rank 0's NCCL id to the other ranks.  The merged answer is verified on every rank (see `verified`)."""
@@ -730,6 +772,11 @@ def run_knn2(args, rank, world, local_rank, dev, barrier, max_over_ranks):
     torch.cuda.synchronize()
     ms = max_over_ranks(ev0.elapsed_time(ev1))
     launches = lib().orbx_launch_count() - l0
+    if outputs is not None:
+        qsel = dump_sample(nq, DUMP_QUERIES, seed=1)
+        sel = torch.as_tensor(qsel, device=dev)
+        outputs.update({"knn2_sample_queries": qsel.astype(np.float64), "knn2_idx": out_idx[sel].cpu().numpy().astype(np.float64),
+                        "knn2_dist": out_dist[sel].cpu().numpy().astype(np.float64)})
     compares = float(nq) * float(ndb) * reps
     cps = compares / (ms * 1e-3)
     popc_peak = orbx.measure_popc_peak(local_rank)
@@ -810,7 +857,13 @@ def main():
     ap.add_argument("--knn-nq", type=int, default=NQ)
     ap.add_argument("--knn-ndb", type=int, default=NDB)
     ap.add_argument("--knn-reps", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last resident extraction step and "
+                    "the 2-NN pass returned as DIR/<name>.npy (float32 / float64, a fixed sample of the frames; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 0)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -3,18 +3,23 @@
 #
 # The reference as a whole cannot be built here (OpenCV / OpenCL / boost / Eigen / Sophus headers and its cmake build are not in
 # this image), but the functions that carry the reference-owned logic of the path are plain C++ over a handful of OpenCV
-# containers.  This recipe slices them — by line range, from the sources WHERE THEY LIE under /root/reference, at build time —
+# containers.  This recipe slices them — by line range, from the sources WHERE THEY LIE in the kpmrozowski/wut-cuda-orb-slam3
+# checkout named by ORB_REFERENCE_ROOT, at build time —
 # into oracle/_ref/gen/*.inc (git-ignored, never committed) and compiles them against oracle/ref_shim/ (container types only;
 # the one OpenCV algorithm a slice calls, cv::FAST, is forwarded to the cv2-pinned oracle).  tests/test_ref_pin.py then checks
-# the oracle against this library and tests/golden/make_ref_golden.py freezes its answers as fixtures for the GPU box.
+# the oracle against this library and tests/golden/make_ref_golden.py freezes its answers as fixtures (tests/golden/ref_golden.json)
+# that tests/test_golden.py checks without the reference.
 #
-# Without /root/reference (the GPU box) the script keeps whatever oracle/_ref/libref.so travelled with the snapshot.
+# Without ORB_REFERENCE_ROOT the script builds nothing (and says so); tests/test_ref_pin.py, tests/test_gpu_ref.py and the
+# reference check of tests/test_gpu_round2.py then compare with the reference's stored answers (tests/golden/ref_pin_golden.json)
+# instead of the live library, and the Frame call-site test skips.
 set -e
 HERE=$(cd "$(dirname "$0")" && pwd)
-REF=${ORB_REFERENCE_ROOT:-/root/reference}
+REF=${ORB_REFERENCE_ROOT:-}
 OUT="$HERE/_ref"
-if [ ! -d "$REF/src" ]; then
-    echo "build_ref: $REF not present, keeping prebuilt $OUT/libref.so (if any)"
+if [ -z "$REF" ] || [ ! -d "$REF/src" ]; then
+    echo "build_ref: set ORB_REFERENCE_ROOT to a kpmrozowski/wut-cuda-orb-slam3 checkout to build oracle/_ref/libref.so;" \
+         "without it the reference tests use the stored answers in tests/golden/ref_pin_golden.json"
     exit 0
 fi
 mkdir -p "$OUT/gen"
@@ -59,7 +64,7 @@ $CXX -O3 -std=c++17 -fPIC -ffp-contract=off -w -I"$HERE/ref_shim" -I"$OUT/gen" -
     "$HERE/ref_shim/ref_wrapper.cpp" "$HERE/ref_shim/ref_dbow2_wrapper.cpp" -L"$HERE/_build" -lorb_oracle -Wl,-rpath,'$ORIGIN/../_build'
 echo "build_ref: built $OUT/libref.so from $REF"
 # The reference's call site of the extractor (Frame ctor accessor block + Frame::ExtractORB) compiled UNCHANGED against the
-# drop-in adapter header; linked against the product library, run on the GPU box by tests/test_gpu_ref.py.
+# drop-in adapter header; linked against the product library, run on the GPU by tests/test_gpu_round2.py.
 ROOT=$(cd "$HERE/.." && pwd)
 if [ -f "$ROOT/wut_cuda_orb_slam3_b200/liborbx.so" ]; then
     $CXX -O2 -std=c++17 -w -pthread -I"$ROOT/tests/cpp/cv_stub" -I"$ROOT/include" -I"$ROOT/wut_cuda_orb_slam3_b200/csrc/adapter" -I"$OUT/gen" \

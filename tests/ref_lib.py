@@ -1,8 +1,11 @@
-"""ctypes binding of oracle/_ref/libref.so — the REFERENCE's own functions of the hot path, compiled from the sources where
-they lie by oracle/build_ref.sh (this container only; the built library travels to the GPU box).  TEST INFRASTRUCTURE ONLY."""
+"""ctypes binding of oracle/_ref/libref.so — the REFERENCE's own functions of the hot path, compiled by oracle/build_ref.sh from
+the reference checkout named by ORB_REFERENCE_ROOT — and Pin, which compares with the reference's answers: live when the library
+is built, else with the CRCs of those answers stored in tests/golden/ref_pin_golden.json.  TEST INFRASTRUCTURE ONLY."""
 import ctypes as C
+import json
 import os
 import subprocess
+import zlib
 
 import numpy as np
 
@@ -18,10 +21,65 @@ def _p(a):
 
 
 def available():
-    if not os.path.exists(SO) and os.path.isdir("/root/reference/src"):
+    if not os.path.exists(SO) and os.path.isdir(os.path.join(os.environ.get("ORB_REFERENCE_ROOT", ""), "src")):
         subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle")])
         subprocess.check_call(["sh", os.path.join(ROOT, "oracle", "build_ref.sh")])
     return os.path.exists(SO)
+
+
+GOLDEN = os.path.join(ROOT, "tests", "golden", "ref_pin_golden.json")
+_golden = None
+
+
+def crc(arrays):
+    c = 0
+    for a in arrays:
+        c = zlib.crc32(np.ascontiguousarray(a).tobytes(), c)
+    return c & 0xFFFFFFFF
+
+
+class Pin:
+    """pin(part, got, want): `got` is a list of arrays computed by the oracle or the CUDA path, `want` the same list from the
+    reference library, or None when libref.so is not built.  With `want`, every array must equal its counterpart (shape and
+    values); without it, the CRC of `got` must equal the CRC stored for this test and part, which is the CRC of the
+    reference's answer.  With ORBX_REF_PIN_RECORD=<file> set, each live comparison that passes records that CRC there (how
+    tests/golden/ref_pin_golden.json is regenerated where the reference is built)."""
+
+    def __init__(self, test_name):
+        self.test_name = test_name
+
+    def __call__(self, part, got, want):
+        global _golden
+        key = self.test_name + ":" + part
+        got = [np.ascontiguousarray(a) for a in got]
+        if want is None:
+            if _golden is None:
+                with open(GOLDEN) as f:
+                    _golden = json.load(f)["crc32"]
+            assert key in _golden, "no stored reference answer for " + key
+            assert crc(got) == _golden[key], "differs from the reference's stored answer: " + key
+            return
+        assert len(got) == len(want), key
+        for i, (a, b) in enumerate(zip(got, want)):
+            b = np.ascontiguousarray(b)
+            assert a.shape == b.shape and np.array_equal(a, b), (key, i)
+        path = os.environ.get("ORBX_REF_PIN_RECORD")
+        if path:
+            rec = json.load(open(path)) if os.path.exists(path) else {}
+            rec[key] = crc(got)
+            with open(path, "w") as f:
+                json.dump(rec, f, indent=1, sort_keys=True)
+
+
+def invz(z):
+    """1.0 / z as refc_search_by_projection_last hands it to the compared side (double division, stored as float)."""
+    return (1.0 / np.asarray(z, np.float64)).astype(np.float32)
+
+
+def dist3d(u, v, z):
+    """|(u, v, z)| as refc_search_by_projection_kf hands it to the compared side (float, left-to-right, no contraction)."""
+    u, v, z = (np.asarray(a, np.float32) for a in (u, v, z))
+    return np.sqrt(u * u + v * v + z * z).astype(np.float32)
 
 
 class Ref:

@@ -77,7 +77,7 @@ def test_cuda_knn2_golden():
 
 def test_oracle_reproduces_reference_golden(oracle):
     """tests/golden/ref_golden.json holds answers of the REFERENCE's own compiled functions (oracle/_ref, made by
-    tests/golden/make_ref_golden.py in the dev container); the oracle must reproduce every one of them."""
+    tests/golden/make_ref_golden.py where the reference is built); the oracle must reproduce every one of them."""
     import json
     import os
 
