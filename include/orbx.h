@@ -413,6 +413,18 @@ int orbx_search_by_projection_kf(int device, const orbx_frame_view* cur, int n_k
                                  const float* v, const float* dist3d, const float* min_dist, const float* max_dist,
                                  const int32_t* level, const float* angle, const uint8_t* desc, float th, int orb_dist,
                                  int check_orientation, int32_t* match_f, int* n_matches);
+/* int ORBmatcher::SearchForInitialization(Frame &F1, Frame &F2, vector<cv::Point2f> &vbPrevMatched, vector<int> &vnMatches12,
+ * int windowSize) — src/ORBmatcher1.cc:650-765, as Tracking::MonocularInitialization calls it (src/Tracking3.cc:740-741).
+ *   kp1 / desc1 = F1.mvKeysUn / F1.mDescriptors (n1 rows); only features with octave <= 0 search (the reference skips level1 > 0),
+ *   in GetFeaturesInArea(vbPrevMatched[i1], windowSize, level1, level1) of f2 (f2->u_right, f2->occupied and the scale factors
+ *   are not read).  Best / second-best with the vMatchedDistance skip, TH_LOW and 'bestDist < (float)bestDist2 * mfNNratio' (no
+ *   second-best always passes); a later feature of F1 that reaches an F2 feature at a smaller distance takes it over.
+ *   prev_matched = vbPrevMatched [n1][2] (x, y), in/out: matched entries become F2.mvKeysUn[vnMatches12[i1]].pt.
+ * Output: matches12[n1] = vnMatches12 (after the rotation filter when check_orientation), *n_matches = the return value.
+ * ORBX_ERR_INVALID_ARG for a keypoint angle pair outside the histogram (the reference asserts). */
+int orbx_search_for_initialization(int device, const orbx_keypoint* kp1, const uint8_t* desc1, int n1, const orbx_frame_view* f2,
+                                   float* prev_matched, int window_size, float nn_ratio, int check_orientation, int32_t* matches12,
+                                   int* n_matches);
 /* Speculation rounds the last projection search on this thread needed (diagnostics; 0 = every query was final at once). */
 int orbx_projection_rounds(void);
 

@@ -91,6 +91,7 @@ SIGNATURES = {
     "orbx_search_by_projection_map": (_i, [_i, _vp, _vp, _f, _i, _f, _f, _vp, _vp]),
     "orbx_search_by_projection_last": (_i, [_i, _vp, _f, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _i, _i, _i, _vp, _vp]),
     "orbx_search_by_projection_kf": (_i, [_i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _i, _i, _vp, _vp]),
+    "orbx_search_for_initialization": (_i, [_i, _vp, _vp, _i, _vp, _vp, _i, _f, _i, _vp, _vp]),
     "orbx_projection_rounds": (_i, []),
     "orbx_undistort_keypoints": (_i, [_i, _vp, _i, _vp, _vp, _i, _vp, _vp]),
     "orbx_rectifier_create": (_i, [_i, _vp, _vp, _sz, _i, _i, C.POINTER(_vp)]),

@@ -11,9 +11,10 @@
 //   int SearchByProjection(Frame& Current, const Frame& Last, th, bMono)             src/ORBmatcher3.cc:256-467
 //   int SearchByBoW(KeyFrame*, Frame&, vector<MapPoint*>& vpMapPointMatches)         src/ORBmatcher1.cc:225-427
 //   int SearchByBoW(KeyFrame*, KeyFrame*, vector<MapPoint*>& vpMatches12)            src/ORBmatcher2.cc:36-171
+//   int SearchForInitialization(Frame&, Frame&, vector<cv::Point2f>&, vector<int>&, windowSize)   src/ORBmatcher1.cc:650-765
 // Not declared (not on the tracking path / out of scope, DESIGN.md §8): the Sim3 SearchByProjection overloads,
-// SearchForInitialization, SearchBySim3, Fuse; SearchForTriangulation is exported by the C ABI (orbx_search_for_triangulation)
-// and takes F12 from the caller.
+// SearchBySim3, Fuse; SearchForTriangulation is exported by the C ABI (orbx_search_for_triangulation) and takes F12 from the
+// caller.
 #ifndef ORBMATCHER_H
 #define ORBMATCHER_H
 
@@ -64,6 +65,12 @@ public:
             }
         }
         return orbx_adapter::SearchByProjectionLast(CurrentFrame, LastFrame, u, v, invz, th, bForward, bBackward, mbCheckOrientation, device);
+    }
+
+    // Matching for the Map Initialization (only used in the monocular case)
+    int SearchForInitialization(Frame& F1, Frame& F2, std::vector<cv::Point2f>& vbPrevMatched, std::vector<int>& vnMatches12, int windowSize = 10)
+    {
+        return orbx_adapter::SearchForInitialization(F1, F2, vbPrevMatched, vnMatches12, windowSize, mfNNratio, mbCheckOrientation, device);
     }
 
     // Search matches between MapPoints in a KeyFrame and ORB in a Frame.

@@ -7,6 +7,8 @@
 //                                      const float thFarPoints)                                     src/ORBmatcher1.cc:45-215
 //   int ORBmatcher::SearchByProjection(Frame &CurrentFrame, const Frame &LastFrame, const float th, const bool bMono)
 //                                                                                                   src/ORBmatcher3.cc:256-467
+//   int ORBmatcher::SearchForInitialization(Frame &F1, Frame &F2, vector<cv::Point2f> &vbPrevMatched, vector<int> &vnMatches12,
+//                                           int windowSize)                                        src/ORBmatcher1.cc:650-765
 // by one-line calls of the functions below (Nleft == -1 rigs; a two-fisheye rig keeps the reference code).
 #pragma once
 #include <cstring>
@@ -95,6 +97,28 @@ inline int SearchByProjectionLast(FrameT& CurrentFrame, const FrameT& LastFrame,
           "SearchByProjection");
     for (int j = 0; j < CurrentFrame.N; ++j)
         if (matchF[j] >= 0) CurrentFrame.mvpMapPoints[j] = LastFrame.mvpMapPoints[matchF[j]];
+    return n;
+}
+
+// ORBmatcher::SearchForInitialization(Frame& F1, Frame& F2, vector<cv::Point2f>& vbPrevMatched, vector<int>& vnMatches12,
+// windowSize) — src/ORBmatcher1.cc:650-765.  `PointT` = cv::Point2f, handed to the C ABI as its [n][2] floats.
+template <class FrameT, class PointT>
+inline int SearchForInitialization(FrameT& F1, FrameT& F2, std::vector<PointT>& vbPrevMatched, std::vector<int>& vnMatches12, int windowSize,
+                                   const float mfNNratio, const bool mbCheckOrientation, int device = 0)
+{
+    static_assert(sizeof(PointT) == 8, "cv::Point2f must be two packed floats");
+    static_assert(sizeof(F1.mvKeysUn[0]) == sizeof(orbx_keypoint), "cv::KeyPoint must be the 28-byte POD");
+    const int n1 = (int)F1.mvKeysUn.size();
+    if ((int)vbPrevMatched.size() < n1) throw std::runtime_error("SearchForInitialization: vbPrevMatched is shorter than F1.mvKeysUn");
+    vnMatches12.assign(n1, -1);
+    const std::vector<uint8_t> none;
+    orbx_frame_view fv = view_of(F2, none);
+    fv.occupied = nullptr; fv.u_right = nullptr;                                // not read by this search
+    int n = 0;
+    check(orbx_search_for_initialization(device, reinterpret_cast<const orbx_keypoint*>(F1.mvKeysUn.data()), n1 ? F1.mDescriptors.ptr(0) : nullptr,
+                                         n1, &fv, reinterpret_cast<float*>(vbPrevMatched.data()), windowSize, mfNNratio, mbCheckOrientation,
+                                         vnMatches12.data(), &n),
+          "SearchForInitialization");
     return n;
 }
 

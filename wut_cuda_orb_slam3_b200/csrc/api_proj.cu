@@ -5,6 +5,7 @@
 //   ORBmatcher::SearchByProjection(Frame&, vector<MapPoint*>&, ...)      src/ORBmatcher1.cc:45-215   (Tracking::SearchLocalPoints)
 //   ORBmatcher::SearchByProjection(Frame& Current, const Frame& Last..)  src/ORBmatcher3.cc:256-467  (Tracking::TrackWithMotionModel)
 //   ORBmatcher::SearchByProjection(Frame& Current, KeyFrame*, ...)       src/ORBmatcher3.cc:469-578  (Tracking::Relocalization)
+//   ORBmatcher::SearchForInitialization(F1, F2, vbPrevMatched, ...)      src/ORBmatcher1.cc:650-765  (Tracking::MonocularInitialization)
 // Each entry point turns the reference's per-map-point pre-checks into window queries (float arithmetic in the reference's
 // order, on the host: a handful of operations per point), ships everything in ONE pinned staging copy, runs the grid build and
 // the window search (kernels_proj.cu) and reads the per-query assignment back in one copy.  The 30-bin rotation histogram runs
@@ -88,7 +89,7 @@ struct Session {
     Lease L;
     ProjArgs A{};
     size_t o_kp = 0, o_desc = 0, o_ur = 0, o_taken = 0, o_q = 0, o_qd = 0, o_cs = 0, o_items = 0, o_cellof = 0, o_claim = 0, o_keys = 0,
-           o_qm = 0, o_la = 0, o_lb = 0, o_rounds = 0, o_area = 0, o_area_n = 0;
+           o_qm = 0, o_la = 0, o_lb = 0, o_rounds = 0, o_area = 0, o_area_n = 0, o_last_acc = 0, o_prev_acc = 0, o_acc_dist = 0;
     int n = 0, nq = 0, area_cap = 0;
     explicit Session(int device) : L(device) {}
 
@@ -100,7 +101,8 @@ struct Session {
         n = f->n; nq = n_queries; area_cap = area_capacity;
         const size_t total = pad((size_t)n * 28) + pad((size_t)n * 32) + pad((size_t)n * 4) + pad((size_t)n * 4) + pad((size_t)nq * sizeof(ProjQuery)) +
                              pad((size_t)nq * 32) + pad((GRID_CELLS + 1) * 4) + pad((size_t)n * 4) + pad((size_t)n * 2) + pad((size_t)n * 4) +
-                             pad((size_t)nq * 16) + 3 * pad((size_t)nq * 4) + pad(4) + pad((size_t)area_cap * 8) + pad(4);
+                             pad((size_t)nq * 16) + 3 * pad((size_t)nq * 4) + pad(4) + pad((size_t)area_cap * 8) + pad(4) +
+                             pad((size_t)n * 4) + 2 * pad((size_t)nq * 4);
         if ((rc = L.reserve(total))) return rc;
         // upload range
         o_kp = L.take<orbx_keypoint>(n);
@@ -122,6 +124,9 @@ struct Session {
         o_lb = L.take<int>(nq);
         o_rounds = L.take<int>(1);
         o_area = L.take<unsigned long long>(area_cap);
+        o_last_acc = L.take<int>(n);
+        o_prev_acc = L.take<int>(nq);
+        o_acc_dist = L.take<int>(nq);
         if (n) memcpy(L.host<orbx_keypoint>(o_kp), f->keys_un, (size_t)n * sizeof(orbx_keypoint));
         if (n && with_desc) memcpy(L.host<uint8_t>(o_desc), f->descriptors, (size_t)n * 32);
         if (n && f->u_right) memcpy(L.host<float>(o_ur), f->u_right, (size_t)n * 4);
@@ -136,6 +141,11 @@ struct Session {
         A.keys = L.dev<unsigned long long>(o_keys); A.qmatch = L.dev<int>(o_qm); A.list_a = L.dev<int>(o_la); A.list_b = L.dev<int>(o_lb);
         A.rounds_out = L.dev<int>(o_rounds);
         return ORBX_OK;
+    }
+    // Mode 2 keeps the acceptances of each feature as a chain; the grid build resets last_acc (before upload_and_grid()).
+    void enable_chains()
+    {
+        A.last_acc = L.dev<int>(o_last_acc); A.prev_acc = L.dev<int>(o_prev_acc); A.acc_dist = L.dev<int>(o_acc_dist);
     }
     ProjQuery* queries() { return L.host<ProjQuery>(o_q); }
     uint8_t* qdesc() { return L.host<uint8_t>(o_qd); }
@@ -374,6 +384,73 @@ int orbx_search_by_projection_kf(int device, const orbx_frame_view* cur, int n_k
     memcpy(S.qdesc(), desc, (size_t)n_kf * 32);
     if ((rc = S.search(1, orb_dist, 0.0f))) return rc;
     return finish_1nn(S, cur, angle, check_orientation, match_f, n_matches);
+}
+
+int orbx_search_for_initialization(int device, const orbx_keypoint* kp1, const uint8_t* desc1, int n1, const orbx_frame_view* f2,
+                                   float* prev_matched, int window_size, float nn_ratio, int check_orientation, int32_t* matches12,
+                                   int* n_matches)
+{
+    int rc;
+    if ((rc = check_frame(f2, false))) return rc;
+    if (f2->n > 0 && !f2->descriptors) return fail(ORBX_ERR_INVALID_ARG, "frame view: descriptors missing");
+    if (n1 < 0 || n1 >= (1 << 24) || !n_matches || (n1 > 0 && (!kp1 || !desc1 || !prev_matched || !matches12)))
+        return fail(ORBX_ERR_INVALID_ARG, "bad arguments");
+    *n_matches = 0;
+    for (int i = 0; i < n1; ++i) matches12[i] = -1;
+    if (n1 == 0 || f2->n == 0) { t_rounds = 0; return ORBX_OK; }
+    // neither mvuRight nor the map points of F2 take part in this search
+    orbx_frame_view v = *f2;
+    v.u_right = nullptr; v.occupied = nullptr;
+    Session S(device);
+    if ((rc = S.begin(device, &v, n1, true))) return rc;
+    S.enable_chains();
+    ProjQuery* q = S.queries();
+    for (int i = 0; i < n1; ++i) {
+        ProjQuery w{};
+        const int level1 = kp1[i].octave;
+        if (level1 <= 0) {                                                   // src/ORBmatcher1.cc:650-765: 'if(level1>0) continue;'
+            w.x = prev_matched[2 * i]; w.y = prev_matched[2 * i + 1];
+            w.r = (float)window_size;
+            w.min_level = level1; w.max_level = level1;                       // GetFeaturesInArea(.., windowSize, level1, level1)
+            w.flags = PROJ_Q_VALID;
+        }
+        q[i] = w;
+    }
+    memcpy(S.qdesc(), desc1, (size_t)n1 * 32);
+    if ((rc = S.search(2, 50 /* TH_LOW, src/ORBmatcher1.cc:37 */, nn_ratio))) return rc;
+    // Replay of the reference's bookkeeping in query order: qmatch holds every acceptance, including the ones a later query
+    // took over (vnMatches21 / vMatchedDistance), and the rotation histogram counts those too.
+    const int H = 30;
+    std::vector<int> m12(n1, -1), m21(f2->n, -1);
+    std::vector<int> rot[H];
+    int nm = 0;
+    for (int i = 0; i < n1; ++i) {
+        const int f = S.qmatch()[i];
+        if (f < 0) continue;
+        if (m21[f] >= 0) { m12[m21[f]] = -1; --nm; }
+        m12[i] = f; m21[f] = i; ++nm;
+        if (check_orientation) {
+            const int b = rotation_bin(kp1[i].angle, f2->keys_un[f].angle);
+            if (b < 0) return fail(ORBX_ERR_INVALID_ARG, "keypoint angles out of range (the reference asserts)");
+            rot[b].push_back(i);
+        }
+    }
+    if (check_orientation) {
+        int count[H], i1, i2, i3;
+        for (int b = 0; b < H; ++b) count[b] = (int)rot[b].size();
+        three_maxima(count, H, i1, i2, i3);
+        for (int b = 0; b < H; ++b) {
+            if (b == i1 || b == i2 || b == i3) continue;
+            for (int i : rot[b])
+                if (m12[i] >= 0) { m12[i] = -1; --nm; }
+        }
+    }
+    for (int i = 0; i < n1; ++i) {
+        matches12[i] = m12[i];
+        if (m12[i] >= 0) { prev_matched[2 * i] = f2->keys_un[m12[i]].x; prev_matched[2 * i + 1] = f2->keys_un[m12[i]].y; }
+    }
+    *n_matches = nm;
+    return ORBX_OK;
 }
 
 }  // extern "C"

@@ -23,6 +23,12 @@
 // on entry) and query q treats f as taken only if taken_by[f] < q — a later query's assignment must stay invisible to an earlier,
 // still undecided one (it may be that query's second-best candidate, which feeds the ratio test).  An earlier query can never
 // take the same feature afterwards: it would have claimed it, and the later query would not have been final.
+//
+// Mode 2 = ORBmatcher::SearchForInitialization src/ORBmatcher1.cc:650-765: one query per level-0 feature of F1, a feature of F2
+// is skipped when vMatchedDistance[f] <= dist, i.e. when an earlier query accepted it at a distance no larger.  Acceptances of
+// one feature happen in query order (the earlier acceptor claims f until it is decided), so they form a chain per feature,
+// newest first: last_acc[f] -> prev_acc[q] -> ...; query q reads vMatchedDistance[f] as the acc_dist of the first acceptor
+// below q on that chain (DESIGN.md §5b).
 #include <climits>
 
 #include "orbx_internal.cuh"
@@ -99,6 +105,15 @@ __device__ __forceinline__ bool in_area(const ProjArgs& a, int idx, float x, flo
     return fabsf(distx) < r && fabsf(disty) < r;
 }
 
+// vMatchedDistance[f] as query qi sees it (mode 2): the distance of the latest acceptance of f by a query below qi, INT_MAX if
+// none.  The chain is newest first and its distances strictly fall from at most TH_LOW, so the walk is short.
+__device__ __forceinline__ int matched_distance(const ProjArgs& a, int f, int qi)
+{
+    int p = __ldcg(a.last_acc + f);
+    while (p >= qi) p = __ldcg(a.prev_acc + p);
+    return p < 0 ? INT_MAX : __ldcg(a.acc_dist + p);
+}
+
 // One warp evaluates one query on the current taken[] state: top-2 keys over its window, and (claim) atomicMin of the query
 // index on every candidate within the distance threshold.
 __device__ void scan_query(const ProjArgs& a, int qi, int lane, unsigned long long& k1, unsigned long long& k2)
@@ -109,13 +124,14 @@ __device__ void scan_query(const ProjArgs& a, int qi, int lane, unsigned long lo
     uint32_t qd[8];
     load_desc(a.qdesc, (size_t)qi, qd);
     const bool check_right = (q.flags & PROJ_Q_CHECK_RIGHT) && a.u_right;
+    const bool init = a.mode == 2;
     for (int ix = w.x0; ix <= w.x1; ++ix) {
         // cells (ix, y0..y1) are consecutive cell ids: one contiguous item range per grid column
         const int t0 = __ldg(a.cell_start + ix * GRID_ROWS + w.y0), t1 = __ldg(a.cell_start + ix * GRID_ROWS + w.y1 + 1);
         for (int t = t0 + lane; t < t1; t += 32) {
             const int idx = __ldg(a.items + t);
             if (!in_area(a, idx, q.x, q.y, q.r, q.min_level, q.max_level)) continue;
-            if (__ldcg(a.taken_by + idx) < qi) continue;                   // mvpMapPoints[idx] with Observations() > 0, as query qi sees it
+            if (!init && __ldcg(a.taken_by + idx) < qi) continue;          // mvpMapPoints[idx] with Observations() > 0, as query qi sees it
             if (check_right) {                                             // src/ORBmatcher1.cc:95-100, ORBmatcher3.cc:330-336
                 const float ur = __ldg(a.u_right + idx);
                 if (ur > 0.0f && fabsf(__fsub_rn(q.ur, ur)) > q.r) continue;
@@ -123,6 +139,7 @@ __device__ void scan_query(const ProjArgs& a, int qi, int lane, unsigned long lo
             uint32_t d[8];
             load_desc(a.desc, (size_t)idx, d);
             const int dist = hamming256(qd, d);
+            if (init && matched_distance(a, idx, qi) <= dist) continue;    // vMatchedDistance[i2] <= dist, before the top-2 update
             top2_push(k1, k2, ((unsigned long long)dist << 48) | ((unsigned long long)__ldg(a.cell_of + idx) << 32) | (unsigned)idx);
             if (dist <= a.th_dist) atomicMin(a.claim + idx, qi);
         }
@@ -138,6 +155,20 @@ __device__ bool decide_query(const ProjArgs& a, int qi)
     const int d1 = (int)(k1 >> 48), f1 = (int)(unsigned)k1;
     if (d1 > a.th_dist) return true;                                       // taking candidates away can only raise the best distance
     if (__ldcg(a.claim + f1) < qi) return false;                           // L2 reads: the claims are L2 atomics
+    if (a.mode == 2) {
+        // src/ORBmatcher1.cc:650-765: bestDist2 starts at INT_MAX, so a candidate at 256 is a real second-best and a query
+        // without one always passes 'bestDist < (float)bestDist2 * mfNNratio'
+        const int f2 = k2 == KEY_NONE ? -1 : (int)(unsigned)k2;
+        if (f2 >= 0 && __ldcg(a.claim + f2) < qi) return false;
+        const int d2 = f2 >= 0 ? (int)(k2 >> 48) : INT_MAX;
+        if (!((float)d1 < __fmul_rn((float)d2, a.nn_ratio))) return true;
+        // at most one query accepts a feature per decide phase (an earlier acceptor claims it until it is decided)
+        __stcg(a.prev_acc + qi, __ldcg(a.last_acc + f1));
+        __stcg(a.acc_dist + qi, d1);
+        __stcg(a.last_acc + f1, qi);
+        a.qmatch[qi] = f1;
+        return true;
+    }
     const int f2 = (k2 >> 48) >= 256 ? -1 : (int)(unsigned)k2;            // 'dist < bestDist2' never fires for 256: no second-best
     if (a.mode == 0) {
         if (f2 >= 0 && __ldcg(a.claim + f2) < qi) return false;
@@ -165,6 +196,7 @@ __global__ void __launch_bounds__(1024) frame_grid_kernel(ProjArgs a)
         a.cell_of[i] = (unsigned short)(c < 0 ? 0xffff : c);
         if (c >= 0) atomicAdd(&s_cnt[c], 1);
         a.claim[i] = INT_MAX;
+        if (a.last_acc) a.last_acc[i] = -1;
     }
     __syncthreads();
     // exclusive scan of 3072 counters: 3 per thread + block scan of the partial sums

@@ -2,7 +2,8 @@
 
 Reference interfaces: Frame::AssignFeaturesToGrid / GetFeaturesInArea (src/Frame.cc:387-418, 687-753) and the three
 ORBmatcher::SearchByProjection overloads of the tracking thread (src/ORBmatcher1.cc:45-215, src/ORBmatcher3.cc:256-467,
-469-578).  Everything computes in liborbx.so on the GPU; there is no CPU fallback.
+469-578) and ORBmatcher::SearchForInitialization (src/ORBmatcher1.cc:650-765).  Everything computes in liborbx.so on the GPU;
+there is no CPU fallback.
 """
 import ctypes as C
 
@@ -97,6 +98,22 @@ def search_by_projection_kf(cur, valid, u, v, dist3d, min_dist, max_dist, level,
                                              ptr(max_dist), ptr(level), ptr(angle), ptr(desc), th, int(orb_dist), int(check_orientation),
                                              ptr(match_f), C.addressof(nm)))
     return match_f[:len(cur)], nm.value
+
+
+def search_for_initialization(kp1, desc1, frame2, prev_matched, window_size=100, nnratio=0.9, check_orientation=True, device=0):
+    """ORBmatcher(nnratio, check_orientation).SearchForInitialization(F1, F2, vbPrevMatched, vnMatches12, window_size).
+
+    kp1 / desc1 = F1.mvKeysUn / F1.mDescriptors, frame2 = a FrameView of F2, prev_matched = vbPrevMatched as [n1][2] (x, y).
+    Returns (matches12[n1], nmatches, prev_matched_out); the input array is left as it is."""
+    kp1 = np.ascontiguousarray(kp1, KP_DTYPE)
+    n1 = len(kp1)
+    desc1 = np.ascontiguousarray(desc1, np.uint8).reshape(n1, 32)
+    prev = np.array(prev_matched, np.float32, copy=True).reshape(n1, 2)
+    matches12 = np.full(max(n1, 1), -1, np.int32)
+    nm = C.c_int(0)
+    check(lib().orbx_search_for_initialization(device, ptr(kp1), ptr(desc1), n1, C.addressof(frame2.c), ptr(prev), int(window_size), nnratio,
+                                               int(check_orientation), ptr(matches12), C.addressof(nm)))
+    return matches12[:n1], nm.value, prev
 
 
 def projection_rounds():
