@@ -425,6 +425,29 @@ int orbx_search_by_projection_kf(int device, const orbx_frame_view* cur, int n_k
 int orbx_search_for_initialization(int device, const orbx_keypoint* kp1, const uint8_t* desc1, int n1, const orbx_frame_view* f2,
                                    float* prev_matched, int window_size, float nn_ratio, int check_orientation, int32_t* matches12,
                                    int* n_matches);
+/* The slice of ORB_SLAM3::KeyFrame that ORBmatcher::Fuse reads (HOST pointers; NLeft == -1). */
+typedef struct orbx_keyframe_view {
+    orbx_frame_view frame;          /* mvKeysUn, mDescriptors, mvuRight (NULL = monocular), bounds, grid, mvScaleFactors; frame.occupied is not read */
+    const float* inv_level_sigma2;  /* mvInvLevelSigma2, frame.n_levels entries */
+    float bf;                       /* mbf */
+} orbx_keyframe_view;
+/* int ORBmatcher::Fuse(KeyFrame* pKF, const vector<MapPoint*>& vpMapPoints, th, bRight = false) — src/ORBmatcher2.cc:420-610, as
+ * LocalMapping::SearchInNeighbors calls it (src/LocalMapping.cc:766-803), for n_kf key frames in one call: the search part.
+ *   Pairs [kf_offsets[k], kf_offsets[k + 1]) belong to key frame kfs[k]; kf_offsets[0] = 0, nq = kf_offsets[n_kf].  Pair q is
+ *   map point point[q] (its descriptor = point_desc row point[q], 0 <= point[q] < n_desc) projected to (u[q], v[q]) with
+ *   invz[q] = 1 / p3Dc(2) and level[q] = pMP->PredictScale(dist3D, pKF).  valid[q] folds the caller's pre-checks: pMP &&
+ *   !isBad() && !IsInKeyFrame(pKF), p3Dc(2) >= 0, the distance window and the viewing angle (Eigen arithmetic, with the caller).
+ *   This call applies IsInImage (x >= mnMinX && x < mnMaxX, the same for y; upper bounds strict), the window
+ *   GetFeaturesInArea(u, v, th * mvScaleFactors[level]), the level gate [level - 1, level], the reprojection gate (mvuRight >= 0:
+ *   e2 * mvInvLevelSigma2 > 7.8 with ur = u - bf * invz, else > 5.99) and the 1-NN by Hamming distance (earliest in the window's
+ *   order on ties) under TH_LOW (50).  Pairs are independent: the candidate loop never reads the key frame's map points.
+ * Output: match[nq] = bestIdx when bestDist <= 50, else -1; n_fused[n_kf] = matches per key frame (the reference's return value
+ *   when no point changes state during the call).  The bookkeeping (AddMapPoint / Replace) stays with the caller.
+ * ORBX_ERR_INVALID_ARG for null arrays, a missing inv_level_sigma2, non-monotone offsets, point[q] outside [0, n_desc) or a level
+ * outside [0, n_levels) on a valid pair.  Uses its own device scratch, so it never waits on the tracking thread's searches. */
+int orbx_fuse(int device, int n_kf, const orbx_keyframe_view* kfs, const int32_t* kf_offsets, int n_desc, const uint8_t* point_desc,
+              const int32_t* point, const uint8_t* valid, const float* u, const float* v, const float* invz, const int32_t* level,
+              float th, int32_t* match, int* n_fused);
 /* Speculation rounds the last projection search on this thread needed (diagnostics; 0 = every query was final at once). */
 int orbx_projection_rounds(void);
 

@@ -92,6 +92,7 @@ SIGNATURES = {
     "orbx_search_by_projection_last": (_i, [_i, _vp, _f, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _i, _i, _i, _vp, _vp]),
     "orbx_search_by_projection_kf": (_i, [_i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _i, _i, _vp, _vp]),
     "orbx_search_for_initialization": (_i, [_i, _vp, _vp, _i, _vp, _vp, _i, _f, _i, _vp, _vp]),
+    "orbx_fuse": (_i, [_i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _vp, _vp]),
     "orbx_projection_rounds": (_i, []),
     "orbx_undistort_keypoints": (_i, [_i, _vp, _i, _vp, _vp, _i, _vp, _vp]),
     "orbx_rectifier_create": (_i, [_i, _vp, _vp, _sz, _i, _i, C.POINTER(_vp)]),
@@ -120,6 +121,11 @@ class FrameViewC(C.Structure):
     _fields_ = [("n", C.c_int), ("keys_un", _vp), ("descriptors", _vp), ("u_right", _vp), ("occupied", _vp),
                 ("min_x", _f), ("min_y", _f), ("max_x", _f), ("max_y", _f), ("grid_w_inv", _f), ("grid_h_inv", _f),
                 ("scale_factors", _vp), ("n_levels", C.c_int)]
+
+
+class KeyFrameViewC(C.Structure):
+    """orbx_keyframe_view (include/orbx.h): a frame view plus mvInvLevelSigma2 and mbf, what ORBmatcher::Fuse reads."""
+    _fields_ = [("frame", FrameViewC), ("inv_level_sigma2", _vp), ("bf", _f)]
 
 
 class TrackPointsC(C.Structure):

@@ -12,13 +12,17 @@
 //   int SearchByBoW(KeyFrame*, Frame&, vector<MapPoint*>& vpMapPointMatches)         src/ORBmatcher1.cc:225-427
 //   int SearchByBoW(KeyFrame*, KeyFrame*, vector<MapPoint*>& vpMatches12)            src/ORBmatcher2.cc:36-171
 //   int SearchForInitialization(Frame&, Frame&, vector<cv::Point2f>&, vector<int>&, windowSize)   src/ORBmatcher1.cc:650-765
+//   int Fuse(KeyFrame*, const vector<MapPoint*>&, th, bRight)                        src/ORBmatcher2.cc:420-610
+//   int Fuse(const vector<KeyFrame*>&, const vector<MapPoint*>&, th)  (added: the forward loop of SearchInNeighbors in one call)
 // Not declared (not on the tracking path / out of scope, DESIGN.md §8): the Sim3 SearchByProjection overloads,
-// SearchBySim3, Fuse; SearchForTriangulation is exported by the C ABI (orbx_search_for_triangulation) and takes F12 from the
+// SearchBySim3, the Sim3 Fuse; SearchForTriangulation is exported by the C ABI (orbx_search_for_triangulation) and takes F12 from the
 // caller.
 #ifndef ORBMATCHER_H
 #define ORBMATCHER_H
 
 #include <cstring>
+#include <stdexcept>
+#include <type_traits>
 #include <vector>
 
 #include "ORBmatcherProjection.h"
@@ -71,6 +75,61 @@ public:
     int SearchForInitialization(Frame& F1, Frame& F2, std::vector<cv::Point2f>& vbPrevMatched, std::vector<int>& vnMatches12, int windowSize = 10)
     {
         return orbx_adapter::SearchForInitialization(F1, F2, vbPrevMatched, vnMatches12, windowSize, mfNNratio, mbCheckOrientation, device);
+    }
+
+    // Project MapPoints into KeyFrame and search for duplicated MapPoints.  (Member templates: the body is compiled only where
+    // Fuse is called, against the complete KeyFrame / MapPoint types.)
+    template <class KF = KeyFrame, class MP = MapPoint>
+    int Fuse(KF* pKF, const std::vector<MP*>& vpMapPoints, const float th = 3.0, const bool bRight = false)
+    {
+        if (bRight) throw std::invalid_argument("ORBmatcher::Fuse: bRight (two-camera rigs keep the reference code)");
+        return Fuse(std::vector<KF*>(1, pKF), vpMapPoints, th);
+    }
+
+    // The same for several key frames: equal to the sum of Fuse(pKFi, vpMapPoints, th) over vpKFs in order (the forward loop of
+    // LocalMapping::SearchInNeighbors), with one search call for all of them (orbx_adapter::FuseApply).
+    template <class KF = KeyFrame, class MP = MapPoint>
+    int Fuse(const std::vector<KF*>& vpKFs, const std::vector<MP*>& vpMapPoints, const float th = 3.0)
+    {
+        const int M = (int)vpMapPoints.size();
+        const size_t nq = vpKFs.size() * (size_t)M;
+        std::vector<uint8_t> valid(nq, 0);
+        std::vector<float> u(nq, 0.f), v(nq, 0.f), invz(nq, 0.f);
+        std::vector<int32_t> level(nq, 0);
+        for (size_t k = 0; k < vpKFs.size(); ++k) {
+            KF* pKF = vpKFs[k];
+            if (pKF->NLeft != -1) throw std::invalid_argument("ORBmatcher::Fuse: NLeft != -1 (two-camera rigs keep the reference code)");
+            // the reference's lines (src/ORBmatcher2.cc:420-610) with Eigen's / Sophus' own arithmetic; the search is orbx_fuse
+            const auto Tcw = pKF->GetPose();
+            const auto Ow = pKF->GetCameraCenter();
+            auto* pCamera = pKF->mpCamera;
+            for (int i = 0; i < M; i++) {
+                MP* pMP = vpMapPoints[i];
+                if (!pMP) continue;
+                if (pMP->isBad()) continue;
+                else if (pMP->IsInKeyFrame(pKF)) continue;
+                using Vec3 = typename std::decay<decltype(pMP->GetWorldPos())>::type;
+                const Vec3 p3Dw = pMP->GetWorldPos();
+                const Vec3 p3Dc = Tcw * p3Dw;
+                // Depth must be positive
+                if (p3Dc(2) < 0.0f) continue;
+                const float invzi = 1 / p3Dc(2);
+                const auto uv = pCamera->project(p3Dc);
+                const float maxDistance = pMP->GetMaxDistanceInvariance();
+                const float minDistance = pMP->GetMinDistanceInvariance();
+                const Vec3 PO = p3Dw - Ow;
+                const float dist3D = PO.norm();
+                // Depth must be inside the scale pyramid of the image
+                if (dist3D < minDistance || dist3D > maxDistance) continue;
+                // Viewing angle must be less than 60 deg
+                const Vec3 Pn = pMP->GetNormal();
+                if (PO.dot(Pn) < 0.5 * dist3D) continue;
+                const size_t q = k * (size_t)M + i;
+                valid[q] = 1; u[q] = uv(0); v[q] = uv(1); invz[q] = invzi;
+                level[q] = pMP->PredictScale(dist3D, pKF);                  // IsInImage and the window: orbx_fuse
+            }
+        }
+        return orbx_adapter::FuseApply(vpKFs, vpMapPoints, th, valid, u, v, invz, level, device);
     }
 
     // Search matches between MapPoints in a KeyFrame and ORB in a Frame.

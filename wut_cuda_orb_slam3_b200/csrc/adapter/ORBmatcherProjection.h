@@ -9,8 +9,10 @@
 //                                                                                                   src/ORBmatcher3.cc:256-467
 //   int ORBmatcher::SearchForInitialization(Frame &F1, Frame &F2, vector<cv::Point2f> &vbPrevMatched, vector<int> &vnMatches12,
 //                                           int windowSize)                                        src/ORBmatcher1.cc:650-765
-// by one-line calls of the functions below (Nleft == -1 rigs; a two-fisheye rig keeps the reference code).
+// by one-line calls of the functions below (Nleft == -1 rigs; a two-fisheye rig keeps the reference code).  FuseApply is the
+// C ABI side and the bookkeeping of ORBmatcher::Fuse (src/ORBmatcher2.cc:420-610); the class keeps the per-point Eigen lines.
 #pragma once
+#include <algorithm>
 #include <cstring>
 #include <stdexcept>
 #include <string>
@@ -120,6 +122,118 @@ inline int SearchForInitialization(FrameT& F1, FrameT& F2, std::vector<PointT>& 
                                          vnMatches12.data(), &n),
           "SearchForInitialization");
     return n;
+}
+
+// What the last Fuse on this thread re-searched because a Replace earlier in the call changed a point's descriptor: pairs
+// re-searched and the extra orbx_fuse calls that took (diagnostics).
+struct FuseDiagnostics { int researched_pairs = 0, extra_calls = 0; };
+inline thread_local FuseDiagnostics fuse_diagnostics;
+
+// The key frame as orbx_fuse reads it (KeyFrame stores the bounds as it stores them: the view takes them as floats).
+template <class KF>
+inline orbx_keyframe_view keyframe_view_of(const KF* pKF)
+{
+    static_assert(sizeof(pKF->mvKeysUn[0]) == sizeof(orbx_keypoint), "cv::KeyPoint must be the 28-byte POD");
+    orbx_keyframe_view k{};
+    orbx_frame_view& v = k.frame;
+    v.n = (int)pKF->mvKeysUn.size();
+    v.keys_un = reinterpret_cast<const orbx_keypoint*>(pKF->mvKeysUn.data());
+    v.descriptors = v.n ? pKF->mDescriptors.ptr(0) : nullptr;
+    v.u_right = pKF->mvuRight.empty() ? nullptr : pKF->mvuRight.data();
+    v.min_x = (float)pKF->mnMinX; v.min_y = (float)pKF->mnMinY; v.max_x = (float)pKF->mnMaxX; v.max_y = (float)pKF->mnMaxY;
+    v.grid_w_inv = pKF->mfGridElementWidthInv; v.grid_h_inv = pKF->mfGridElementHeightInv;
+    v.scale_factors = pKF->mvScaleFactors.data();
+    v.n_levels = (int)pKF->mvScaleFactors.size();
+    k.inv_level_sigma2 = pKF->mvInvLevelSigma2.data();
+    k.bf = pKF->mbf;
+    return k;
+}
+
+// ORBmatcher::Fuse over the key frames vpKFs in order, each with all of vpMapPoints: pair q = k * M + i.  The caller has run the
+// reference's per-point lines: valid[q] (pMP && !isBad() && !IsInKeyFrame(pKF), depth, distance window, viewing angle), the
+// projection (u, v, invz) and level (PredictScale).  One orbx_fuse call searches every pair; then per key frame, in order:
+// pairs whose point's live descriptor differs from the one searched with (a Replace in an earlier key frame of the call) are
+// re-searched in one extra call, and the reference's tail is replayed with isBad() / IsInKeyFrame(pKF) re-evaluated live.
+template <class KF, class MP>
+inline int FuseApply(const std::vector<KF*>& vpKFs, const std::vector<MP*>& vpMapPoints, const float th, const std::vector<uint8_t>& valid,
+                     const std::vector<float>& u, const std::vector<float>& v, const std::vector<float>& invz, const std::vector<int32_t>& level,
+                     int device = 0)
+{
+    const int nK = (int)vpKFs.size(), M = (int)vpMapPoints.size();
+    const size_t nq = (size_t)nK * M;
+    fuse_diagnostics = FuseDiagnostics{};
+    // descriptors the pairs were searched with: rows of `rows`, row_of[q]; the first M rows are the snapshot of the points
+    std::vector<uint8_t> rows((size_t)M * 32, 0);
+    for (int i = 0; i < M; ++i)
+        if (vpMapPoints[i] && !vpMapPoints[i]->isBad()) std::memcpy(&rows[(size_t)32 * i], vpMapPoints[i]->GetDescriptor().ptr(0), 32);
+    std::vector<int32_t> row_of(nq), point(nq), match(nq, -1), offs(nK + 1), nf(std::max(nK, 1));
+    for (size_t q = 0; q < nq; ++q) row_of[q] = point[q] = (int32_t)(q % (size_t)std::max(M, 1));
+    for (int k = 0; k <= nK; ++k) offs[k] = k * M;
+    std::vector<orbx_keyframe_view> views(nK);
+    for (int k = 0; k < nK; ++k) views[k] = keyframe_view_of(vpKFs[k]);
+    check(orbx_fuse(device, nK, views.data(), offs.data(), M, rows.data(), point.data(), valid.data(), u.data(), v.data(), invz.data(),
+                    level.data(), th, match.data(), nf.data()),
+          "Fuse");
+    // re-search pairs qs of key frame k with the points' live descriptors (appended to rows)
+    auto research = [&](int k, const std::vector<size_t>& qs) {
+        const int n = (int)qs.size();
+        std::vector<uint8_t> d((size_t)n * 32), ok(n, 1);
+        std::vector<int32_t> pt(n), lv(n), m(n), o = {0, n};
+        std::vector<float> uu(n), vv(n), iz(n);
+        for (int j = 0; j < n; ++j) {
+            const size_t q = qs[j];
+            std::memcpy(&d[(size_t)32 * j], vpMapPoints[point[q]]->GetDescriptor().ptr(0), 32);
+            pt[j] = j; uu[j] = u[q]; vv[j] = v[q]; iz[j] = invz[q]; lv[j] = level[q];
+        }
+        int nfk = 0;
+        check(orbx_fuse(device, 1, &views[k], o.data(), n, d.data(), pt.data(), ok.data(), uu.data(), vv.data(), iz.data(), lv.data(), th,
+                        m.data(), &nfk),
+              "Fuse");
+        for (int j = 0; j < n; ++j) {
+            row_of[qs[j]] = (int32_t)(rows.size() / 32);
+            rows.insert(rows.end(), d.begin() + (size_t)32 * j, d.begin() + (size_t)32 * (j + 1));
+            match[qs[j]] = m[j];
+        }
+        fuse_diagnostics.researched_pairs += n;
+        fuse_diagnostics.extra_calls += 1;
+    };
+    auto live = [&](size_t q, KF* pKF) {
+        MP* pMP = vpMapPoints[point[q]];
+        return valid[q] && pMP && !pMP->isBad() && !pMP->IsInKeyFrame(pKF);
+    };
+    auto stale = [&](size_t q) { return std::memcmp(vpMapPoints[point[q]]->GetDescriptor().ptr(0), &rows[(size_t)32 * row_of[q]], 32) != 0; };
+    int nFused = 0;
+    for (int k = 0; k < nK; ++k) {
+        KF* pKF = vpKFs[k];
+        if (k > 0) {
+            std::vector<size_t> qs;
+            for (size_t q = (size_t)k * M; q < (size_t)(k + 1) * M; ++q)
+                if (live(q, pKF) && stale(q)) qs.push_back(q);
+            if (!qs.empty()) research(k, qs);
+        }
+        for (size_t q = (size_t)k * M; q < (size_t)(k + 1) * M; ++q) {
+            if (!live(q, pKF)) continue;
+            if (stale(q)) research(k, std::vector<size_t>(1, q));   // vpMapPoints holds the point twice (see DESIGN.md §5b)
+            const int bestIdx = match[q];
+            if (bestIdx < 0) continue;
+            MP* pMP = vpMapPoints[point[q]];
+            // If there is already a MapPoint replace otherwise add new measurement (src/ORBmatcher2.cc:420-610)
+            MP* pMPinKF = pKF->GetMapPoint(bestIdx);
+            if (pMPinKF) {
+                if (!pMPinKF->isBad()) {
+                    if (pMPinKF->Observations() > pMP->Observations())
+                        pMP->Replace(pMPinKF);
+                    else
+                        pMPinKF->Replace(pMP);
+                }
+            } else {
+                pMP->AddObservation(pKF, bestIdx);
+                pKF->AddMapPoint(pMP, bestIdx);
+            }
+            nFused++;
+        }
+    }
+    return nFused;
 }
 
 }  // namespace orbx_adapter

@@ -6,6 +6,7 @@
 //   ORBmatcher::SearchByProjection(Frame& Current, const Frame& Last..)  src/ORBmatcher3.cc:256-467  (Tracking::TrackWithMotionModel)
 //   ORBmatcher::SearchByProjection(Frame& Current, KeyFrame*, ...)       src/ORBmatcher3.cc:469-578  (Tracking::Relocalization)
 //   ORBmatcher::SearchForInitialization(F1, F2, vbPrevMatched, ...)      src/ORBmatcher1.cc:650-765  (Tracking::MonocularInitialization)
+//   ORBmatcher::Fuse(KeyFrame*, const vector<MapPoint*>&, th, bRight)     src/ORBmatcher2.cc:420-610  (LocalMapping::SearchInNeighbors)
 // Each entry point turns the reference's per-map-point pre-checks into window queries (float arithmetic in the reference's
 // order, on the host: a handful of operations per point), ships everything in ONE pinned staging copy, runs the grid build and
 // the window search (kernels_proj.cu) and reads the per-query assignment back in one copy.  The 30-bin rotation histogram runs
@@ -34,6 +35,8 @@ struct ProjArena {
     cudaStream_t st = nullptr;
 };
 ProjArena g_arena[64];
+// orbx_fuse runs on the local-mapping thread: its own arenas, so a large Fuse never holds the lock a tracking-thread search waits on
+ProjArena g_fuse_arena[64];
 
 // One call = one lease: a bump allocator that hands out matching (pinned host, device) ranges so that all inputs travel in
 // one cudaMemcpyAsync.  Inputs are allocated first (the upload range), device-only scratch and outputs after.
@@ -41,7 +44,7 @@ struct Lease {
     ProjArena& A;
     std::unique_lock<std::mutex> lock;
     size_t off = 0, upload_end = 0;
-    explicit Lease(int device) : A(g_arena[device & 63]), lock(A.mu) {}
+    explicit Lease(int device, ProjArena* arenas = g_arena) : A(arenas[device & 63]), lock(A.mu) {}
     int reserve(size_t bytes)
     {
         bytes += 8192;
@@ -450,6 +453,108 @@ int orbx_search_for_initialization(int device, const orbx_keypoint* kp1, const u
         if (m12[i] >= 0) { prev_matched[2 * i] = f2->keys_un[m12[i]].x; prev_matched[2 * i + 1] = f2->keys_un[m12[i]].y; }
     }
     *n_matches = nm;
+    return ORBX_OK;
+}
+
+int orbx_fuse(int device, int n_kf, const orbx_keyframe_view* kfs, const int32_t* kf_offsets, int n_desc, const uint8_t* point_desc,
+              const int32_t* point, const uint8_t* valid, const float* u, const float* v, const float* invz, const int32_t* level,
+              float th, int32_t* match, int* n_fused)
+{
+    int rc;
+    if (n_kf < 0 || n_desc < 0 || !kf_offsets || (n_kf > 0 && (!kfs || !n_fused))) return fail(ORBX_ERR_INVALID_ARG, "fuse: bad arguments");
+    if (kf_offsets[0] != 0) return fail(ORBX_ERR_INVALID_ARG, "fuse: kf_offsets[0] must be 0");
+    for (int k = 0; k < n_kf; ++k)
+        if (kf_offsets[k + 1] < kf_offsets[k]) return fail(ORBX_ERR_INVALID_ARG, "fuse: kf_offsets not monotone at %d", k);
+    const int nq = kf_offsets[n_kf];
+    if (nq > 0 && (!point || !valid || !u || !v || !invz || !level || !match)) return fail(ORBX_ERR_INVALID_ARG, "fuse: missing pair arrays");
+    if (n_desc > 0 && !point_desc) return fail(ORBX_ERR_INVALID_ARG, "fuse: point_desc missing");
+    long long n_feat = 0;
+    for (int k = 0; k < n_kf; ++k) {
+        if ((rc = check_frame(&kfs[k].frame, true))) return rc;
+        if (!kfs[k].inv_level_sigma2) return fail(ORBX_ERR_INVALID_ARG, "fuse: key frame %d: inv_level_sigma2 missing", k);
+        n_feat += kfs[k].frame.n;
+    }
+    if (n_feat >= (1LL << 31) / 32) return fail(ORBX_ERR_UNSUPPORTED, "fuse: too many key-frame features");
+    // pre-checks of the caller (valid), then KeyFrame::IsInImage with strict upper bounds; the rest are compacted away
+    std::vector<int> live;
+    for (int k = 0; k < n_kf; ++k) {
+        const orbx_frame_view& f = kfs[k].frame;
+        for (int q = kf_offsets[k]; q < kf_offsets[k + 1]; ++q) {
+            if (point[q] < 0 || point[q] >= n_desc) return fail(ORBX_ERR_INVALID_ARG, "fuse: pair %d: point %d outside [0, %d)", q, point[q], n_desc);
+            if (!valid[q]) continue;
+            if (level[q] < 0 || level[q] >= f.n_levels) return fail(ORBX_ERR_INVALID_ARG, "fuse: pair %d: level %d out of range", q, level[q]);
+            if (!(u[q] >= f.min_x && u[q] < f.max_x && v[q] >= f.min_y && v[q] < f.max_y)) continue;
+            if (f.n > 0) live.push_back(q);
+        }
+    }
+    for (int q = 0; q < nq; ++q) match[q] = -1;
+    for (int k = 0; k < n_kf; ++k) n_fused[k] = 0;
+    if (live.empty()) return ORBX_OK;
+    const int nv = (int)live.size();
+    if ((rc = set_device(device))) return rc;
+    Lease L(device, g_fuse_arena);
+    const size_t total = pad((size_t)n_kf * sizeof(FuseKF)) + pad((size_t)n_feat * 28) + pad((size_t)n_feat * 32) + pad((size_t)n_feat * 4) +
+                         pad((size_t)nv * sizeof(FuseQuery)) + pad((size_t)n_desc * 32) + pad((size_t)n_kf * (GRID_CELLS + 1) * 4) +
+                         pad((size_t)n_feat * 4) + pad((size_t)n_feat * 2) + pad((size_t)nv * 4);
+    if ((rc = L.reserve(total))) return rc;
+    // upload range
+    const size_t o_kf = L.take<FuseKF>(n_kf), o_kp = L.take<orbx_keypoint>(n_feat), o_desc = L.take<uint8_t>((size_t)n_feat * 32),
+                 o_ur = L.take<float>(n_feat), o_q = L.take<FuseQuery>(nv), o_pd = L.take<uint8_t>((size_t)n_desc * 32);
+    L.upload_end = L.off;
+    // device-only scratch / outputs
+    const size_t o_cs = L.take<int>((size_t)n_kf * (GRID_CELLS + 1)), o_items = L.take<int>(n_feat), o_cellof = L.take<unsigned short>(n_feat),
+                 o_match = L.take<int>(nv);
+    FuseKF* K = L.host<FuseKF>(o_kf);
+    size_t base = 0;
+    for (int k = 0; k < n_kf; ++k) {
+        const orbx_keyframe_view& kv = kfs[k];
+        const orbx_frame_view& f = kv.frame;
+        FuseKF e{};
+        e.n = f.n;
+        e.kp = L.dev<orbx_keypoint>(o_kp) + base; e.desc = L.dev<uint8_t>(o_desc) + base * 32;
+        e.u_right = f.u_right ? L.dev<float>(o_ur) + base : nullptr;
+        e.min_x = f.min_x; e.min_y = f.min_y; e.grid_w_inv = f.grid_w_inv; e.grid_h_inv = f.grid_h_inv;
+        e.cell_start = L.dev<int>(o_cs) + (size_t)k * (GRID_CELLS + 1);
+        e.items = L.dev<int>(o_items) + base; e.cell_of = L.dev<unsigned short>(o_cellof) + base;
+        for (int l = 0; l < f.n_levels; ++l) e.inv_sigma2[l] = kv.inv_level_sigma2[l];
+        K[k] = e;
+        if (f.n) {
+            memcpy(L.host<orbx_keypoint>(o_kp) + base, f.keys_un, (size_t)f.n * sizeof(orbx_keypoint));
+            memcpy(L.host<uint8_t>(o_desc) + base * 32, f.descriptors, (size_t)f.n * 32);
+            if (f.u_right) memcpy(L.host<float>(o_ur) + base, f.u_right, (size_t)f.n * 4);
+        }
+        base += (size_t)f.n;
+    }
+    FuseQuery* Q = L.host<FuseQuery>(o_q);
+    int k = 0;
+    for (int i = 0; i < nv; ++i) {
+        const int q = live[i];
+        while (q >= kf_offsets[k + 1]) ++k;
+        FuseQuery w{};
+        w.u = u[q]; w.v = v[q];
+        w.r = th * kfs[k].frame.scale_factors[level[q]];                     // src/ORBmatcher2.cc: radius = th * mvScaleFactors[nPredictedLevel]
+        w.ur = u[q] - kfs[k].bf * invz[q];                                  // ur = uv(0) - bf * invz
+        w.kf = k; w.point = point[q]; w.level = level[q];
+        Q[i] = w;
+    }
+    if (n_desc) memcpy(L.host<uint8_t>(o_pd), point_desc, (size_t)n_desc * 32);
+    FuseArgs A{};
+    A.n_kf = n_kf; A.kfs = L.dev<FuseKF>(o_kf); A.nq = nv; A.q = L.dev<FuseQuery>(o_q); A.pdesc = L.dev<uint8_t>(o_pd);
+    A.th_dist = 50;                                                          // TH_LOW, src/ORBmatcher1.cc:37
+    A.match = L.dev<int>(o_match);
+    cudaStream_t st = L.A.st;
+    cudaError_t e = cudaMemcpyAsync(L.A.d, L.A.h, L.upload_end, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = launch_fuse(A, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(L.host<int>(o_match), A.match, (size_t)nv * 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "fuse: %s", cudaGetErrorString(e));
+    const int* m = L.host<int>(o_match);
+    k = 0;
+    for (int i = 0; i < nv; ++i) {
+        const int q = live[i];
+        while (q >= kf_offsets[k + 1]) ++k;
+        if (m[i] >= 0) { match[q] = m[i]; ++n_fused[k]; }
+    }
     return ORBX_OK;
 }
 

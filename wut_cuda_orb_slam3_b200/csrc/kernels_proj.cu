@@ -29,6 +29,9 @@
 // one feature happen in query order (the earlier acceptor claims f until it is decided), so they form a chain per feature,
 // newest first: last_acc[f] -> prev_acc[q] -> ...; query q reads vMatchedDistance[f] as the acc_dist of the first acceptor
 // below q on that chain (DESIGN.md §5b).
+//
+// ORBmatcher::Fuse src/ORBmatcher2.cc:420-610 (fuse_grid_kernel, fuse_scan_kernel): the candidate loop never reads the key
+// frame's map points, so every (key frame, point) pair is independent — one wide launch, no rounds (DESIGN.md §5b).
 #include <climits>
 
 #include "orbx_internal.cuh"
@@ -181,13 +184,10 @@ __device__ bool decide_query(const ProjArgs& a, int qi)
     return true;
 }
 
-}  // namespace
-
-// ---- grid build: one CTA, counting sort by cell id (ix * 48 + iy), in-cell order = ascending feature index ----------------
-__global__ void __launch_bounds__(1024) frame_grid_kernel(ProjArgs a)
+// ---- grid build: one CTA per frame, counting sort by cell id (ix * 48 + iy), in-cell order = ascending feature index --------
+// Reads a.n, a.kp, the grid geometry; writes a.cell_of, a.cell_start, a.items.  Every thread of the CTA calls it.
+__device__ void build_grid(const ProjArgs& a, int* s_cnt, int* s_part)
 {
-    __shared__ int s_cnt[GRID_CELLS];
-    __shared__ int s_part[1024];
     const int tid = threadIdx.x;
     for (int c = tid; c < GRID_CELLS; c += 1024) s_cnt[c] = 0;
     __syncthreads();
@@ -195,8 +195,6 @@ __global__ void __launch_bounds__(1024) frame_grid_kernel(ProjArgs a)
         const int c = cell_of_point(a, a.kp[i].x, a.kp[i].y);
         a.cell_of[i] = (unsigned short)(c < 0 ? 0xffff : c);
         if (c >= 0) atomicAdd(&s_cnt[c], 1);
-        a.claim[i] = INT_MAX;
-        if (a.last_acc) a.last_acc[i] = -1;
     }
     __syncthreads();
     // exclusive scan of 3072 counters: 3 per thread + block scan of the partial sums
@@ -229,6 +227,89 @@ __global__ void __launch_bounds__(1024) frame_grid_kernel(ProjArgs a)
             a.items[j + 1] = v;
         }
     }
+}
+
+// The fields of ProjArgs that build_grid / window_cells / in_area read, for one key frame of orbx_fuse.
+__device__ __forceinline__ ProjArgs kf_args(const FuseKF& k)
+{
+    ProjArgs a{};
+    a.n = k.n; a.kp = k.kp; a.desc = k.desc; a.u_right = k.u_right;
+    a.min_x = k.min_x; a.min_y = k.min_y; a.grid_w_inv = k.grid_w_inv; a.grid_h_inv = k.grid_h_inv;
+    a.cell_start = k.cell_start; a.items = k.items; a.cell_of = k.cell_of;
+    return a;
+}
+
+}  // namespace
+
+__global__ void __launch_bounds__(1024) frame_grid_kernel(ProjArgs a)
+{
+    __shared__ int s_cnt[GRID_CELLS];
+    __shared__ int s_part[1024];
+    for (int i = threadIdx.x; i < a.n; i += 1024) {
+        a.claim[i] = INT_MAX;
+        if (a.last_acc) a.last_acc[i] = -1;
+    }
+    build_grid(a, s_cnt, s_part);
+}
+
+// ---- orbx_fuse: the grids of all key frames of the call in one launch, one CTA per key frame ------------------------------
+__global__ void __launch_bounds__(1024) fuse_grid_kernel(FuseArgs f)
+{
+    __shared__ int s_cnt[GRID_CELLS];
+    __shared__ int s_part[1024];
+    build_grid(kf_args(f.kfs[blockIdx.x]), s_cnt, s_part);
+}
+
+// ---- ORBmatcher::Fuse (src/ORBmatcher2.cc:420-610), the candidate loop: one warp per (key frame, point) pair -----------------
+// The loop never reads the key frame's map points, so every pair is independent.  KeyFrame::GetFeaturesInArea is the window of
+// Frame::GetFeaturesInArea without levels; the level gate [level - 1, level] comes first in the loop, so it is folded into the
+// window's membership test.  The least key (distance, cell id, index) is the earliest candidate at the least distance, which is
+// what strict '<' keeps.
+__global__ void __launch_bounds__(256) fuse_scan_kernel(FuseArgs f)
+{
+    const int lane = threadIdx.x & 31;
+    const int qi = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (qi >= f.nq) return;
+    const FuseQuery q = f.q[qi];
+    const FuseKF& K = f.kfs[q.kf];
+    const ProjArgs a = kf_args(K);
+    const Window w = window_cells(a, q.u, q.v, q.r);
+    uint32_t qd[8];
+    load_desc(f.pdesc, (size_t)q.point, qd);
+    unsigned long long k1 = KEY_NONE;
+    for (int ix = w.x0; ix <= w.x1; ++ix) {
+        const int t0 = __ldg(a.cell_start + ix * GRID_ROWS + w.y0), t1 = __ldg(a.cell_start + ix * GRID_ROWS + w.y1 + 1);
+        for (int t = t0 + lane; t < t1; t += 32) {
+            const int idx = __ldg(a.items + t);
+            // kpLevel < nPredictedLevel - 1 || kpLevel > nPredictedLevel (an octave of -1 would index mvInvLevelSigma2[-1])
+            if (!in_area(a, idx, q.u, q.v, q.r, max(q.level - 1, 0), q.level)) continue;
+            const orbx_keypoint* kp = a.kp + idx;
+            const int oct = __ldg(&kp->octave);
+            const float inv = K.inv_sigma2[oct];
+            const float ex = __fsub_rn(q.u, __ldg(&kp->x)), ey = __fsub_rn(q.v, __ldg(&kp->y));
+            const float kpr = a.u_right ? __ldg(a.u_right + idx) : -1.0f;
+            // float e2, every product and sum rounded; 'e2 * inv' rounded to float, then compared with the double constant
+            if (kpr >= 0.0f) {
+                const float er = __fsub_rn(q.ur, kpr);
+                const float e2 = __fadd_rn(__fadd_rn(__fmul_rn(ex, ex), __fmul_rn(ey, ey)), __fmul_rn(er, er));
+                if ((double)__fmul_rn(e2, inv) > 7.8) continue;
+            } else {
+                const float e2 = __fadd_rn(__fmul_rn(ex, ex), __fmul_rn(ey, ey));
+                if ((double)__fmul_rn(e2, inv) > 5.99) continue;
+            }
+            uint32_t d[8];
+            load_desc(a.desc, (size_t)idx, d);
+            const unsigned long long key =
+                ((unsigned long long)hamming256(qd, d) << 48) | ((unsigned long long)__ldg(a.cell_of + idx) << 32) | (unsigned)idx;
+            if (key < k1) k1 = key;
+        }
+    }
+#pragma unroll
+    for (int s = 16; s >= 1; s >>= 1) {
+        const unsigned long long o = __shfl_xor_sync(0xffffffffu, k1, s);
+        if (o < k1) k1 = o;
+    }
+    if (lane == 0) f.match[qi] = (k1 != KEY_NONE && (int)(k1 >> 48) <= f.th_dist) ? (int)(unsigned)k1 : -1;
 }
 
 // ---- round 0, wide: every valid query scans and claims on the initial state -------------------------------------------------
@@ -312,6 +393,14 @@ cudaError_t launch_proj_search(const ProjArgs& a, cudaStream_t st)
     proj_scan_kernel<<<(a.nq + 7) / 8, 256, 0, st>>>(a);
     proj_resolve_kernel<<<1, 1024, 0, st>>>(a);
     count_launch(2);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_fuse(const FuseArgs& a, cudaStream_t st)
+{
+    if (a.n_kf > 0) fuse_grid_kernel<<<a.n_kf, 1024, 0, st>>>(a);
+    if (a.nq > 0) fuse_scan_kernel<<<(a.nq + 7) / 8, 256, 0, st>>>(a);
+    count_launch((a.n_kf > 0) + (a.nq > 0));
     return cudaGetLastError();
 }
 

@@ -241,6 +241,28 @@ struct ProjArgs {
 };
 cudaError_t launch_frame_grid(const ProjArgs& a, cudaStream_t st);
 cudaError_t launch_proj_search(const ProjArgs& a, cudaStream_t st);
+// ORBmatcher::Fuse (ORBmatcher2.cc:420-610) over many key frames: one grid per key frame, one warp per (key frame, point) pair
+struct FuseKF {                  // one key frame on the device
+    const orbx_keypoint* kp; const uint8_t* desc; const float* u_right;   // u_right null = monocular (mvuRight all -1)
+    int n;
+    float min_x, min_y, grid_w_inv, grid_h_inv;
+    int* cell_start;             // [64*48 + 1]
+    int* items;                  // [n]
+    unsigned short* cell_of;     // [n]
+    float inv_sigma2[kMaxLevels];   // mvInvLevelSigma2
+};
+struct FuseQuery {               // one pair that passed the caller's pre-checks and IsInImage (32 bytes)
+    float u, v, r, ur;           // projection, window half size th * mvScaleFactors[level], ur = u - bf * invz
+    int kf, point, level, pad;
+};
+struct FuseArgs {
+    int n_kf; const FuseKF* kfs;
+    int nq; const FuseQuery* q;
+    const uint8_t* pdesc;        // [n_desc][32] map point descriptors, indexed by FuseQuery::point
+    int th_dist;                 // TH_LOW
+    int* match;                  // [nq] bestIdx or -1
+};
+cudaError_t launch_fuse(const FuseArgs& a, cudaStream_t st);
 cudaError_t launch_features_in_area(const ProjArgs& a, float x, float y, float r, int min_level, int max_level,
                                     unsigned long long* d_out, int capacity, int* d_n_out, cudaStream_t st);
 
