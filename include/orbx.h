@@ -448,6 +448,40 @@ typedef struct orbx_keyframe_view {
 int orbx_fuse(int device, int n_kf, const orbx_keyframe_view* kfs, const int32_t* kf_offsets, int n_desc, const uint8_t* point_desc,
               const int32_t* point, const uint8_t* valid, const float* u, const float* v, const float* invz, const int32_t* level,
               float th, int32_t* match, int* n_fused);
+/* int ORBmatcher::SearchByProjection(KeyFrame* pKF, Sophus::Sim3f& Scw, const vector<MapPoint*>& vpPoints,
+ * [const vector<KeyFrame*>& vpPointsKFs,] vector<MapPoint*>& vpMatched, [vector<KeyFrame*>& vpMatchedKF,] int th,
+ * float ratioHamming) — src/ORBmatcher1.cc:429-648 (NLeft == -1), as loop closing calls it (LoopClosing::DetectCommonRegionsFromBoW,
+ * FindMatchesByProjection).  Point i is vpPoints[i] projected with Tcw = SE3(Scw.rotationMatrix(), Scw.translation() / Scw.scale())
+ * to (u[i], v[i]), level[i] = pMP->PredictScale(dist, pKF), desc = pMP->GetDescriptor() (n_points x 32).
+ *   valid[i] folds the caller's checks: !isBad(), not in spAlreadyFound (the non-NULL entries of vpMatched on entry),
+ *   p3Dc(2) >= 0, the distance window and the viewing angle (Eigen arithmetic, with the caller).
+ *   kf->occupied[idx] != 0 <=> vpMatched[idx] != NULL on entry; kf->u_right is not read.
+ *   This call applies IsInImage (x >= mnMinX && x < mnMaxX, the same for y; upper bounds strict), the window
+ *   GetFeaturesInArea(u, v, th * mvScaleFactors[level]), the level gate [level - 1, level] and the 1-NN by Hamming distance
+ *   (earliest in the window's order on ties) accepted when bestDist <= TH_LOW * ratio_hamming (in float).  A feature taken by an
+ *   earlier point of the call is skipped by later ones exactly as the sequential loop does.
+ * Output: match_f[kf->n] = index of the point assigned to the feature by THIS call, -1 = untouched; *n_matches = the return value.
+ * Sets orbx_projection_rounds().  ORBX_ERR_INVALID_ARG for null arrays, a level outside [0, n_levels) on a valid point, and
+ * 50 * ratio_hamming >= 256 or NaN (where the reference would write vpMatched[-1]).  Uses the loop-closing thread's own device
+ * scratch. */
+int orbx_search_by_projection_sim3(int device, const orbx_frame_view* kf, int n_points, const uint8_t* valid, const float* u,
+                                   const float* v, const int32_t* level, const uint8_t* desc, float th, float ratio_hamming,
+                                   int32_t* match_f, int* n_matches);
+/* int ORBmatcher::Fuse(KeyFrame* pKF, Sophus::Sim3f& Scw, const vector<MapPoint*>& vpPoints, float th,
+ * vector<MapPoint*>& vpReplacePoint) — src/ORBmatcher2.cc:612-729, as LoopClosing::SearchAndFuse calls it (both overloads), for
+ * n_kf key frames in one call: the search part.  The layout of orbx_fuse without invz: pairs [kf_offsets[k], kf_offsets[k + 1])
+ * belong to kfs[k]; pair q is point point[q] (a row of point_desc) at (u[q], v[q]) with level[q] = PredictScale.  valid[q] folds
+ * the caller's pre-checks: !isBad(), not in pKF->GetMapPoints() on entry, p3Dc(2) >= 0, the distance window, the viewing angle.
+ *   This call applies IsInImage (upper bounds strict), the window GetFeaturesInArea(u, v, th * mvScaleFactors[level]), the level
+ *   gate [level - 1, level] and the 1-NN by Hamming distance (earliest in the window's order on ties) under TH_LOW (50).  There is
+ *   no reprojection gate: kfs[k].inv_level_sigma2, kfs[k].bf and kfs[k].frame.u_right are not read and may be NULL / 0.
+ * Output: match[nq] = bestIdx when bestDist <= 50, else -1; n_fused[n_kf] = acceptances per key frame (the reference's return
+ *   value).  The bookkeeping (vpReplacePoint, AddMapPoint, the Replace loop of SearchAndFuse) stays with the caller.
+ * ORBX_ERR_INVALID_ARG as orbx_fuse (without the inv_level_sigma2 case).  Uses the loop-closing thread's own device scratch, so
+ * it never waits on the tracking thread's searches or on orbx_fuse. */
+int orbx_fuse_sim3(int device, int n_kf, const orbx_keyframe_view* kfs, const int32_t* kf_offsets, int n_desc, const uint8_t* point_desc,
+                   const int32_t* point, const uint8_t* valid, const float* u, const float* v, const int32_t* level, float th,
+                   int32_t* match, int* n_fused);
 /* Speculation rounds the last projection search on this thread needed (diagnostics; 0 = every query was final at once). */
 int orbx_projection_rounds(void);
 

@@ -9,8 +9,8 @@ from .capi import KP_DTYPE, OrbxError, lib  # noqa: F401
 from .bow import FeatureVector, ORBVocabulary, search_by_bow, search_for_triangulation  # noqa: F401
 from .extractor import ORBextractor, compute_tables, distribute_octree  # noqa: F401
 from .prep import Rectifier, undistort_keypoints  # noqa: F401
-from .projection import (FrameView, KeyFrameView, fuse, projection_rounds, search_by_projection_kf,  # noqa: F401
-                         search_by_projection_last, search_by_projection_map, search_for_initialization)
+from .projection import (FrameView, KeyFrameView, fuse, fuse_sim3, projection_rounds, search_by_projection_kf,  # noqa: F401
+                         search_by_projection_last, search_by_projection_map, search_by_projection_sim3, search_for_initialization)
 from . import io  # noqa: F401
 from .matcher import (ORBmatcher, ShardedMatcher, compute_stereo_matches, distinctive_descriptor, distinctive_descriptors, extract_stereo,  # noqa: F401
                       knn2_device, knn2_merge_device, measure_popc_peak, rotation_consistency)

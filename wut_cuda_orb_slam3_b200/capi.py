@@ -93,6 +93,8 @@ SIGNATURES = {
     "orbx_search_by_projection_kf": (_i, [_i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _i, _i, _vp, _vp]),
     "orbx_search_for_initialization": (_i, [_i, _vp, _vp, _i, _vp, _vp, _i, _f, _i, _vp, _vp]),
     "orbx_fuse": (_i, [_i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _vp, _vp]),
+    "orbx_search_by_projection_sim3": (_i, [_i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _f, _f, _vp, _vp]),
+    "orbx_fuse_sim3": (_i, [_i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _f, _vp, _vp]),
     "orbx_projection_rounds": (_i, []),
     "orbx_undistort_keypoints": (_i, [_i, _vp, _i, _vp, _vp, _i, _vp, _vp]),
     "orbx_rectifier_create": (_i, [_i, _vp, _vp, _sz, _i, _i, C.POINTER(_vp)]),

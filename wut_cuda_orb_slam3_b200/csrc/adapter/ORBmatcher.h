@@ -14,13 +14,19 @@
 //   int SearchForInitialization(Frame&, Frame&, vector<cv::Point2f>&, vector<int>&, windowSize)   src/ORBmatcher1.cc:650-765
 //   int Fuse(KeyFrame*, const vector<MapPoint*>&, th, bRight)                        src/ORBmatcher2.cc:420-610
 //   int Fuse(const vector<KeyFrame*>&, const vector<MapPoint*>&, th)  (added: the forward loop of SearchInNeighbors in one call)
-// Not declared (not on the tracking path / out of scope, DESIGN.md §8): the Sim3 SearchByProjection overloads,
-// SearchBySim3, the Sim3 Fuse; SearchForTriangulation is exported by the C ABI (orbx_search_for_triangulation) and takes F12 from the
-// caller.
+//   int SearchByProjection(KeyFrame*, Sim3f&, vpPoints, vpMatched, th, ratioHamming)                    src/ORBmatcher1.cc:429-648
+//   int SearchByProjection(KeyFrame*, Sim3f&, vpPoints, vpPointsKFs, vpMatched, vpMatchedKF, th, ratioHamming)
+//   int Fuse(KeyFrame*, Sim3f&, const vector<MapPoint*>&, th, vector<MapPoint*>& vpReplacePoint)       src/ORBmatcher2.cc:612-729
+//   int SearchAndFuse(const vector<KeyFrame*>&, const vector<Sim3f>&, const vector<MapPoint*>&, th)
+//                                     (added: the loop body of both LoopClosing::SearchAndFuse overloads in one call)
+// Not declared (no live caller / out of scope, DESIGN.md §8): SearchBySim3; SearchForTriangulation is exported by the C ABI
+// (orbx_search_for_triangulation) and takes F12 from the caller.
 #ifndef ORBMATCHER_H
 #define ORBMATCHER_H
 
 #include <cstring>
+#include <mutex>
+#include <set>
 #include <stdexcept>
 #include <type_traits>
 #include <vector>
@@ -132,6 +138,56 @@ public:
         return orbx_adapter::FuseApply(vpKFs, vpMapPoints, th, valid, u, v, invz, level, device);
     }
 
+    // Project MapPoints using a Similarity Transformation and search matches.
+    // Used in loop detection (Loop Closing)
+    // (Member templates like Fuse: the Sim3 type is deduced from the argument, Sophus::Sim3f in ORB-SLAM3.)
+    template <class KF = KeyFrame, class Sim3T, class MP = MapPoint>
+    int SearchByProjection(KF* pKF, Sim3T& Scw, const std::vector<MP*>& vpPoints, std::vector<MP*>& vpMatched, int th, float ratioHamming = 1.0)
+    {
+        return SearchByProjectionSim3<KF, Sim3T, MP>(pKF, Scw, vpPoints, nullptr, vpMatched, nullptr, th, ratioHamming);
+    }
+
+    // Project MapPoints using a Similarity Transformation and search matches.
+    // Used in Place Recognition (Loop Closing and Merging)
+    template <class KF = KeyFrame, class Sim3T, class MP = MapPoint>
+    int SearchByProjection(KF* pKF, Sim3T& Scw, const std::vector<MP*>& vpPoints, const std::vector<KF*>& vpPointsKFs, std::vector<MP*>& vpMatched,
+                           std::vector<KF*>& vpMatchedKF, int th, float ratioHamming = 1.0)
+    {
+        if (vpPointsKFs.size() < vpPoints.size()) throw std::invalid_argument("ORBmatcher::SearchByProjection: vpPointsKFs is shorter than vpPoints");
+        if ((int)vpMatchedKF.size() != pKF->N) throw std::invalid_argument("ORBmatcher::SearchByProjection: vpMatchedKF must have pKF->N entries");
+        return SearchByProjectionSim3<KF, Sim3T, MP>(pKF, Scw, vpPoints, &vpPointsKFs, vpMatched, &vpMatchedKF, th, ratioHamming);
+    }
+
+    // Project MapPoints into KeyFrame using a given Sim3 and search for duplicated MapPoints.
+    template <class KF = KeyFrame, class Sim3T, class MP = MapPoint>
+    int Fuse(KF* pKF, Sim3T& Scw, const std::vector<MP*>& vpPoints, float th, std::vector<MP*>& vpReplacePoint)
+    {
+        if (vpReplacePoint.size() < vpPoints.size()) throw std::invalid_argument("ORBmatcher::Fuse: vpReplacePoint is shorter than vpPoints");
+        return FuseSim3(std::vector<KF*>(1, pKF), std::vector<typename std::remove_const<Sim3T>::type>(1, Scw), vpPoints, th, vpReplacePoint, [](int) {});
+    }
+
+    // The loop body of both LoopClosing::SearchAndFuse overloads (loop correction and map merge) for the key frames vpKFs with
+    // their corrected poses vScw, in order: per key frame, vpReplacePoints(M, NULL), Fuse(pKFi, Scw_i, vpMapPoints, th,
+    // vpReplacePoints), then under pKFi->GetMap()->mMutexMapUpdate pRep->Replace(vpMapPoints[i]) for every non-NULL pRep.
+    // One orbx_fuse_sim3 call for all key frames, plus one re-search call before a key frame whose points a Replace loop gave
+    // new descriptors (orbx_adapter::FuseSim3Apply).  Returns the sum of the Fuse return values.
+    template <class KF = KeyFrame, class Sim3T, class MP = MapPoint>
+    int SearchAndFuse(const std::vector<KF*>& vpKFs, const std::vector<Sim3T>& vScw, const std::vector<MP*>& vpMapPoints, const float th = 4)
+    {
+        if (vScw.size() != vpKFs.size()) throw std::invalid_argument("ORBmatcher::SearchAndFuse: one Sim3 per key frame");
+        std::vector<MP*> vpReplacePoints(vpMapPoints.size(), static_cast<MP*>(NULL));
+        return FuseSim3(vpKFs, vScw, vpMapPoints, th, vpReplacePoints, [&](int k) {
+            // Get Map Mutex
+            std::unique_lock<std::mutex> lock(vpKFs[k]->GetMap()->mMutexMapUpdate);
+            const int nLP = (int)vpMapPoints.size();
+            for (int i = 0; i < nLP; i++) {
+                MP* pRep = vpReplacePoints[i];
+                if (pRep) pRep->Replace(vpMapPoints[i]);
+            }
+            std::fill(vpReplacePoints.begin(), vpReplacePoints.end(), static_cast<MP*>(NULL));   // the next key frame's vpReplacePoints
+        });
+    }
+
     // Search matches between MapPoints in a KeyFrame and ORB in a Frame.
     // Brute force constrained to ORB that belong to the same vocabulary node (at a certain level)
     // Used in Relocalisation and Loop Detection
@@ -185,6 +241,83 @@ public:
     static const int HISTO_LENGTH = 30;
 
 protected:
+    // The per-point lines of the Sim3 searches (src/ORBmatcher1.cc:429-648, ORBmatcher2.cc:612-729) after the isBad() /
+    // spAlreadyFound test `keep`, with Eigen's / Sophus' own arithmetic: Tcw = SE3(R, t / s), depth, projection, distance window,
+    // viewing angle, PredictScale.  IsInImage and the window are the C ABI's.  Fills entries [0, M) of valid / u / v / level.
+    template <class KF, class Sim3T, class MP, class Keep>
+    static void Sim3Project(KF* pKF, const Sim3T& Scw, const std::vector<MP*>& vpPoints, Keep keep, uint8_t* valid, float* u, float* v, int32_t* level)
+    {
+        if (pKF->NLeft != -1) throw std::invalid_argument("ORBmatcher: NLeft != -1 (two-camera rigs keep the reference code)");
+        // Decompose Scw
+        using SE3 = typename std::decay<decltype(pKF->GetPose())>::type;
+        const SE3 Tcw = SE3(Scw.rotationMatrix(), Scw.translation() / Scw.scale());
+        const auto Ow = Tcw.inverse().translation();
+        for (int iMP = 0, iendMP = (int)vpPoints.size(); iMP < iendMP; iMP++) {
+            MP* pMP = vpPoints[iMP];
+            if (!pMP) continue;                                             // (the reference dereferences it)
+            // Discard Bad MapPoints and already found
+            if (pMP->isBad() || !keep(pMP)) continue;
+            using Vec3 = typename std::decay<decltype(pMP->GetWorldPos())>::type;
+            // Get 3D Coords.
+            const Vec3 p3Dw = pMP->GetWorldPos();
+            // Transform into Camera Coords.
+            const Vec3 p3Dc = Tcw * p3Dw;
+            // Depth must be positive
+            if (p3Dc(2) < 0.0f) continue;
+            // Project into Image
+            const auto uv = pKF->mpCamera->project(p3Dc);
+            // Depth must be inside the scale invariance region of the point
+            const float maxDistance = pMP->GetMaxDistanceInvariance();
+            const float minDistance = pMP->GetMinDistanceInvariance();
+            const Vec3 PO = p3Dw - Ow;
+            const float dist = PO.norm();
+            if (dist < minDistance || dist > maxDistance) continue;
+            // Viewing angle must be less than 60 deg
+            const Vec3 Pn = pMP->GetNormal();
+            if (PO.dot(Pn) < 0.5 * dist) continue;
+            valid[iMP] = 1; u[iMP] = uv(0); v[iMP] = uv(1);
+            level[iMP] = pMP->PredictScale(dist, pKF);                     // IsInImage and the window: the C ABI
+        }
+    }
+
+    template <class KF, class Sim3T, class MP>
+    int SearchByProjectionSim3(KF* pKF, Sim3T& Scw, const std::vector<MP*>& vpPoints, const std::vector<KF*>* vpPointsKFs,
+                               std::vector<MP*>& vpMatched, std::vector<KF*>* vpMatchedKF, int th, float ratioHamming)
+    {
+        if ((int)vpMatched.size() != pKF->N) throw std::invalid_argument("ORBmatcher::SearchByProjection: vpMatched must have pKF->N entries");
+        const int M = (int)vpPoints.size();
+        std::vector<uint8_t> valid(M, 0);
+        std::vector<float> u(M, 0.f), v(M, 0.f);
+        std::vector<int32_t> level(M, 0), matchF;
+        // Set of MapPoints already found in the KeyFrame
+        std::set<MP*> spAlreadyFound(vpMatched.begin(), vpMatched.end());
+        spAlreadyFound.erase(static_cast<MP*>(NULL));
+        Sim3Project(pKF, Scw, vpPoints, [&](MP* pMP) { return !spAlreadyFound.count(pMP); }, valid.data(), u.data(), v.data(), level.data());
+        const int nmatches = orbx_adapter::SearchByProjectionSim3(pKF, vpPoints, vpMatched, valid, u, v, level, th, ratioHamming, matchF, device);
+        for (int idx = 0; idx < pKF->N; ++idx) {
+            if (matchF[idx] < 0) continue;
+            vpMatched[idx] = vpPoints[matchF[idx]];
+            if (vpMatchedKF) (*vpMatchedKF)[idx] = (*vpPointsKFs)[matchF[idx]];
+        }
+        return nmatches;
+    }
+
+    // The Sim3 Fuse of vpPoints into each of vpKFs with its Sim3, in order; after(k) runs once key frame k is applied.
+    template <class KF, class Sim3T, class MP, class After>
+    int FuseSim3(const std::vector<KF*>& vpKFs, const std::vector<Sim3T>& vScw, const std::vector<MP*>& vpPoints, const float th,
+                 std::vector<MP*>& vpReplacePoint, After after)
+    {
+        const size_t M = vpPoints.size(), nq = vpKFs.size() * M;
+        std::vector<uint8_t> valid(nq, 0);
+        std::vector<float> u(nq, 0.f), v(nq, 0.f);
+        std::vector<int32_t> level(nq, 0);
+        // spAlreadyFound = pKF->GetMapPoints() is taken at the start of each key frame, by FuseSim3Apply
+        for (size_t k = 0; k < vpKFs.size(); ++k)
+            Sim3Project(vpKFs[k], vScw[k], vpPoints, [](MP*) { return true; }, valid.data() + k * M, u.data() + k * M, v.data() + k * M,
+                        level.data() + k * M);
+        return orbx_adapter::FuseSim3Apply(vpKFs, vpPoints, th, valid, u, v, level, vpReplacePoint, after, device);
+    }
+
     // DBoW2::FeatureVector (std::map<NodeId, std::vector<unsigned int>>, Thirdparty/DBoW2/DBoW2/FeatureVector.h:23-25) -> CSR
     struct Csr {
         std::vector<uint32_t> nodes, indices;

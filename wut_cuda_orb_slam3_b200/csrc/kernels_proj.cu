@@ -31,7 +31,9 @@
 // below q on that chain (DESIGN.md §5b).
 //
 // ORBmatcher::Fuse src/ORBmatcher2.cc:420-610 (fuse_grid_kernel, fuse_scan_kernel): the candidate loop never reads the key
-// frame's map points, so every (key frame, point) pair is independent — one wide launch, no rounds (DESIGN.md §5b).
+// frame's map points, so every (key frame, point) pair is independent — one wide launch, no rounds (DESIGN.md §5b).  The Sim3
+// Fuse of loop closing (src/ORBmatcher2.cc:612-729) is the same loop without the reprojection gate (fuse_scan_kernel<false>);
+// the Sim3 SearchByProjection (src/ORBmatcher1.cc:429-648) is mode 1 above.
 #include <climits>
 
 #include "orbx_internal.cuh"
@@ -264,7 +266,9 @@ __global__ void __launch_bounds__(1024) fuse_grid_kernel(FuseArgs f)
 // The loop never reads the key frame's map points, so every pair is independent.  KeyFrame::GetFeaturesInArea is the window of
 // Frame::GetFeaturesInArea without levels; the level gate [level - 1, level] comes first in the loop, so it is folded into the
 // window's membership test.  The least key (distance, cell id, index) is the earliest candidate at the least distance, which is
-// what strict '<' keeps.
+// what strict '<' keeps.  kReprojGate = false is the Sim3 Fuse (src/ORBmatcher2.cc:612-729): no reprojection gate, so neither
+// inv_sigma2 nor u_right is read (its bestDist starts at INT_MAX instead of 256, which changes nothing under TH_LOW).
+template <bool kReprojGate>
 __global__ void __launch_bounds__(256) fuse_scan_kernel(FuseArgs f)
 {
     const int lane = threadIdx.x & 31;
@@ -283,19 +287,21 @@ __global__ void __launch_bounds__(256) fuse_scan_kernel(FuseArgs f)
             const int idx = __ldg(a.items + t);
             // kpLevel < nPredictedLevel - 1 || kpLevel > nPredictedLevel (an octave of -1 would index mvInvLevelSigma2[-1])
             if (!in_area(a, idx, q.u, q.v, q.r, max(q.level - 1, 0), q.level)) continue;
-            const orbx_keypoint* kp = a.kp + idx;
-            const int oct = __ldg(&kp->octave);
-            const float inv = K.inv_sigma2[oct];
-            const float ex = __fsub_rn(q.u, __ldg(&kp->x)), ey = __fsub_rn(q.v, __ldg(&kp->y));
-            const float kpr = a.u_right ? __ldg(a.u_right + idx) : -1.0f;
-            // float e2, every product and sum rounded; 'e2 * inv' rounded to float, then compared with the double constant
-            if (kpr >= 0.0f) {
-                const float er = __fsub_rn(q.ur, kpr);
-                const float e2 = __fadd_rn(__fadd_rn(__fmul_rn(ex, ex), __fmul_rn(ey, ey)), __fmul_rn(er, er));
-                if ((double)__fmul_rn(e2, inv) > 7.8) continue;
-            } else {
-                const float e2 = __fadd_rn(__fmul_rn(ex, ex), __fmul_rn(ey, ey));
-                if ((double)__fmul_rn(e2, inv) > 5.99) continue;
+            if constexpr (kReprojGate) {
+                const orbx_keypoint* kp = a.kp + idx;
+                const int oct = __ldg(&kp->octave);
+                const float inv = K.inv_sigma2[oct];
+                const float ex = __fsub_rn(q.u, __ldg(&kp->x)), ey = __fsub_rn(q.v, __ldg(&kp->y));
+                const float kpr = a.u_right ? __ldg(a.u_right + idx) : -1.0f;
+                // float e2, every product and sum rounded; 'e2 * inv' rounded to float, then compared with the double constant
+                if (kpr >= 0.0f) {
+                    const float er = __fsub_rn(q.ur, kpr);
+                    const float e2 = __fadd_rn(__fadd_rn(__fmul_rn(ex, ex), __fmul_rn(ey, ey)), __fmul_rn(er, er));
+                    if ((double)__fmul_rn(e2, inv) > 7.8) continue;
+                } else {
+                    const float e2 = __fadd_rn(__fmul_rn(ex, ex), __fmul_rn(ey, ey));
+                    if ((double)__fmul_rn(e2, inv) > 5.99) continue;
+                }
             }
             uint32_t d[8];
             load_desc(a.desc, (size_t)idx, d);
@@ -396,10 +402,13 @@ cudaError_t launch_proj_search(const ProjArgs& a, cudaStream_t st)
     return cudaGetLastError();
 }
 
-cudaError_t launch_fuse(const FuseArgs& a, cudaStream_t st)
+cudaError_t launch_fuse(const FuseArgs& a, bool reproj_gate, cudaStream_t st)
 {
     if (a.n_kf > 0) fuse_grid_kernel<<<a.n_kf, 1024, 0, st>>>(a);
-    if (a.nq > 0) fuse_scan_kernel<<<(a.nq + 7) / 8, 256, 0, st>>>(a);
+    if (a.nq > 0) {
+        if (reproj_gate) fuse_scan_kernel<true><<<(a.nq + 7) / 8, 256, 0, st>>>(a);
+        else fuse_scan_kernel<false><<<(a.nq + 7) / 8, 256, 0, st>>>(a);
+    }
     count_launch((a.n_kf > 0) + (a.nq > 0));
     return cudaGetLastError();
 }
