@@ -355,22 +355,36 @@ def test_batch_pyramid_streaming_kernel_is_bit_exact(oracle, cols, rows, nlevels
         assert np.array_equal(ex.pyramid_level(l, with_border=True), got[1][l]), l
 
 
-def test_tiled_pyramid_kernel_matches_streaming_kernel():
-    """ORBX_PYR_PIPE=0 selects the tiled resize kernel (the fallback of the streaming one, e.g. without tensor maps): a child
-    process with the switch set must produce the same bordered pyramid bytes as this process (streaming kernel, compared with
-    the oracle in the tests above)."""
-    import hashlib, os, subprocess, sys
+def test_fallback_kernels_match_default_kernels():
+    """Test hooks that reach the fallback kernels: ORBX_PYR_PIPE=0 selects the tiled resize kernel instead of the streaming one,
+    ORBX_NO_TMA=1 builds no tensor maps (as when cuTensorMapEncodeTiled fails or a box does not fit), so the tiled resize stages
+    its window with vector loads, the blur takes the register-streaming kernel and rBRIEF gathers from global memory.  A child
+    process under each hook must produce the same bordered pyramid bytes, keypoints and descriptors as one under the default
+    (compared with the oracle in the tests above), for single frames and for a 9-frame batch."""
+    import os, subprocess, sys
     code = ("import hashlib, numpy as np, wut_cuda_orb_slam3_b200 as orbx\n"
             "from wut_cuda_orb_slam3_b200 import synth\n"
             "h = hashlib.sha1()\n"
             "for cols, rows, scale in ((752, 480, 1.2), (333, 211, 1.3)):\n"
             "    ex = orbx.ORBextractor(500, scale, 6, 20, 7)\n"
-            "    ex(synth.image(77, cols, rows))\n"
+            "    nm, kps, desc = ex(synth.image(77, cols, rows))\n"
+            "    h.update(np.int32(nm).tobytes()); h.update(kps.tobytes()); h.update(desc.tobytes())\n"
             "    for l in range(6): h.update(ex.pyramid_level(l, with_border=True).tobytes())\n"
-            "print(h.hexdigest())\n")
+            "F = 9\n"
+            "imgs = np.stack([synth.image(600 + f, 752, 480) for f in range(F)])\n"
+            "ex = orbx.ORBextractor(1000, 1.2, 8, 20, 7, max_batch=F)\n"
+            "nm, n, kps, desc = ex.extract_batch(imgs)\n"
+            "h.update(nm.tobytes()); h.update(n.tobytes())\n"
+            "for f in range(F):\n"
+            "    h.update(kps[f, :n[f]].tobytes()); h.update(desc[f, :n[f]].tobytes())\n"
+            "    for l in range(8): h.update(ex.pyramid_level(l, frame=f, with_border=True).tobytes())\n"
+            "print(int(n.min()), h.hexdigest())\n")
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    base = {k: v for k, v in os.environ.items() if k not in ("ORBX_PYR_PIPE", "ORBX_NO_TMA")}
+    base["PYTHONPATH"] = root + os.pathsep + os.environ.get("PYTHONPATH", "")
     digests = []
-    for v in ("0", "1"):
-        env = dict(os.environ, ORBX_PYR_PIPE=v, PYTHONPATH=root + os.pathsep + os.environ.get("PYTHONPATH", ""))
-        digests.append(subprocess.check_output([sys.executable, "-c", code], env=env, text=True, cwd=root).strip().splitlines()[-1])
-    assert digests[0] == digests[1]
+    for hook in ({}, {"ORBX_PYR_PIPE": "0"}, {"ORBX_NO_TMA": "1"}):
+        out = subprocess.check_output([sys.executable, "-c", code], env=dict(base, **hook), text=True, cwd=root)
+        digests.append(out.strip().splitlines()[-1])
+    assert int(digests[0].split()[0]) > 100, digests[0]
+    assert digests[1] == digests[0] and digests[2] == digests[0], digests

@@ -575,7 +575,8 @@ static int ensure_slot(orbx_extractor* ex, Slot& s, int frames)
         CUtensorMap* d_maps = nullptr;
         if ((rc = dev_alloc(s, &d_maps, maps.size()))) return rc;
         CU(cudaMemcpy(d_maps, maps.data(), maps.size() * sizeof(CUtensorMap), cudaMemcpyHostToDevice));
-        static const bool no_tma = getenv("ORBX_NO_TMA") != nullptr;      // A/B switch for measurements
+        // ORBX_NO_TMA: a test hook, the only way the suite reaches the kernels taken when no tensor maps can be built
+        static const bool no_tma = getenv("ORBX_NO_TMA") != nullptr;
         if (ok_resize && !no_tma) s.ws.tmap_resize = d_maps;
         if (ok_blur && !no_tma) s.ws.tmap_blur = d_maps + kMaxLevels;
         if (ok_rpipe && !no_tma) s.ws.tmap_rpipe = d_maps + 2 * kMaxLevels;
@@ -669,10 +670,8 @@ static int run_chunk(orbx_extractor* ex, Slot& s, const uint8_t* d_images, size_
     // launches ends with a tail of half-empty SMs, and the blur's persistent CTAs fill those: 3.163 -> 3.088 ms per 512 frames.
     // (The blur beside the octree instead: no gain — the octree's four CTAs hold the whole register file of an SM.  FAST's three
     // launches alternating between two streams: 3.17 ms.  The octree of the first FAST group's levels beside the later FAST launches: 3.13 ms.)  Not while
-    // profiling (the per-stage events assume one stream), not for a few frames (run_single_forked forks per level);
-    // ORBX_BATCH_FORK=0 keeps everything on one stream.
-    static const char* fork_env = getenv("ORBX_BATCH_FORK");
-    const bool fork = (fork_env ? atoi(fork_env) != 0 : true) && !ex->profiling && frames >= 8;
+    // profiling (the per-stage events assume one stream), not for a few frames (run_single_forked forks per level).
+    const bool fork = !ex->profiling && frames >= 8;
     if (fork) {
         if (!ex->side[0]) CU(cudaStreamCreateWithFlags(&ex->side[0], cudaStreamNonBlocking));
         if (!ex->ev_lvl[0]) CU(cudaEventCreateWithFlags(&ex->ev_lvl[0], cudaEventDisableTiming));
@@ -778,13 +777,11 @@ static int enqueue_single(orbx_extractor* ex, const uint8_t* image, int rows, in
     if ((rc = ensure_mirror(ex, st))) return rc;
     if (step == (size_t)cols) CU(cudaMemcpyAsync(s.d_in, image, dframe, cudaMemcpyHostToDevice, st));
     else CU(cudaMemcpy2DAsync(s.d_in, dpitch, image, step, cols, rows, cudaMemcpyHostToDevice, st));
-    static const bool graphs = !(getenv("ORBX_GRAPH") && atoi(getenv("ORBX_GRAPH")) == 0);
-    static const bool forked = !(getenv("ORBX_SINGLE_FORK") && atoi(getenv("ORBX_SINGLE_FORK")) == 0);   // A/B switch
     auto body = [&](cudaStream_t cs) -> int {
-        if ((forked && !ex->profiling) || ex->mirror) return run_single_forked(ex, s, s.d_in, dpitch, lap0, lap1, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm, cs);
+        if (!ex->profiling || ex->mirror) return run_single_forked(ex, s, s.d_in, dpitch, lap0, lap1, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm, cs);
         return run_chunk(ex, s, s.d_in, dframe, dpitch, 1, lap0, lap1, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm, cs);
     };
-    if (graphs && !ex->profiling && !ex->force_eager && ex->single_calls++ > 0) {
+    if (!ex->profiling && !ex->force_eager && ex->single_calls++ > 0) {
         orbx_extractor::GraphKey key;
         key.rows = rows; key.cols = cols; key.lap0 = lap0; key.lap1 = lap1; key.capacity = capacity;
         key.pyr = s.ws.pyr; key.d_in = s.d_in; key.d_kps = s.d_kps; key.cand = s.ws.cand;
@@ -1041,36 +1038,25 @@ int orbx_extract_batch(orbx_extractor* ex, const uint8_t* const* images, int n_f
     const int chunk = ex->max_batch > 0 ? std::min(ex->max_batch, n_frames) : std::min(n_frames, 64);
     // Chunk schedule: the first host->device copy cannot overlap any compute, so the pipeline ramps up with a quarter and a
     // half chunk before it settles on full chunks (shorter un-overlapped prologue; the tail is whatever remains).
-    std::vector<std::pair<int, int>> sched;          // (first frame, frames)
-    int max_chunk = chunk;
+    std::vector<std::pair<int, int>> sched;          // (first frame, frames); no entry exceeds `chunk`
     {
         int f0 = 0;
-        const char* env = getenv("ORBX_BATCH_SCHED");            // measurement override: "64,192,256" (last entry repeats)
-        if (env && *env) {
-            std::vector<int> sizes;
-            for (const char* p = env; *p;) { sizes.push_back(std::max(atoi(p), 1)); while (*p && *p != ',') ++p; if (*p == ',') ++p; }
-            for (size_t i = 0; f0 < n_frames; ++i) {
-                const int nf = std::min(sizes[std::min(i, sizes.size() - 1)], n_frames - f0);
-                sched.emplace_back(f0, nf); f0 += nf; max_chunk = std::max(max_chunk, nf);
-            }
-        } else {
-            const int ramp[2] = {std::max(chunk / 4, 1), std::max(chunk / 2, 1)};
-            for (int r = 0; r < 2 && n_frames - f0 > 2 * chunk; ++r) { sched.emplace_back(f0, ramp[r]); f0 += ramp[r]; }
-            // ... and ramps down the same way: the compute of a chunk trails its upload, so what is left after the LAST upload
-            // is one chunk of compute + its download — a quarter chunk instead of a full one (trace of a 4096-frame call:
-            // 2.8 ms of tail behind 27.3 ms of back-to-back uploads)
-            const int tail = n_frames - f0 > 3 * chunk ? ramp[0] + ramp[1] : 0;
-            while (f0 < n_frames - tail) { const int nf = std::min(chunk, n_frames - tail - f0); sched.emplace_back(f0, nf); f0 += nf; }
-            if (tail) { sched.emplace_back(f0, ramp[1]); f0 += ramp[1]; sched.emplace_back(f0, ramp[0]); f0 += ramp[0]; }
-        }
+        const int ramp[2] = {std::max(chunk / 4, 1), std::max(chunk / 2, 1)};
+        for (int r = 0; r < 2 && n_frames - f0 > 2 * chunk; ++r) { sched.emplace_back(f0, ramp[r]); f0 += ramp[r]; }
+        // ... and ramps down the same way: the compute of a chunk trails its upload, so what is left after the LAST upload
+        // is one chunk of compute + its download — a quarter chunk instead of a full one (trace of a 4096-frame call:
+        // 2.8 ms of tail behind 27.3 ms of back-to-back uploads)
+        const int tail = n_frames - f0 > 3 * chunk ? ramp[0] + ramp[1] : 0;
+        while (f0 < n_frames - tail) { const int nf = std::min(chunk, n_frames - tail - f0); sched.emplace_back(f0, nf); f0 += nf; }
+        if (tail) { sched.emplace_back(f0, ramp[1]); f0 += ramp[1]; sched.emplace_back(f0, ramp[0]); f0 += ramp[0]; }
     }
     const int nchunks = (int)sched.size();
     const int nslots = std::min(nchunks, (int)orbx_extractor::kSlots);
-    if ((rc = ensure_capacity(ex, max_chunk, nslots))) return rc;
+    if ((rc = ensure_capacity(ex, chunk, nslots))) return rc;
     const size_t dpitch = (size_t)cols;
     const size_t dframe = dpitch * rows;
     for (int i = 0; i < nslots; ++i)
-        if ((rc = ensure_host_staging(ex->slots[i], dframe * max_chunk, max_chunk, capacity))) return rc;
+        if ((rc = ensure_host_staging(ex->slots[i], dframe * chunk, chunk, capacity))) return rc;
     // ORBX_TRACE_BATCH=1: per-chunk timeline (H2D start/end, compute end, D2H end; ms since the first H2D) on stderr
     static const bool trace = getenv("ORBX_TRACE_BATCH") != nullptr;
     std::vector<cudaEvent_t> tev;                    // [chunk][4]: H2D start / end, compute end (= D2H may start), D2H end
@@ -1085,9 +1071,7 @@ int orbx_extract_batch(orbx_extractor* ex, const uint8_t* const* images, int n_f
     // exactly three streams — H2D, compute, D2H — tied by per-slot events: with one copy stream per slot (seven streams) two of
     // them regularly landed on the same hardware connection (8 by default) and a chunk's D2H or the next H2D queued behind an
     // unrelated copy (90.5 k frames/s; 97.9 k with CUDA_DEVICE_MAX_CONNECTIONS=32; 98 k with three streams at any setting).
-    // ORBX_BATCH_SERIAL=0/1 overrides.
-    static const char* serial_env = getenv("ORBX_BATCH_SERIAL");
-    const bool serial = serial_env ? atoi(serial_env) != 0 : max_chunk >= 128;
+    const bool serial = chunk >= 128;
     if (serial && !ex->compute) {
         CU(cudaStreamCreateWithFlags(&ex->compute, cudaStreamNonBlocking));
         CU(cudaStreamCreateWithFlags(&ex->copy_in, cudaStreamNonBlocking));
@@ -1099,19 +1083,15 @@ int orbx_extract_batch(orbx_extractor* ex, const uint8_t* const* images, int n_f
     // then asks for the keypoint / descriptor rows every frame of the chunk actually has — one strided copy per array, row
     // count = the chunk's largest n_out — instead of `capacity` rows per frame.  The host looks at the counts of chunk c - 2
     // after it has queued chunk c, so two chunks of compute are always queued behind the one it waits for and the next
-    // upload never starts late.  ORBX_D2H_FULL=1 copies whole slabs as before (A/B switch).
-    static const bool d2h_full = getenv("ORBX_D2H_FULL") && atoi(getenv("ORBX_D2H_FULL")) != 0;
+    // upload never starts late.
     auto finish = [&](int c) -> int {
         Slot& s = ex->slots[c % nslots];
         const int f0 = sched[c].first, nf = sched[c].second;
         cudaStream_t ost = serial ? ex->copy_out : s.stream;
-        int rows_out = capacity;
-        if (!d2h_full) {
-            CU(cudaEventSynchronize(s.ev_cnt));
-            int mx = 0;
-            for (int f = 0; f < nf; ++f) mx = std::max(mx, n_out[f0 + f]);
-            rows_out = std::min(mx, capacity);         // a frame over capacity wrote nothing: the call fails below
-        }
+        CU(cudaEventSynchronize(s.ev_cnt));
+        int mx = 0;
+        for (int f = 0; f < nf; ++f) mx = std::max(mx, n_out[f0 + f]);
+        const int rows_out = std::min(mx, capacity);   // a frame over capacity wrote nothing: the call fails below
         if (rows_out > 0) {
             CU(cudaMemcpy2DAsync(keypoints + (size_t)f0 * capacity, sizeof(orbx_keypoint) * (size_t)capacity, s.d_kps,
                                  sizeof(orbx_keypoint) * (size_t)capacity, sizeof(orbx_keypoint) * (size_t)rows_out, nf, cudaMemcpyDeviceToHost, ost));

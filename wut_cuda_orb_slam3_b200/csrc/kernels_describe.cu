@@ -11,7 +11,6 @@
 #include <float.h>
 
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 
 #include "orbx_internal.cuh"
@@ -583,11 +582,9 @@ __global__ void __launch_bounds__(T) pack_kernel(const __grid_constant__ FrameGe
 
 cudaError_t launch_blur(const FrameGeom& fg, const Workspace& ws, int n_frames, cudaStream_t st)
 {
-    static const char* mode = getenv("ORBX_BLUR");                      // A/B switch: "pipe" (default with TMA) | "stream" | "tiled"
-    // default: the TMA-pipelined kernel for batches, the tiled kernel (more parallel units) for a few frames, the
-    // register-streaming kernel when no tensor maps are available
-    const char m0 = mode ? mode[0] : (!ws.tmap_blur ? 's' : (n_frames >= 8 ? 'p' : 't'));
-    if (m0 == 'p' && ws.tmap_blur) {
+    // the TMA-pipelined kernel for batches, the tiled kernel (more parallel units) for a few frames, the register-streaming
+    // kernel when no tensor maps are available or a batch has too many items for the pipelined kernel
+    if (ws.tmap_blur && n_frames >= 8) {
         int ipf = 0;
         for (int l = 0; l < fg.nlevels; ++l) ipf += ((fg.L[l].w + 127) / 128) * ((fg.L[l].h + 31) / 32);
         const long long total = (long long)ipf * n_frames;
@@ -610,8 +607,7 @@ cudaError_t launch_blur(const FrameGeom& fg, const Workspace& ws, int n_frames, 
             return cudaGetLastError();
         }
     }
-    const bool tiled = m0 == 't';
-    if (!tiled) {
+    if (!ws.tmap_blur || n_frames >= 8) {
         int items = 0;
         for (int l = 0; l < fg.nlevels; ++l) items += ((fg.L[l].w + 127) / 128) * ((fg.L[l].h + BS_ROWS - 1) / BS_ROWS);
         dim3 sgrid((items + 3) / 4, n_frames);
@@ -660,10 +656,9 @@ cudaError_t launch_orient_describe(const FrameGeom& fg, const Workspace& ws, int
                                    orbx_keypoint* d_kps, uint8_t* d_desc, int capacity, int* d_n_out, int* d_n_mono, bool* fused)
 {
     FusedPack fp{};
-    static const bool no_fuse = getenv("ORBX_NO_FUSED_PACK") != nullptr;        // A/B switch
     // a few frames only: the fused stores are scattered (7 lanes x 4 bytes per keypoint), which costs a 512-frame batch more than
     // the separate pack pass (measured 0.607 vs 0.557 + 0.024 ms), while a single frame saves a whole launch on its critical path
-    if (d_kps && d_desc && d_n_out && d_n_mono && !no_fuse && fg.kp_slots > 0 && n_frames < 8) {
+    if (d_kps && d_desc && d_n_out && d_n_mono && fg.kp_slots > 0 && n_frames < 8) {
         // output x = level x * scale lies in [19, cols): the lapping test px >= lap0 && px <= lap1 is decided by the bounds
         if (lap1 < kEdge || lap0 >= fg.cols || lap0 > lap1) fp.mode = 1;
         else if (lap0 <= kEdge && lap1 >= fg.cols) fp.mode = 2;
@@ -681,8 +676,7 @@ cudaError_t launch_orient_describe(const FrameGeom& fg, const Workspace& ws, int
         filled[dev & 63] = true;
     }
     dim3 grid((fg.kp_slots + 7) / 8, n_frames);
-    static const char* od_env = getenv("ORBX_DESC_STAGED");           // A/B switch: 0 = global gathers
-    if (ws.tmap_desc && (od_env ? atoi(od_env) != 0 : true)) orient_describe_kernel<true><<<grid, 256, 8 * kOdStage, st>>>(fg, ws, fp);
+    if (ws.tmap_desc) orient_describe_kernel<true><<<grid, 256, 8 * kOdStage, st>>>(fg, ws, fp);
     else orient_describe_kernel<false><<<grid, 256, 0, st>>>(fg, ws, fp);
     count_launch();
     return cudaGetLastError();

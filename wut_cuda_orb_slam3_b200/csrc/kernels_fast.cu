@@ -16,7 +16,6 @@
 #include "orbx_internal.cuh"
 
 #include <algorithm>
-#include <cstdlib>
 
 namespace orbx {
 
@@ -606,10 +605,7 @@ cudaError_t launch_fast(const FrameGeom& fg, const Workspace& ws, int n_frames, 
     if (level_hi <= 0) level_hi = fg.nlevels;
     if (fg.total_cells == 0 || level_lo >= level_hi) return cudaSuccess;
     // Small jobs (single frames: the SLAM tracking case) keep one CTA per cell for latency; batches use one warp per cell.
-    static const char* force = getenv("ORBX_FAST_KERNEL");      // "cta" | "warp": A/B switch for tests and measurements
-    bool use_warp = (long long)fg.total_cells * n_frames >= 8192;
-    if (force) use_warp = force[0] == 'w';
-    if (!use_warp) {
+    if ((long long)fg.total_cells * n_frames < 8192) {
         const int cell_lo = fg.L[level_lo].cell_base;
         const int cell_hi = fg.L[level_hi - 1].cell_base + fg.L[level_hi - 1].nCols * fg.L[level_hi - 1].nRows;
         if (cell_hi <= cell_lo) return cudaSuccess;

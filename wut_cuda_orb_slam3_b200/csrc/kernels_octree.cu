@@ -18,8 +18,6 @@
 //    nodes with std::sort(compareNodes) — replayed exactly (introsort_replay.h) because ties are broken by the
 //    algorithm's internal permutation — and splits from the back until size >= N.
 //  * Retain (756-771): first key with maximal response per node, in list order.
-#include <stdlib.h>
-
 #include <mutex>
 
 #include "introsort_replay.h"
@@ -693,12 +691,6 @@ cudaError_t octree_prepare()
 {
     cudaError_t e = cudaFuncSetAttribute(octree_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(octree_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(octree_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(octree_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return e;
     return cudaFuncSetAttribute(octree_kernel<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
 }
 
@@ -743,9 +735,6 @@ cudaError_t launch_octree(const FrameGeom& fg, const Workspace& ws, int n_frames
     // Batches: 256-thread CTAs (measured on 512-frame batches: 128 threads +7 %, 64 threads +36 %, 512 threads ~30 % slower:
     // the parallel phases need the lanes, the single-lane parts need many resident CTAs).
     // A few frames: the level-0 CTA is the critical path of the whole extraction, so give it more lanes.
-    static const int t_override = getenv("ORBX_OCTREE_THREADS") ? atoi(getenv("ORBX_OCTREE_THREADS")) : 0;
-    int T = n_frames >= 8 ? 256 : 1024;
-    if (t_override == 64 || t_override == 128 || t_override == 256 || t_override == 512 || t_override == 1024) T = t_override;
     const size_t smem = octree_smem_bytes(M, NB);
     if (smem > 200 * 1024) return cudaErrorInvalidConfiguration;
     int dev = 0;
@@ -762,11 +751,8 @@ cudaError_t launch_octree(const FrameGeom& fg, const Workspace& ws, int n_frames
         }
     }
     dim3 grid(n_frames, level_hi - level_lo);
-    if (T == 64) octree_kernel<64><<<grid, 64, smem, st>>>(fg, ws, M, NB, level_lo, g_err_flag[dev & 63]);
-    else if (T == 128) octree_kernel<128><<<grid, 128, smem, st>>>(fg, ws, M, NB, level_lo, g_err_flag[dev & 63]);
-    else if (T == 1024) octree_kernel<1024><<<grid, 1024, smem, st>>>(fg, ws, M, NB, level_lo, g_err_flag[dev & 63]);
-    else if (T == 512) octree_kernel<512><<<grid, 512, smem, st>>>(fg, ws, M, NB, level_lo, g_err_flag[dev & 63]);
-    else octree_kernel<256><<<grid, 256, smem, st>>>(fg, ws, M, NB, level_lo, g_err_flag[dev & 63]);
+    if (n_frames >= 8) octree_kernel<256><<<grid, 256, smem, st>>>(fg, ws, M, NB, level_lo, g_err_flag[dev & 63]);
+    else octree_kernel<1024><<<grid, 1024, smem, st>>>(fg, ws, M, NB, level_lo, g_err_flag[dev & 63]);
     count_launch();
     return cudaGetLastError();
 }

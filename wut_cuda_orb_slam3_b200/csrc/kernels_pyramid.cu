@@ -16,7 +16,6 @@
 //   pyr_resize_pipe_kernel    levels >= 1, the production path: one warp per 128 x 16 item of the BORDERED level, source window
 //                             by TMA into the warp's stage, IDP.2A horizontal pass, row sums in registers (scale <= 1.5)
 //   pyr_resize_tiled_kernel   levels >= 1 without tensor maps / scale in (1.5, 2]: 128 x 32 (128 x 16) tiles, u16 sum plane
-//   pyr_multilevel_kernel     all levels in one cooperative launch (opt-in, slower on batches)
 //   pyr_level0_kernel, pyr_resize_kernel   generic per-word fallbacks (tiny levels, scale > 2): each thread produces one aligned
 //                             32-bit word of a bordered row
 //   cvt_gray_kernel           cv::cvtColor RGB/BGR(A) -> grey of Tracking::GrabImage*
@@ -24,8 +23,6 @@
 #include <stdlib.h>
 
 #include <algorithm>
-
-#include <cooperative_groups.h>
 
 #include "orbx_internal.cuh"
 
@@ -163,8 +160,8 @@ constexpr int L0_H = 32;                     // level-0 copy tile height
 // pitch = cols) a 16-byte segment is read as its 4 - 5 covering aligned words and realigned with funnel shifts; the misalignment
 // differs from row to row.  `img_end` = one past the last image byte: the fifth word is only read when it lies inside the images.
 __device__ __forceinline__ void level0_tile(const LevelGeom& g, const Workspace& ws, const uint8_t* __restrict__ images, size_t frame_stride,
-                                            size_t in_pitch, uint8_t* t, int tid, int x0, int y0, int frame, bool aligned = true,
-                                            const uint8_t* img_end = nullptr)
+                                            size_t in_pitch, uint8_t* t, int tid, int x0, int y0, int frame, bool aligned,
+                                            const uint8_t* img_end)
 {
     const int tw = min(PT_W, g.w - x0), th = min(L0_H, g.h - y0);
     const uint8_t* S = images + (size_t)frame * frame_stride;
@@ -457,133 +454,6 @@ __global__ void __launch_bounds__(32 * kRpWarps) pyr_resize_pipe_kernel(const __
     }
 }
 
-// ---- ComputePyramid as ONE launch -------------------------------------------------------------------------------------------
-// All levels in one cooperative kernel: the CTAs walk the 128 x 32 tiles of level 0 (copy + border), meet at a grid-wide
-// barrier, walk the tiles of level 1 (source windows of level 0 staged by TMA: cp.async.bulk.tensor + mbarrier, one mbarrier per
-// CTA whose phase bit flips with every tile), meet again, and so on: level l + 1 only ever reads the finished level l.  Tiles are
-// dealt round-robin (tile id = blockIdx.x + k * gridDim.x over frames x tile rows x tile columns), the grid is one resident
-// wave.  Same tile code as the per-level kernels above, so the result is bit-identical by construction.
-namespace cg = cooperative_groups;
-
-__global__ void __launch_bounds__(PT_THREADS, PT_MINB) pyr_multilevel_kernel(const __grid_constant__ FrameGeom fg, Workspace ws,
-                                                                            const uint8_t* __restrict__ images, size_t frame_stride,
-                                                                            size_t in_pitch, int n_frames)
-{
-    constexpr int PT_H = 32, PT_SR = 52, PT_SP = 224;
-    __shared__ __align__(128) uint8_t src[PT_SR * PT_SP];
-    __shared__ __align__(16) uint16_t hbuf[PT_SR * PT_W];
-    __shared__ __align__(16) uint8_t outt[PT_H * PT_W];
-    __shared__ uint2 ytl[PT_H];
-    __shared__ __align__(8) uint64_t bar;
-    cg::grid_group grid = cg::this_grid();
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    uint32_t phase = 0;
-    if (tid == 0) mbar_init(&bar, 1);
-    __syncthreads();
-
-    {   // level 0
-        const LevelGeom& g = fg.L[0];
-        const int ntx = (g.w + PT_W - 1) / PT_W, nty = (g.h + L0_H - 1) / L0_H;
-        const long long ntiles = (long long)ntx * nty * n_frames;
-        for (long long t = blockIdx.x; t < ntiles; t += gridDim.x) {
-            const int frame = (int)(t / (ntx * nty)), r = (int)(t - (long long)frame * ntx * nty);
-            level0_tile(g, ws, images, frame_stride, in_pitch, outt, tid, (r % ntx) * PT_W, (r / ntx) * L0_H, frame);
-            __syncthreads();
-        }
-    }
-    for (int level = 1; level < fg.nlevels; ++level) {
-        __threadfence();
-        grid.sync();
-        const LevelGeom& g = fg.L[level];
-        const LevelGeom& p = fg.L[level - 1];
-        const int ntx = (g.w + PT_W - 1) / PT_W, nty = (g.h + PT_H - 1) / PT_H;
-        const long long ntiles = (long long)ntx * nty * n_frames;
-        for (long long t = blockIdx.x; t < ntiles; t += gridDim.x) {
-            const int frame = (int)(t / (ntx * nty)), r = (int)(t - (long long)frame * ntx * nty);
-            const int x0 = (r % ntx) * PT_W, y0 = (r / ntx) * PT_H;
-            const int tw = min(PT_W, g.w - x0), th = min(PT_H, g.h - y0);
-            const int tx = tid & (PT_W - 1);
-            const uint2 xt = __ldg(g.xtab + kEdge + x0 + min(tx, tw - 1));
-            if (tid < PT_H) ytl[tid] = __ldg(g.ytab + kEdge + y0 + min(tid, th - 1));
-            const uint2 xfirst = __ldg(g.xtab + kEdge + x0), xlast = __ldg(g.xtab + kEdge + x0 + tw - 1);
-            const uint2 yfirst = __ldg(g.ytab + kEdge + y0), ylast = __ldg(g.ytab + kEdge + y0 + th - 1);
-            const int sxmin = (int)(xfirst.x & 0xffff), sxmax = (int)(xlast.x >> 16);
-            const int symin = (int)(yfirst.x & 0xffff), symax = (int)(ylast.x >> 16);
-            const int nrows = symax - symin + 1;
-            const int cbase = sxmin & ~15;
-            int spitch;
-            if (ws.tmap_resize) {
-                spitch = p.tma_box_w;
-                if (tid == 0) {
-                    // the generic-proxy writes of the previous level (other CTAs, before the grid barrier) and of this CTA's
-                    // last tile are ordered before the async-proxy read of the bulk copy
-                    asm volatile("fence.proxy.async;" ::: "memory");
-                    mbar_expect_tx(&bar, (uint32_t)(p.tma_box_w * p.tma_box_h));
-                    tma_load_3d(src, ws.tmap_resize + (level - 1), &bar, kXPad + cbase, kEdge + symin, frame);
-                }
-                mbar_wait(&bar, phase);
-                phase ^= 1u;
-            } else {
-                spitch = PT_SP;
-                const int nvec = ((sxmax - cbase) >> 4) + 1;
-                const uint8_t* P = level_interior((const uint8_t*)ws.pyr, p, frame) + (size_t)symin * p.pitch + cbase;
-                if (lane < nvec)
-                    for (int rr = warp; rr < nrows; rr += PT_THREADS / 32)
-                        *reinterpret_cast<uint4*>(src + rr * PT_SP + lane * 16) = *(reinterpret_cast<const uint4*>(P + (size_t)rr * p.pitch) + lane);
-                __syncthreads();
-            }
-            resize_tile_passes<PT_H>(g, ws, src, hbuf, outt, ytl, xt, tid, tx, x0, y0, frame, tw, th, cbase, spitch, symin, nrows);
-            __syncthreads();
-        }
-    }
-}
-
-// One cooperative launch for all levels when every level takes the 128 x 32 tiled path; false = not applicable / not supported.
-static bool launch_pyramid_multilevel(const FrameGeom& fg, const Workspace& ws, const uint8_t* d_images, size_t frame_stride, size_t pitch,
-                                      int n_frames, cudaStream_t st, cudaError_t* err)
-{
-    *err = cudaSuccess;
-    const bool aligned = ((uintptr_t)d_images & 15) == 0 && (frame_stride & 15) == 0 && (pitch & 15) == 0;
-    if (!aligned) return false;
-    for (int l = 0; l < fg.nlevels; ++l) {
-        const LevelGeom& g = fg.L[l];
-        if (!(g.w >= 2 * kEdge + 2 && g.h >= 2 * kEdge + 2)) return false;
-        if (l > 0) {
-            const LevelGeom& p = fg.L[l - 1];
-            if (!(2LL * p.w <= 3LL * g.w && 2LL * p.h <= 3LL * g.h)) return false;
-            if (!ws.tmap_resize) {                      // the staged window must fit the fixed buffer of the non-TMA path
-                if ((long long)p.w * 32 / g.w + 4 > 52 || (long long)p.w * 128 / g.w + 36 > 224) return false;
-            }
-        }
-    }
-    static int resident[64] = {0};          // co-resident CTAs of the kernel per device (one wave)
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (resident[dev & 63] == 0) {
-        int coop = 0, per_sm = 0, sms = 0;
-        cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (!coop || cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pyr_multilevel_kernel, PT_THREADS, 0) != cudaSuccess || per_sm <= 0) {
-            cudaGetLastError();
-            resident[dev & 63] = -1;
-        } else {
-            resident[dev & 63] = per_sm * sms;
-        }
-    }
-    if (resident[dev & 63] <= 0) return false;
-    long long most = 0;
-    for (int l = 0; l < fg.nlevels; ++l) {
-        const int hh = l == 0 ? L0_H : 32;
-        most = std::max(most, (long long)((fg.L[l].w + PT_W - 1) / PT_W) * ((fg.L[l].h + hh - 1) / hh) * n_frames);
-    }
-    const int grid = (int)std::min<long long>(most, resident[dev & 63]);
-    const FrameGeom* pfg = &fg; const Workspace* pws = &ws;
-    void* args[] = {(void*)pfg, (void*)pws, (void*)&d_images, (void*)&frame_stride, (void*)&pitch, (void*)&n_frames};
-    *err = cudaLaunchCooperativeKernel((const void*)pyr_multilevel_kernel, dim3(grid), dim3(PT_THREADS), args, 0, st);
-    if (*err == cudaSuccess) count_launch();
-    return true;
-}
-
 // One level with the warp-streaming kernel; false = not applicable (the caller falls back to the tiled kernel).
 static bool launch_resize_pipe(const FrameGeom& fg, const Workspace& ws, int level, int n_frames, cudaStream_t st)
 {
@@ -611,8 +481,7 @@ static bool launch_resize_pipe(const FrameGeom& fg, const Workspace& ws, int lev
         }
     }
     if (n_sm_dev[dev & 63] < 0) return false;
-    static const char* per_env = getenv("ORBX_PYR_PIPE_CTAS");
-    int per_sm = std::min(per_env ? atoi(per_env) : 9, std::max(1, (200 * 1024) / (smem + 1024)));
+    const int per_sm = std::min(9, std::max(1, (200 * 1024) / (smem + 1024)));
     const int ctas = (int)std::min<long long>((total + kRpWarps - 1) / kRpWarps, (long long)n_sm_dev[dev & 63] * per_sm);
     const uint32_t magic_frame = (uint32_t)((1ULL << 32) / (uint64_t)(ntx * nstrips)), magic_ntx = (uint32_t)((1ULL << 32) / (uint64_t)ntx);
     pyr_resize_pipe_kernel<<<ctas, 32 * kRpWarps, smem, st>>>(fg, ws, level, stage_bytes, ntx, nstrips, (int)total,
@@ -625,16 +494,10 @@ cudaError_t launch_pyramid(const FrameGeom& fg, const Workspace& ws, const uint8
                            size_t pitch, int n_frames, cudaStream_t st, int level_lo, int level_hi)
 {
     if (level_hi <= 0) level_hi = fg.nlevels;
-    // The whole pyramid in one cooperative launch: ORBX_PYR_MULTILEVEL=1.  Off by default — measured on 512-frame batches the
-    // eight dependent launches are FASTER (0.81 ms vs 1.19 ms): a resident wave of persistent CTAs that walks its tiles in a
-    // fixed order and stops at seven grid-wide barriers loses more to imbalance and to the exposed TMA round trip of every
-    // tile than the launches lose at their boundaries (the hardware deals CTAs out as SMs free up).
-    static const char* ml_env = getenv("ORBX_PYR_MULTILEVEL");
-    const bool want_ml = ml_env ? atoi(ml_env) != 0 : false;
-    if (want_ml && level_lo == 0 && level_hi == fg.nlevels && fg.nlevels > 1) {
-        cudaError_t e = cudaSuccess;
-        if (launch_pyramid_multilevel(fg, ws, d_images, frame_stride, pitch, n_frames, st, &e)) return e;
-    }
+    // One launch per level.  A cooperative kernel for the whole pyramid was measured slower on 512-frame batches (1.19 ms vs
+    // 0.81 ms for the eight dependent launches): a resident wave of persistent CTAs that walks its tiles in a fixed order and
+    // stops at seven grid-wide barriers loses more to imbalance and to the exposed TMA round trip of every tile than the
+    // launches lose at their boundaries (the hardware deals CTAs out as SMs free up).
     for (int l = level_lo; l < level_hi; ++l) {
         const LevelGeom& g = fg.L[l];
         const int words = g.pitch / 4;
@@ -653,7 +516,8 @@ cudaError_t launch_pyramid(const FrameGeom& fg, const Workspace& ws, const uint8
             const bool s15 = 2LL * p.w <= 3LL * g.w && 2LL * p.h <= 3LL * g.h;
             const bool s20 = (long long)p.w <= 2LL * g.w && (long long)p.h <= 2LL * g.h;
             // warp-streaming kernel whenever it applies (batches: 0.45 vs 0.81 ms per 512 frames; a single frame: 49 vs 52 us for
-            // the eight levels, a stereo pair 236 vs 247 us); ORBX_PYR_PIPE=0 forces the tiled kernel (A/B switch)
+            // the eight levels, a stereo pair 236 vs 247 us).  ORBX_PYR_PIPE=0 forces the tiled kernel: a test hook, the only way
+            // the suite reaches the kernel that levels the streaming resize does not apply to take
             static const char* rp_env = getenv("ORBX_PYR_PIPE");
             const bool want_pipe = rp_env ? atoi(rp_env) != 0 : true;
             if (big && s15 && !g.area2x && want_pipe && ws.tmap_rpipe && launch_resize_pipe(fg, ws, l, n_frames, st)) {
