@@ -258,6 +258,32 @@ int orbx_extract_stereo(orbx_extractor* exL, orbx_extractor* exR, const uint8_t*
                         size_t step, orbx_keypoint* kpL, uint8_t* descL, int* nL, orbx_keypoint* kpR, uint8_t* descR, int* nR,
                         int capacity, float bf, float maxD, float* uRight, float* depth);
 
+/* orbx_extract_stereo over a batch of rectified pairs of one shape, with ONE handle for both sides: the reference builds its
+ * left and right extractors from the same settings, and results depend only on those and the image.  For every pair the
+ * outputs equal what orbx_extract_stereo returns for it, bit for bit.  n_pairs HOST pairs imagesL[i] / imagesR[i] (rows x cols,
+ * `step` bytes per row).  Outputs are [n_pairs][capacity] slabs: keypoints (28 B), descriptors (32 B) and mvuRight / mvDepth
+ * floats; nL / nR are [n_pairs].  Only the first nL[i] rows of a pair's uRight / depth are defined.  Host<->device copies are
+ * pipelined against compute when the host buffers are page-locked.
+ * n_pairs == 0 returns ORBX_OK and does nothing; n_pairs < 0, a NULL output, capacity <= 0 or step < cols: ORBX_ERR_INVALID_ARG;
+ * a NULL image array or image, rows or cols <= 0: ORBX_ERR_EMPTY_IMAGE; capacity >= 2^20: ORBX_ERR_UNSUPPORTED; a pair with more
+ * than `capacity` keypoints on either side: ORBX_ERR_CAPACITY (the rows of that pair are undefined; nothing is written past the
+ * slabs).
+ * The pyramids of a stereo batch are not kept for inspection: afterwards the stage probes, orbx_get_pyramid_level and
+ * orbx_stereo_match refuse every frame index (ORBX_ERR_INVALID_ARG) until the next extraction. */
+int orbx_extract_stereo_batch(orbx_extractor* ex, const uint8_t* const* imagesL, const uint8_t* const* imagesR, int n_pairs,
+                              int rows, int cols, size_t step, float bf, float maxD, orbx_keypoint* kpL, uint8_t* descL, int* nL,
+                              orbx_keypoint* kpR, uint8_t* descR, int* nR, int capacity, float* uRight, float* depth);
+/* The same on DEVICE-resident pairs: pair i at d_imagesL + i * frame_stride and d_imagesR + i * frame_stride (`pitch` bytes per
+ * row); every output is DEVICE memory with the slab layout above.  Asynchronous on `stream` (NULL = the extractor's own):
+ * orbx_sync and the next call on the handle wait for it, exactly as for orbx_extract_batch_device.  A pair over capacity is
+ * reported only through its device counts (*d_nL / *d_nR > capacity; the rows of that pair are undefined), as in
+ * orbx_extract_batch_device.  Rows
+ * of d_uRight / d_depth at or past a pair's *d_nL are left untouched. */
+int orbx_extract_stereo_batch_device(orbx_extractor* ex, const uint8_t* d_imagesL, const uint8_t* d_imagesR, size_t frame_stride,
+                                     int n_pairs, int rows, int cols, size_t pitch, float bf, float maxD, orbx_keypoint* d_kpL,
+                                     uint8_t* d_descL, int* d_nL, orbx_keypoint* d_kpR, uint8_t* d_descR, int* d_nR, int capacity,
+                                     float* d_uRight, float* d_depth, void* stream);
+
 /* ---- bag-of-words transform and vocabulary-guided matching (SURVEY.md §8 rows A13, A14 and (f)1) -------------------- */
 
 /* DBoW2::TemplatedVocabulary<FORB::TDescriptor, FORB> (Thirdparty/DBoW2/DBoW2/TemplatedVocabulary.h): a k-ary tree of

@@ -69,6 +69,8 @@ SIGNATURES = {
     "orbx_stereo_match": (_i, [_vp, _i, _vp, _i, _vp, _vp, _i, _vp, _vp, _i, _f, _f, _vp, _vp]),
     "orbx_stereo_match_device": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i, _f, _f, _vp, _vp, _vp]),
     "orbx_extract_stereo": (_i, [_vp, _vp, _vp, _vp, _i, _i, _sz, _vp, _vp, _vp, _vp, _vp, _vp, _i, _f, _f, _vp, _vp]),
+    "orbx_extract_stereo_batch": (_i, [_vp, _vp, _vp, _i, _i, _i, _sz, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
+    "orbx_extract_stereo_batch_device": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _sz, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "orbx_comm_unique_id": (_i, [_vp]),
     "orbx_comm_create": (_i, [_i, _i, _i, _vp, C.POINTER(_vp)]),
     "orbx_comm_from_nccl": (_i, [_i, _vp, _i, _i, C.POINTER(_vp)]),

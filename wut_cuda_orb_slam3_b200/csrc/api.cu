@@ -116,6 +116,10 @@ struct Slot {
     orbx_keypoint* d_kps = nullptr; uint8_t* d_desc = nullptr; int* d_n = nullptr; int* d_nm = nullptr;
     size_t out_cap = 0;            // keypoint rows the output staging holds
     int out_frames = 0;            // frames the per-frame counters hold
+    // stereo batches: mvuRight / mvDepth staging of the host-buffer call and the matcher's SAD scratch, [pairs][capacity]
+    float* d_su = nullptr; float* d_sd = nullptr; int* d_sad = nullptr;
+    int* d_snm = nullptr;          // [2 * pairs] monoIndex scratch of the device call (stereo outputs have no n_mono)
+    size_t stereo_rows = 0; int stereo_pairs = 0;
     std::vector<void*> allocs;
 };
 
@@ -240,6 +244,7 @@ static void free_slot(Slot& s)
     s.cap_frames = 0;
     s.d_in = nullptr; s.d_in_bytes = 0; s.d_color = nullptr; s.d_color_bytes = 0; s.d_kps = nullptr; s.d_desc = nullptr; s.d_n = nullptr; s.d_nm = nullptr;
     s.out_cap = 0; s.out_frames = 0;
+    s.d_su = nullptr; s.d_sd = nullptr; s.d_sad = nullptr; s.d_snm = nullptr; s.stereo_rows = 0; s.stereo_pairs = 0;
 }
 
 // release one buffer of a slot early (a staging buffer that is being replaced by a larger one)
@@ -640,6 +645,42 @@ static int ensure_host_staging(Slot& s, size_t in_bytes, int frames, int capacit
     return ORBX_OK;
 }
 
+// Matcher staging of a stereo chunk of `pairs` pairs.  As above: nothing may be in flight on the slot.
+static bool stereo_staging_fits(const Slot& s, int pairs, int capacity)
+{
+    return s.stereo_pairs >= pairs && s.stereo_rows >= (size_t)pairs * capacity;
+}
+static int ensure_stereo_staging(Slot& s, int pairs, int capacity)
+{
+    if (stereo_staging_fits(s, pairs, capacity)) return ORBX_OK;
+    dev_release(s, s.d_su); dev_release(s, s.d_sd); dev_release(s, s.d_sad); dev_release(s, s.d_snm);
+    s.stereo_rows = 0; s.stereo_pairs = 0;
+    const size_t rows = (size_t)pairs * capacity;
+    int rc;
+    if ((rc = dev_alloc(s, &s.d_su, rows)) || (rc = dev_alloc(s, &s.d_sd, rows)) || (rc = dev_alloc(s, &s.d_sad, rows)) ||
+        (rc = dev_alloc(s, &s.d_snm, 2 * (size_t)pairs)))
+        return rc;
+    s.stereo_rows = rows; s.stereo_pairs = pairs;
+    return ORBX_OK;
+}
+
+// Chunk schedule of the host-buffer batches: the first host->device copy cannot overlap any compute, so the pipeline ramps
+// up with a quarter and a half chunk before it settles on full chunks (shorter un-overlapped prologue) ...
+static std::vector<std::pair<int, int>> chunk_schedule(int n, int chunk)
+{
+    std::vector<std::pair<int, int>> sched;          // (first item, items); no entry exceeds `chunk`
+    int f0 = 0;
+    const int ramp[2] = {std::max(chunk / 4, 1), std::max(chunk / 2, 1)};
+    for (int r = 0; r < 2 && n - f0 > 2 * chunk; ++r) { sched.emplace_back(f0, ramp[r]); f0 += ramp[r]; }
+    // ... and ramps down the same way: the compute of a chunk trails its upload, so what is left after the LAST upload
+    // is one chunk of compute + its download — a quarter chunk instead of a full one (trace of a 4096-frame call:
+    // 2.8 ms of tail behind 27.3 ms of back-to-back uploads)
+    const int tail = n - f0 > 3 * chunk ? ramp[0] + ramp[1] : 0;
+    while (f0 < n - tail) { const int nf = std::min(chunk, n - tail - f0); sched.emplace_back(f0, nf); f0 += nf; }
+    if (tail) { sched.emplace_back(f0, ramp[1]); f0 += ramp[1]; sched.emplace_back(f0, ramp[0]); f0 += ramp[0]; }
+    return sched;
+}
+
 // The whole per-chunk pipeline on one stream.
 static const int kStages = 6;   // pyramid, fast, blur, octree, orient+describe, pack
 
@@ -655,15 +696,13 @@ static int prof_mark(orbx_extractor* ex, cudaStream_t st)
     return ORBX_OK;
 }
 
-static int run_chunk(orbx_extractor* ex, Slot& s, const uint8_t* d_images, size_t frame_stride, size_t pitch, int frames,
-                     int lap0, int lap1, orbx_keypoint* d_kps, uint8_t* d_desc, int capacity, int* d_n, int* d_nm,
-                     cudaStream_t st)
+static int run_chunk(orbx_extractor* ex, Slot& s, const ChunkIO& io, int frames, int lap0, int lap1, cudaStream_t st)
 {
     const FrameGeom& fg = ex->fg;
     int rc;
     ex->mirror_valid = false;          // only the forked single-frame pipeline sends the levels home
     if ((rc = prof_mark(ex, st))) return rc;
-    CU(launch_pyramid(fg, s.ws, d_images, frame_stride, pitch, frames, st));
+    CU(launch_pyramid(fg, s.ws, io, frames, st));
     if ((rc = prof_mark(ex, st))) return rc;
     // The blur depends on the pyramid only: for batches it runs on a side stream beside FAST and the octree.  While a FAST launch
     // is at full occupancy there is no room for a blur CTA (shared memory and registers are taken), but each of FAST's three
@@ -692,9 +731,9 @@ static int run_chunk(orbx_extractor* ex, Slot& s, const uint8_t* d_images, size_
     }
     if ((rc = prof_mark(ex, st))) return rc;
     bool fused = false;
-    CU(launch_orient_describe(fg, s.ws, frames, st, lap0, lap1, d_kps, d_desc, capacity, d_n, d_nm, &fused));
+    CU(launch_orient_describe(fg, s.ws, frames, st, lap0, lap1, io, &fused));
     if ((rc = prof_mark(ex, st))) return rc;
-    if (!fused) CU(launch_pack(fg, s.ws, frames, lap0, lap1, d_kps, d_desc, capacity, d_n, d_nm, st));
+    if (!fused) CU(launch_pack(fg, s.ws, frames, lap0, lap1, io, st));
     if ((rc = prof_mark(ex, st))) return rc;
     return ORBX_OK;
 }
@@ -708,13 +747,14 @@ static int run_single_forked(orbx_extractor* ex, Slot& s, const uint8_t* d_image
                              orbx_keypoint* d_kps, uint8_t* d_desc, int capacity, int* d_n, int* d_nm, cudaStream_t st)
 {
     const FrameGeom& fg = ex->fg;
+    const ChunkIO io = one_set_io(d_image, pitch * fg.rows, pitch, d_kps, d_desc, capacity, d_n, d_nm);
     for (int l = 0; l < fg.nlevels; ++l) {
         if (!ex->side[l]) CU(cudaStreamCreateWithFlags(&ex->side[l], cudaStreamNonBlocking));
         if (!ex->ev_lvl[l]) CU(cudaEventCreateWithFlags(&ex->ev_lvl[l], cudaEventDisableTiming));
         if (!ex->ev_side[l]) CU(cudaEventCreateWithFlags(&ex->ev_side[l], cudaEventDisableTiming));
     }
     for (int l = 0; l < fg.nlevels; ++l) {
-        CU(launch_pyramid(fg, s.ws, d_image, pitch * fg.rows, pitch, 1, st, l, l + 1));
+        CU(launch_pyramid(fg, s.ws, io, 1, st, l, l + 1));
         CU(cudaEventRecord(ex->ev_lvl[l], st));
         if (ex->mirror) {           // the level goes home while the later stages run
             const LevelGeom& g = fg.L[l];
@@ -731,8 +771,8 @@ static int run_single_forked(orbx_extractor* ex, Slot& s, const uint8_t* d_image
     CU(launch_blur(fg, s.ws, 1, st));
     for (int l = 0; l < fg.nlevels; ++l) CU(cudaStreamWaitEvent(st, ex->ev_side[l], 0));
     bool fused = false;
-    CU(launch_orient_describe(fg, s.ws, 1, st, lap0, lap1, d_kps, d_desc, capacity, d_n, d_nm, &fused));
-    if (!fused) CU(launch_pack(fg, s.ws, 1, lap0, lap1, d_kps, d_desc, capacity, d_n, d_nm, st));
+    CU(launch_orient_describe(fg, s.ws, 1, st, lap0, lap1, io, &fused));
+    if (!fused) CU(launch_pack(fg, s.ws, 1, lap0, lap1, io, st));
     if (ex->mirror) { CU(cudaEventRecord(ex->ev_mirror, ex->mirror_stream)); CU(cudaStreamWaitEvent(st, ex->ev_mirror, 0)); }
     ex->mirror_valid = ex->mirror;
     return ORBX_OK;
@@ -779,7 +819,7 @@ static int enqueue_single(orbx_extractor* ex, const uint8_t* image, int rows, in
     else CU(cudaMemcpy2DAsync(s.d_in, dpitch, image, step, cols, rows, cudaMemcpyHostToDevice, st));
     auto body = [&](cudaStream_t cs) -> int {
         if (!ex->profiling || ex->mirror) return run_single_forked(ex, s, s.d_in, dpitch, lap0, lap1, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm, cs);
-        return run_chunk(ex, s, s.d_in, dframe, dpitch, 1, lap0, lap1, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm, cs);
+        return run_chunk(ex, s, one_set_io(s.d_in, dframe, dpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), 1, lap0, lap1, cs);
     };
     if (!ex->profiling && !ex->force_eager && ex->single_calls++ > 0) {
         orbx_extractor::GraphKey key;
@@ -1010,9 +1050,9 @@ int orbx_extract_batch_device(orbx_extractor* ex, const uint8_t* d_images, size_
     if (st != s.stream) { CU(cudaEventRecord(s.ev_done, s.stream)); CU(cudaStreamWaitEvent(st, s.ev_done, 0)); }
     for (int f0 = 0; f0 < n_frames; f0 += chunk) {
         const int nf = std::min(chunk, n_frames - f0);
-        rc = run_chunk(ex, s, d_images + (size_t)f0 * frame_stride, frame_stride, pitch, nf, lap0, lap1,
-                       d_keypoints + (size_t)f0 * capacity, d_descriptors + (size_t)f0 * capacity * 32, capacity, d_n_out + f0,
-                       d_n_mono + f0, st);
+        rc = run_chunk(ex, s, one_set_io(d_images + (size_t)f0 * frame_stride, frame_stride, pitch, d_keypoints + (size_t)f0 * capacity,
+                                         d_descriptors + (size_t)f0 * capacity * 32, capacity, d_n_out + f0, d_n_mono + f0),
+                       nf, lap0, lap1, st);
         if (rc) return rc;
         ex->last_frames = nf;
     }
@@ -1036,20 +1076,7 @@ int orbx_extract_batch(orbx_extractor* ex, const uint8_t* const* images, int n_f
     if ((rc = configure(ex, rows, cols))) return rc;
     wait_user_work(ex);
     const int chunk = ex->max_batch > 0 ? std::min(ex->max_batch, n_frames) : std::min(n_frames, 64);
-    // Chunk schedule: the first host->device copy cannot overlap any compute, so the pipeline ramps up with a quarter and a
-    // half chunk before it settles on full chunks (shorter un-overlapped prologue; the tail is whatever remains).
-    std::vector<std::pair<int, int>> sched;          // (first frame, frames); no entry exceeds `chunk`
-    {
-        int f0 = 0;
-        const int ramp[2] = {std::max(chunk / 4, 1), std::max(chunk / 2, 1)};
-        for (int r = 0; r < 2 && n_frames - f0 > 2 * chunk; ++r) { sched.emplace_back(f0, ramp[r]); f0 += ramp[r]; }
-        // ... and ramps down the same way: the compute of a chunk trails its upload, so what is left after the LAST upload
-        // is one chunk of compute + its download — a quarter chunk instead of a full one (trace of a 4096-frame call:
-        // 2.8 ms of tail behind 27.3 ms of back-to-back uploads)
-        const int tail = n_frames - f0 > 3 * chunk ? ramp[0] + ramp[1] : 0;
-        while (f0 < n_frames - tail) { const int nf = std::min(chunk, n_frames - tail - f0); sched.emplace_back(f0, nf); f0 += nf; }
-        if (tail) { sched.emplace_back(f0, ramp[1]); f0 += ramp[1]; sched.emplace_back(f0, ramp[0]); f0 += ramp[0]; }
-    }
+    const std::vector<std::pair<int, int>> sched = chunk_schedule(n_frames, chunk);   // (first frame, frames)
     const int nchunks = (int)sched.size();
     const int nslots = std::min(nchunks, (int)orbx_extractor::kSlots);
     if ((rc = ensure_capacity(ex, chunk, nslots))) return rc;
@@ -1123,7 +1150,7 @@ int orbx_extract_batch(orbx_extractor* ex, const uint8_t* const* images, int n_f
         }
         mark(ist, c, 1);
         if (serial) { CU(cudaEventRecord(s.ev_in, ist)); CU(cudaStreamWaitEvent(cst, s.ev_in, 0)); }
-        if ((rc = run_chunk(ex, s, s.d_in, dframe, dpitch, nf, lap0, lap1, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm, cst))) return rc;
+        if ((rc = run_chunk(ex, s, one_set_io(s.d_in, dframe, dpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), nf, lap0, lap1, cst))) return rc;
         if (serial) { CU(cudaEventRecord(s.ev_done, cst)); CU(cudaStreamWaitEvent(ost, s.ev_done, 0)); }
         mark(ost, c, 2);
         CU(cudaMemcpyAsync(n_out + f0, s.d_n, sizeof(int) * nf, cudaMemcpyDeviceToHost, ost));
@@ -1225,7 +1252,7 @@ int orbx_extract_color(orbx_extractor* ex, const uint8_t* image, int rows, int c
     CU(launch_cvt_gray(s.d_color, cpitch, 0, channels, rgb, 1, rows, cols, s.d_in, gpitch, 0, s.stream));
     // same per-level fork / join as orbx_extract (launched eagerly: the colour staging buffer is not part of the captured graph)
     if ((rc = ensure_mirror(ex, s.stream))) return rc;
-    if (ex->profiling) rc = run_chunk(ex, s, s.d_in, gpitch * rows, gpitch, 1, lap0, lap1, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm, s.stream);
+    if (ex->profiling) rc = run_chunk(ex, s, one_set_io(s.d_in, gpitch * rows, gpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), 1, lap0, lap1, s.stream);
     else rc = run_single_forked(ex, s, s.d_in, gpitch, lap0, lap1, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm, s.stream);
     if (rc) return rc;
     CU(cudaMemcpyAsync(keypoints, s.d_kps, sizeof(orbx_keypoint) * (size_t)capacity, cudaMemcpyDeviceToHost, s.stream));
@@ -1544,7 +1571,7 @@ static int stereo_prepare(orbx_extractor* exL, int frameL, orbx_extractor* exR, 
     // Scale tables: the reference reads Frame::mvScaleFactors / mvInvScaleFactors — the LEFT extractor's — for both sides
     // (src/Frame.cc:112-118, 859, 933); the level sizes and pitches follow from the shape, which is shared.  What is NOT
     // shared is where each extractor put its level slabs (that depends on its own slot capacity).
-    A.pyrL = exL->slots[0].ws.pyr; A.pyrR = exR->slots[0].ws.pyr; A.frameL = frameL; A.frameR = frameR;
+    A.pyrL = exL->slots[0].ws.pyr; A.pyrR = exR->slots[0].ws.pyr; A.frameL = frameL; A.frameR = frameR; A.n_pairs = 1;
     for (int l = 0; l < exR->nlevels; ++l) A.offR[l] = exR->fg.L[l].pyr_off;
     return ORBX_OK;
 }
@@ -1656,6 +1683,188 @@ int orbx_extract_stereo(orbx_extractor* exL, orbx_extractor* exR, const uint8_t*
     CU(cudaStreamSynchronize(sL.stream));
     CU(cudaStreamSynchronize(sR.stream));
     if (*nL > capacity || *nR > capacity) return fail(ORBX_ERR_CAPACITY, "%d / %d keypoints, capacity %d", *nL, *nR, capacity);
+    return ORBX_OK;
+}
+
+// ---- stereo batches -----------------------------------------------------------------------------------------------------
+// A chunk of P pairs is 2P frames of one slot: the pairs' left images, then their right images.  Both images of a pair are
+// extracted in the same chunk and the pair is matched on the chunk's stream from that slot's pyramids, before the slot can be
+// reused.  One handle serves both sides: results depend only on its parameters and the image, and the reference's matcher reads
+// the left extractor's scale tables for both sides (src/Frame.cc:112-118).
+
+static int stereo_batch_args(orbx_extractor* ex, int n_pairs, int rows, int cols, bool images_ok, bool outputs_ok, size_t step,
+                             int capacity)
+{
+    if (!ex) return fail(ORBX_ERR_INVALID_ARG, "extractor is NULL");
+    if (n_pairs < 0) return fail(ORBX_ERR_INVALID_ARG, "n_pairs %d < 0", n_pairs);
+    if (n_pairs == 0) return ORBX_OK;
+    if (!images_ok || rows <= 0 || cols <= 0) return fail(ORBX_ERR_EMPTY_IMAGE, "empty image");
+    if (!outputs_ok || capacity <= 0 || step < (size_t)cols) return fail(ORBX_ERR_INVALID_ARG, "bad output buffers / step");
+    if (capacity >= (1 << 20)) return fail(ORBX_ERR_UNSUPPORTED, "capacity %d: the stereo kernels index at most 2^20 - 1 rows", capacity);
+    return ORBX_OK;
+}
+
+// Matcher arguments of pairs [p, p + np) whose 2 np frames the slot's pyramid holds (left frames 0.., right frames np..)
+static StereoArgs stereo_chunk_args(const orbx_extractor* ex, const Slot& s, int np, const orbx_keypoint* kpL, const uint8_t* descL,
+                                    const int* d_nL, const orbx_keypoint* kpR, const uint8_t* descR, const int* d_nR, int capacity,
+                                    float bf, float maxD, float* uRight, float* depth)
+{
+    StereoArgs A{};
+    A.pyrL = A.pyrR = s.ws.pyr;
+    for (int l = 0; l < ex->nlevels; ++l) A.offR[l] = ex->fg.L[l].pyr_off;
+    A.frameL = 0; A.frameR = np; A.n_pairs = np;
+    A.kpL = kpL; A.descL = descL; A.nL = capacity; A.d_nL = d_nL;
+    A.kpR = kpR; A.descR = descR; A.nR = capacity; A.d_nR = d_nR;
+    A.bf = bf; A.maxD = maxD; A.uRight = uRight; A.depth = depth; A.sad = s.d_sad;
+    return A;
+}
+
+int orbx_extract_stereo_batch(orbx_extractor* ex, const uint8_t* const* imagesL, const uint8_t* const* imagesR, int n_pairs, int rows,
+                              int cols, size_t step, float bf, float maxD, orbx_keypoint* kpL, uint8_t* descL, int* nL,
+                              orbx_keypoint* kpR, uint8_t* descR, int* nR, int capacity, float* uRight, float* depth)
+{
+    bool images_ok = imagesL && imagesR;
+    for (int i = 0; images_ok && i < n_pairs; ++i) images_ok = imagesL[i] && imagesR[i];
+    int rc = stereo_batch_args(ex, n_pairs, rows, cols, images_ok, kpL && descL && nL && kpR && descR && nR && uRight && depth, step,
+                               capacity);
+    if (rc || n_pairs == 0) return rc;
+    if ((rc = set_device(ex->device))) return rc;
+    if ((rc = configure(ex, rows, cols))) return rc;
+    wait_user_work(ex);
+    ex->last_frames = 0;
+    // orbx_extract_batch's chunking and ramp schedule, in whole pairs
+    const int chunk_frames = ex->max_batch > 0 ? std::min(ex->max_batch, 2 * n_pairs) : std::min(2 * n_pairs, 64);
+    const int chunk = std::max(chunk_frames / 2, 1);
+    const std::vector<std::pair<int, int>> sched = chunk_schedule(n_pairs, chunk);   // (first pair, pairs)
+    const int nchunks = (int)sched.size();
+    const int nslots = std::min(nchunks, (int)orbx_extractor::kSlots);
+    if ((rc = ensure_capacity(ex, 2 * chunk, nslots))) return rc;
+    const size_t dpitch = (size_t)cols, dframe = dpitch * rows;
+    for (int i = 0; i < nslots; ++i) {
+        Slot& s = ex->slots[i];
+        if (s.d_in_bytes < dframe * 2 * chunk || s.out_cap < (size_t)2 * chunk * capacity || s.out_frames < 2 * chunk ||
+            !stereo_staging_fits(s, chunk, capacity))
+            CU(cudaStreamSynchronize(s.stream));
+        if ((rc = ensure_host_staging(s, dframe * 2 * chunk, 2 * chunk, capacity))) return rc;
+        if ((rc = ensure_stereo_staging(s, chunk, capacity))) return rc;
+    }
+    // the two pipelines of orbx_extract_batch (there: why), chosen by the chunk's frame count
+    const bool serial = 2 * chunk >= 128;
+    if (serial && !ex->compute) {
+        CU(cudaStreamCreateWithFlags(&ex->compute, cudaStreamNonBlocking));
+        CU(cudaStreamCreateWithFlags(&ex->copy_in, cudaStreamNonBlocking));
+        CU(cudaStreamCreateWithFlags(&ex->copy_out, cudaStreamNonBlocking));
+    }
+    if (serial)
+        for (int i = 0; i < nslots; ++i) CU(cudaStreamSynchronize(ex->slots[i].stream));
+    // trimmed downloads as in orbx_extract_batch: counts first, then the rows the chunk's pairs have
+    auto finish = [&](int c) -> int {
+        Slot& s = ex->slots[c % nslots];
+        const int p0 = sched[c].first, np = sched[c].second;
+        cudaStream_t ost = serial ? ex->copy_out : s.stream;
+        CU(cudaEventSynchronize(s.ev_cnt));
+        int mxL = 0, mxR = 0;
+        for (int p = 0; p < np; ++p) { mxL = std::max(mxL, nL[p0 + p]); mxR = std::max(mxR, nR[p0 + p]); }
+        const size_t kpitch = sizeof(orbx_keypoint) * (size_t)capacity, dpitch32 = (size_t)capacity * 32, fpitch = sizeof(float) * (size_t)capacity;
+        const int rowsL = std::min(mxL, capacity), rowsR = std::min(mxR, capacity);   // a pair over capacity fails the call below
+        if (rowsL > 0) {
+            CU(cudaMemcpy2DAsync(kpL + (size_t)p0 * capacity, kpitch, s.d_kps, kpitch, sizeof(orbx_keypoint) * (size_t)rowsL, np, cudaMemcpyDeviceToHost, ost));
+            CU(cudaMemcpy2DAsync(descL + (size_t)p0 * capacity * 32, dpitch32, s.d_desc, dpitch32, (size_t)rowsL * 32, np, cudaMemcpyDeviceToHost, ost));
+            CU(cudaMemcpy2DAsync(uRight + (size_t)p0 * capacity, fpitch, s.d_su, fpitch, sizeof(float) * (size_t)rowsL, np, cudaMemcpyDeviceToHost, ost));
+            CU(cudaMemcpy2DAsync(depth + (size_t)p0 * capacity, fpitch, s.d_sd, fpitch, sizeof(float) * (size_t)rowsL, np, cudaMemcpyDeviceToHost, ost));
+        }
+        if (rowsR > 0) {
+            CU(cudaMemcpy2DAsync(kpR + (size_t)p0 * capacity, kpitch, s.d_kps + (size_t)np * capacity, kpitch, sizeof(orbx_keypoint) * (size_t)rowsR, np,
+                                 cudaMemcpyDeviceToHost, ost));
+            CU(cudaMemcpy2DAsync(descR + (size_t)p0 * capacity * 32, dpitch32, s.d_desc + (size_t)np * capacity * 32, dpitch32, (size_t)rowsR * 32, np,
+                                 cudaMemcpyDeviceToHost, ost));
+        }
+        if (serial) CU(cudaEventRecord(s.ev_out, ost));
+        return ORBX_OK;
+    };
+    auto upload = [&](const uint8_t* const* images, int p0, int np, uint8_t* dst, cudaStream_t ist) -> int {
+        bool contiguous = step == (size_t)cols;
+        for (int p = 1; p < np && contiguous; ++p) contiguous = images[p0 + p] == images[p0 + p - 1] + dframe;
+        if (contiguous) {
+            CU(cudaMemcpyAsync(dst, images[p0], dframe * np, cudaMemcpyHostToDevice, ist));
+        } else {
+            for (int p = 0; p < np; ++p)
+                CU(cudaMemcpy2DAsync(dst + (size_t)p * dframe, dpitch, images[p0 + p], step, cols, rows, cudaMemcpyHostToDevice, ist));
+        }
+        return ORBX_OK;
+    };
+    const int lag = 2;
+    for (int c = 0; c < nchunks; ++c) {
+        Slot& s = ex->slots[c % nslots];
+        const int p0 = sched[c].first, np = sched[c].second;
+        cudaStream_t cst = serial ? ex->compute : s.stream;
+        cudaStream_t ist = serial ? ex->copy_in : s.stream, ost = serial ? ex->copy_out : s.stream;
+        if (serial && c >= nslots) { CU(cudaStreamWaitEvent(ist, s.ev_done, 0)); CU(cudaStreamWaitEvent(cst, s.ev_out, 0)); }
+        if ((rc = upload(imagesL, p0, np, s.d_in, ist)) || (rc = upload(imagesR, p0, np, s.d_in + (size_t)np * dframe, ist))) return rc;
+        if (serial) { CU(cudaEventRecord(s.ev_in, ist)); CU(cudaStreamWaitEvent(cst, s.ev_in, 0)); }
+        // the staging holds both sides back to back: one set of 2 np frames (vLappingArea = {0, 0}, src/Frame.cc:124-125)
+        if ((rc = run_chunk(ex, s, one_set_io(s.d_in, dframe, dpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), 2 * np, 0, 0, cst))) return rc;
+        const size_t r = (size_t)np * capacity;
+        const StereoArgs A = stereo_chunk_args(ex, s, np, s.d_kps, s.d_desc, s.d_n, s.d_kps + r, s.d_desc + r * 32, s.d_n + np, capacity, bf, maxD,
+                                               s.d_su, s.d_sd);
+        CU(launch_stereo(ex->fg, A, cst));
+        if (serial) { CU(cudaEventRecord(s.ev_done, cst)); CU(cudaStreamWaitEvent(ost, s.ev_done, 0)); }
+        CU(cudaMemcpyAsync(nL + p0, s.d_n, sizeof(int) * np, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpyAsync(nR + p0, s.d_n + np, sizeof(int) * np, cudaMemcpyDeviceToHost, ost));
+        CU(cudaEventRecord(s.ev_cnt, ost));
+        if (c >= lag && (rc = finish(c - lag))) return rc;
+    }
+    for (int c = std::max(nchunks - lag, 0); c < nchunks; ++c)
+        if ((rc = finish(c))) return rc;
+    if (serial) { CU(cudaStreamSynchronize(ex->copy_out)); CU(cudaStreamSynchronize(ex->compute)); CU(cudaStreamSynchronize(ex->copy_in)); }
+    for (int i = 0; i < nslots; ++i) CU(cudaStreamSynchronize(ex->slots[i].stream));
+    for (int p = 0; p < n_pairs; ++p)
+        if (nL[p] > capacity || nR[p] > capacity)
+            return fail(ORBX_ERR_CAPACITY, "pair %d has %d / %d keypoints, capacity %d", p, nL[p], nR[p], capacity);
+    return ORBX_OK;
+}
+
+int orbx_extract_stereo_batch_device(orbx_extractor* ex, const uint8_t* d_imagesL, const uint8_t* d_imagesR, size_t frame_stride,
+                                     int n_pairs, int rows, int cols, size_t pitch, float bf, float maxD, orbx_keypoint* d_kpL,
+                                     uint8_t* d_descL, int* d_nL, orbx_keypoint* d_kpR, uint8_t* d_descR, int* d_nR, int capacity,
+                                     float* d_uRight, float* d_depth, void* stream)
+{
+    int rc = stereo_batch_args(ex, n_pairs, rows, cols, d_imagesL && d_imagesR,
+                               d_kpL && d_descL && d_nL && d_kpR && d_descR && d_nR && d_uRight && d_depth, pitch, capacity);
+    if (rc || n_pairs == 0) return rc;
+    if ((rc = set_device(ex->device))) return rc;
+    if ((rc = configure(ex, rows, cols))) return rc;
+    ex->last_frames = 0;
+    const int chunk_frames = ex->max_batch > 0 ? std::min(ex->max_batch, 2 * n_pairs) : std::min(2 * n_pairs, 256);
+    const int chunk = std::max(chunk_frames / 2, 1);
+    if ((rc = ensure_capacity(ex, 2 * chunk, 1))) return rc;
+    Slot& s = ex->slots[0];
+    if (!stereo_staging_fits(s, chunk, capacity)) {          // replaced below: earlier work on any stream must be done with it
+        wait_user_work(ex);
+        CU(cudaStreamSynchronize(s.stream));
+        if ((rc = ensure_stereo_staging(s, chunk, capacity))) return rc;
+    }
+    cudaStream_t st = stream ? (cudaStream_t)stream : s.stream;
+    if (!ex->ev_user) CU(cudaEventCreateWithFlags(&ex->ev_user, cudaEventDisableTiming));
+    if (ex->user_pending) CU(cudaStreamWaitEvent(st, ex->ev_user, 0));
+    if (st != s.stream) { CU(cudaEventRecord(s.ev_done, s.stream)); CU(cudaStreamWaitEvent(st, s.ev_done, 0)); }
+    for (int p0 = 0; p0 < n_pairs; p0 += chunk) {
+        const int np = std::min(chunk, n_pairs - p0);
+        const size_t r = (size_t)p0 * capacity;
+        // level 0 reads the left images from one base and the right images from the other; the results go straight to the
+        // caller's slabs
+        ChunkIO io{};
+        io.img0 = d_imagesL + (size_t)p0 * frame_stride; io.img1 = d_imagesR + (size_t)p0 * frame_stride;
+        io.frame_stride = frame_stride; io.pitch = pitch;
+        io.kps0 = d_kpL + r; io.kps1 = d_kpR + r; io.desc0 = d_descL + r * 32; io.desc1 = d_descR + r * 32;
+        io.n_out0 = d_nL + p0; io.n_out1 = d_nR + p0; io.n_mono0 = s.d_snm; io.n_mono1 = s.d_snm + np;
+        io.capacity = capacity; io.split = np;
+        if ((rc = run_chunk(ex, s, io, 2 * np, 0, 0, st))) return rc;
+        const StereoArgs A = stereo_chunk_args(ex, s, np, d_kpL + r, d_descL + r * 32, d_nL + p0, d_kpR + r, d_descR + r * 32, d_nR + p0,
+                                               capacity, bf, maxD, d_uRight + r, d_depth + r);
+        CU(launch_stereo(ex->fg, A, st));
+    }
+    if (st != s.stream) { CU(cudaEventRecord(ex->ev_user, st)); ex->user_pending = true; }
     return ORBX_OK;
 }
 

@@ -330,7 +330,7 @@ __global__ void __launch_bounds__(32 * kBpWarps) blur_pipe_kernel(const __grid_c
 // monocular, src/Frame.cc:313) -> row nkp - 1 - t.  Anything else (a fisheye lapping area) takes pack_kernel.
 struct FusedPack {
     int mode;                 // 0 = separate pack kernel, 1 = nothing lapping, 2 = everything lapping
-    orbx_keypoint* kps; uint8_t* desc; int capacity; int* n_out; int* n_mono;
+    ChunkIO io;
 };
 
 // grid = (ceil(kp_slots / 8), n_frames), 8 warps per CTA, one warp per keypoint slot.
@@ -369,8 +369,8 @@ __global__ void __launch_bounds__(256, STAGED ? ORBX_OD_MINB : 1) orient_describ
         t_out = __shfl_sync(0xffffffffu, incl - c, level) + i;
         nkp = __shfl_sync(0xffffffffu, incl, 31);
         if (slot == 0 && lane == 0) {                       // the frame's counters (src 1306: the return value is monoIndex)
-            fp.n_out[frame] = nkp;
-            fp.n_mono[frame] = nkp > fp.capacity ? -1 : (fp.mode == 1 ? nkp : 0);
+            *fp.io.n_out(frame) = nkp;
+            *fp.io.n_mono(frame) = nkp > fp.io.capacity ? -1 : (fp.mode == 1 ? nkp : 0);
         }
     } else {
         n_level = ws.lvl_n[(size_t)frame * fg.nlevels + level];
@@ -484,9 +484,9 @@ __global__ void __launch_bounds__(256, STAGED ? ORBX_OD_MINB : 1) orient_describ
     }
     ws.lvl_desc[((size_t)frame * fg.kp_slots + slot) * 32 + lane] = (uint8_t)val;
     if (lane == 0) ws.lvl_angle[(size_t)frame * fg.kp_slots + slot] = angle;
-    if (fp.mode && nkp <= fp.capacity) {
+    if (fp.mode && nkp <= fp.io.capacity) {
         const int dst = fp.mode == 1 ? t_out : nkp - 1 - t_out;
-        fp.desc[((size_t)frame * fp.capacity + dst) * 32 + lane] = (uint8_t)val;
+        fp.io.desc(frame)[(size_t)dst * 32 + lane] = (uint8_t)val;
         if (lane < 7) {                                     // the 28-byte keypoint, one 32-bit field per lane
             float px = (float)x, py = (float)y;
             if (level != 0) { px = __fmul_rn(px, g.scale); py = __fmul_rn(py, g.scale); }       // src 1289-1291
@@ -500,7 +500,7 @@ __global__ void __launch_bounds__(256, STAGED ? ORBX_OD_MINB : 1) orient_describ
                 case 5: w = (uint32_t)level; break;
                 default: w = 0xffffffffu; break;            // class_id = -1
             }
-            reinterpret_cast<uint32_t*>(fp.kps + (size_t)frame * fp.capacity + dst)[lane] = w;
+            reinterpret_cast<uint32_t*>(fp.io.kps(frame) + dst)[lane] = w;
         }
     }
 }
@@ -509,9 +509,7 @@ __global__ void __launch_bounds__(256, STAGED ? ORBX_OD_MINB : 1) orient_describ
 // flight), 1024 for a few frames: the whole frame is then one pass with two barriers — the kernel sits on the critical path
 // of the single-frame call.
 template <int T>
-__global__ void __launch_bounds__(T) pack_kernel(const __grid_constant__ FrameGeom fg, Workspace ws, int lap0, int lap1,
-                                                 orbx_keypoint* __restrict__ kps, uint8_t* __restrict__ desc, int capacity,
-                                                 int* __restrict__ n_out, int* __restrict__ n_mono)
+__global__ void __launch_bounds__(T) pack_kernel(const __grid_constant__ FrameGeom fg, Workspace ws, int lap0, int lap1, const ChunkIO io)
 {
     __shared__ int lvl_off[kMaxLevels + 1];
     __shared__ int warp_cnt[T / 32];
@@ -533,12 +531,15 @@ __global__ void __launch_bounds__(T) pack_kernel(const __grid_constant__ FrameGe
     }
     __syncthreads();
     const int nkp = lvl_off[fg.nlevels];
+    const int capacity = io.capacity;
+    int* n_out = io.n_out(frame);
+    int* n_mono = io.n_mono(frame);
     if (nkp > capacity) {
-        if (tid == 0) { n_out[frame] = nkp; n_mono[frame] = -1; }
+        if (tid == 0) { *n_out = nkp; *n_mono = -1; }
         return;
     }
-    orbx_keypoint* okp = kps + (size_t)frame * capacity;
-    uint8_t* odesc = desc + (size_t)frame * capacity * 32;
+    orbx_keypoint* okp = io.kps(frame);
+    uint8_t* odesc = io.desc(frame);
     const float flap0 = (float)lap0, flap1 = (float)lap1;
     for (int base = 0; base < nkp; base += T) {
         const int t = base + tid;
@@ -577,7 +578,7 @@ __global__ void __launch_bounds__(T) pack_kernel(const __grid_constant__ FrameGe
         if (tid == 0) { int c = carry; for (int w = 0; w < T / 32; ++w) c += warp_cnt[w]; carry = c; }
         __syncthreads();
     }
-    if (tid == 0) { n_out[frame] = nkp; n_mono[frame] = nkp - carry; }
+    if (tid == 0) { *n_out = nkp; *n_mono = nkp - carry; }
 }
 
 cudaError_t launch_blur(const FrameGeom& fg, const Workspace& ws, int n_frames, cudaStream_t st)
@@ -650,19 +651,19 @@ static cudaError_t fill_describe_tables()
     return cudaMemcpyToSymbol(d_mom_mask, mask, sizeof mask);
 }
 
-// With d_kps != nullptr the packing is fused when the lapping area allows it; *fused tells the caller whether pack_kernel is
-// still needed.
+// The packing into io's slabs is fused when the lapping area allows it; *fused tells the caller whether pack_kernel is still
+// needed.
 cudaError_t launch_orient_describe(const FrameGeom& fg, const Workspace& ws, int n_frames, cudaStream_t st, int lap0, int lap1,
-                                   orbx_keypoint* d_kps, uint8_t* d_desc, int capacity, int* d_n_out, int* d_n_mono, bool* fused)
+                                   const ChunkIO& io, bool* fused)
 {
     FusedPack fp{};
     // a few frames only: the fused stores are scattered (7 lanes x 4 bytes per keypoint), which costs a 512-frame batch more than
     // the separate pack pass (measured 0.607 vs 0.557 + 0.024 ms), while a single frame saves a whole launch on its critical path
-    if (d_kps && d_desc && d_n_out && d_n_mono && fg.kp_slots > 0 && n_frames < 8) {
+    if (fg.kp_slots > 0 && n_frames < 8) {
         // output x = level x * scale lies in [19, cols): the lapping test px >= lap0 && px <= lap1 is decided by the bounds
         if (lap1 < kEdge || lap0 >= fg.cols || lap0 > lap1) fp.mode = 1;
         else if (lap0 <= kEdge && lap1 >= fg.cols) fp.mode = 2;
-        fp.kps = d_kps; fp.desc = d_desc; fp.capacity = capacity; fp.n_out = d_n_out; fp.n_mono = d_n_mono;
+        fp.io = io;
     }
     if (fused) *fused = fp.mode != 0;
     static bool filled[64] = {false};      // per device (the tables are __device__ symbols, one copy per context)
@@ -682,11 +683,10 @@ cudaError_t launch_orient_describe(const FrameGeom& fg, const Workspace& ws, int
     return cudaGetLastError();
 }
 
-cudaError_t launch_pack(const FrameGeom& fg, const Workspace& ws, int n_frames, int lap0, int lap1, orbx_keypoint* d_kps,
-                        uint8_t* d_desc, int capacity, int* d_n_out, int* d_n_mono, cudaStream_t st)
+cudaError_t launch_pack(const FrameGeom& fg, const Workspace& ws, int n_frames, int lap0, int lap1, const ChunkIO& io, cudaStream_t st)
 {
-    if (n_frames >= 8) pack_kernel<256><<<n_frames, 256, 0, st>>>(fg, ws, lap0, lap1, d_kps, d_desc, capacity, d_n_out, d_n_mono);
-    else pack_kernel<1024><<<n_frames, 1024, 0, st>>>(fg, ws, lap0, lap1, d_kps, d_desc, capacity, d_n_out, d_n_mono);
+    if (n_frames >= 8) pack_kernel<256><<<n_frames, 256, 0, st>>>(fg, ws, lap0, lap1, io);
+    else pack_kernel<1024><<<n_frames, 1024, 0, st>>>(fg, ws, lap0, lap1, io);
     count_launch();
     return cudaGetLastError();
 }

@@ -36,9 +36,7 @@ __device__ __forceinline__ int reflect101_dev(int i, int n)
 }
 
 // Level 0: copy + border.  grid = (ceil(words/128), rows_alloc, frames)
-__global__ void __launch_bounds__(128) pyr_level0_kernel(const __grid_constant__ FrameGeom fg, Workspace ws,
-                                                         const uint8_t* __restrict__ images, size_t frame_stride,
-                                                         size_t in_pitch)
+__global__ void __launch_bounds__(128) pyr_level0_kernel(const __grid_constant__ FrameGeom fg, Workspace ws, const ChunkIO io)
 {
     const LevelGeom& g = fg.L[0];
     const int word = blockIdx.x * blockDim.x + threadIdx.x;
@@ -46,7 +44,7 @@ __global__ void __launch_bounds__(128) pyr_level0_kernel(const __grid_constant__
     const int frame = blockIdx.z;
     if (word * 4 >= g.pitch) return;
     const int sy = reflect101_dev(brow - kEdge, g.h);
-    const uint8_t* src = images + (size_t)frame * frame_stride + (size_t)sy * in_pitch;
+    const uint8_t* src = io.image(frame) + (size_t)sy * io.pitch;
     uint32_t out = 0;
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
@@ -159,12 +157,10 @@ constexpr int L0_H = 32;                     // level-0 copy tile height
 // `aligned`: image base, frame stride and pitch are multiples of 16 (16-byte loads).  Otherwise (e.g. 1241-pixel KITTI rows at
 // pitch = cols) a 16-byte segment is read as its 4 - 5 covering aligned words and realigned with funnel shifts; the misalignment
 // differs from row to row.  `img_end` = one past the last image byte: the fifth word is only read when it lies inside the images.
-__device__ __forceinline__ void level0_tile(const LevelGeom& g, const Workspace& ws, const uint8_t* __restrict__ images, size_t frame_stride,
-                                            size_t in_pitch, uint8_t* t, int tid, int x0, int y0, int frame, bool aligned,
-                                            const uint8_t* img_end)
+__device__ __forceinline__ void level0_tile(const LevelGeom& g, const Workspace& ws, const uint8_t* __restrict__ S, size_t in_pitch,
+                                            uint8_t* t, int tid, int x0, int y0, int frame, bool aligned, const uint8_t* img_end)
 {
     const int tw = min(PT_W, g.w - x0), th = min(L0_H, g.h - y0);
-    const uint8_t* S = images + (size_t)frame * frame_stride;
     uint8_t* D = level_interior(ws.pyr, g, frame);
     if (tid < L0_H * (PT_W / 16)) {
         const int ty = tid >> 3, v = tid & 7;
@@ -200,12 +196,14 @@ __device__ __forceinline__ void level0_tile(const LevelGeom& g, const Workspace&
     write_border_mirrors<PT_W>(D, g.pitch, g.w, g.h, x0, y0, tw, th, t, tid, PT_THREADS);
 }
 
-__global__ void __launch_bounds__(PT_THREADS) pyr_level0_tiled_kernel(const __grid_constant__ FrameGeom fg, Workspace ws,
-                                                                     const uint8_t* __restrict__ images, size_t frame_stride, size_t in_pitch,
-                                                                     int aligned, const uint8_t* img_end)
+// img_end[k]: one past the last image byte of set k
+__global__ void __launch_bounds__(PT_THREADS) pyr_level0_tiled_kernel(const __grid_constant__ FrameGeom fg, Workspace ws, const ChunkIO io,
+                                                                     int aligned, const uint8_t* img_end0, const uint8_t* img_end1)
 {
     __shared__ __align__(16) uint8_t t[L0_H * PT_W];
-    level0_tile(fg.L[0], ws, images, frame_stride, in_pitch, t, threadIdx.x, blockIdx.x * PT_W, blockIdx.y * L0_H, blockIdx.z, aligned != 0, img_end);
+    const int frame = blockIdx.z;
+    level0_tile(fg.L[0], ws, io.image(frame), io.pitch, t, threadIdx.x, blockIdx.x * PT_W, blockIdx.y * L0_H, frame, aligned != 0,
+                frame >= io.split ? img_end1 : img_end0);
 }
 
 // The two fixed-point passes, the interior stores and the border mirrors of one 128 x PT_H tile whose source window is already
@@ -490,8 +488,8 @@ static bool launch_resize_pipe(const FrameGeom& fg, const Workspace& ws, int lev
 }
 
 // Levels [level_lo, level_hi) (level_hi <= 0: all); level l >= 1 reads level l - 1, which must be complete on `st`.
-cudaError_t launch_pyramid(const FrameGeom& fg, const Workspace& ws, const uint8_t* d_images, size_t frame_stride,
-                           size_t pitch, int n_frames, cudaStream_t st, int level_lo, int level_hi)
+cudaError_t launch_pyramid(const FrameGeom& fg, const Workspace& ws, const ChunkIO& io, int n_frames, cudaStream_t st, int level_lo,
+                           int level_hi)
 {
     if (level_hi <= 0) level_hi = fg.nlevels;
     // One launch per level.  A cooperative kernel for the whole pyramid was measured slower on 512-frame batches (1.19 ms vs
@@ -504,12 +502,16 @@ cudaError_t launch_pyramid(const FrameGeom& fg, const Workspace& ws, const uint8
         dim3 grid((words + 127) / 128, g.rows_alloc, n_frames);
         const bool big = g.w >= 2 * kEdge + 2 && g.h >= 2 * kEdge + 2;      // border band narrower than the level
         if (l == 0) {
-            const bool aligned = ((uintptr_t)d_images & 15) == 0 && (frame_stride & 15) == 0 && (pitch & 15) == 0;
+            const int n0 = std::min(io.split, n_frames), n1 = n_frames - n0;
+            const bool aligned = (((uintptr_t)io.img0 | (n1 > 0 ? (uintptr_t)io.img1 : 0)) & 15) == 0 && (io.frame_stride & 15) == 0 &&
+                                 (io.pitch & 15) == 0;
             dim3 tgrid((g.w + PT_W - 1) / PT_W, (g.h + L0_H - 1) / L0_H, n_frames);
-            // one past the last byte the caller's images hold (the last row of the last frame ends at its last pixel)
-            const uint8_t* img_end = d_images + (size_t)(n_frames - 1) * frame_stride + (size_t)(g.h - 1) * pitch + g.w;
-            if (big) pyr_level0_tiled_kernel<<<tgrid, PT_THREADS, 0, st>>>(fg, ws, d_images, frame_stride, pitch, aligned ? 1 : 0, img_end);
-            else pyr_level0_kernel<<<grid, 128, 0, st>>>(fg, ws, d_images, frame_stride, pitch);
+            // one past the last byte the caller's images of each set hold (the last row of the last frame ends at its last pixel)
+            auto img_end = [&](const uint8_t* img, int n) {
+                return n > 0 ? img + (size_t)(n - 1) * io.frame_stride + (size_t)(g.h - 1) * io.pitch + g.w : nullptr;
+            };
+            if (big) pyr_level0_tiled_kernel<<<tgrid, PT_THREADS, 0, st>>>(fg, ws, io, aligned ? 1 : 0, img_end(io.img0, n0), img_end(io.img1, n1));
+            else pyr_level0_kernel<<<grid, 128, 0, st>>>(fg, ws, io);
         } else {
             const LevelGeom& p = fg.L[l - 1];
             // source footprint of a tile must fit the staged window: scale <= 1.5 -> 128x32 tiles, <= 2 -> 128x16 tiles

@@ -127,22 +127,49 @@ __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* m
 }
 #endif
 
+// Where the frames of a chunk read their image and write their results.  The frames form one or two sets: frames [0, split)
+// are set 0, frames [split, n) set 1, and frame f is element f - (set ? split : 0) of its set.  A mono batch is one set
+// (split >= n); a stereo chunk of P pairs has split = P: the pairs' left images, then their right images, each side read
+// from and written to the caller's own arrays.
+// (Named fields and selects, not [2] arrays: a dynamically indexed kernel parameter is copied to the stack.)
+struct ChunkIO {
+    const uint8_t* img0; const uint8_t* img1;  // frame i of a set: img + i * frame_stride, `pitch` bytes per row
+    size_t frame_stride, pitch;
+    orbx_keypoint* kps0; orbx_keypoint* kps1;  // [capacity] rows per frame
+    uint8_t* desc0; uint8_t* desc1;            // [capacity][32] per frame
+    int* n_out0; int* n_out1; int* n_mono0; int* n_mono1;   // one count per frame
+    int capacity;
+    int split;
+    __host__ __device__ size_t index(int f) const { return (size_t)(f >= split ? f - split : f); }
+    __host__ __device__ const uint8_t* image(int f) const { return (f >= split ? img1 : img0) + index(f) * frame_stride; }
+    __host__ __device__ orbx_keypoint* kps(int f) const { return (f >= split ? kps1 : kps0) + index(f) * capacity; }
+    __host__ __device__ uint8_t* desc(int f) const { return (f >= split ? desc1 : desc0) + index(f) * capacity * 32; }
+    __host__ __device__ int* n_out(int f) const { return (f >= split ? n_out1 : n_out0) + index(f); }
+    __host__ __device__ int* n_mono(int f) const { return (f >= split ? n_mono1 : n_mono0) + index(f); }
+};
+inline ChunkIO one_set_io(const uint8_t* images, size_t frame_stride, size_t pitch, orbx_keypoint* kps, uint8_t* desc, int capacity,
+                          int* n_out, int* n_mono)
+{
+    ChunkIO io{};
+    io.img0 = io.img1 = images; io.frame_stride = frame_stride; io.pitch = pitch;
+    io.kps0 = io.kps1 = kps; io.desc0 = io.desc1 = desc; io.n_out0 = io.n_out1 = n_out; io.n_mono0 = io.n_mono1 = n_mono;
+    io.capacity = capacity; io.split = 1 << 30;
+    return io;
+}
+
 // ---- launchers (defined in the kernel translation units) ---------------------------------------------------
 void count_launch(int n = 1);
 
-cudaError_t launch_pyramid(const FrameGeom& fg, const Workspace& ws, const uint8_t* d_images, size_t frame_stride,
-                           size_t pitch, int n_frames, cudaStream_t st, int level_lo = 0, int level_hi = 0);
+cudaError_t launch_pyramid(const FrameGeom& fg, const Workspace& ws, const ChunkIO& io, int n_frames, cudaStream_t st, int level_lo = 0,
+                           int level_hi = 0);
 cudaError_t launch_cvt_gray(const uint8_t* d_src, size_t src_pitch, size_t src_frame_stride, int channels, int rgb, int n_frames,
                             int rows, int cols, uint8_t* d_dst, size_t dst_pitch, size_t dst_frame_stride, cudaStream_t st);
 cudaError_t launch_fast(const FrameGeom& fg, const Workspace& ws, int n_frames, cudaStream_t st, int level_lo = 0, int level_hi = 0);
 cudaError_t launch_blur(const FrameGeom& fg, const Workspace& ws, int n_frames, cudaStream_t st);
 cudaError_t launch_octree(const FrameGeom& fg, const Workspace& ws, int n_frames, cudaStream_t st, int level_lo = 0, int level_hi = 0);
-cudaError_t launch_orient_describe(const FrameGeom& fg, const Workspace& ws, int n_frames, cudaStream_t st, int lap0 = 0, int lap1 = 0,
-                                   orbx_keypoint* d_kps = nullptr, uint8_t* d_desc = nullptr, int capacity = 0, int* d_n_out = nullptr,
-                                   int* d_n_mono = nullptr, bool* fused = nullptr);
-cudaError_t launch_pack(const FrameGeom& fg, const Workspace& ws, int n_frames, int lap0, int lap1,
-                        orbx_keypoint* d_kps, uint8_t* d_desc, int capacity, int* d_n_out, int* d_n_mono,
-                        cudaStream_t st);
+cudaError_t launch_orient_describe(const FrameGeom& fg, const Workspace& ws, int n_frames, cudaStream_t st, int lap0, int lap1,
+                                   const ChunkIO& io, bool* fused);
+cudaError_t launch_pack(const FrameGeom& fg, const Workspace& ws, int n_frames, int lap0, int lap1, const ChunkIO& io, cudaStream_t st);
 size_t octree_smem_for(const FrameGeom& fg, int level_lo, int level_hi);   // dynamic shared memory of octree_kernel for these levels
 int octree_take_error_flag();   // depth-overflow flag of the current device (duplicate pixels); reading clears it; synchronises
 cudaError_t octree_prepare();   // opt in to large dynamic shared memory
@@ -154,16 +181,20 @@ cudaError_t launch_knn2_merge(const int32_t* d_idx_sh, const int32_t* d_dist_sh,
                               int32_t* d_dist, cudaStream_t st, size_t shard_stride = 0);   // stride in int32 elements, 0 = 2 * nq
 cudaError_t launch_popc_bench(unsigned long long* d_sink, int iters, int blocks, cudaStream_t st);
 
+// Frame::ComputeStereoMatches over n_pairs pairs (blockIdx.y of the match kernel, blockIdx.x of the median kernel).  Pair p
+// reads pyramid frames frameL + p / frameR + p, keypoints / descriptors at row p * nL (left) and p * nR (right), counts
+// d_nL[p] / d_nR[p], and writes rows p * nL of uRight / depth / sad.
 struct StereoArgs {
     const uint8_t* pyrL; const uint8_t* pyrR;       // pyramid allocations: same level sizes and pitches, but each extractor lays its
     unsigned long long offR[kMaxLevels];            // level slabs out for its own slot capacity -> the right pyramid's level offsets
     int frameL, frameR;
+    int n_pairs;
     const orbx_keypoint* kpL; const uint8_t* descL; int nL;      // nL / nR: counts, or (with d_nL / d_nR) the capacity bound
     const orbx_keypoint* kpR; const uint8_t* descR; int nR;
     const int* d_nL; const int* d_nR;               // optional device-resident counts (results of an extraction still in flight)
     float bf, maxD;
-    float* uRight; float* depth;                    // [nL]
-    int* sad;                                       // [nL] scratch: SAD of accepted matches, -1 otherwise
+    float* uRight; float* depth;                    // [n_pairs][nL]
+    int* sad;                                       // [n_pairs][nL] scratch: SAD of accepted matches, -1 otherwise
 };
 cudaError_t launch_stereo(const FrameGeom& fg, const StereoArgs& a, cudaStream_t st);
 

@@ -135,6 +135,34 @@ class ORBextractor:
                                               ptr(stream) if stream else None))
         self._shape = (rows, cols)
 
+    def extract_stereo_batch(self, left, right, bf, maxD):
+        """The stereo Frame constructor (src/Frame.cc:124-143) over N rectified pairs on this one handle: left / right are [N,H,W]
+        uint8 numpy arrays (host, ideally page-locked).  Returns (nL[N], nR[N], kpL[N,cap], descL[N,cap,32], kpR[N,cap],
+        descR[N,cap,32], uRight[N,cap], depth[N,cap]); rows of pair i past nL[i] / nR[i] are undefined."""
+        assert left.dtype == np.uint8 and right.dtype == np.uint8 and left.ndim == 3 and left.shape == right.shape
+        assert left.strides == right.strides and left.strides[2] == 1
+        N, rows, cols = left.shape
+        cap = self.max_keypoints(rows, cols)
+        kL = np.zeros((N, cap), KP_DTYPE); kR = np.zeros((N, cap), KP_DTYPE)
+        dL = np.zeros((N, cap, 32), np.uint8); dR = np.zeros((N, cap, 32), np.uint8)
+        u = np.full((N, cap), -1.0, np.float32); d = np.full((N, cap), -1.0, np.float32)
+        nL = np.zeros(N, np.int32); nR = np.zeros(N, np.int32)
+        pl = (C.c_void_p * max(N, 1))(*[left.ctypes.data + i * left.strides[0] for i in range(N)])
+        pr = (C.c_void_p * max(N, 1))(*[right.ctypes.data + i * right.strides[0] for i in range(N)])
+        check(lib().orbx_extract_stereo_batch(self._h, pl, pr, N, rows, cols, left.strides[1], float(bf), float(maxD), ptr(kL), ptr(dL),
+                                              ptr(nL), ptr(kR), ptr(dR), ptr(nR), cap, ptr(u), ptr(d)))
+        self._shape = (rows, cols)
+        return nL, nR, kL, dL, kR, dR, u, d
+
+    def extract_stereo_batch_device(self, d_left, d_right, n_pairs, rows, cols, pitch, frame_stride, bf, maxD, d_kpL, d_descL, d_nL,
+                                    d_kpR, d_descR, d_nR, capacity, d_uRight, d_depth, stream=None):
+        """Device-resident stereo batch: every argument named d_* is a device pointer (int) or a torch CUDA tensor; the outputs are
+        [n_pairs][capacity] slabs (counts [n_pairs])."""
+        check(lib().orbx_extract_stereo_batch_device(self._h, ptr(d_left), ptr(d_right), frame_stride, n_pairs, rows, cols, pitch,
+                                                     float(bf), float(maxD), ptr(d_kpL), ptr(d_descL), ptr(d_nL), ptr(d_kpR), ptr(d_descR),
+                                                     ptr(d_nR), capacity, ptr(d_uRight), ptr(d_depth), ptr(stream) if stream else None))
+        self._shape = (rows, cols)
+
     def sync(self):
         check(lib().orbx_sync(self._h))
 
