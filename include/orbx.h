@@ -365,6 +365,37 @@ int orbx_search_for_triangulation(int device, const orbx_keypoint* kp_a, const u
                                   const float* sigma2_b, int n_levels, int only_stereo, int coarse, int check_orientation,
                                   int32_t* match_a, int* n_matches);
 
+/* One neighbour (pKF2) of orbx_search_for_triangulation_batch: the KF2 arguments of orbx_search_for_triangulation, plus the
+ * neighbour's own bCoarse (HOST pointers). */
+typedef struct orbx_triangulation_view {
+    int n;                          /* KF2's N */
+    const orbx_keypoint* kp;        /* mvKeysUn */
+    const uint8_t* desc;            /* mDescriptors, n x 32 */
+    const uint8_t* free;            /* [n] != 0 <=> no map point yet */
+    const uint8_t* stereo;          /* [n] != 0 <=> mvuRight[j] >= 0 */
+    orbx_feature_vector fv;         /* mFeatVec */
+    float F12[9];                   /* row-major K1^-T [t12]x R12 K2^-1 (Pinhole.cpp:109-112) */
+    float ep[2];                    /* KF1's camera centre projected into KF2 */
+    const float* scale;             /* mvScaleFactors, n_levels entries */
+    const float* sigma2;            /* mvLevelSigma2, n_levels entries */
+    int n_levels;
+    int coarse;                     /* bCoarse */
+} orbx_triangulation_view;
+/* orbx_search_for_triangulation of KF1 against n_kf neighbours in one call (the neighbour loop of
+ * LocalMapping::CreateNewMapPoints, src/LocalMapping.cc): KF1 is uploaded once, the neighbours in one packed copy, the
+ * jobs are built on the GPU and one launch scans them all.  For every neighbour k the result is bit-identical to
+ * orbx_search_for_triangulation(KF1, kfs[k], ..., only_stereo, kfs[k].coarse, check_orientation):
+ *   match[k * n_a + i] = index in kfs[k] or -1 (after the rotation filter when check_orientation), n_matches[k] = its return value.
+ * The neighbours are searched against the same free_a: the caller that adds map points to KF1 between neighbours drops the
+ * later neighbours' matches of those features itself (the C++ adapter does; DESIGN.md §5d).  n_kf == 0 does nothing.
+ * ORBX_ERR_INVALID_ARG per neighbour as the single call: null arrays, a malformed feature vector, n_levels outside
+ * [1, ORBX_MAX_LEVELS], an octave outside [0, n_levels).  Uses local mapping's device scratch (that of orbx_fuse), so it never
+ * waits on the tracking thread's searches. */
+int orbx_search_for_triangulation_batch(int device, const orbx_keypoint* kp_a, const uint8_t* desc_a, const uint8_t* free_a,
+                                        const uint8_t* stereo_a, int n_a, const orbx_feature_vector* fv_a, int n_kf,
+                                        const orbx_triangulation_view* kfs, int only_stereo, int check_orientation,
+                                        int32_t* match, int* n_matches);
+
 /* ---- the frame grid and the projection-guided searches (SURVEY.md §8(f)2) ---------------------------------- */
 
 #define ORBX_FRAME_GRID_ROWS 48   /* include/Frame.h:44 */

@@ -6,7 +6,8 @@ the built library raises (no CPU fallback).
 """
 from . import capi, synth  # noqa: F401
 from .capi import KP_DTYPE, OrbxError, lib  # noqa: F401
-from .bow import FeatureVector, ORBVocabulary, search_by_bow, search_for_triangulation  # noqa: F401
+from .bow import (FeatureVector, ORBVocabulary, search_by_bow, search_for_triangulation,  # noqa: F401
+                  search_for_triangulation_batch)
 from .extractor import ORBextractor, compute_tables, distribute_octree  # noqa: F401
 from .prep import Rectifier, undistort_keypoints  # noqa: F401
 from .projection import (FrameView, KeyFrameView, fuse, fuse_sim3, projection_rounds, search_by_projection_kf,  # noqa: F401

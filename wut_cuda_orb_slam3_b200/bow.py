@@ -5,7 +5,7 @@ import ctypes as C
 
 import numpy as np
 
-from .capi import FeatureVectorC, KP_DTYPE, check, lib, ptr
+from .capi import FeatureVectorC, KP_DTYPE, TriangulationViewC, check, lib, ptr
 
 TF_IDF, TF, IDF, BINARY = 0, 1, 2, 3
 L1_NORM, L2_NORM, CHI_SQUARE, KL, BHATTACHARYYA, DOT_PRODUCT = 0, 1, 2, 3, 4, 5
@@ -127,3 +127,33 @@ def search_for_triangulation(kp_a, desc_a, free_a, stereo_a, fv_a, kp_b, desc_b,
                                               ptr(frb), ptr(sb), len(kb), C.addressof(fb), ptr(F), ptr(e), ptr(sc), ptr(sg), len(sc),
                                               int(only_stereo), int(coarse), int(check_orientation), ptr(ma), C.byref(nm)))
     return ma, nm.value
+
+
+def search_for_triangulation_batch(kp_a, desc_a, free_a, stereo_a, fv_a, neighbours, only_stereo=False, check_orientation=True,
+                                   device=0):
+    """ORBmatcher::SearchForTriangulation of KF1 against many neighbours in one call (orbx_search_for_triangulation_batch).
+    `neighbours` is a sequence of dicts with the KF2 arguments of search_for_triangulation: kp, desc, free, stereo, fv, F12, ep,
+    scale, sigma2 and optionally coarse (default False).  Returns (match [n_kf, n_a] as KF2 indices, nmatches [n_kf]); row k
+    equals search_for_triangulation(KF1, neighbour k, ...)."""
+    ka = np.ascontiguousarray(kp_a, KP_DTYPE)
+    da = np.ascontiguousarray(desc_a, np.uint8).reshape(-1, 32)
+    fra = np.ascontiguousarray(free_a, np.uint8); sa = np.ascontiguousarray(stereo_a, np.uint8)
+    n_kf = len(neighbours)
+    keep = []                                  # the arrays the views point into stay alive for the call
+    views = (TriangulationViewC * max(n_kf, 1))()
+    for k, nb in enumerate(neighbours):
+        kb = np.ascontiguousarray(nb["kp"], KP_DTYPE); db = np.ascontiguousarray(nb["desc"], np.uint8).reshape(-1, 32)
+        frb = np.ascontiguousarray(nb["free"], np.uint8); sb = np.ascontiguousarray(nb["stereo"], np.uint8)
+        sc = np.ascontiguousarray(nb["scale"], np.float32); sg = np.ascontiguousarray(nb["sigma2"], np.float32)
+        keep += [kb, db, frb, sb, sc, sg, nb["fv"]]
+        v = views[k]
+        v.n = len(kb); v.kp = ptr(kb); v.desc = ptr(db); v.free = ptr(frb); v.stereo = ptr(sb); v.fv = nb["fv"].c_struct()
+        v.F12[:] = [float(x) for x in np.asarray(nb["F12"], np.float32).reshape(9)]
+        v.ep[:] = [float(x) for x in np.asarray(nb["ep"], np.float32).reshape(2)]
+        v.scale = ptr(sc); v.sigma2 = ptr(sg); v.n_levels = len(sc); v.coarse = int(bool(nb.get("coarse", False)))
+    match = np.full((n_kf, len(ka)), -1, np.int32)
+    nm = np.zeros(n_kf, np.int32)
+    fa = fv_a.c_struct()
+    check(lib().orbx_search_for_triangulation_batch(device, ptr(ka), ptr(da), ptr(fra), ptr(sa), len(ka), C.addressof(fa), n_kf,
+                                                    C.addressof(views), int(only_stereo), int(check_orientation), ptr(match), ptr(nm)))
+    return match, nm

@@ -88,6 +88,7 @@ SIGNATURES = {
     "orbx_search_by_bow": (_i, [_i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _vp, _i, _f, _i, _vp, _vp, _vp]),
     "orbx_search_for_triangulation": (_i, [_i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _i,
                                            _i, _i, _vp, _vp]),
+    "orbx_search_for_triangulation_batch": (_i, [_i, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _i, _i, _vp, _vp]),
     "orbx_assign_features_to_grid": (_i, [_i, _vp, _vp, _vp]),
     "orbx_get_features_in_area": (_i, [_i, _vp, _f, _f, _f, _i, _i, _vp, _i, _vp]),
     "orbx_search_by_projection_map": (_i, [_i, _vp, _vp, _f, _i, _f, _f, _vp, _vp]),
@@ -118,6 +119,12 @@ SIGNATURES = {
 class FeatureVectorC(C.Structure):
     """orbx_feature_vector (include/orbx.h): a DBoW2::FeatureVector in CSR form."""
     _fields_ = [("n_nodes", C.c_int), ("node_ids", _vp), ("offsets", _vp), ("indices", _vp)]
+
+
+class TriangulationViewC(C.Structure):
+    """orbx_triangulation_view (include/orbx.h): one neighbour of orbx_search_for_triangulation_batch."""
+    _fields_ = [("n", C.c_int), ("kp", _vp), ("desc", _vp), ("free", _vp), ("stereo", _vp), ("fv", FeatureVectorC),
+                ("F12", _f * 9), ("ep", _f * 2), ("scale", _vp), ("sigma2", _vp), ("n_levels", C.c_int), ("coarse", C.c_int)]
 
 
 class FrameViewC(C.Structure):

@@ -19,8 +19,10 @@
 //   int Fuse(KeyFrame*, Sim3f&, const vector<MapPoint*>&, th, vector<MapPoint*>& vpReplacePoint)       src/ORBmatcher2.cc:612-729
 //   int SearchAndFuse(const vector<KeyFrame*>&, const vector<Sim3f>&, const vector<MapPoint*>&, th)
 //                                     (added: the loop body of both LoopClosing::SearchAndFuse overloads in one call)
-// Not declared (no live caller / out of scope, DESIGN.md §8): SearchBySim3; SearchForTriangulation is exported by the C ABI
-// (orbx_search_for_triangulation) and takes F12 from the caller.
+//   int SearchForTriangulation(KeyFrame*, KeyFrame*, vector<pair<size_t, size_t>>&, bOnlyStereo, bCoarse)  src/ORBmatcher2.cc:173-471
+//   int SearchForTriangulation(KeyFrame*, const vector<KeyFrame*>&, const vector<char>& vbCoarse, bOnlyStereo, body)
+//                                     (added: the neighbour loop of LocalMapping::CreateNewMapPoints in one call)
+// Not declared (no live caller / out of scope, DESIGN.md §8): SearchBySim3.
 #ifndef ORBMATCHER_H
 #define ORBMATCHER_H
 
@@ -29,6 +31,7 @@
 #include <set>
 #include <stdexcept>
 #include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "ORBmatcherProjection.h"
@@ -186,6 +189,131 @@ public:
             }
             std::fill(vpReplacePoints.begin(), vpReplacePoints.end(), static_cast<MP*>(NULL));   // the next key frame's vpReplacePoints
         });
+    }
+
+    // Search matches for triangulation of new MapPoints between two key frames; checks the epipolar constraint.  (Member
+    // templates like Fuse.)  Equal to the batched overload below with the one neighbour pKF2.
+    template <class KF = KeyFrame>
+    int SearchForTriangulation(KF* pKF1, KF* pKF2, std::vector<std::pair<size_t, size_t>>& vMatchedPairs, const bool bOnlyStereo,
+                               const bool bCoarse = false)
+    {
+        vMatchedPairs.clear();
+        return SearchForTriangulation(pKF1, std::vector<KF*>(1, pKF2), std::vector<char>(1, (char)bCoarse), bOnlyStereo,
+                                      [&](int, std::vector<std::pair<size_t, size_t>>& v) { vMatchedPairs.swap(v); return true; });
+    }
+
+    // The neighbour loop of LocalMapping::CreateNewMapPoints: for k = 0, 1, ... in order, body(k, vMatchedPairs) receives exactly
+    // what SearchForTriangulation(pKF1, vpKF2[k], vMatchedPairs, bOnlyStereo, vbCoarse[k]) returns at that moment; body returns
+    // false to stop (the CheckNewKeyFrames() return).  One orbx_search_for_triangulation_batch call searches every neighbour
+    // against the KF1 features free at entry; before neighbour k is delivered its matches of KF1 features that gained a map point
+    // since then are dropped, a neighbour whose own slots changed since entry is searched again (one extra call), and the
+    // rotation filter runs on what is left (DESIGN.md §5d).  Poses are read at entry.  Returns the matches delivered.
+    template <class KF = KeyFrame, class Body>
+    int SearchForTriangulation(KF* pKF1, const std::vector<KF*>& vpKF2, const std::vector<char>& vbCoarse, const bool bOnlyStereo, Body body)
+    {
+        const int nK = (int)vpKF2.size();
+        if ((int)vbCoarse.size() != nK) throw std::invalid_argument("ORBmatcher::SearchForTriangulation: one bCoarse per neighbour");
+        auto single_camera = [](KF* pKF) {
+            if (pKF->mpCamera2 || pKF->NLeft != -1)
+                throw std::invalid_argument("ORBmatcher::SearchForTriangulation: two-camera key frame (two-camera rigs keep the reference code)");
+        };
+        single_camera(pKF1);
+        for (KF* pKF2 : vpKF2) single_camera(pKF2);
+        orbx_adapter::triangulation_diagnostics = orbx_adapter::TriangulationDiagnostics{};
+        if (nK == 0) return 0;
+        static_assert(sizeof(pKF1->mvKeysUn[0]) == sizeof(orbx_keypoint), "cv::KeyPoint must be the 28-byte POD");
+        const int N1 = (int)pKF1->mvKeysUn.size();
+        const orbx_keypoint* kp1 = reinterpret_cast<const orbx_keypoint*>(pKF1->mvKeysUn.data());
+        std::vector<uint8_t> free1(N1), stereo1(N1);
+        for (int i = 0; i < N1; ++i) { free1[i] = pKF1->GetMapPoint(i) == nullptr; stereo1[i] = pKF1->mvuRight[i] >= 0; }   // :246-258
+        Csr fv1(pKF1->mFeatVec);
+        const orbx_feature_vector va = fv1.view();
+        std::vector<Csr> fv2;
+        std::vector<std::vector<uint8_t>> free2(nK), stereo2(nK);
+        std::vector<orbx_triangulation_view> views(nK);
+        fv2.reserve(nK);
+        for (int k = 0; k < nK; ++k) {
+            KF* pKF2 = vpKF2[k];
+            orbx_triangulation_view& V = views[k];
+            // the reference's Sophus / Eigen lines (src/ORBmatcher2.cc:173-471) with the types' own arithmetic
+            //Compute epipole in second image
+            const auto T1w = pKF1->GetPose();
+            const auto T2w = pKF2->GetPose();
+            const auto Tw2 = pKF2->GetPoseInverse();
+            const auto Cw = pKF1->GetCameraCenter();
+            const auto C2 = T2w * Cw;
+            const auto ep = pKF2->mpCamera->project(C2);
+            const auto T12 = T1w * Tw2;
+            const auto R12 = T12.rotationMatrix();
+            const auto t12 = T12.translation();
+            // Pinhole::epipolarConstrain (src/CameraModels/Pinhole.cpp:107-112): F12 = K1^-T [t12]x R12 K2^-1
+            using SO3 = typename std::decay<decltype(T12.so3())>::type;
+            const auto t12x = SO3::hat(t12);
+            const auto K1 = pKF1->mpCamera->toK_();
+            const auto K2 = pKF2->mpCamera->toK_();
+            using Mat3 = typename std::decay<decltype(R12)>::type;
+            const Mat3 F12 = K1.transpose().inverse() * t12x * R12 * K2.inverse();
+            for (int r = 0; r < 3; ++r)
+                for (int c = 0; c < 3; ++c) V.F12[r * 3 + c] = F12(r, c);
+            V.ep[0] = ep(0); V.ep[1] = ep(1);
+            const int N2 = (int)pKF2->mvKeysUn.size();
+            free2[k].resize(N2); stereo2[k].resize(N2);
+            for (int j = 0; j < N2; ++j) { free2[k][j] = pKF2->GetMapPoint(j) == nullptr; stereo2[k][j] = pKF2->mvuRight[j] >= 0; }   // :273-279
+            fv2.emplace_back(pKF2->mFeatVec);
+            V.n = N2;
+            V.kp = reinterpret_cast<const orbx_keypoint*>(pKF2->mvKeysUn.data());
+            V.desc = N2 ? pKF2->mDescriptors.ptr(0) : nullptr;
+            V.free = free2[k].data(); V.stereo = stereo2[k].data();
+            V.fv = fv2.back().view();
+            V.scale = pKF2->mvScaleFactors.data(); V.sigma2 = pKF2->mvLevelSigma2.data();
+            V.n_levels = (int)pKF2->mvScaleFactors.size();
+            V.coarse = vbCoarse[k] != 0;
+        }
+        std::vector<int32_t> match((size_t)nK * N1, -1);
+        std::vector<int> nm(nK, 0);
+        orbx_adapter::check(orbx_search_for_triangulation_batch(device, kp1, N1 ? pKF1->mDescriptors.ptr(0) : nullptr, free1.data(), stereo1.data(), N1,
+                                                                &va, nK, views.data(), bOnlyStereo, 0, match.data(), nm.data()),
+                            "SearchForTriangulation");
+        int total = 0;
+        std::vector<std::pair<size_t, size_t>> vMatchedPairs;
+        for (int k = 0; k < nK; ++k) {
+            KF* pKF2 = vpKF2[k];
+            int32_t* m = &match[(size_t)k * N1];
+            orbx_triangulation_view& V = views[k];
+            // a slot of pKF2 changed since entry (not by the loop itself: it adds map points to pKF1 and the searched neighbour
+            // only): search this neighbour again with the live slots of both key frames
+            bool changed = false;
+            for (int j = 0; j < V.n && !changed; ++j) changed = (pKF2->GetMapPoint(j) == nullptr) != (free2[k][j] != 0);
+            if (changed) {
+                for (int j = 0; j < V.n; ++j) free2[k][j] = pKF2->GetMapPoint(j) == nullptr;
+                for (int i = 0; i < N1; ++i) free1[i] = pKF1->GetMapPoint(i) == nullptr;
+                int n = 0;
+                orbx_adapter::check(orbx_search_for_triangulation(device, kp1, N1 ? pKF1->mDescriptors.ptr(0) : nullptr, free1.data(), stereo1.data(), N1,
+                                                                  &va, V.kp, V.desc, V.free, V.stereo, V.n, &V.fv, V.F12, V.ep, V.scale, V.sigma2,
+                                                                  V.n_levels, bOnlyStereo, V.coarse, 0, m, &n),
+                                    "SearchForTriangulation");
+                orbx_adapter::triangulation_diagnostics.researched_kfs += 1;
+            }
+            // KF1 features that gained a map point since entry: the reference skips them (pMP1 = pKF1->GetMapPoint(idx1); if (pMP1) continue;)
+            for (int i = 0; i < N1; ++i)
+                if (m[i] >= 0 && pKF1->GetMapPoint(i)) { m[i] = -1; orbx_adapter::triangulation_diagnostics.dropped += 1; }
+            if (mbCheckOrientation) {                                       // :429-447, on the matches the reference would have made
+                std::vector<int> idx;
+                std::vector<float> a1, a2;
+                for (int i = 0; i < N1; ++i)
+                    if (m[i] >= 0) { idx.push_back(i); a1.push_back(pKF1->mvKeysUn[i].angle); a2.push_back(pKF2->mvKeysUn[m[i]].angle); }
+                std::vector<uint8_t> keep(idx.size());
+                orbx_adapter::check(orbx_rotation_consistency(a1.data(), a2.data(), (int)idx.size(), keep.data()), "SearchForTriangulation");
+                for (size_t t = 0; t < idx.size(); ++t)
+                    if (!keep[t]) m[idx[t]] = -1;
+            }
+            vMatchedPairs.clear();
+            for (int i = 0; i < N1; ++i)
+                if (m[i] >= 0) vMatchedPairs.push_back(std::make_pair((size_t)i, (size_t)m[i]));
+            total += (int)vMatchedPairs.size();
+            if (!body(k, vMatchedPairs)) break;
+        }
+        return total;
     }
 
     // Search matches between MapPoints in a KeyFrame and ORB in a Frame.

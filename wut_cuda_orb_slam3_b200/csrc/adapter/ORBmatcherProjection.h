@@ -348,5 +348,10 @@ inline int FuseSim3Apply(const std::vector<KF*>& vpKFs, const std::vector<MP*>& 
     return nFused;
 }
 
+// What the last batched SearchForTriangulation on this thread did besides delivering the batch: neighbours searched again because
+// their map-point slots changed after entry, and matches dropped because their KF1 feature gained a map point (diagnostics).
+struct TriangulationDiagnostics { int researched_kfs = 0, dropped = 0; };
+inline thread_local TriangulationDiagnostics triangulation_diagnostics;
+
 }  // namespace orbx_adapter
 }  // namespace ORB_SLAM3

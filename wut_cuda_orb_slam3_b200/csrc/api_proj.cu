@@ -25,61 +25,37 @@
 
 namespace orbx {
 
-namespace {
-
-constexpr int GRID_CELLS = ORBX_FRAME_GRID_COLS * ORBX_FRAME_GRID_ROWS;
-thread_local int t_rounds = 0;
-
-struct ProjArena {
-    std::mutex mu;
-    unsigned char* d = nullptr; size_t d_bytes = 0;
-    unsigned char* h = nullptr; size_t h_bytes = 0;
-    cudaStream_t st = nullptr;
-};
 ProjArena g_arena[64];
-// orbx_fuse runs on the local-mapping thread: its own arenas, so a large Fuse never holds the lock a tracking-thread search waits on
+// orbx_fuse and orbx_search_for_triangulation_batch run on the local-mapping thread: their own arenas, so a large Fuse never
+// holds the lock a tracking-thread search waits on
 ProjArena g_fuse_arena[64];
 // the Sim3 searches run on the loop-closing thread: a third set, so they never hold a lock the other two threads wait on
 ProjArena g_loop_arena[64];
 
-// One call = one lease: a bump allocator that hands out matching (pinned host, device) ranges so that all inputs travel in
-// one cudaMemcpyAsync.  Inputs are allocated first (the upload range), device-only scratch and outputs after.
-struct Lease {
-    ProjArena& A;
-    std::unique_lock<std::mutex> lock;
-    size_t off = 0, upload_end = 0;
-    explicit Lease(int device, ProjArena* arenas = g_arena) : A(arenas[device & 63]), lock(A.mu) {}
-    int reserve(size_t bytes)
-    {
-        bytes += 8192;
-        if (!A.st) {
-            cudaError_t e = cudaStreamCreateWithFlags(&A.st, cudaStreamNonBlocking);
-            if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
-        }
-        if (A.d_bytes < bytes) {
-            if (A.d) cudaFree(A.d);
-            if (A.h) cudaFreeHost(A.h);
-            A.d = A.h = nullptr; A.d_bytes = A.h_bytes = 0;
-            const size_t want = bytes + bytes / 2;
-            cudaError_t e = cudaMalloc((void**)&A.d, want);
-            if (e == cudaSuccess) e = cudaMallocHost((void**)&A.h, want);
-            if (e != cudaSuccess) return fail(ORBX_ERR_OOM, "projection scratch (%zu bytes): %s", want, cudaGetErrorString(e));
-            A.d_bytes = A.h_bytes = want;
-        }
-        return ORBX_OK;
+int Lease::reserve(size_t bytes)
+{
+    bytes += 8192;
+    if (!A.st) {
+        cudaError_t e = cudaStreamCreateWithFlags(&A.st, cudaStreamNonBlocking);
+        if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
     }
-    template <typename T> size_t take(size_t count)
-    {
-        off = (off + 255) & ~(size_t)255;
-        const size_t o = off;
-        off += std::max<size_t>(count, 1) * sizeof(T);
-        return o;
+    if (A.d_bytes < bytes) {
+        if (A.d) cudaFree(A.d);
+        if (A.h) cudaFreeHost(A.h);
+        A.d = A.h = nullptr; A.d_bytes = A.h_bytes = 0;
+        const size_t want = bytes + bytes / 2;
+        cudaError_t e = cudaMalloc((void**)&A.d, want);
+        if (e == cudaSuccess) e = cudaMallocHost((void**)&A.h, want);
+        if (e != cudaSuccess) return fail(ORBX_ERR_OOM, "projection scratch (%zu bytes): %s", want, cudaGetErrorString(e));
+        A.d_bytes = A.h_bytes = want;
     }
-    template <typename T> T* dev(size_t o) const { return reinterpret_cast<T*>(A.d + o); }
-    template <typename T> T* host(size_t o) const { return reinterpret_cast<T*>(A.h + o); }
-};
+    return ORBX_OK;
+}
 
-size_t pad(size_t bytes) { return ((bytes + 255) & ~(size_t)255) + 256; }
+namespace {
+
+constexpr int GRID_CELLS = ORBX_FRAME_GRID_COLS * ORBX_FRAME_GRID_ROWS;
+thread_local int t_rounds = 0;
 
 int check_frame(const orbx_frame_view* f, bool need_desc)
 {
@@ -106,10 +82,10 @@ struct Session {
         int rc;
         if ((rc = set_device(device))) return rc;
         n = f->n; nq = n_queries; area_cap = area_capacity;
-        const size_t total = pad((size_t)n * 28) + pad((size_t)n * 32) + pad((size_t)n * 4) + pad((size_t)n * 4) + pad((size_t)nq * sizeof(ProjQuery)) +
-                             pad((size_t)nq * 32) + pad((GRID_CELLS + 1) * 4) + pad((size_t)n * 4) + pad((size_t)n * 2) + pad((size_t)n * 4) +
-                             pad((size_t)nq * 16) + 3 * pad((size_t)nq * 4) + pad(4) + pad((size_t)area_cap * 8) + pad(4) +
-                             pad((size_t)n * 4) + 2 * pad((size_t)nq * 4);
+        const size_t total = lease_pad((size_t)n * 28) + lease_pad((size_t)n * 32) + lease_pad((size_t)n * 4) + lease_pad((size_t)n * 4) + lease_pad((size_t)nq * sizeof(ProjQuery)) +
+                             lease_pad((size_t)nq * 32) + lease_pad((GRID_CELLS + 1) * 4) + lease_pad((size_t)n * 4) + lease_pad((size_t)n * 2) + lease_pad((size_t)n * 4) +
+                             lease_pad((size_t)nq * 16) + 3 * lease_pad((size_t)nq * 4) + lease_pad(4) + lease_pad((size_t)area_cap * 8) + lease_pad(4) +
+                             lease_pad((size_t)n * 4) + 2 * lease_pad((size_t)nq * 4);
         if ((rc = L.reserve(total))) return rc;
         // upload range
         o_kp = L.take<orbx_keypoint>(n);
@@ -263,9 +239,9 @@ int fuse_search(int device, ProjArena* arenas, const char* name, bool gate, int 
     if ((rc = set_device(device))) return rc;
     Lease L(device, arenas);
     const size_t n_ur = gate ? (size_t)n_feat : 0;
-    const size_t total = pad((size_t)n_kf * sizeof(FuseKF)) + pad((size_t)n_feat * 28) + pad((size_t)n_feat * 32) + pad(n_ur * 4) +
-                         pad((size_t)nv * sizeof(FuseQuery)) + pad((size_t)n_desc * 32) + pad((size_t)n_kf * (GRID_CELLS + 1) * 4) +
-                         pad((size_t)n_feat * 4) + pad((size_t)n_feat * 2) + pad((size_t)nv * 4);
+    const size_t total = lease_pad((size_t)n_kf * sizeof(FuseKF)) + lease_pad((size_t)n_feat * 28) + lease_pad((size_t)n_feat * 32) + lease_pad(n_ur * 4) +
+                         lease_pad((size_t)nv * sizeof(FuseQuery)) + lease_pad((size_t)n_desc * 32) + lease_pad((size_t)n_kf * (GRID_CELLS + 1) * 4) +
+                         lease_pad((size_t)n_feat * 4) + lease_pad((size_t)n_feat * 2) + lease_pad((size_t)nv * 4);
     if ((rc = L.reserve(total))) return rc;
     // upload range
     const size_t o_kf = L.take<FuseKF>(n_kf), o_kp = L.take<orbx_keypoint>(n_feat), o_desc = L.take<uint8_t>((size_t)n_feat * 32),

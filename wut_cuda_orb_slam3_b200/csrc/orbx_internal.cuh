@@ -4,6 +4,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <mutex>
+
 #include "../../include/orbx.h"
 
 namespace orbx {
@@ -238,6 +240,26 @@ struct TriSearchArgs {
 };
 cudaError_t launch_search_triangulation(const TriSearchArgs& a, cudaStream_t st);
 
+// SearchForTriangulation of one KF1 against many neighbours: a job-build kernel (one CTA per neighbour) writes the jobs of
+// neighbour k into jobs[k * n_a, k * n_a + job_count[k]) and sets match row k to -1; the scan kernel takes the neighbour as
+// blockIdx.y.  Feature indices inside a neighbour are its own (0 .. n - 1); its arrays point into the packed upload.
+struct TriKF {
+    const orbx_keypoint* kp; const uint8_t* desc; const uint8_t* free; const uint8_t* stereo;
+    const uint32_t* node_ids; const int32_t* offsets; const uint32_t* indices;   // mFeatVec in CSR form
+    int n, n_nodes, coarse, pad;
+    float F12[9]; float ep[2]; float scale[kMaxLevels]; float sigma2[kMaxLevels];
+};
+struct TriBatchArgs {
+    int n_kf; const TriKF* kfs;
+    int n_a; const orbx_keypoint* kp_a; const uint8_t* desc_a; const uint8_t* free_a; const uint8_t* stereo_a;
+    int a_nodes; const uint32_t* a_node_ids; const int32_t* a_offsets; const uint32_t* a_indices;
+    int only_stereo;
+    int4* jobs;                  // [n_kf][n_a] (iA, b_begin, b_end, 0), b_* into the neighbour's indices
+    int* job_count;              // [n_kf]
+    int* match;                  // [n_kf][n_a]
+};
+cudaError_t launch_search_triangulation_batch(const TriBatchArgs& a, cudaStream_t st);
+
 
 // ---- frame grid + projection-guided window searches (kernels_proj.cu, api_proj.cu) ----------------------------------------
 enum { PROJ_Q_VALID = 1, PROJ_Q_CHECK_RIGHT = 2, PROJ_Q_TAKES = 4 };
@@ -311,6 +333,36 @@ cudaError_t launch_remap(const uint8_t* d_src, int sw, int sh, size_t spitch, si
                          int dh, size_t dpitch, size_t dframe, int n_frames, cudaStream_t st);
 cudaError_t launch_resize(const uint8_t* d_src, size_t spitch, size_t sframe, const uint2* d_xtab, const uint2* d_ytab, int area2x,
                           uint8_t* d_dst, int dw, int dh, size_t dpitch, size_t dframe, int n_frames, cudaStream_t st);
+
+// Per-device grow-only scratch of the matcher calls (api_proj.cu): device memory, a pinned staging buffer of the same size and
+// a stream.  One call = one Lease: a bump allocator that hands out matching (pinned host, device) ranges so that all inputs
+// travel in one cudaMemcpyAsync.  Inputs are allocated first (the upload range), device-only scratch and outputs after.
+struct ProjArena {
+    std::mutex mu;
+    unsigned char* d = nullptr; size_t d_bytes = 0;
+    unsigned char* h = nullptr; size_t h_bytes = 0;
+    cudaStream_t st = nullptr;
+};
+extern ProjArena g_arena[64];          // the tracking thread's searches
+extern ProjArena g_fuse_arena[64];     // local mapping: orbx_fuse, orbx_search_for_triangulation_batch
+extern ProjArena g_loop_arena[64];     // loop closing: the Sim3 searches
+struct Lease {
+    ProjArena& A;
+    std::unique_lock<std::mutex> lock;
+    size_t off = 0, upload_end = 0;
+    explicit Lease(int device, ProjArena* arenas = g_arena) : A(arenas[device & 63]), lock(A.mu) {}
+    int reserve(size_t bytes);
+    template <typename T> size_t take(size_t count)
+    {
+        off = (off + 255) & ~(size_t)255;
+        const size_t o = off;
+        off += (count > 1 ? count : 1) * sizeof(T);
+        return o;
+    }
+    template <typename T> T* dev(size_t o) const { return reinterpret_cast<T*>(A.d + o); }
+    template <typename T> T* host(size_t o) const { return reinterpret_cast<T*>(A.h + o); }
+};
+inline size_t lease_pad(size_t bytes) { return ((bytes + 255) & ~(size_t)255) + 256; }   // bytes of one take() in reserve()
 
 // host helpers shared by api.cu / api_bow.cu / api_proj.cu
 int fail(int code, const char* fmt, ...);
