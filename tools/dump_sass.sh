@@ -11,7 +11,7 @@ echo "cuobjdump -sass of $SO ($(date -u +%Y-%m-%dT%H:%MZ)); arch: $(cuobjdump -l
 cuobjdump -sass $SO 2>/dev/null | awk '
   /Function :/ { fn=$3 }
   /^[ \t]+\/\*[0-9a-f]+\*\/[ \t]+[A-Z@]/ { line=$0; sub(/^[ \t]+\/\*[0-9a-f]+\*\/[ \t]+/, "", line); sub(/[ \t]*\/\*.*$/, "", line); print fn "\t" line }' > /tmp/all_sass.tsv
-for pat in pyr_resize_pipe_kernel pyr_resize_tiled_kernelILi32 pyr_level0_tiled blur_pipe_kernel fast_cells_warp_kernelILi48 fast_cells_kernel octree_kernelILi256 octree_kernelILi1024 orient_describe_kernelILb1 orient_describe_kernelILb0 pack_kernelILi256 knn2_imma_kernel knn2_kernelILi6 knn2_merge stereo_match_kernel remap_tiled resize_tiled distinctive_kernel; do
+for pat in pyr_resize_pipe_kernel pyr_resize_tiled_kernelILi32 pyr_level0_tiled blur_mma_kernel fast_cells_warp_kernelILi48 fast_cells_kernel octree_kernelILi256 octree_kernelILi1024 orient_describe_kernelILb1 orient_describe_kernelILb0 pack_kernelILi256 knn2_imma_kernel knn2_kernelILi6 knn2_merge stereo_match_kernel remap_tiled resize_tiled distinctive_kernel; do
   fn=$(cut -f1 /tmp/all_sass.tsv | grep "$pat" | sort -u | head -1)
   [ -z "$fn" ] && { echo "missing $pat" >> $SUM; continue; }
   short=$(echo $pat | sed 's/ILi/_/')

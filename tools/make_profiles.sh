@@ -21,7 +21,7 @@ ncu --set full --clock-control none --import-source on -k regex:knn2_kernel -s 1
 python bench.py $ARGS > $OUT/plain.log 2>&1 && \
 ncu --metrics dram__bytes_read.sum,dram__bytes_write.sum --clock-control none -k regex:fast_cells_warp -s 3 -c 3 --csv --log-file $OUT/${TAG}_fast_dram.csv python bench.py $ARGS > $OUT/ncu_d.log 2>&1
 python bench.py $ARGS > $OUT/plain.log 2>&1 && \
-ncu --set full --clock-control none --import-source on -k regex:blur_pipe -s 1 -c 1 -f -o $OUT/${TAG}_blur_pipe python bench.py $ARGS > $OUT/ncu_b.log 2>&1
+ncu --set full --clock-control none --import-source on -k regex:blur_mma -s 1 -c 1 -f -o $OUT/${TAG}_blur_mma python bench.py $ARGS > $OUT/ncu_b.log 2>&1
 python tools/latency.py > $OUT/${TAG}_single_frame_latency.txt 2>&1
 # rectification / resize kernels and the projection-guided searches (SURVEY.md §8(f)2-3)
 python tools/prep_bench.py > $OUT/${TAG}_prep_bench.json 2> $OUT/prep_bench.err && \

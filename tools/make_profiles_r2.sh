@@ -12,7 +12,7 @@ ncu --metrics gpu__time_duration.sum --clock-control none -c 120 --csv --log-fil
 python tools/launch_shares.py $OUT/${TAG}_launches_b512.csv $OUT/${TAG}_bench.json 512 > $OUT/${TAG}_launch_shares_b512.txt 2>&1
 ARGS="--steps 1 --warmup 1 --batch 64 --no-knn2 --no-cpu --no-other --no-cfg4"
 python bench.py $ARGS > $OUT/plain.log 2>&1 || { tail -5 $OUT/plain.log; exit 1; }
-for K in fast_cells_warp:3 octree_kernel:1 orient_describe:1 pyr_resize_pipe:7 blur_pipe:1; do
+for K in fast_cells_warp:3 octree_kernel:1 orient_describe:1 pyr_resize_pipe:7 blur_mma:1; do
   NAME=${K%%:*}; SKIP=${K##*:}
   ncu --set full --clock-control none --import-source on -k regex:$NAME -s $SKIP -c 1 -f -o $OUT/${TAG}_$NAME python bench.py $ARGS > $OUT/ncu_$NAME.log 2>&1
   tail -n 1 $OUT/ncu_$NAME.log

@@ -572,7 +572,7 @@ static int ensure_slot(orbx_extractor* ex, Slot& s, int frames)
                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
                     ok_desc = false;
             }
-            const cuuint32_t bbox[3] = {160, 38, 1};
+            const cuuint32_t bbox[3] = {kBlurBoxW, kBlurBoxH, 1};
             if (enc(&maps[kMaxLevels + l], CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, base, dims, strides, bbox, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
                 ok_blur = false;
@@ -706,7 +706,9 @@ static int run_chunk(orbx_extractor* ex, Slot& s, const ChunkIO& io, int frames,
     if ((rc = prof_mark(ex, st))) return rc;
     // The blur depends on the pyramid only: for batches it runs on a side stream beside FAST and the octree.  While a FAST launch
     // is at full occupancy there is no room for a blur CTA (shared memory and registers are taken), but each of FAST's three
-    // launches ends with a tail of half-empty SMs, and the blur's persistent CTAs fill those: 3.163 -> 3.088 ms per 512 frames.
+    // launches ends with a tail of half-empty SMs, and the blur's persistent CTAs fill those.  With the tensor-core blur (0.31 ms
+    // alone) the step is 2.990 ms per 512 frames this way and 3.031 ms with the blur on this stream (B200, 1000 W; with the
+    // earlier scalar blur, 0.44 ms alone: 3.088 vs 3.163 ms).
     // (The blur beside the octree instead: no gain — the octree's four CTAs hold the whole register file of an SM.  FAST's three
     // launches alternating between two streams: 3.17 ms.  The octree of the first FAST group's levels beside the later FAST launches: 3.13 ms.)  Not while
     // profiling (the per-stage events assume one stream), not for a few frames (run_single_forked forks per level).

@@ -28,7 +28,7 @@ __device__ float4 d_pattern_f[8][32];
 __device__ uint4 d_mom_mask[16][2];
 
 constexpr int BT_W = 128, BT_H = 32;          // blur tile
-constexpr int BIN_P = 160;                    // input tile pitch (bytes): image columns x0-16 .. x0+143 (16-byte aligned)
+constexpr int BIN_P = kBlurBoxW;              // input tile pitch (bytes): image columns x0-16 .. x0+159 (16-byte aligned)
 constexpr int BIN_R = BT_H + 6;
 
 // cv::fastAtan2 (OpenCV mathfuncs_core atan_f32): float32, no FMA contraction.
@@ -60,7 +60,7 @@ __device__ __forceinline__ float fast_atan2_dev(float y, float x)
 // sliding 32-bit window using the kernel's symmetry; the tile leaves through shared memory as 16-byte stores.
 __global__ void __launch_bounds__(256) blur_kernel(const __grid_constant__ FrameGeom fg, Workspace ws)
 {
-    __shared__ __align__(128) uint8_t in[BIN_R * BIN_P];
+    __shared__ __align__(128) uint8_t in[kBlurBoxH * BIN_P];
     __shared__ __align__(16) uint32_t hb[BIN_R * BT_W];
     __shared__ __align__(16) uint8_t outt[BT_H * BT_W];
     const int tid = threadIdx.x;
@@ -81,12 +81,13 @@ __global__ void __launch_bounds__(256) blur_kernel(const __grid_constant__ Frame
     // input tile: buffer rows (ty0 - 3 + 19) .., buffer byte columns (tx0 - 16 + 32) .. : 16-byte aligned
     const int brow0 = ty0 - 3 + kEdge, bcol0 = tx0 - 16 + kXPad;
     if (ws.tmap_blur) {
-        // TMA: 160 x 38 box of the bordered level (out-of-range rows/columns are zero-filled by the copy engine)
+        // TMA: kBlurBoxW x kBlurBoxH box of the bordered level (out-of-range rows/columns are zero-filled by the copy engine);
+        // its last two rows are not used here
         __shared__ __align__(8) uint64_t bar;
         if (tid == 0) mbar_init(&bar, 1);
         __syncthreads();
         if (tid == 0) {
-            mbar_expect_tx(&bar, BIN_R * BIN_P);
+            mbar_expect_tx(&bar, kBlurBoxH * BIN_P);
             tma_load_3d(in, ws.tmap_blur + level, &bar, bcol0, brow0, frame);
         }
         mbar_wait(&bar, 0);
@@ -223,34 +224,68 @@ __global__ void __launch_bounds__(128) blur_stream_kernel(const __grid_constant_
     }
 }
 
-// TMA-pipelined blur (default when tensor maps are available): the register-streaming arithmetic of blur_stream_kernel, fed
-// from shared memory by a per-warp ring of TMA boxes.  Both kernels above are bound by memory-level parallelism (long-scoreboard
-// stalls, ~30 % of HBM peak): a warp that loads its rows itself keeps ~3 lines in flight.  Here every warp is persistent, owns
-// kBpStages shared-memory stages of one 160 x 38 box each (128 columns + 16-byte aligned halo, 32 rows + 6 halo rows) and lane 0
-// keeps kBpStages bulk copies in flight (cp.async.bulk.tensor.3d -> mbarrier complete_tx); the copy engine zero-fills what
-// lies outside the bordered level.  No CTA-wide barrier: a stage is refilled by the same warp that has just consumed it.
-constexpr int kBpStages = 1;
-constexpr int kBpStageBytes = 6144;               // 160 * 38 = 6080, padded to a multiple of 128
-constexpr int kBpWarps = 4;
+// Tensor-core blur (default for batches when tensor maps are available).  The filter is an integer linear map, exact in int32
+// up to the single final rounding, so int8 MMAs (imma_16832_u8) produce the same bytes as the scalar kernels in any summation
+// order.  Every warp is persistent and owns one stage of one kBlurBoxW x kBlurBoxH TMA box (completion on an mbarrier); an item is a
+// 128-column x 32-row band, worked as 8 column tiles of 16 outputs (g = lane / 4, t = lane % 4):
+//  * Horizontal pass, transposed: H^T (16 columns x 8 rows) = Wh (16 x 32) . I^T (32 input columns x 8 rows).  The K window of a
+//    tile starts one word left of it (input column c0 - 4), so Wh[m][k] = w[k - m - 1] is constant and a B register is 4
+//    consecutive bytes of one staged row: one conflict-free 32-bit shared load.  Five such MMAs cover the 40 rows of the box.
+//  * Vertical pass: S (16 rows x 8 columns) = Wv (16 x 32) . H (32 H rows x 8 columns).  The horizontal accumulators leave a
+//    thread the H values of columns g and g + 8 in rows 2 t, 2 t + 1 of every 8-row block.  With K permuted (slot 16 u + 4 t + i
+//    <-> H row 16 u + 8 (i / 2) + 2 t + i % 2) these are exactly its B slots, so Wv carries the permutation and no data moves
+//    between lanes.  Row tile T uses the blocks 2T .. 2T+2; the fourth block of its K window has zero weight.
+//  * H < 2^16 is split into bytes with PRMT: S = 256 acc_hi + acc_lo, acc_lo seeded with the rounding constant 2^15, and the output
+//    byte is byte 2 of S (S < 2^24).  Per 16 x 16 outputs: 2.5 horizontal and 4 vertical MMAs.
+//  * Two shuffles over the lane quad give each lane 8 consecutive output bytes of one row; they go to the columns of the stage the
+//    tile has consumed (16 j .. 16 j + 15), and the finished band leaves as 16-byte stores, 128 contiguous bytes per row.
+constexpr int kBmWarps = 4;
+constexpr int kBmStageBytes = kBlurBoxW * kBlurBoxH;          // 7040, a multiple of 128 (TMA destination alignment)
 
-__global__ void __launch_bounds__(32 * kBpWarps) blur_pipe_kernel(const __grid_constant__ FrameGeom fg, Workspace ws, int items_per_frame,
-                                                                  int total_items)
+__device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel)
 {
-    extern __shared__ __align__(128) uint8_t bp_smem[];
-    __shared__ __align__(8) uint64_t bars[kBpWarps][kBpStages];
+    uint32_t d;
+    asm("prmt.b32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(sel));
+    return d;
+}
+
+__global__ void __launch_bounds__(32 * kBmWarps) blur_mma_kernel(const __grid_constant__ FrameGeom fg, Workspace ws, int items_per_frame,
+                                                                 int total_items)
+{
+    extern __shared__ __align__(128) uint8_t bm_smem[];
+    __shared__ __align__(8) uint64_t bars[kBmWarps];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint8_t* stage0 = bp_smem + (size_t)warp * kBpStages * kBpStageBytes;
-    if (lane == 0) {
-#pragma unroll
-        for (int sgi = 0; sgi < kBpStages; ++sgi) mbar_init(&bars[warp][sgi], 1);
-    }
+    const int g = lane >> 2, t = lane & 3;
+    uint8_t* stage = bm_smem + (size_t)warp * kBmStageBytes;
+    uint64_t* bar = &bars[warp];
+    if (lane == 0) mbar_init(bar, 1);
     __syncwarp();
-    const int gw = blockIdx.x * kBpWarps + warp, nw = gridDim.x * kBpWarps;
+    const int gw = blockIdx.x * kBmWarps + warp, nw = gridDim.x * kBmWarps;
+
+    // constant A fragments: taps w[0..6] = bytes of kTaps (byte 7 = 0)
+    uint32_t ah[4], av[4];
+    {
+        constexpr unsigned long long kTaps = 0x0012223038302212ull;
+        auto tap = [](int d) -> uint32_t { return d >= 0 && d < 8 ? (uint32_t)(kTaps >> (8 * d)) & 0xffu : 0u; };
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const int m = g + 8 * (q & 1);
+            ah[q] = av[q] = 0;
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                ah[q] |= tap(16 * (q >> 1) + 4 * t + i - m - 1) << (8 * i);
+                av[q] |= tap(16 * (q >> 1) + 8 * (i >> 1) + 2 * t + (i & 1) - m) << (8 * i);
+            }
+        }
+    }
+    // the quad transpose of the output: round 1 (lanes t, t ^ 1) exchanges rows, round 2 (t, t ^ 2) exchanges column halves
+    const int a = t & 1, hb = t >> 1;
+    const uint32_t sel0 = a ? 0x1054u : 0x5410u, sel1 = a ? 0x3276u : 0x7632u;
 
     // item -> (frame, level, x0, y0)
     auto decode = [&](int item, int& frame, int& level, int& x0, int& y0) {
         frame = item / items_per_frame;
-        int t = item - frame * items_per_frame;
+        int r = item - frame * items_per_frame;
         level = 0;
         int sx_n = 1;
 #pragma unroll 1
@@ -258,69 +293,87 @@ __global__ void __launch_bounds__(32 * kBpWarps) blur_pipe_kernel(const __grid_c
             sx_n = (fg.L[l].w + 127) / 128;
             const int nt = sx_n * ((fg.L[l].h + 31) / 32);
             level = l;
-            if (t < nt) break;
-            t -= nt;
+            if (r < nt) break;
+            r -= nt;
         }
-        const int band = t / sx_n;
-        x0 = (t - band * sx_n) * 128;
+        const int band = r / sx_n;
+        x0 = (r - band * sx_n) * 128;
         y0 = band * 32;
     };
-    auto issue = [&](int item, int sgi) {          // lane 0 only
+    auto issue = [&](int item) {          // lane 0 only
         int frame, level, x0, y0;
         decode(item, frame, level, x0, y0);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        mbar_expect_tx(&bars[warp][sgi], 160 * 38);
-        tma_load_3d(stage0 + (size_t)sgi * kBpStageBytes, ws.tmap_blur + level, &bars[warp][sgi], kXPad + x0 - 16, kEdge + y0 - 3, frame);
+        mbar_expect_tx(bar, kBmStageBytes);
+        tma_load_3d(stage, ws.tmap_blur + level, bar, kXPad + x0 - 16, kEdge + y0 - 3, frame);
     };
 
-    if (lane == 0) {
-#pragma unroll
-        for (int sgi = 0; sgi < kBpStages; ++sgi)
-            if (gw + sgi * nw < total_items) issue(gw + sgi * nw, sgi);
-    }
+    if (lane == 0 && gw < total_items) issue(gw);
     int k = 0;
     for (int item = gw; item < total_items; item += nw, ++k) {
-        const int sgi = k % kBpStages;
         int frame, level, x0, y0;
         decode(item, frame, level, x0, y0);
-        const LevelGeom& g = fg.L[level];
-        mbar_wait(&bars[warp][sgi], (uint32_t)((k / kBpStages) & 1));
-        const int x = x0 + 4 * lane;
-        if (x < g.w) {
-            const int rows = min(32, g.h - y0);
-            const uint32_t sb = (uint32_t)__cvta_generic_to_shared(stage0 + (size_t)sgi * kBpStageBytes) + 12 + 4 * lane;   // word left of the lane's 4 pixels
-            uint8_t* out = ws.blur + g.blur_off + (size_t)frame * g.blur_frame_stride + (size_t)y0 * g.bpitch + x;
-            const int bpitch = g.bpitch;
-            uint32_t W[7][4];
-            auto hrow = [&](int r, uint32_t h[4]) {
-                uint32_t w[3];
-                asm volatile("ld.shared.u32 %0, [%1];" : "=r"(w[0]) : "r"(sb + r * 160));
-                asm volatile("ld.shared.u32 %0, [%1+4];" : "=r"(w[1]) : "r"(sb + r * 160));
-                asm volatile("ld.shared.u32 %0, [%1+8];" : "=r"(w[2]) : "r"(sb + r * 160));
-                blur_hsum(w, h);
-            };
+        const LevelGeom& lg = fg.L[level];
+        mbar_wait(bar, (uint32_t)(k & 1));
+        const int ntiles = min(8, (lg.w - x0 + 15) >> 4);
+#pragma unroll 1
+        for (int j = 0; j < ntiles; ++j) {
+            // horizontal pass: per 8-row block b and column half h, q = (H lo, H lo, H hi, H hi) of rows 2 t, 2 t + 1
+            uint32_t hq[5][2];
+            const uint8_t* bp = stage + g * kBlurBoxW + 16 * j + 12 + 4 * t;
 #pragma unroll
-            for (int i = 0; i < 6; ++i) hrow(i, W[i]);
-            for (int r = 0; r < rows; r += 7) {
+            for (int b = 0; b < 5; ++b) {
+                const uint32_t b0 = *reinterpret_cast<const uint32_t*>(bp + 8 * b * kBlurBoxW);
+                const uint32_t b1 = *reinterpret_cast<const uint32_t*>(bp + 8 * b * kBlurBoxW + 16);
+                int c[4] = {0, 0, 0, 0};
+                imma_16832_u8(c, ah, b0, b1);
+                hq[b][0] = prmt(c[0], c[1], 0x5140u);
+                hq[b][1] = prmt(c[2], c[3], 0x5140u);
+            }
 #pragma unroll
-                for (int kk = 0; kk < 7; ++kk) {
-                    if (r + kk < rows) {                            // warp-uniform
-                        hrow(r + kk + 6, W[(kk + 6) % 7]);
-                        uint32_t o = 0;
+            for (int T = 0; T < 2; ++T) {
+                // vertical pass: s[h][c] = S + 2^15 of row g + 8 (c >> 1), column 8 h + 2 t + (c & 1)
+                int s[2][4];
 #pragma unroll
-                        for (int j = 0; j < 4; ++j) {
-                            const uint32_t sum = 18u * (W[kk % 7][j] + W[(kk + 6) % 7][j]) + 34u * (W[(kk + 1) % 7][j] + W[(kk + 5) % 7][j]) +
-                                                 48u * (W[(kk + 2) % 7][j] + W[(kk + 4) % 7][j]) + 56u * W[(kk + 3) % 7][j];
-                            o |= ((sum + 32768u) >> 16) << (8 * j);
-                        }
-                        *reinterpret_cast<uint32_t*>(out) = o;
-                        out += bpitch;
-                    }
+                for (int h = 0; h < 2; ++h) {
+                    const uint32_t qa = hq[2 * T][h], qb = hq[2 * T + 1][h], qc = hq[2 * T + 2][h];
+                    int lo[4] = {32768, 32768, 32768, 32768}, hi[4] = {0, 0, 0, 0};
+                    imma_16832_u8(lo, av, prmt(qa, qb, 0x5410u), qc);          // qc's upper half sits in zero-weight slots
+                    imma_16832_u8(hi, av, prmt(qa, qb, 0x7632u), qc >> 16);
+#pragma unroll
+                    for (int c = 0; c < 4; ++c) s[h][c] = lo[c] + (hi[c] << 8);
+                }
+                // w[r] = output bytes of row g + 8 r, columns 8 h + 2 t + {0, 1} for h = 0, 1
+                uint32_t w[2];
+#pragma unroll
+                for (int r = 0; r < 2; ++r)
+                    w[r] = prmt(prmt(s[0][2 * r], s[0][2 * r + 1], 0x62u), prmt(s[1][2 * r], s[1][2 * r + 1], 0x62u), 0x5410u);
+                const uint32_t rx = __shfl_xor_sync(0xffffffffu, a ? w[0] : w[1], 1);
+                const uint32_t keep = a ? w[1] : w[0];
+                // row g + 8 a, columns 8 h + 4 hb .. + 3
+                const uint32_t kh0 = prmt(keep, rx, sel0), kh1 = prmt(keep, rx, sel1);
+                const uint32_t ry = __shfl_xor_sync(0xffffffffu, hb ? kh0 : kh1, 2);
+                const uint32_t kk = hb ? kh1 : kh0;
+                *reinterpret_cast<uint2*>(stage + (16 * T + g + 8 * a) * kBlurBoxW + 16 * j + 8 * hb) = hb ? make_uint2(ry, kk) : make_uint2(kk, ry);
+            }
+        }
+        __syncwarp();
+        {
+            // the band leaves: lane = (row quarter, 16-byte column); the blurred level's pitch is a multiple of 16, so the last
+            // vector of a row may spill into padding
+            const int rows = min(32, lg.h - y0);
+            const int cx = 16 * (lane & 7);
+            uint8_t* out = ws.blur + lg.blur_off + (size_t)frame * lg.blur_frame_stride + (size_t)y0 * lg.bpitch + x0 + cx;
+            if (x0 + cx < lg.w) {
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    const int r = 4 * i + (lane >> 3);
+                    if (r < rows) *reinterpret_cast<uint4*>(out + (size_t)r * lg.bpitch) = *reinterpret_cast<const uint4*>(stage + r * kBlurBoxW + cx);
                 }
             }
         }
         __syncwarp();                                               // every lane is done reading the stage
-        if (lane == 0 && item + kBpStages * nw < total_items) issue(item + kBpStages * nw, sgi);
+        if (lane == 0 && item + nw < total_items) issue(item + nw);
     }
 }
 
@@ -583,27 +636,26 @@ __global__ void __launch_bounds__(T) pack_kernel(const __grid_constant__ FrameGe
 
 cudaError_t launch_blur(const FrameGeom& fg, const Workspace& ws, int n_frames, cudaStream_t st)
 {
-    // the TMA-pipelined kernel for batches, the tiled kernel (more parallel units) for a few frames, the register-streaming
-    // kernel when no tensor maps are available or a batch has too many items for the pipelined kernel
+    // the tensor-core kernel for batches, the tiled kernel (more parallel units) for a few frames, the register-streaming
+    // kernel when no tensor maps are available or a batch has too many items for the persistent kernel
     if (ws.tmap_blur && n_frames >= 8) {
         int ipf = 0;
         for (int l = 0; l < fg.nlevels; ++l) ipf += ((fg.L[l].w + 127) / 128) * ((fg.L[l].h + 31) / 32);
         const long long total = (long long)ipf * n_frames;
         if (total > 0 && total < (1LL << 31)) {
-            static int n_sm_dev[64] = {0};               // per device (a process may drive several GPUs)
-            const int smem = kBpWarps * kBpStages * kBpStageBytes;
+            static int resident_ctas[64] = {0};          // per device (a process may drive several GPUs)
+            const int smem = kBmWarps * kBmStageBytes;
             int dev = 0;
             cudaGetDevice(&dev);
-            if (n_sm_dev[dev & 63] == 0) {
-                int n = 0;
-                cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-                cudaError_t e = cudaFuncSetAttribute(blur_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+            if (resident_ctas[dev & 63] == 0) {
+                int n_sm = 0, per_sm = 0;
+                cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
+                cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, blur_mma_kernel, 32 * kBmWarps, smem);
                 if (e != cudaSuccess) return e;
-                n_sm_dev[dev & 63] = n > 0 ? n : 148;
+                resident_ctas[dev & 63] = std::max(n_sm, 1) * std::max(per_sm, 1);
             }
-            const int n_sm = n_sm_dev[dev & 63];
-            const int ctas = (int)std::min<long long>((total + kBpWarps - 1) / kBpWarps, (long long)n_sm * 9);
-            blur_pipe_kernel<<<ctas, 32 * kBpWarps, smem, st>>>(fg, ws, ipf, (int)total);
+            const int ctas = (int)std::min<long long>((total + kBmWarps - 1) / kBmWarps, (long long)resident_ctas[dev & 63]);
+            blur_mma_kernel<<<ctas, 32 * kBmWarps, smem, st>>>(fg, ws, ipf, (int)total);
             count_launch();
             return cudaGetLastError();
         }

@@ -208,12 +208,6 @@ constexpr int KI_WARPS = 8, KI_QTILE = KI_WARPS * 32, KI_DT = 128;
 #endif
 constexpr int kKiUnroll = ORBX_KI_UNROLL;
 
-__device__ __forceinline__ void imma_16832_u8(int (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1)
-{
-    asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.u8.u8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
 __global__ void __launch_bounds__(32 * KI_WARPS, 2) knn2_imma_kernel(const uint32_t* __restrict__ q, int nq, const uint4* __restrict__ db,
                                                                     long long ndb, int index_base, long long rows_per_chunk,
                                                                     int32_t* __restrict__ out_idx, int32_t* __restrict__ out_dist)

@@ -20,6 +20,10 @@ constexpr int kHalfPatch = 15;
 // window of a blurred level staged per keypoint for rBRIEF: |dx|, |dy| <= 19, + 15 bytes of alignment; a row pitch of 80 bytes spreads
 // the rows over 8 shared-memory bank offsets (64 bytes: 2)
 constexpr int kDescBoxW = 80, kDescBoxH = 40;
+// box of the blur's tensor maps over a bordered level: 128 output columns + 16-byte aligned halo (columns x0 - 16 .. x0 + 159) by
+// 32 output rows + 3 above + 5 below (blur_mma_kernel works in 8-row blocks); a pitch of 176 bytes (44 words, 12 mod 32) puts the
+// 32-bit loads of 8 rows x 4 consecutive words on distinct banks
+constexpr int kBlurBoxW = 176, kBlurBoxH = 40;
 
 // Geometry of one pyramid level for the current image shape (host-computed, passed to kernels by value).
 struct LevelGeom {
@@ -126,6 +130,14 @@ __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* m
     asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
                  ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(map), "r"(x), "r"(y), "r"(z),
                  "r"((uint32_t)__cvta_generic_to_shared(bar)) : "memory");
+}
+// c += A . B, int8 MMA m16n8k32 (u8 x u8 -> s32; SASS IMMA.16832.U8.U8).  PTX fragment layout, g = lane / 4, t = lane % 4:
+// a[q] = A row g + 8 (q & 1), k = 16 (q >> 1) + 4 t + byte;  b0 / b1 = B k = 4 t + byte / + 16, n = g;
+// c0, c1 = C row g, n = 2 t, 2 t + 1;  c2, c3 = row g + 8.
+__device__ __forceinline__ void imma_16832_u8(int (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1)
+{
+    asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.u8.u8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+                 : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
 #endif
 
