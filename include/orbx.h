@@ -164,7 +164,8 @@ int orbx_descriptor_distance(const uint8_t* a, const uint8_t* b);
 
 /* Brute-force 2-NN (cv::BFMatcher(NORM_HAMMING).knnMatch(k=2), src/Frame.cc:45,1174; identical (d1,i1,d2) to the
  * strict-'<' best/second scan of src/ORBmatcher1.cc:283-300 and src/ORBmatcher2.cc:84-118 over the whole set).
- * HOST buffers; idx/dist are [nq][2], ascending distance, ties -> lower database index; missing = (-1, INT32_MAX). */
+ * HOST buffers; idx/dist are [nq][2], ascending distance, ties -> lower database index; missing = (-1, INT32_MAX).  Uses the
+ * tracking thread's device scratch; the database is copied straight from `database` (it is not staged in pinned memory). */
 int orbx_knn2(int device, const uint8_t* queries, int nq, const uint8_t* database, int64_t ndb, int32_t* idx,
               int32_t* dist);
 /* Device-resident variant on `stream`; database rows are numbered index_base + row (for sharded databases).  Re-entrant:
@@ -219,7 +220,8 @@ int orbx_distinctive_descriptor(const uint8_t* descriptors, int n, int* best_idx
 /* The same for MANY map points in one call, on the GPU (one warp per map point): the observations of point p are the
  * descriptors [offsets[p], offsets[p + 1]) of `descriptors` (HOST, rows of 32 bytes; offsets[0] == 0).  best_idx[p] = index
  * INSIDE the point's own list, -1 for a point without observations.  What LocalMapping does point by point after every key
- * frame (src/LocalMapping.cc -> MapPoint::ComputeDistinctiveDescriptors, src/MapPoint.cc:329-401). */
+ * frame (src/LocalMapping.cc -> MapPoint::ComputeDistinctiveDescriptors, src/MapPoint.cc:329-401).  Uses local mapping's
+ * device scratch. */
 int orbx_distinctive_descriptors(int device, const uint8_t* descriptors, const int32_t* offsets, int n_points, int32_t* best_idx);
 
 /* ---- the on-disk form of descriptors and key points (SURVEY.md §8(f)4) --------------------------------------------------
@@ -238,7 +240,8 @@ int64_t orbx_deserialize_keypoints(int text, const uint8_t* src, size_t src_len,
 /* void Frame::ComputeStereoMatches() — src/Frame.cc:841-1011.  Uses the un-blurred pyramids of frame `frameL` /
  * `frameR` of the LAST calls on exL / exR (which must live on the same device; they may be the same handle) and
  * HOST keypoints/descriptors as returned by orbx_extract.  bf = mbf; maxD = mbf/mb is explicit because the
- * reference reads mb before it is assigned (src/Frame.cc:143 vs 176).  Outputs mvuRight / mvDepth (-1 = no match). */
+ * reference reads mb before it is assigned (src/Frame.cc:143 vs 176).  Outputs mvuRight / mvDepth (-1 = no match).  Uses the
+ * tracking thread's device scratch. */
 int orbx_stereo_match(orbx_extractor* exL, int frameL, orbx_extractor* exR, int frameR, const orbx_keypoint* kpL,
                       const uint8_t* descL, int nL, const orbx_keypoint* kpR, const uint8_t* descR, int nR, float bf,
                       float maxD, float* uRight, float* depth);
@@ -253,7 +256,9 @@ int orbx_stereo_match_device(orbx_extractor* exL, int frameL, orbx_extractor* ex
 /* The stereo Frame constructor in one call — src/Frame.cc:124-143: ExtractORB(0, imLeft) and ExtractORB(1, imRight) (two
  * std::threads in the reference, two CUDA streams here, vLappingArea = {0, 0}) followed by ComputeStereoMatches().  HOST images
  * in; HOST keypoints / descriptors of both sides (capacity rows each, *nL / *nR valid), mvuRight / mvDepth [capacity] out.
- * The matcher reads keypoints, descriptors and pyramids where the extractors left them on the device. */
+ * The matcher reads keypoints, descriptors and pyramids where the extractors left them on the device; its outputs and scratch
+ * are exL's stereo staging (that of orbx_extract_stereo_batch).  Every argument is checked before any work is queued:
+ * capacity >= 2^20 returns ORBX_ERR_UNSUPPORTED with the outputs untouched. */
 int orbx_extract_stereo(orbx_extractor* exL, orbx_extractor* exR, const uint8_t* imageL, const uint8_t* imageR, int rows, int cols,
                         size_t step, orbx_keypoint* kpL, uint8_t* descL, int* nL, orbx_keypoint* kpR, uint8_t* descR, int* nR,
                         int capacity, float bf, float maxD, float* uRight, float* depth);
@@ -306,7 +311,8 @@ int orbx_vocab_info(const orbx_vocabulary* voc, int* n_nodes, int* n_words, int*
 
 /* transform(feature, word_id, weight, &nid, levelsup) for every feature (TemplatedVocabulary.h:1217-1259): greedy descent,
  * the child with the least Hamming distance wins, ties -> the first child; node_id = the node met at level L - levelsup
- * (0 = root when L - levelsup <= 0).  HOST arrays of n entries; any output may be NULL.  Runs on the GPU. */
+ * (0 = root when L - levelsup <= 0).  HOST arrays of n entries; any output may be NULL.  Runs on the GPU, in the tracking
+ * thread's device scratch (Frame::ComputeBoW). */
 int orbx_bow_transform(const orbx_vocabulary* voc, const uint8_t* descriptors, int n, int levelsup, uint32_t* word_id,
                        double* weight, uint32_t* node_id);
 /* Frame::ComputeBoW / KeyFrame::ComputeBoW (src/Frame.cc:768-775): transform(features, BowVector, FeatureVector, levelsup)
@@ -340,7 +346,8 @@ typedef struct orbx_feature_vector {
  * sequential dependence is honoured (one warp walks a node's A-list in order; lanes scan the B-list).
  * Outputs: mode 0: match_b[nB] = index of the A feature whose map point was assigned to B's feature j (vpMapPointMatches),
  *          mode 1: match_a[nA] = index of the B feature matched to A's feature i (vpMatches12), -1 = none; the other array
- *          (may be NULL) receives the inverse map.  *n_matches = the reference's return value (after the rotation filter). */
+ *          (may be NULL) receives the inverse map.  *n_matches = the reference's return value (after the rotation filter).
+ * Mode 0 uses the tracking thread's device scratch, mode 1 the loop-closing thread's. */
 int orbx_search_by_bow(int device, int mode, const uint8_t* desc_a, const float* angle_a, const uint8_t* valid_a, int n_a,
                        const orbx_feature_vector* fv_a, const uint8_t* desc_b, const float* angle_b, const uint8_t* valid_b,
                        int n_b, const orbx_feature_vector* fv_b, int nleft_b, float nn_ratio, int check_orientation,
@@ -357,7 +364,8 @@ int orbx_search_by_bow(int device, int mode, const uint8_t* desc_a, const float*
  *   F12[9]           = row-major K1^-T [t12]x R12 K2^-1 computed by the caller exactly as Pinhole.cpp:109-112 does
  *   ep[2]            = projection of KF1's camera centre into KF2 (:186-189); scale_b / sigma2_b = mvScaleFactors and mvLevelSigma2
  *                      of KF2, n_levels entries (Pinhole::epipolarConstrain ignores its sigmaLevel argument, KF1's sigma)
- * Output: match_a[nA] = index in B or -1 (vMatches12 after the rotation filter); *n_matches = the return value. */
+ * Output: match_a[nA] = index in B or -1 (vMatches12 after the rotation filter); *n_matches = the return value.
+ * orbx_search_for_triangulation_batch with this one neighbour: the same checks, results and device scratch. */
 int orbx_search_for_triangulation(int device, const orbx_keypoint* kp_a, const uint8_t* desc_a, const uint8_t* free_a,
                                   const uint8_t* stereo_a, int n_a, const orbx_feature_vector* fv_a, const orbx_keypoint* kp_b,
                                   const uint8_t* desc_b, const uint8_t* free_b, const uint8_t* stereo_b, int n_b,
@@ -501,7 +509,7 @@ typedef struct orbx_keyframe_view {
  * Output: match[nq] = bestIdx when bestDist <= 50, else -1; n_fused[n_kf] = matches per key frame (the reference's return value
  *   when no point changes state during the call).  The bookkeeping (AddMapPoint / Replace) stays with the caller.
  * ORBX_ERR_INVALID_ARG for null arrays, a missing inv_level_sigma2, non-monotone offsets, point[q] outside [0, n_desc) or a level
- * outside [0, n_levels) on a valid pair.  Uses its own device scratch, so it never waits on the tracking thread's searches. */
+ * outside [0, n_levels) on a valid pair.  Uses local mapping's device scratch, so it never waits on the tracking thread's searches. */
 int orbx_fuse(int device, int n_kf, const orbx_keyframe_view* kfs, const int32_t* kf_offsets, int n_desc, const uint8_t* point_desc,
               const int32_t* point, const uint8_t* valid, const float* u, const float* v, const float* invz, const int32_t* level,
               float th, int32_t* match, int* n_fused);
@@ -547,7 +555,8 @@ int orbx_projection_rounds(void);
 /* void Frame::UndistortKeyPoints() — src/Frame.cc:777-810 = cv::undistortPoints(mvKeys, K, mDistCoef, cv::Mat(), mK).
  *   K[4] / new_K[4] = (fx, fy, cx, cy) of Pinhole::toK() and of mK; dist = mDistCoef (CV_32F: k1 k2 p1 p2 [k3 [k4 k5 k6]]),
  *   n_dist in {0, 4, 5, 8, 12}.  dist[0] == 0 (or n_dist == 0) copies the key points, as the reference does (:779-783).
- * HOST arrays; out may alias keypoints.  Computes on the GPU in double, bit-identical to OpenCV's scalar code. */
+ * HOST arrays; out may alias keypoints.  Computes on the GPU in double, bit-identical to OpenCV's scalar code, in the tracking
+ * thread's device scratch. */
 int orbx_undistort_keypoints(int device, const orbx_keypoint* keypoints, int n, const float* K, const float* dist, int n_dist,
                              const float* new_K, orbx_keypoint* out);
 

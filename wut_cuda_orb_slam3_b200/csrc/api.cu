@@ -222,7 +222,7 @@ int set_device(int device)
     }
     if (device < 0 || device >= n) return fail(ORBX_ERR_INVALID_ARG, "device %d out of range (%d visible)", device, n);
     CU(cudaSetDevice(device));
-    // stream-ordered scratch (cudaMallocAsync in the matcher entry points) should stay in the pool between calls
+    // stream-ordered scratch (cudaMallocAsync in the device-resident matcher entry points) should stay in the pool between calls
     static std::atomic<unsigned long long> pool_ready{0};
     if (device < 64 && !(pool_ready.load(std::memory_order_relaxed) & (1ull << device))) {
         cudaMemPool_t pool = nullptr;
@@ -232,6 +232,37 @@ int set_device(int device)
         }
         cudaGetLastError();
         pool_ready.fetch_or(1ull << device, std::memory_order_relaxed);
+    }
+    return ORBX_OK;
+}
+
+ProjArena g_arena[64];
+ProjArena g_fuse_arena[64];
+ProjArena g_loop_arena[64];
+
+int Lease::reserve(size_t bytes, size_t staged)
+{
+    staged = std::min(staged, bytes) + 8192;
+    bytes += 8192;
+    if (!A.st) {
+        cudaError_t e = cudaStreamCreateWithFlags(&A.st, cudaStreamNonBlocking);
+        if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
+    }
+    if (A.d_bytes < bytes) {
+        if (A.d) cudaFree(A.d);
+        A.d = nullptr; A.d_bytes = 0;
+        const size_t want = bytes + bytes / 2;
+        cudaError_t e = cudaMalloc((void**)&A.d, want);
+        if (e != cudaSuccess) return fail(ORBX_ERR_OOM, "scratch (%zu device bytes): %s", want, cudaGetErrorString(e));
+        A.d_bytes = want;
+    }
+    if (A.h_bytes < staged) {
+        if (A.h) cudaFreeHost(A.h);
+        A.h = nullptr; A.h_bytes = 0;
+        const size_t want = staged + staged / 2;
+        cudaError_t e = cudaMallocHost((void**)&A.h, want);
+        if (e != cudaSuccess) return fail(ORBX_ERR_OOM, "staging (%zu pinned bytes): %s", want, cudaGetErrorString(e));
+        A.h_bytes = want;
     }
     return ORBX_OK;
 }
@@ -852,40 +883,6 @@ static int enqueue_single(orbx_extractor* ex, const uint8_t* image, int rows, in
     return ORBX_OK;
 }
 
-// Grow-only device scratch per device for the matcher entry points that take host buffers (orbx_knn2, orbx_stereo_match): a
-// cudaMalloc/cudaFree pair per call costs more than the kernels on frame-sized inputs.  One call at a time per device holds it.
-struct ScratchArena {
-    std::mutex mu;
-    unsigned char* base = nullptr;
-    size_t bytes = 0;
-};
-static ScratchArena g_scratch[64];
-
-struct ScratchLease {
-    ScratchArena& a;
-    std::unique_lock<std::mutex> lock;
-    size_t off = 0;
-    explicit ScratchLease(int device) : a(g_scratch[device & 63]), lock(a.mu) {}
-    int reserve(size_t total)
-    {
-        total += 4096;
-        if (a.bytes >= total) return ORBX_OK;
-        if (a.base) cudaFree(a.base);
-        a.base = nullptr; a.bytes = 0;
-        cudaError_t e = cudaMalloc(&a.base, total);
-        if (e != cudaSuccess) return fail(ORBX_ERR_OOM, "cudaMalloc(%zu): %s", total, cudaGetErrorString(e));
-        a.bytes = total;
-        return ORBX_OK;
-    }
-    template <typename T> T* take(size_t count)
-    {
-        off = (off + 255) & ~(size_t)255;
-        T* p = reinterpret_cast<T*>(a.base + off);
-        off += std::max<size_t>(count, 1) * sizeof(T);
-        return p;
-    }
-};
-
 }  // namespace orbx
 
 // =====================================================================================================================
@@ -1435,7 +1432,7 @@ int orbx_distribute_octree(int device, const int* xs, const int* ys, const int* 
     cudaMemcpy(ws.cand, packed.data(), sizeof(uint32_t) * packed.size(), cudaMemcpyHostToDevice);
     cudaMemcpy(ws.cell_count, &one, sizeof(int), cudaMemcpyHostToDevice);
     cudaError_t e = launch_octree(fg, ws, 1, 0);
-    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    if (e == cudaSuccess) e = cudaStreamSynchronize(0);
     if (e != cudaSuccess) { cleanup(); return fail(ORBX_ERR_CUDA, "octree kernel: %s", cudaGetErrorString(e)); }
     if (octree_take_error_flag()) { cleanup(); return fail(ORBX_ERR_INVALID_ARG, "quadtree depth exhausted (candidates not separable)"); }
     int m = 0;
@@ -1491,19 +1488,24 @@ int orbx_knn2(int device, const uint8_t* queries, int nq, const uint8_t* databas
     if (nq == 0) return ORBX_OK;
     int rc = set_device(device);
     if (rc) return rc;
-    ScratchLease L(device);
-    const size_t ws_bytes = knn2_workspace_bytes(nq, ndb);
-    if ((rc = L.reserve((size_t)nq * 32 + (size_t)std::max<int64_t>(ndb, 1) * 32 + (size_t)nq * 16 + ws_bytes + 5 * 256))) return rc;
-    uint8_t* dq = L.take<uint8_t>((size_t)nq * 32);
-    uint8_t* ddb = L.take<uint8_t>((size_t)std::max<int64_t>(ndb, 1) * 32);
-    int32_t* di = L.take<int32_t>((size_t)nq * 2);
-    int32_t* dd = L.take<int32_t>((size_t)nq * 2);
-    void* dws = ws_bytes ? (void*)L.take<uint8_t>(ws_bytes) : nullptr;
-    cudaError_t e = cudaMemcpy(dq, queries, (size_t)nq * 32, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && ndb > 0) e = cudaMemcpy(ddb, database, (size_t)ndb * 32, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = launch_knn2(dq, nq, ddb, ndb, 0, di, dd, 0, dws);
-    if (e == cudaSuccess) e = cudaMemcpy(idx, di, (size_t)nq * 8, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaMemcpy(dist, dd, (size_t)nq * 8, cudaMemcpyDeviceToHost);
+    Lease L(device);
+    const size_t ws_bytes = knn2_workspace_bytes(nq, ndb), db_bytes = (size_t)std::max<int64_t>(ndb, 1) * 32;
+    // the queries are staged; the database (up to hundreds of MB) is copied straight from the caller into the device-only tail
+    const size_t staged = lease_pad((size_t)nq * 32);
+    if ((rc = L.reserve(staged + lease_pad(db_bytes) + 2 * lease_pad((size_t)nq * 8) + lease_pad(ws_bytes), staged))) return rc;
+    const size_t o_q = L.take<uint8_t>((size_t)nq * 32);
+    L.upload_end = L.off;
+    const size_t o_db = L.take<uint8_t>(db_bytes), o_i = L.take<int32_t>((size_t)nq * 2), o_d = L.take<int32_t>((size_t)nq * 2),
+                 o_ws = L.take<uint8_t>(ws_bytes);
+    memcpy(L.host<uint8_t>(o_q), queries, (size_t)nq * 32);
+    cudaStream_t st = L.A.st;
+    cudaError_t e = cudaMemcpyAsync(L.A.d, L.A.h, L.upload_end, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess && ndb > 0) e = cudaMemcpyAsync(L.dev<uint8_t>(o_db), database, (size_t)ndb * 32, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess)
+        e = launch_knn2(L.dev<uint8_t>(o_q), nq, L.dev<uint8_t>(o_db), ndb, 0, L.dev<int32_t>(o_i), L.dev<int32_t>(o_d), st, L.dev<uint8_t>(o_ws));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(idx, L.dev<int32_t>(o_i), (size_t)nq * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dist, L.dev<int32_t>(o_d), (size_t)nq * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "knn2: %s", cudaGetErrorString(e));
     return ORBX_OK;
 }
@@ -1595,24 +1597,30 @@ int orbx_stereo_match(orbx_extractor* exL, int frameL, orbx_extractor* exR, int 
         if (kpL[i].octave < 0 || kpL[i].octave >= exL->nlevels) return fail(ORBX_ERR_INVALID_ARG, "left keypoint %d octave", i);
     for (int i = 0; i < nR; ++i)
         if (kpR[i].octave < 0 || kpR[i].octave >= exL->nlevels) return fail(ORBX_ERR_INVALID_ARG, "right keypoint %d octave", i);
-    ScratchLease Ls(exL->device);
-    const size_t nRa = (size_t)std::max(nR, 1);
-    if ((rc = Ls.reserve(((size_t)nL + nRa) * (sizeof(orbx_keypoint) + 32) + (size_t)nL * 12 + 8 * 256))) return rc;
-    orbx_keypoint* dkL = Ls.take<orbx_keypoint>((size_t)nL);
-    uint8_t* ddL = Ls.take<uint8_t>((size_t)nL * 32);
-    orbx_keypoint* dkR = Ls.take<orbx_keypoint>(nRa);
-    uint8_t* ddR = Ls.take<uint8_t>(nRa * 32);
-    A.uRight = Ls.take<float>((size_t)nL); A.depth = Ls.take<float>((size_t)nL); A.sad = Ls.take<int>((size_t)nL);
-    cudaStream_t st = exL->slots[0].stream;          // idle: orbx_sync above
-    cudaError_t e = cudaMemcpyAsync(dkL, kpL, sizeof(orbx_keypoint) * nL, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(ddL, descL, (size_t)nL * 32, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess && nR > 0) e = cudaMemcpyAsync(dkR, kpR, sizeof(orbx_keypoint) * nR, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess && nR > 0) e = cudaMemcpyAsync(ddR, descR, (size_t)nR * 32, cudaMemcpyHostToDevice, st);
-    A.kpL = dkL; A.descL = ddL; A.nL = nL; A.kpR = dkR; A.descR = ddR; A.nR = nR; A.bf = bf; A.maxD = maxD;
+    Lease L(exL->device);          // the pyramids are complete: orbx_sync above
+    const size_t kb = sizeof(orbx_keypoint);
+    if ((rc = L.reserve(lease_pad((size_t)nL * kb) + lease_pad((size_t)nL * 32) + lease_pad((size_t)nR * kb) + lease_pad((size_t)nR * 32) +
+                        3 * lease_pad((size_t)nL * 4))))
+        return rc;
+    const size_t o_kL = L.take<orbx_keypoint>(nL), o_dL = L.take<uint8_t>((size_t)nL * 32), o_kR = L.take<orbx_keypoint>(nR),
+                 o_dR = L.take<uint8_t>((size_t)nR * 32);
+    L.upload_end = L.off;
+    const size_t o_u = L.take<float>(nL), o_depth = L.take<float>(nL), o_sad = L.take<int>(nL);
+    memcpy(L.host<orbx_keypoint>(o_kL), kpL, (size_t)nL * kb);
+    memcpy(L.host<uint8_t>(o_dL), descL, (size_t)nL * 32);
+    if (nR > 0) {
+        memcpy(L.host<orbx_keypoint>(o_kR), kpR, (size_t)nR * kb);
+        memcpy(L.host<uint8_t>(o_dR), descR, (size_t)nR * 32);
+    }
+    A.kpL = L.dev<orbx_keypoint>(o_kL); A.descL = L.dev<uint8_t>(o_dL); A.nL = nL;
+    A.kpR = L.dev<orbx_keypoint>(o_kR); A.descR = L.dev<uint8_t>(o_dR); A.nR = nR; A.bf = bf; A.maxD = maxD;
+    A.uRight = L.dev<float>(o_u); A.depth = L.dev<float>(o_depth); A.sad = L.dev<int>(o_sad);
+    cudaStream_t st = L.A.st;
+    cudaError_t e = cudaMemcpyAsync(L.A.d, L.A.h, L.upload_end, cudaMemcpyHostToDevice, st);
     if (e == cudaSuccess) e = launch_stereo(exL->fg, A, st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(uRight, A.uRight, sizeof(float) * nL, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(depth, A.depth, sizeof(float) * nL, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);          // the lease (scratch) is released on return
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "stereo: %s", cudaGetErrorString(e));
     return ORBX_OK;
 }
@@ -1652,13 +1660,23 @@ int orbx_extract_stereo(orbx_extractor* exL, orbx_extractor* exR, const uint8_t*
     if (!imageL || !imageR || rows <= 0 || cols <= 0) return fail(ORBX_ERR_EMPTY_IMAGE, "empty image");
     if (!kpL || !descL || !nL || !kpR || !descR || !nR || !uRight || !depth || capacity <= 0 || step < (size_t)cols)
         return fail(ORBX_ERR_INVALID_ARG, "bad output buffers / step");
-    if (exL->device != exR->device) return fail(ORBX_ERR_INVALID_ARG, "left/right extractors must share a device");
+    if (exL->device != exR->device || exL->nlevels != exR->nlevels || exL->scaleFactorF != exR->scaleFactorF)
+        return fail(ORBX_ERR_INVALID_ARG, "left/right extractors must share device, levels and scale factor");
+    if (capacity >= (1 << 20)) return fail(ORBX_ERR_UNSUPPORTED, "capacity %d: the stereo kernels index at most 2^20 - 1 rows", capacity);
     // vLappingArea = {0, 0} for both cameras of a rectified pair (src/Frame.cc:124-125)
     int rc;
     if ((rc = enqueue_single(exL, imageL, rows, cols, step, 0, 0, capacity))) return rc;
     if ((rc = enqueue_single(exR, imageR, rows, cols, step, 0, 0, capacity))) return rc;
     Slot& sL = exL->slots[0];
     Slot& sR = exR->slots[0];
+    // the matcher's outputs and scratch: slot 0's stereo staging (that of orbx_extract_stereo_batch), replaced only while the
+    // slot's stream is idle
+    if (!stereo_staging_fits(sL, 1, capacity)) {
+        CU(cudaStreamSynchronize(sL.stream));
+        if ((rc = ensure_stereo_staging(sL, 1, capacity))) return rc;
+    }
+    StereoArgs A{};
+    if ((rc = stereo_prepare(exL, 0, exR, 0, A))) return rc;          // (cannot fail after the checks above)
     // right side: its results go home on its own stream while the matcher runs
     CU(cudaEventRecord(sR.ev_done, sR.stream));
     CU(cudaMemcpyAsync(kpR, sR.d_kps, sizeof(orbx_keypoint) * (size_t)capacity, cudaMemcpyDeviceToHost, sR.stream));
@@ -1666,22 +1684,15 @@ int orbx_extract_stereo(orbx_extractor* exL, orbx_extractor* exR, const uint8_t*
     CU(cudaMemcpyAsync(nR, sR.d_n, sizeof(int), cudaMemcpyDeviceToHost, sR.stream));
     // left side: wait for the right extraction, match on the device, then copy everything back
     CU(cudaStreamWaitEvent(sL.stream, sR.ev_done, 0));
-    ScratchLease Ls(exL->device);
-    if ((rc = Ls.reserve((size_t)capacity * 12 + 4 * 256))) return rc;
-    float* d_u = Ls.take<float>((size_t)capacity);
-    float* d_d = Ls.take<float>((size_t)capacity);
-    StereoArgs A{};
-    if ((rc = stereo_prepare(exL, 0, exR, 0, A))) return rc;
     A.kpL = sL.d_kps; A.descL = sL.d_desc; A.nL = capacity; A.d_nL = sL.d_n;
     A.kpR = sR.d_kps; A.descR = sR.d_desc; A.nR = capacity; A.d_nR = sR.d_n;
-    A.bf = bf; A.maxD = maxD; A.uRight = d_u; A.depth = d_d; A.sad = Ls.take<int>((size_t)capacity);
-    if (capacity >= (1 << 20)) return fail(ORBX_ERR_UNSUPPORTED, "too many right keypoints");
+    A.bf = bf; A.maxD = maxD; A.uRight = sL.d_su; A.depth = sL.d_sd; A.sad = sL.d_sad;
     CU(launch_stereo(exL->fg, A, sL.stream));
     CU(cudaMemcpyAsync(kpL, sL.d_kps, sizeof(orbx_keypoint) * (size_t)capacity, cudaMemcpyDeviceToHost, sL.stream));
     CU(cudaMemcpyAsync(descL, sL.d_desc, (size_t)capacity * 32, cudaMemcpyDeviceToHost, sL.stream));
     CU(cudaMemcpyAsync(nL, sL.d_n, sizeof(int), cudaMemcpyDeviceToHost, sL.stream));
-    CU(cudaMemcpyAsync(uRight, d_u, sizeof(float) * (size_t)capacity, cudaMemcpyDeviceToHost, sL.stream));
-    CU(cudaMemcpyAsync(depth, d_d, sizeof(float) * (size_t)capacity, cudaMemcpyDeviceToHost, sL.stream));
+    CU(cudaMemcpyAsync(uRight, sL.d_su, sizeof(float) * (size_t)capacity, cudaMemcpyDeviceToHost, sL.stream));
+    CU(cudaMemcpyAsync(depth, sL.d_sd, sizeof(float) * (size_t)capacity, cudaMemcpyDeviceToHost, sL.stream));
     CU(cudaStreamSynchronize(sL.stream));
     CU(cudaStreamSynchronize(sR.stream));
     if (*nL > capacity || *nR > capacity) return fail(ORBX_ERR_CAPACITY, "%d / %d keypoints, capacity %d", *nL, *nR, capacity);

@@ -36,32 +36,6 @@ namespace orbx {
 
 namespace {
 
-struct DevBuf {                      // RAII bag of device allocations for one call
-    std::vector<void*> ptrs;
-    ~DevBuf() { for (void* p : ptrs) cudaFree(p); }
-    template <typename T>
-    int alloc(T** out, size_t count)
-    {
-        void* p = nullptr;
-        cudaError_t e = cudaMalloc(&p, std::max<size_t>(count, 1) * sizeof(T));
-        if (e != cudaSuccess) return fail(ORBX_ERR_OOM, "cudaMalloc(%zu): %s", count * sizeof(T), cudaGetErrorString(e));
-        ptrs.push_back(p);
-        *out = (T*)p;
-        return ORBX_OK;
-    }
-    template <typename T>
-    int upload(T** out, const T* host, size_t count)
-    {
-        int rc = alloc(out, count);
-        if (rc) return rc;
-        if (count) {
-            cudaError_t e = cudaMemcpy(*out, host, count * sizeof(T), cudaMemcpyHostToDevice);
-            if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "cudaMemcpy H2D: %s", cudaGetErrorString(e));
-        }
-        return ORBX_OK;
-    }
-};
-
 int check_fv(const orbx_feature_vector* fv, int n_features, const char* name)
 {
     if (!fv || fv->n_nodes < 0 || (fv->n_nodes > 0 && (!fv->node_ids || !fv->offsets))) return fail(ORBX_ERR_INVALID_ARG, "%s: bad feature vector", name);
@@ -229,16 +203,22 @@ int orbx_bow_transform(const orbx_vocabulary* v, const uint8_t* descriptors, int
     if (v->n_nodes < 2) return fail(ORBX_ERR_INVALID_ARG, "empty vocabulary");
     int rc = set_device(v->device);
     if (rc) return rc;
-    DevBuf B;
-    uint8_t* d_desc; uint32_t *d_word, *d_node; double* d_w;
-    if ((rc = B.upload(&d_desc, descriptors, (size_t)n * 32)) || (rc = B.alloc(&d_word, (size_t)n)) || (rc = B.alloc(&d_node, (size_t)n)) ||
-        (rc = B.alloc(&d_w, (size_t)n)))
-        return rc;
-    cudaError_t e = launch_bow_descend(v->dev, d_desc, n, v->L - levelsup, d_word, d_w, d_node, 0);
-    if (e == cudaSuccess && word_id) e = cudaMemcpy(word_id, d_word, (size_t)n * 4, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess && weight) e = cudaMemcpy(weight, d_w, (size_t)n * 8, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess && node_id) e = cudaMemcpy(node_id, d_node, (size_t)n * 4, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    Lease L(v->device);
+    if ((rc = L.reserve(lease_pad((size_t)n * 32) + 2 * lease_pad((size_t)n * 4) + lease_pad((size_t)n * 8)))) return rc;
+    const size_t o_desc = L.take<uint8_t>((size_t)n * 32);
+    L.upload_end = L.off;
+    const size_t o_word = L.take<uint32_t>(n), o_node = L.take<uint32_t>(n), o_w = L.take<double>(n);
+    memcpy(L.host<uint8_t>(o_desc), descriptors, (size_t)n * 32);
+    cudaStream_t st = L.A.st;
+    uint32_t* d_word = L.dev<uint32_t>(o_word);
+    uint32_t* d_node = L.dev<uint32_t>(o_node);
+    double* d_w = L.dev<double>(o_w);
+    cudaError_t e = cudaMemcpyAsync(L.A.d, L.A.h, L.upload_end, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = launch_bow_descend(v->dev, L.dev<uint8_t>(o_desc), n, v->L - levelsup, d_word, d_w, d_node, st);
+    if (e == cudaSuccess && word_id) e = cudaMemcpyAsync(word_id, d_word, (size_t)n * 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess && weight) e = cudaMemcpyAsync(weight, d_w, (size_t)n * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess && node_id) e = cudaMemcpyAsync(node_id, d_node, (size_t)n * 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "bow_transform: %s", cudaGetErrorString(e));
     return ORBX_OK;
 }
@@ -326,22 +306,39 @@ int orbx_search_by_bow(int device, int mode, const uint8_t* desc_a, const float*
         std::vector<int4> pairs;
         for (auto& c : common)
             pairs.push_back(make_int4(fv_a->offsets[c.first], fv_a->offsets[c.first + 1], fv_b->offsets[c.second], fv_b->offsets[c.second + 1]));
-        DevBuf B;
-        BowSearchArgs A{};
-        int4* d_pairs; uint32_t *d_ia, *d_ib; uint8_t *d_da, *d_db, *d_va, *d_vb = nullptr; int *d_mb, *d_ma, *d_mar;
-        if ((rc = B.upload(&d_pairs, pairs.data(), pairs.size())) || (rc = B.upload(&d_ia, fv_a->indices, (size_t)fv_a->offsets[fv_a->n_nodes])) ||
-            (rc = B.upload(&d_ib, fv_b->indices, (size_t)fv_b->offsets[fv_b->n_nodes])) || (rc = B.upload(&d_da, desc_a, (size_t)n_a * 32)) ||
-            (rc = B.upload(&d_db, desc_b, (size_t)n_b * 32)) || (rc = B.upload(&d_va, valid_a, (size_t)n_a)) ||
-            (mode == 1 && (rc = B.upload(&d_vb, valid_b, (size_t)n_b))) || (rc = B.upload(&d_mb, mB.data(), (size_t)n_b)) ||
-            (rc = B.upload(&d_ma, mA.data(), (size_t)n_a)) || (rc = B.upload(&d_mar, mAR.data(), (size_t)n_a)))
+        // KF -> Frame runs on the tracking thread, KF <-> KF on loop closing
+        Lease L(device, mode == 0 ? g_arena : g_loop_arena);
+        const size_t ia = (size_t)fv_a->offsets[fv_a->n_nodes], ib = (size_t)fv_b->offsets[fv_b->n_nodes], vb = mode == 1 ? (size_t)n_b : 0;
+        if ((rc = L.reserve(lease_pad(pairs.size() * 16) + lease_pad(ia * 4) + lease_pad(ib * 4) + lease_pad((size_t)n_a * 32) +
+                            lease_pad((size_t)n_b * 32) + lease_pad((size_t)n_a) + lease_pad(vb) + lease_pad((size_t)n_b * 4) +
+                            2 * lease_pad((size_t)n_a * 4))))
             return rc;
-        A.mode = mode; A.n_pairs = (int)pairs.size(); A.pairs = d_pairs; A.idx_a = d_ia; A.idx_b = d_ib; A.desc_a = d_da; A.desc_b = d_db;
-        A.valid_a = d_va; A.valid_b = d_vb; A.nleft_b = nleft_b; A.nn_ratio = nn_ratio; A.match_b = d_mb; A.match_a = d_ma; A.match_a_right = d_mar;
-        cudaError_t e = launch_search_by_bow(A, 0);
-        if (e == cudaSuccess) e = cudaMemcpy(mB.data(), d_mb, (size_t)n_b * 4, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(mA.data(), d_ma, (size_t)n_a * 4, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(mAR.data(), d_mar, (size_t)n_a * 4, cudaMemcpyDeviceToHost);
+        // upload range; the three match arrays (initialised to -1) come back in one copy
+        const size_t o_pairs = L.take<int4>(pairs.size()), o_ia = L.take<uint32_t>(ia), o_ib = L.take<uint32_t>(ib),
+                     o_da = L.take<uint8_t>((size_t)n_a * 32), o_db = L.take<uint8_t>((size_t)n_b * 32), o_va = L.take<uint8_t>(n_a),
+                     o_vb = L.take<uint8_t>(vb), o_mb = L.take<int>(n_b), o_ma = L.take<int>(n_a), o_mar = L.take<int>(n_a);
+        L.upload_end = L.off;
+        memcpy(L.host<int4>(o_pairs), pairs.data(), pairs.size() * 16);
+        memcpy(L.host<uint32_t>(o_ia), fv_a->indices, ia * 4);
+        memcpy(L.host<uint32_t>(o_ib), fv_b->indices, ib * 4);
+        memcpy(L.host<uint8_t>(o_da), desc_a, (size_t)n_a * 32);
+        memcpy(L.host<uint8_t>(o_db), desc_b, (size_t)n_b * 32);
+        memcpy(L.host<uint8_t>(o_va), valid_a, (size_t)n_a);
+        if (vb) memcpy(L.host<uint8_t>(o_vb), valid_b, vb);
+        memset(L.host<uint8_t>(o_mb), 0xff, L.upload_end - o_mb);
+        BowSearchArgs A{};
+        A.mode = mode; A.n_pairs = (int)pairs.size(); A.pairs = L.dev<int4>(o_pairs); A.idx_a = L.dev<uint32_t>(o_ia); A.idx_b = L.dev<uint32_t>(o_ib);
+        A.desc_a = L.dev<uint8_t>(o_da); A.desc_b = L.dev<uint8_t>(o_db); A.valid_a = L.dev<uint8_t>(o_va); A.valid_b = vb ? L.dev<uint8_t>(o_vb) : nullptr;
+        A.nleft_b = nleft_b; A.nn_ratio = nn_ratio; A.match_b = L.dev<int>(o_mb); A.match_a = L.dev<int>(o_ma); A.match_a_right = L.dev<int>(o_mar);
+        cudaStream_t st = L.A.st;
+        cudaError_t e = cudaMemcpyAsync(L.A.d, L.A.h, L.upload_end, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) e = launch_search_by_bow(A, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(L.host<int>(o_mb), A.match_b, L.upload_end - o_mb, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
         if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "search_by_bow: %s", cudaGetErrorString(e));
+        memcpy(mB.data(), L.host<int>(o_mb), (size_t)n_b * 4);
+        memcpy(mA.data(), L.host<int>(o_ma), (size_t)n_a * 4);
+        memcpy(mAR.data(), L.host<int>(o_mar), (size_t)n_a * 4);
     }
     // rotation histogram + ComputeThreeMaxima (src/ORBmatcher1.cc:344-356, 406-427; src/ORBmatcher2.cc:127-139, 152-169).
     // One histogram entry per accepted match; the filter depends on bin sizes only, so the entry order is irrelevant.
@@ -381,49 +378,15 @@ int orbx_search_for_triangulation(int device, const orbx_keypoint* kp_a, const u
                                   const float* sigma2_b, int n_levels, int only_stereo, int coarse, int check_orientation,
                                   int32_t* match_a, int* n_matches)
 {
-    if (n_a < 0 || n_b < 0 || !n_matches || !F12 || !ep || !scale_b || !sigma2_b || n_levels < 1 || n_levels > kMaxLevels ||
-        (n_a > 0 && (!kp_a || !desc_a || !free_a || !stereo_a || !match_a)) || (n_b > 0 && (!kp_b || !desc_b || !free_b || !stereo_b)))
-        return fail(ORBX_ERR_INVALID_ARG, "bad arguments");
-    int rc;
-    if ((rc = check_fv(fv_a, n_a, "fv_a")) || (rc = check_fv(fv_b, n_b, "fv_b"))) return rc;
-    for (int j = 0; j < n_b; ++j)
-        if (kp_b[j].octave < 0 || kp_b[j].octave >= n_levels) return fail(ORBX_ERR_INVALID_ARG, "kp_b[%d].octave out of range", j);
+    // the one-neighbour batch; these are the arguments the view cannot carry (the batch checks the rest)
+    if (!n_matches || !F12 || !ep || !fv_b) return fail(ORBX_ERR_INVALID_ARG, "bad arguments");
+    orbx_triangulation_view V{};
+    V.n = n_b; V.kp = kp_b; V.desc = desc_b; V.free = free_b; V.stereo = stereo_b; V.fv = *fv_b;
+    memcpy(V.F12, F12, sizeof V.F12); memcpy(V.ep, ep, sizeof V.ep);
+    V.scale = scale_b; V.sigma2 = sigma2_b; V.n_levels = n_levels; V.coarse = coarse;
     *n_matches = 0;
-    std::vector<int32_t> mA(n_a, -1);
-    std::vector<std::pair<int, int>> common;
-    common_nodes(fv_a, fv_b, common);
-    std::vector<int4> jobs;
-    for (auto& c : common)
-        for (int t = fv_a->offsets[c.first]; t < fv_a->offsets[c.first + 1]; ++t) {
-            const int iA = (int)fv_a->indices[t];
-            if (!free_a[iA]) continue;                                   // already has a MapPoint (src/ORBmatcher2.cc:246-252)
-            if (only_stereo && !stereo_a[iA]) continue;                  // :256-258
-            jobs.push_back(make_int4(iA, fv_b->offsets[c.second], fv_b->offsets[c.second + 1], 0));
-        }
-    if (!jobs.empty() && n_b > 0) {
-        if ((rc = set_device(device))) return rc;
-        DevBuf B;
-        TriSearchArgs A{};
-        int4* d_jobs; uint32_t* d_ib; orbx_keypoint *d_ka, *d_kb; uint8_t *d_da, *d_db, *d_sa, *d_sb, *d_fb; int* d_ma;
-        if ((rc = B.upload(&d_jobs, jobs.data(), jobs.size())) || (rc = B.upload(&d_ib, fv_b->indices, (size_t)fv_b->offsets[fv_b->n_nodes])) ||
-            (rc = B.upload(&d_ka, kp_a, (size_t)n_a)) || (rc = B.upload(&d_kb, kp_b, (size_t)n_b)) || (rc = B.upload(&d_da, desc_a, (size_t)n_a * 32)) ||
-            (rc = B.upload(&d_db, desc_b, (size_t)n_b * 32)) || (rc = B.upload(&d_sa, stereo_a, (size_t)n_a)) || (rc = B.upload(&d_sb, stereo_b, (size_t)n_b)) ||
-            (rc = B.upload(&d_fb, free_b, (size_t)n_b)) || (rc = B.upload(&d_ma, mA.data(), (size_t)n_a)))
-            return rc;
-        A.n_jobs = (int)jobs.size(); A.jobs = d_jobs; A.idx_b = d_ib; A.kp_a = d_ka; A.kp_b = d_kb; A.desc_a = d_da; A.desc_b = d_db;
-        A.stereo_a = d_sa; A.stereo_b = d_sb; A.free_b = d_fb; A.only_stereo = only_stereo; A.coarse = coarse; A.match_a = d_ma;
-        memcpy(A.F12, F12, sizeof A.F12); memcpy(A.ep, ep, sizeof A.ep);
-        for (int l = 0; l < n_levels; ++l) { A.scale_b[l] = scale_b[l]; A.sigma2_b[l] = sigma2_b[l]; }
-        cudaError_t e = launch_search_triangulation(A, 0);
-        if (e == cudaSuccess) e = cudaMemcpy(mA.data(), d_ma, (size_t)n_a * 4, cudaMemcpyDeviceToHost);
-        if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "search_for_triangulation: %s", cudaGetErrorString(e));
-    }
-    int nm = 0;
-    for (int i = 0; i < n_a; ++i) nm += mA[i] >= 0;
-    if (check_orientation && (rc = tri_rotation_filter(kp_a, kp_b, n_a, mA.data(), &nm))) return rc;
-    for (int i = 0; i < n_a; ++i) match_a[i] = mA[i];
-    *n_matches = nm;
-    return ORBX_OK;
+    return orbx_search_for_triangulation_batch(device, kp_a, desc_a, free_a, stereo_a, n_a, fv_a, 1, &V, only_stereo, check_orientation,
+                                               match_a, n_matches);
 }
 
 int orbx_search_for_triangulation_batch(int device, const orbx_keypoint* kp_a, const uint8_t* desc_a, const uint8_t* free_a,
@@ -431,11 +394,11 @@ int orbx_search_for_triangulation_batch(int device, const orbx_keypoint* kp_a, c
                                         const orbx_triangulation_view* kfs, int only_stereo, int check_orientation, int32_t* match,
                                         int* n_matches)
 {
-    if (n_kf < 0) return fail(ORBX_ERR_INVALID_ARG, "search_for_triangulation_batch: n_kf < 0");
+    if (n_kf < 0) return fail(ORBX_ERR_INVALID_ARG, "search_for_triangulation: n_kf < 0");
     if (n_kf == 0) return ORBX_OK;
-    if (n_kf > 65535) return fail(ORBX_ERR_UNSUPPORTED, "search_for_triangulation_batch: more than 65535 neighbours");
+    if (n_kf > 65535) return fail(ORBX_ERR_UNSUPPORTED, "search_for_triangulation: more than 65535 neighbours");
     if (!kfs || !n_matches || n_a < 0 || (n_a > 0 && (!kp_a || !desc_a || !free_a || !stereo_a || !match)))
-        return fail(ORBX_ERR_INVALID_ARG, "search_for_triangulation_batch: bad arguments");
+        return fail(ORBX_ERR_INVALID_ARG, "search_for_triangulation: bad arguments");
     int rc;
     if ((rc = check_fv(fv_a, n_a, "fv_a"))) return rc;
     // the single call's checks, per neighbour
@@ -444,13 +407,13 @@ int orbx_search_for_triangulation_batch(int device, const orbx_keypoint* kp_a, c
         const orbx_triangulation_view& V = kfs[k];
         if (V.n < 0 || !V.scale || !V.sigma2 || V.n_levels < 1 || V.n_levels > kMaxLevels ||
             (V.n > 0 && (!V.kp || !V.desc || !V.free || !V.stereo)))
-            return fail(ORBX_ERR_INVALID_ARG, "search_for_triangulation_batch: kfs[%d]: bad arguments", k);
+            return fail(ORBX_ERR_INVALID_ARG, "search_for_triangulation: kfs[%d]: bad arguments", k);
         char name[32];
         snprintf(name, sizeof name, "kfs[%d].fv", k);
         if ((rc = check_fv(&V.fv, V.n, name))) return rc;
         for (int j = 0; j < V.n; ++j)
             if (V.kp[j].octave < 0 || V.kp[j].octave >= V.n_levels)
-                return fail(ORBX_ERR_INVALID_ARG, "search_for_triangulation_batch: kfs[%d].kp[%d].octave out of range", k, j);
+                return fail(ORBX_ERR_INVALID_ARG, "search_for_triangulation: kfs[%d].kp[%d].octave out of range", k, j);
         n_feat += (size_t)V.n; n_nodes += (size_t)V.fv.n_nodes; n_idx += V.fv.n_nodes ? (size_t)V.fv.offsets[V.fv.n_nodes] : 0;
     }
     const size_t rows = (size_t)n_kf * n_a;
@@ -520,7 +483,7 @@ int orbx_search_for_triangulation_batch(int device, const orbx_keypoint* kp_a, c
         if (e == cudaSuccess) e = launch_search_triangulation_batch(A, st);
         if (e == cudaSuccess) e = cudaMemcpyAsync(match, A.match, rows * 4, cudaMemcpyDeviceToHost, st);
         if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-        if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "search_for_triangulation_batch: %s", cudaGetErrorString(e));
+        if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "search_for_triangulation: %s", cudaGetErrorString(e));
     }
     // the return value and the rotation filter per neighbour, on the host as in the single call
     for (int k = 0; k < n_kf; ++k) {

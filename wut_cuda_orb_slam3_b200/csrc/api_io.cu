@@ -193,25 +193,24 @@ extern "C" int orbx_distinctive_descriptors(int device, const uint8_t* descripto
     if (total > 0 && !descriptors) return fail(ORBX_ERR_INVALID_ARG, "descriptors is NULL");
     int rc = set_device(device);
     if (rc) return rc;
-    uint8_t* d_desc = nullptr; int* d_off = nullptr; int* d_best = nullptr;
-    cudaStream_t st = nullptr;
-    cudaError_t e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaMallocAsync((void**)&d_desc, (size_t)std::max(total, 1) * 32, st);
-    if (e == cudaSuccess) e = cudaMallocAsync((void**)&d_off, sizeof(int) * ((size_t)n_points + 1), st);
-    if (e == cudaSuccess) e = cudaMallocAsync((void**)&d_best, sizeof(int) * (size_t)n_points, st);
-    if (e == cudaSuccess && total > 0) e = cudaMemcpyAsync(d_desc, descriptors, (size_t)total * 32, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_off, offsets, sizeof(int) * ((size_t)n_points + 1), cudaMemcpyHostToDevice, st);
+    Lease L(device, g_fuse_arena);          // MapPoint::ComputeDistinctiveDescriptors runs on the local-mapping thread
+    const size_t n_off = (size_t)n_points + 1;
+    if ((rc = L.reserve(lease_pad((size_t)total * 32) + lease_pad(n_off * 4) + lease_pad((size_t)n_points * 4)))) return rc;
+    const size_t o_desc = L.take<uint8_t>((size_t)total * 32), o_off = L.take<int>(n_off);
+    L.upload_end = L.off;
+    const size_t o_best = L.take<int>(n_points);
+    if (total > 0) memcpy(L.host<uint8_t>(o_desc), descriptors, (size_t)total * 32);
+    memcpy(L.host<int>(o_off), offsets, n_off * 4);
+    cudaStream_t st = L.A.st;
+    cudaError_t e = cudaMemcpyAsync(L.A.d, L.A.h, L.upload_end, cudaMemcpyHostToDevice, st);
     if (e == cudaSuccess) {
-        distinctive_kernel<<<(n_points + kDdWarps - 1) / kDdWarps, 32 * kDdWarps, 0, st>>>(d_desc, d_off, n_points, d_best);
+        distinctive_kernel<<<(n_points + kDdWarps - 1) / kDdWarps, 32 * kDdWarps, 0, st>>>(L.dev<uint8_t>(o_desc), L.dev<int>(o_off), n_points,
+                                                                                         L.dev<int>(o_best));
         count_launch();
         e = cudaGetLastError();
     }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(best_idx, d_best, sizeof(int) * (size_t)n_points, cudaMemcpyDeviceToHost, st);
-    if (d_desc) cudaFreeAsync(d_desc, st);
-    if (d_off) cudaFreeAsync(d_off, st);
-    if (d_best) cudaFreeAsync(d_best, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(best_idx, L.dev<int>(o_best), sizeof(int) * (size_t)n_points, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (st) cudaStreamDestroy(st);
     if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "distinctive descriptors: %s", cudaGetErrorString(e));
     // map points with more than 64 observations: the single-point host entry (same arithmetic)
     for (int p = 0; p < n_points; ++p)

@@ -6,7 +6,6 @@
 #include <cfloat>
 #include <cmath>
 #include <cstring>
-#include <mutex>
 #include <vector>
 
 #include "orbx_internal.cuh"
@@ -22,19 +21,6 @@ struct orbx_rectifier {
 };
 
 using namespace orbx;
-
-namespace {
-// Grow-only device + pinned staging per device for orbx_undistort_keypoints: the call sits on the per-frame path of the
-// tracking thread (Frame constructor), a cudaMalloc / cudaFree pair per call cost more than everything else in it.
-struct UndistortArena {
-    std::mutex mu;
-    orbx_keypoint* d = nullptr;
-    orbx_keypoint* h = nullptr;
-    size_t cap = 0;
-    cudaStream_t st = nullptr;
-};
-UndistortArena g_undistort[64];
-}  // namespace
 
 extern "C" {
 
@@ -55,28 +41,18 @@ int orbx_undistort_keypoints(int device, const orbx_keypoint* keypoints, int n, 
     p.nfx = new_K[0]; p.nfy = new_K[1]; p.ncx = new_K[2]; p.ncy = new_K[3];
     for (int i = 0; i < n_dist; ++i) p.k[i] = dist[i];
     p.n_dist = n_dist;
-    UndistortArena& A = g_undistort[device & 63];
-    std::lock_guard<std::mutex> lock(A.mu);
-    cudaError_t e = cudaSuccess;
-    if (!A.st) e = cudaStreamCreateWithFlags(&A.st, cudaStreamNonBlocking);
-    if (e == cudaSuccess && A.cap < (size_t)n) {
-        if (A.d) cudaFree(A.d);
-        if (A.h) cudaFreeHost(A.h);
-        A.d = A.h = nullptr; A.cap = 0;
-        const size_t want = (size_t)n + (size_t)n / 2 + 256;
-        e = cudaMalloc(&A.d, want * sizeof(orbx_keypoint));
-        if (e == cudaSuccess) e = cudaMallocHost(&A.h, want * sizeof(orbx_keypoint));
-        if (e != cudaSuccess) return fail(ORBX_ERR_OOM, "undistort scratch: %s", cudaGetErrorString(e));
-        A.cap = want;
-    }
-    if (e == cudaSuccess) {
-        memcpy(A.h, keypoints, (size_t)n * sizeof(orbx_keypoint));
-        e = cudaMemcpyAsync(A.d, A.h, (size_t)n * sizeof(orbx_keypoint), cudaMemcpyHostToDevice, A.st);
-    }
-    if (e == cudaSuccess) e = launch_undistort(A.d, n, p, A.d, A.st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(A.h, A.d, (size_t)n * sizeof(orbx_keypoint), cudaMemcpyDeviceToHost, A.st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(A.st);
-    if (e == cudaSuccess) memcpy(out, A.h, (size_t)n * sizeof(orbx_keypoint));
+    const size_t bytes = (size_t)n * sizeof(orbx_keypoint);
+    Lease L(device);
+    if ((rc = L.reserve(lease_pad(bytes)))) return rc;
+    const size_t o_kp = L.take<orbx_keypoint>(n);
+    L.upload_end = L.off;
+    memcpy(L.host<orbx_keypoint>(o_kp), keypoints, bytes);
+    orbx_keypoint* d_kp = L.dev<orbx_keypoint>(o_kp);
+    cudaError_t e = cudaMemcpyAsync(L.A.d, L.A.h, L.upload_end, cudaMemcpyHostToDevice, L.A.st);
+    if (e == cudaSuccess) e = launch_undistort(d_kp, n, p, d_kp, L.A.st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(L.host<orbx_keypoint>(o_kp), d_kp, bytes, cudaMemcpyDeviceToHost, L.A.st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(L.A.st);
+    if (e == cudaSuccess) memcpy(out, L.host<orbx_keypoint>(o_kp), bytes);
     if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "undistort_keypoints: %s", cudaGetErrorString(e));
     return ORBX_OK;
 }

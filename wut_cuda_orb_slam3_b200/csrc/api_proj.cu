@@ -12,8 +12,8 @@
 // Each entry point turns the reference's per-map-point pre-checks into window queries (float arithmetic in the reference's
 // order, on the host: a handful of operations per point), ships everything in ONE pinned staging copy, runs the grid build and
 // the window search (kernels_proj.cu) and reads the per-query assignment back in one copy.  The 30-bin rotation histogram runs
-// on the host afterwards (it depends on the accepted matches only).  These calls sit on the tracking thread's per-frame path,
-// so the device scratch, the pinned staging buffer and the stream live in a per-device grow-only arena (no cudaMalloc per call).
+// on the host afterwards (it depends on the accepted matches only).  The device scratch, the pinned staging buffer and the
+// stream come from the calling thread's arena (ProjArena / Lease, orbx_internal.cuh).
 #include <algorithm>
 #include <climits>
 #include <cmath>
@@ -24,33 +24,6 @@
 #include "orbx_internal.cuh"
 
 namespace orbx {
-
-ProjArena g_arena[64];
-// orbx_fuse and orbx_search_for_triangulation_batch run on the local-mapping thread: their own arenas, so a large Fuse never
-// holds the lock a tracking-thread search waits on
-ProjArena g_fuse_arena[64];
-// the Sim3 searches run on the loop-closing thread: a third set, so they never hold a lock the other two threads wait on
-ProjArena g_loop_arena[64];
-
-int Lease::reserve(size_t bytes)
-{
-    bytes += 8192;
-    if (!A.st) {
-        cudaError_t e = cudaStreamCreateWithFlags(&A.st, cudaStreamNonBlocking);
-        if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
-    }
-    if (A.d_bytes < bytes) {
-        if (A.d) cudaFree(A.d);
-        if (A.h) cudaFreeHost(A.h);
-        A.d = A.h = nullptr; A.d_bytes = A.h_bytes = 0;
-        const size_t want = bytes + bytes / 2;
-        cudaError_t e = cudaMalloc((void**)&A.d, want);
-        if (e == cudaSuccess) e = cudaMallocHost((void**)&A.h, want);
-        if (e != cudaSuccess) return fail(ORBX_ERR_OOM, "projection scratch (%zu bytes): %s", want, cudaGetErrorString(e));
-        A.d_bytes = A.h_bytes = want;
-    }
-    return ORBX_OK;
-}
 
 namespace {
 
@@ -325,8 +298,10 @@ int orbx_assign_features_to_grid(int device, const orbx_frame_view* frame, int32
     if ((rc = S.upload_and_grid())) return rc;
     cudaError_t e = cudaMemcpyAsync(cell_start, S.A.cell_start, (GRID_CELLS + 1) * 4, cudaMemcpyDeviceToHost, S.stream());
     if (e == cudaSuccess) e = cudaStreamSynchronize(S.stream());
-    if (e == cudaSuccess && cell_start[GRID_CELLS] > 0)
-        e = cudaMemcpy(items, S.A.items, (size_t)cell_start[GRID_CELLS] * 4, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess && cell_start[GRID_CELLS] > 0) {
+        e = cudaMemcpyAsync(items, S.A.items, (size_t)cell_start[GRID_CELLS] * 4, cudaMemcpyDeviceToHost, S.stream());
+        if (e == cudaSuccess) e = cudaStreamSynchronize(S.stream());
+    }
     if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "assign_features_to_grid: %s", cudaGetErrorString(e));
     return ORBX_OK;
 }
@@ -347,7 +322,10 @@ int orbx_get_features_in_area(int device, const orbx_frame_view* frame, float x,
     if (e == cudaSuccess) e = cudaMemcpyAsync(&cnt, d_n, 4, cudaMemcpyDeviceToHost, S.stream());
     if (e == cudaSuccess) e = cudaStreamSynchronize(S.stream());
     std::vector<unsigned long long> keys(cnt);
-    if (e == cudaSuccess && cnt) e = cudaMemcpy(keys.data(), d_out, (size_t)cnt * 8, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess && cnt) {
+        e = cudaMemcpyAsync(keys.data(), d_out, (size_t)cnt * 8, cudaMemcpyDeviceToHost, S.stream());
+        if (e == cudaSuccess) e = cudaStreamSynchronize(S.stream());
+    }
     if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "get_features_in_area: %s", cudaGetErrorString(e));
     *n_out = cnt;
     if (cnt > capacity) return fail(ORBX_ERR_CAPACITY, "get_features_in_area: %d candidates, capacity %d", cnt, capacity);

@@ -174,7 +174,7 @@ namespace {
 
 // The scan of one (A feature, common node) job by one warp: the least distance <= TH_LOW among gate-passing candidates
 // idx_b[b_begin, b_end), the LAST one in list order on ties ('dist > bestDist' is the skip test, src/ORBmatcher2.cc:289).
-// Returns the KF2 index or -1 (on every lane).  F / scale_b / sigma2_b are the pair's tables (kernel parameters or global).
+// Returns the KF2 index or -1 (on every lane).  F / scale_b / sigma2_b are the pair's tables (global: the neighbour's TriKF).
 __device__ __forceinline__ int tri_scan(int lane, const uint32_t q[8], const orbx_keypoint& k1, bool stereo1, const float* F, float ep0,
                                         float ep1, const float* scale_b, const float* sigma2_b, bool only_stereo, bool coarse,
                                         const uint32_t* __restrict__ idx_b, const uint8_t* __restrict__ free_b,
@@ -216,31 +216,6 @@ __device__ __forceinline__ int tri_scan(int lane, const uint32_t q[8], const orb
 }
 
 }  // namespace
-
-// One warp per (A feature, common node) job.
-__global__ void __launch_bounds__(128) search_triangulation_kernel(TriSearchArgs a)
-{
-    const int lane = threadIdx.x & 31;
-    const int jb = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (jb >= a.n_jobs) return;
-    const int4 job = __ldg(a.jobs + jb);                     // (iA, b_begin, b_end, unused)
-    const int iA = job.x;
-    const orbx_keypoint k1 = a.kp_a[iA];
-    const bool stereo1 = __ldg(a.stereo_a + iA) != 0;
-    uint32_t q[8];
-    load_desc(a.desc_a, (size_t)iA, q);
-    const int m = tri_scan(lane, q, k1, stereo1, a.F12, a.ep[0], a.ep[1], a.scale_b, a.sigma2_b, a.only_stereo, a.coarse, a.idx_b, a.free_b,
-                           a.stereo_b, a.desc_b, a.kp_b, job.y, job.z);
-    if (lane == 0) a.match_a[iA] = m;
-}
-
-cudaError_t launch_search_triangulation(const TriSearchArgs& a, cudaStream_t st)
-{
-    if (a.n_jobs <= 0) return cudaSuccess;
-    search_triangulation_kernel<<<(a.n_jobs + 3) / 4, 128, 0, st>>>(a);
-    count_launch();
-    return cudaGetLastError();
-}
 
 // Job build of neighbour blockIdx.x: match row k = -1, then the common nodes of the two ascending node lists (a node of A is
 // looked up in B's list by binary search: the node ids are strictly ascending, so the equal pairs are those of the lock-step

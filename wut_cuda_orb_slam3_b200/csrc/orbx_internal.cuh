@@ -239,19 +239,6 @@ struct BowSearchArgs {
 };
 cudaError_t launch_search_by_bow(const BowSearchArgs& a, cudaStream_t st);
 
-struct TriSearchArgs {
-    int n_jobs;
-    const int4* jobs;            // (iA, b_begin, b_end, 0)
-    const uint32_t* idx_b;
-    const orbx_keypoint* kp_a; const orbx_keypoint* kp_b;
-    const uint8_t* desc_a; const uint8_t* desc_b;
-    const uint8_t* stereo_a; const uint8_t* stereo_b; const uint8_t* free_b;
-    float F12[9]; float ep[2]; float scale_b[kMaxLevels]; float sigma2_b[kMaxLevels];
-    int only_stereo, coarse;
-    int* match_a;                // [nA] init -1
-};
-cudaError_t launch_search_triangulation(const TriSearchArgs& a, cudaStream_t st);
-
 // SearchForTriangulation of one KF1 against many neighbours: a job-build kernel (one CTA per neighbour) writes the jobs of
 // neighbour k into jobs[k * n_a, k * n_a + job_count[k]) and sets match row k to -1; the scan kernel takes the neighbour as
 // blockIdx.y.  Feature indices inside a neighbour are its own (0 .. n - 1); its arrays point into the packed upload.
@@ -346,24 +333,32 @@ cudaError_t launch_remap(const uint8_t* d_src, int sw, int sh, size_t spitch, si
 cudaError_t launch_resize(const uint8_t* d_src, size_t spitch, size_t sframe, const uint2* d_xtab, const uint2* d_ytab, int area2x,
                           uint8_t* d_dst, int dw, int dh, size_t dpitch, size_t dframe, int n_frames, cudaStream_t st);
 
-// Per-device grow-only scratch of the matcher calls (api_proj.cu): device memory, a pinned staging buffer of the same size and
-// a stream.  One call = one Lease: a bump allocator that hands out matching (pinned host, device) ranges so that all inputs
-// travel in one cudaMemcpyAsync.  Inputs are allocated first (the upload range), device-only scratch and outputs after.
+// Per-device grow-only scratch of every call that takes host buffers (api.cu): device memory, a pinned staging buffer and a
+// non-blocking stream.  One call = one Lease: a bump allocator that hands out matching (pinned host, device) ranges so that all
+// inputs travel in one cudaMemcpyAsync.  Inputs are allocated first (the upload range), device-only scratch and outputs after.
+// The call queues everything on A.st and ends with one cudaStreamSynchronize(A.st), so the arena is idle whenever it is leased.
+// Each thread of an ORB-SLAM3 system has its own set, so a call never waits for another thread's lock or work.
 struct ProjArena {
     std::mutex mu;
     unsigned char* d = nullptr; size_t d_bytes = 0;
     unsigned char* h = nullptr; size_t h_bytes = 0;
     cudaStream_t st = nullptr;
 };
-extern ProjArena g_arena[64];          // the tracking thread's searches
-extern ProjArena g_fuse_arena[64];     // local mapping: orbx_fuse, orbx_search_for_triangulation_batch
-extern ProjArena g_loop_arena[64];     // loop closing: the Sim3 searches
+// tracking: the Frame / KF->Frame searches, orbx_knn2, orbx_stereo_match, orbx_undistort_keypoints, orbx_bow_transform,
+// orbx_search_by_bow mode 0
+extern ProjArena g_arena[64];
+// local mapping: orbx_fuse, orbx_search_for_triangulation(_batch), orbx_distinctive_descriptors
+extern ProjArena g_fuse_arena[64];
+// loop closing: the Sim3 searches, orbx_search_by_bow mode 1
+extern ProjArena g_loop_arena[64];
 struct Lease {
     ProjArena& A;
     std::unique_lock<std::mutex> lock;
     size_t off = 0, upload_end = 0;
     explicit Lease(int device, ProjArena* arenas = g_arena) : A(arenas[device & 63]), lock(A.mu) {}
-    int reserve(size_t bytes);
+    // Device bytes for the whole layout; only its first `staged` bytes have a pinned host mirror (a large device-only tail, such
+    // as orbx_knn2's database, is not pinned twice).
+    int reserve(size_t bytes, size_t staged = SIZE_MAX);
     template <typename T> size_t take(size_t count)
     {
         off = (off + 255) & ~(size_t)255;
