@@ -289,6 +289,52 @@ int orbx_extract_stereo_batch_device(orbx_extractor* ex, const uint8_t* d_images
                                      uint8_t* d_descL, int* d_nL, orbx_keypoint* d_kpR, uint8_t* d_descR, int* d_nR, int capacity,
                                      float* d_uRight, float* d_depth, void* stream);
 
+/* ---- RGB-D frames ------------------------------------------------------------------------------------------------ */
+
+/* What the RGB-D Frame constructor reads besides the images (src/Frame.cc:202-260, Tracking::GrabImageRGBD in src/Tracking2.cc). */
+typedef struct orbx_rgbd_calib {
+    float K[4];           /* fx, fy, cx, cy = Pinhole::toK() == mK */
+    const float* dist;    /* mDistCoef: k1 k2 p1 p2 [k3 [k4 k5 k6 [s1..s4]]], n_dist in {0, 4, 5, 8, 12} */
+    int n_dist;
+    float bf;             /* mbf */
+    float depth_factor;   /* Tracking::mDepthMapFactor: already the multiplier (1 / RGBD.DepthMapFactor, or 1) */
+} orbx_rgbd_calib;
+
+/* The RGB-D Frame constructor in one call — Tracking::GrabImageRGBD's colour conversion and depth conversion, then
+ * Frame::Frame(imGray, imDepth, ...) (src/Frame.cc:202-260): ExtractORB(0, imGray, 0, 0), UndistortKeyPoints() and
+ * ComputeStereoFromRGBD(imDepth).  HOST inputs: `image` rows x cols of `channels` (1, 3 or 4; `rgb` as in orbx_extract_color),
+ * `depth` the RAW rows x cols depth map, depth_type 0 = CV_16U, 1 = CV_32F, depth_step bytes per row.  GrabImageRGBD's
+ * convertTo(CV_32F, depth_factor) applies when |depth_factor - 1| > 1e-5 or the map is not CV_32F; it is evaluated on the
+ * sampled pixels only (it is element-wise), so the caller passes the map unconverted.  HOST outputs, capacity rows each:
+ * mvKeys, mvKeysUn, descriptors, *n_out = N, mvuRight and mvDepth (-1 where the depth is not > 0).  Rows past *n_out are
+ * undefined.  Every argument is checked before any work is queued: a NULL handle, output, depth or calib, a bad depth_type,
+ * depth_step < cols * element size, channels not 1 / 3 / 4, step < cols * channels, capacity <= 0, n_dist not in
+ * {0, 4, 5, 8, 12} or a NULL dist with n_dist > 0: ORBX_ERR_INVALID_ARG; a NULL image, rows or cols <= 0:
+ * ORBX_ERR_EMPTY_IMAGE; more than `capacity` keypoints: ORBX_ERR_CAPACITY.  Frame 0 stays inspectable through the probes and
+ * the pyramid mirror is filled, as after orbx_extract. */
+int orbx_extract_rgbd(orbx_extractor* ex, const uint8_t* image, int rows, int cols, size_t step, int channels, int rgb,
+                      const void* depth, int depth_type, size_t depth_step, const orbx_rgbd_calib* calib, orbx_keypoint* kp,
+                      orbx_keypoint* kp_un, uint8_t* desc, int capacity, int* n_out, float* uRight, float* depth_out);
+/* orbx_extract_rgbd over n_frames HOST grey frames images[i] (rows x cols, `step` bytes per row) and depth maps depths[i] of one
+ * type and shape.  Outputs are [n_frames][capacity] slabs; n_out is [n_frames]; for every frame they equal what
+ * orbx_extract_rgbd returns, bit for bit.  Copies are pipelined against compute when the host buffers are page-locked.
+ * n_frames == 0 returns ORBX_OK and does nothing; a frame over capacity: ORBX_ERR_CAPACITY (its rows are undefined; nothing is
+ * written past the slabs).  Afterwards the probes refuse every frame index until the next extraction, as after a stereo batch. */
+int orbx_extract_rgbd_batch(orbx_extractor* ex, const uint8_t* const* images, const void* const* depths, int n_frames, int rows,
+                            int cols, size_t step, int depth_type, size_t depth_step, const orbx_rgbd_calib* calib, orbx_keypoint* kp,
+                            orbx_keypoint* kp_un, uint8_t* desc, int capacity, int* n_out, float* uRight, float* depth_out);
+/* The same on DEVICE-resident grey frames (frame f at d_images + f * frame_stride, `pitch` bytes per row) and depth maps (at
+ * d_depths + f * depth_frame_stride, depth_pitch bytes per row; base, pitch and stride multiples of the element size); every
+ * output is DEVICE memory with the slab layout above.  Asynchronous on `stream` (NULL = the extractor's own): orbx_sync and the
+ * next call on the handle wait for it, as for orbx_extract_batch_device.  A frame over capacity shows only in its device count
+ * (*d_n_out > capacity; its rows are undefined).  Rows of d_kp_un / d_uRight / d_depth at or past a frame's count are left
+ * untouched.  Colour frames: run
+ * orbx_cvt_gray_device in front on the same stream. */
+int orbx_extract_rgbd_batch_device(orbx_extractor* ex, const uint8_t* d_images, size_t frame_stride, size_t pitch, const void* d_depths,
+                                   size_t depth_frame_stride, size_t depth_pitch, int depth_type, int n_frames, int rows, int cols,
+                                   const orbx_rgbd_calib* calib, orbx_keypoint* d_kp, orbx_keypoint* d_kp_un, uint8_t* d_desc,
+                                   int capacity, int* d_n_out, float* d_uRight, float* d_depth, void* stream);
+
 /* ---- bag-of-words transform and vocabulary-guided matching (SURVEY.md §8 rows A13, A14 and (f)1) -------------------- */
 
 /* DBoW2::TemplatedVocabulary<FORB::TDescriptor, FORB> (Thirdparty/DBoW2/DBoW2/TemplatedVocabulary.h): a k-ary tree of

@@ -9,7 +9,7 @@ from .capi import KP_DTYPE, OrbxError, lib  # noqa: F401
 from .bow import (FeatureVector, ORBVocabulary, search_by_bow, search_for_triangulation,  # noqa: F401
                   search_for_triangulation_batch)
 from .extractor import ORBextractor, compute_tables, distribute_octree  # noqa: F401
-from .prep import Rectifier, undistort_keypoints  # noqa: F401
+from .prep import Rectifier, extract_rgbd, undistort_keypoints  # noqa: F401
 from .projection import (FrameView, KeyFrameView, fuse, fuse_sim3, projection_rounds, search_by_projection_kf,  # noqa: F401
                          search_by_projection_last, search_by_projection_map, search_by_projection_sim3, search_for_initialization)
 from . import io  # noqa: F401

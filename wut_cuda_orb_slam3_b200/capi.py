@@ -71,6 +71,9 @@ SIGNATURES = {
     "orbx_extract_stereo": (_i, [_vp, _vp, _vp, _vp, _i, _i, _sz, _vp, _vp, _vp, _vp, _vp, _vp, _i, _f, _f, _vp, _vp]),
     "orbx_extract_stereo_batch": (_i, [_vp, _vp, _vp, _i, _i, _i, _sz, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
     "orbx_extract_stereo_batch_device": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _sz, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
+    "orbx_extract_rgbd": (_i, [_vp, _vp, _i, _i, _sz, _i, _i, _vp, _i, _sz, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
+    "orbx_extract_rgbd_batch": (_i, [_vp, _vp, _vp, _i, _i, _i, _sz, _i, _sz, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
+    "orbx_extract_rgbd_batch_device": (_i, [_vp, _vp, _sz, _sz, _vp, _sz, _sz, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "orbx_comm_unique_id": (_i, [_vp]),
     "orbx_comm_create": (_i, [_i, _i, _i, _vp, C.POINTER(_vp)]),
     "orbx_comm_from_nccl": (_i, [_i, _vp, _i, _i, C.POINTER(_vp)]),
@@ -143,6 +146,11 @@ class TrackPointsC(C.Structure):
     """orbx_track_points (include/orbx.h)."""
     _fields_ = [("n", C.c_int), ("in_view", _vp), ("bad", _vp), ("proj_x", _vp), ("proj_y", _vp), ("proj_xr", _vp),
                 ("view_cos", _vp), ("track_depth", _vp), ("scale_level", _vp), ("n_obs", _vp), ("descriptors", _vp)]
+
+
+class RgbdCalibC(C.Structure):
+    """orbx_rgbd_calib (include/orbx.h): mK, mDistCoef, mbf and Tracking::mDepthMapFactor."""
+    _fields_ = [("K", _f * 4), ("dist", _vp), ("n_dist", C.c_int), ("bf", _f), ("depth_factor", _f)]
 
 
 class OrbxError(RuntimeError):

@@ -12,6 +12,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <mutex>
 #include <string>
 #include <unordered_map>
@@ -120,6 +121,9 @@ struct Slot {
     float* d_su = nullptr; float* d_sd = nullptr; int* d_sad = nullptr;
     int* d_snm = nullptr;          // [2 * pairs] monoIndex scratch of the device call (stereo outputs have no n_mono)
     size_t stereo_rows = 0; int stereo_pairs = 0;
+    // RGB-D frames: the raw depth maps of the host-buffer calls and the mvKeysUn slab (mvuRight / mvDepth use d_su / d_sd)
+    uint8_t* d_depth = nullptr; size_t d_depth_bytes = 0;
+    orbx_keypoint* d_kpun = nullptr; size_t kpun_rows = 0;
     std::vector<void*> allocs;
 };
 
@@ -194,6 +198,9 @@ struct orbx_extractor {
     size_t mirror_off[ORBX_MAX_LEVELS] = {0};
     cudaStream_t mirror_stream = nullptr;
     cudaEvent_t ev_mirror = nullptr;
+    // orbx_extract_rgbd: the depth map goes up on its own stream while the extraction runs
+    cudaStream_t depth_stream = nullptr;
+    cudaEvent_t ev_depth = nullptr;
     bool force_eager = false;      // debug hooks that patch the workspace (orbx_debug_octree_timing) must not replay a captured graph
     // fork / join of the single-frame pipeline: FAST + octree of level l run on side[l] as soon as level l of the pyramid exists
     cudaStream_t side[ORBX_MAX_LEVELS] = {nullptr};
@@ -276,6 +283,7 @@ static void free_slot(Slot& s)
     s.d_in = nullptr; s.d_in_bytes = 0; s.d_color = nullptr; s.d_color_bytes = 0; s.d_kps = nullptr; s.d_desc = nullptr; s.d_n = nullptr; s.d_nm = nullptr;
     s.out_cap = 0; s.out_frames = 0;
     s.d_su = nullptr; s.d_sd = nullptr; s.d_sad = nullptr; s.d_snm = nullptr; s.stereo_rows = 0; s.stereo_pairs = 0;
+    s.d_depth = nullptr; s.d_depth_bytes = 0; s.d_kpun = nullptr; s.kpun_rows = 0;
 }
 
 // release one buffer of a slot early (a staging buffer that is being replaced by a larger one)
@@ -695,6 +703,29 @@ static int ensure_stereo_staging(Slot& s, int pairs, int capacity)
     return ORBX_OK;
 }
 
+// RGB-D staging of the host-buffer calls: raw depth maps and mvKeysUn rows.  As above: nothing may be in flight on the slot.
+static bool rgbd_staging_fits(const Slot& s, size_t depth_bytes, size_t rows)
+{
+    return s.d_depth_bytes >= depth_bytes && s.kpun_rows >= rows;
+}
+static int ensure_rgbd_staging(Slot& s, size_t depth_bytes, size_t rows)
+{
+    int rc;
+    if (s.d_depth_bytes < depth_bytes) {
+        dev_release(s, s.d_depth);
+        s.d_depth_bytes = 0;
+        if ((rc = dev_alloc(s, &s.d_depth, depth_bytes))) return rc;
+        s.d_depth_bytes = depth_bytes;
+    }
+    if (s.kpun_rows < rows) {
+        dev_release(s, s.d_kpun);
+        s.kpun_rows = 0;
+        if ((rc = dev_alloc(s, &s.d_kpun, rows))) return rc;
+        s.kpun_rows = rows;
+    }
+    return ORBX_OK;
+}
+
 // Chunk schedule of the host-buffer batches: the first host->device copy cannot overlap any compute, so the pipeline ramps
 // up with a quarter and a half chunk before it settles on full chunks (shorter un-overlapped prologue) ...
 static std::vector<std::pair<int, int>> chunk_schedule(int n, int chunk)
@@ -710,6 +741,77 @@ static std::vector<std::pair<int, int>> chunk_schedule(int n, int chunk)
     while (f0 < n - tail) { const int nf = std::min(chunk, n - tail - f0); sched.emplace_back(f0, nf); f0 += nf; }
     if (tail) { sched.emplace_back(f0, ramp[1]); f0 += ramp[1]; sched.emplace_back(f0, ramp[0]); f0 += ramp[0]; }
     return sched;
+}
+
+// Host frames [i0, i0 + n) of `src` (rows of row_bytes, `step` bytes apart) into dst back to back: one copy when they already are.
+template <typename T>
+static int upload_frames(const T* const* src, int i0, int n, uint8_t* dst, size_t row_bytes, int rows, size_t step, cudaStream_t st)
+{
+    const size_t frame = row_bytes * rows;
+    bool contiguous = step == row_bytes;
+    for (int i = 1; i < n && contiguous; ++i)
+        contiguous = (const uint8_t*)src[i0 + i] == (const uint8_t*)src[i0 + i - 1] + frame;
+    if (contiguous) {
+        CU(cudaMemcpyAsync(dst, src[i0], frame * n, cudaMemcpyHostToDevice, st));
+    } else {
+        for (int i = 0; i < n; ++i)
+            CU(cudaMemcpy2DAsync(dst + (size_t)i * frame, row_bytes, src[i0 + i], step, row_bytes, rows, cudaMemcpyHostToDevice, st));
+    }
+    return ORBX_OK;
+}
+
+// The driver loop of the host-buffer batches of stereo pairs and RGB-D frames.  Chunk c of `sched` (first item, items) runs on
+// slot c % nslots, whose staging the caller has sized.  serial = false: each chunk runs whole on its slot's stream; serial = true:
+// orbx_extract_batch's three-stream pipeline (there: why), tied by the slot's events.  Results go home trimmed, as in
+// orbx_extract_batch: `counts` queues the copy of a chunk's per-item counts, and the host reads them after it has queued chunk
+// c + 2, then `download` asks for the rows the chunk's items actually have.
+struct HostPipeline {
+    // (slot, first item, items, stream): upload on the H2D stream, compute on the compute stream, counts and download on the D2H
+    // stream (all three are the slot's stream when not serial)
+    std::function<int(Slot&, int, int, cudaStream_t)> upload, compute, counts, download;
+};
+static int run_host_pipeline(orbx_extractor* ex, const std::vector<std::pair<int, int>>& sched, int nslots, bool serial, const HostPipeline& h)
+{
+    const int nchunks = (int)sched.size();
+    int rc;
+    if (serial && !ex->compute) {
+        CU(cudaStreamCreateWithFlags(&ex->compute, cudaStreamNonBlocking));
+        CU(cudaStreamCreateWithFlags(&ex->copy_in, cudaStreamNonBlocking));
+        CU(cudaStreamCreateWithFlags(&ex->copy_out, cudaStreamNonBlocking));
+    }
+    if (serial)      // earlier work of this extractor on the slot streams must be complete
+        for (int i = 0; i < nslots; ++i) CU(cudaStreamSynchronize(ex->slots[i].stream));
+    auto finish = [&](int c) -> int {
+        Slot& s = ex->slots[c % nslots];
+        cudaStream_t ost = serial ? ex->copy_out : s.stream;
+        CU(cudaEventSynchronize(s.ev_cnt));
+        int rc2 = h.download(s, sched[c].first, sched[c].second, ost);
+        if (rc2) return rc2;
+        if (serial) CU(cudaEventRecord(s.ev_out, ost));
+        return ORBX_OK;
+    };
+    const int lag = 2;
+    for (int c = 0; c < nchunks; ++c) {
+        Slot& s = ex->slots[c % nslots];
+        const int i0 = sched[c].first, ni = sched[c].second;
+        cudaStream_t cst = serial ? ex->compute : s.stream;
+        cudaStream_t ist = serial ? ex->copy_in : s.stream, ost = serial ? ex->copy_out : s.stream;
+        // reuse of a slot: its input staging is free once the chunk that used it has been computed, its output staging once that
+        // chunk's D2H has completed (queued when chunk c - nslots + lag was; nslots > lag whenever a slot is reused)
+        if (serial && c >= nslots) { CU(cudaStreamWaitEvent(ist, s.ev_done, 0)); CU(cudaStreamWaitEvent(cst, s.ev_out, 0)); }
+        if ((rc = h.upload(s, i0, ni, ist))) return rc;
+        if (serial) { CU(cudaEventRecord(s.ev_in, ist)); CU(cudaStreamWaitEvent(cst, s.ev_in, 0)); }
+        if ((rc = h.compute(s, i0, ni, cst))) return rc;
+        if (serial) { CU(cudaEventRecord(s.ev_done, cst)); CU(cudaStreamWaitEvent(ost, s.ev_done, 0)); }
+        if ((rc = h.counts(s, i0, ni, ost))) return rc;
+        CU(cudaEventRecord(s.ev_cnt, ost));
+        if (c >= lag && (rc = finish(c - lag))) return rc;
+    }
+    for (int c = std::max(nchunks - lag, 0); c < nchunks; ++c)
+        if ((rc = finish(c))) return rc;
+    if (serial) { CU(cudaStreamSynchronize(ex->copy_out)); CU(cudaStreamSynchronize(ex->compute)); CU(cudaStreamSynchronize(ex->copy_in)); }
+    for (int i = 0; i < nslots; ++i) CU(cudaStreamSynchronize(ex->slots[i].stream));
+    return ORBX_OK;
 }
 
 // The whole per-chunk pipeline on one stream.
@@ -883,6 +985,33 @@ static int enqueue_single(orbx_extractor* ex, const uint8_t* image, int rows, in
     return ORBX_OK;
 }
 
+// The same for a host colour image (channels 3 or 4): upload into the slot's colour staging, convert to grey into its input
+// staging, and the per-level fork / join of orbx_extract launched eagerly (the colour staging is not part of the captured graph).
+static int enqueue_color(orbx_extractor* ex, const uint8_t* image, int rows, int cols, size_t step, int channels, int rgb, int lap0,
+                         int lap1, int capacity)
+{
+    int rc = set_device(ex->device);
+    if (rc) return rc;
+    if ((rc = configure(ex, rows, cols))) return rc;
+    wait_user_work(ex);
+    if ((rc = ensure_capacity(ex, 1, 1))) return rc;
+    Slot& s = ex->slots[0];
+    const size_t gpitch = (size_t)cols, cpitch = align_up((size_t)cols * channels, 16);
+    if ((rc = ensure_host_staging(s, gpitch * rows, 1, capacity))) return rc;
+    if (s.d_color_bytes < cpitch * rows) {
+        if ((rc = dev_alloc(s, &s.d_color, cpitch * rows))) return rc;
+        s.d_color_bytes = cpitch * rows;
+    }
+    CU(cudaMemcpy2DAsync(s.d_color, cpitch, image, step, (size_t)cols * channels, rows, cudaMemcpyHostToDevice, s.stream));
+    CU(launch_cvt_gray(s.d_color, cpitch, 0, channels, rgb, 1, rows, cols, s.d_in, gpitch, 0, s.stream));
+    if ((rc = ensure_mirror(ex, s.stream))) return rc;
+    if (ex->profiling) rc = run_chunk(ex, s, one_set_io(s.d_in, gpitch * rows, gpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), 1, lap0, lap1, s.stream);
+    else rc = run_single_forked(ex, s, s.d_in, gpitch, lap0, lap1, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm, s.stream);
+    if (rc) return rc;
+    ex->last_frames = 1;
+    return ORBX_OK;
+}
+
 }  // namespace orbx
 
 // =====================================================================================================================
@@ -962,6 +1091,8 @@ void orbx_destroy(orbx_extractor* ex)
     if (ex->mirror_stream) { cudaStreamSynchronize(ex->mirror_stream); cudaStreamDestroy(ex->mirror_stream); }
     if (ex->ev_mirror) cudaEventDestroy(ex->ev_mirror);
     if (ex->h_mirror) cudaFreeHost(ex->h_mirror);
+    if (ex->depth_stream) { cudaStreamSynchronize(ex->depth_stream); cudaStreamDestroy(ex->depth_stream); }
+    if (ex->ev_depth) cudaEventDestroy(ex->ev_depth);
     for (int l = 0; l < ORBX_MAX_LEVELS; ++l) {
         if (ex->side[l]) { cudaStreamSynchronize(ex->side[l]); cudaStreamDestroy(ex->side[l]); }
         if (ex->ev_lvl[l]) cudaEventDestroy(ex->ev_lvl[l]);
@@ -1235,31 +1366,14 @@ int orbx_extract_color(orbx_extractor* ex, const uint8_t* image, int rows, int c
     if (channels == 1) return orbx_extract(ex, image, rows, cols, step, lap0, lap1, keypoints, descriptors, capacity, n_out, n_mono);
     if ((channels != 3 && channels != 4) || step < (size_t)cols * channels) return fail(ORBX_ERR_INVALID_ARG, "channels must be 1, 3 or 4");
     if (!keypoints || !descriptors || !n_out || !n_mono || capacity <= 0) return fail(ORBX_ERR_INVALID_ARG, "bad output buffers");
-    int rc = set_device(ex->device);
+    int rc = enqueue_color(ex, image, rows, cols, step, channels, rgb, lap0, lap1, capacity);
     if (rc) return rc;
-    if ((rc = configure(ex, rows, cols))) return rc;
-    wait_user_work(ex);
-    if ((rc = ensure_capacity(ex, 1, 1))) return rc;
     Slot& s = ex->slots[0];
-    const size_t gpitch = (size_t)cols, cpitch = align_up((size_t)cols * channels, 16);
-    if ((rc = ensure_host_staging(s, gpitch * rows, 1, capacity))) return rc;
-    if (s.d_color_bytes < cpitch * rows) {
-        if ((rc = dev_alloc(s, &s.d_color, cpitch * rows))) return rc;
-        s.d_color_bytes = cpitch * rows;
-    }
-    CU(cudaMemcpy2DAsync(s.d_color, cpitch, image, step, (size_t)cols * channels, rows, cudaMemcpyHostToDevice, s.stream));
-    CU(launch_cvt_gray(s.d_color, cpitch, 0, channels, rgb, 1, rows, cols, s.d_in, gpitch, 0, s.stream));
-    // same per-level fork / join as orbx_extract (launched eagerly: the colour staging buffer is not part of the captured graph)
-    if ((rc = ensure_mirror(ex, s.stream))) return rc;
-    if (ex->profiling) rc = run_chunk(ex, s, one_set_io(s.d_in, gpitch * rows, gpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), 1, lap0, lap1, s.stream);
-    else rc = run_single_forked(ex, s, s.d_in, gpitch, lap0, lap1, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm, s.stream);
-    if (rc) return rc;
     CU(cudaMemcpyAsync(keypoints, s.d_kps, sizeof(orbx_keypoint) * (size_t)capacity, cudaMemcpyDeviceToHost, s.stream));
     CU(cudaMemcpyAsync(descriptors, s.d_desc, (size_t)capacity * 32, cudaMemcpyDeviceToHost, s.stream));
     CU(cudaMemcpyAsync(n_out, s.d_n, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
     CU(cudaMemcpyAsync(n_mono, s.d_nm, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
     CU(cudaStreamSynchronize(s.stream));
-    ex->last_frames = 1;
     if (*n_out > capacity) return fail(ORBX_ERR_CAPACITY, "%d keypoints, capacity %d", *n_out, capacity);
     return ORBX_OK;
 }
@@ -1761,21 +1875,28 @@ int orbx_extract_stereo_batch(orbx_extractor* ex, const uint8_t* const* imagesL,
         if ((rc = ensure_host_staging(s, dframe * 2 * chunk, 2 * chunk, capacity))) return rc;
         if ((rc = ensure_stereo_staging(s, chunk, capacity))) return rc;
     }
-    // the two pipelines of orbx_extract_batch (there: why), chosen by the chunk's frame count
-    const bool serial = 2 * chunk >= 128;
-    if (serial && !ex->compute) {
-        CU(cudaStreamCreateWithFlags(&ex->compute, cudaStreamNonBlocking));
-        CU(cudaStreamCreateWithFlags(&ex->copy_in, cudaStreamNonBlocking));
-        CU(cudaStreamCreateWithFlags(&ex->copy_out, cudaStreamNonBlocking));
-    }
-    if (serial)
-        for (int i = 0; i < nslots; ++i) CU(cudaStreamSynchronize(ex->slots[i].stream));
-    // trimmed downloads as in orbx_extract_batch: counts first, then the rows the chunk's pairs have
-    auto finish = [&](int c) -> int {
-        Slot& s = ex->slots[c % nslots];
-        const int p0 = sched[c].first, np = sched[c].second;
-        cudaStream_t ost = serial ? ex->copy_out : s.stream;
-        CU(cudaEventSynchronize(s.ev_cnt));
+    HostPipeline h;
+    h.upload = [&](Slot& s, int p0, int np, cudaStream_t ist) -> int {
+        int rc2 = upload_frames(imagesL, p0, np, s.d_in, dpitch, rows, step, ist);
+        return rc2 ? rc2 : upload_frames(imagesR, p0, np, s.d_in + (size_t)np * dframe, dpitch, rows, step, ist);
+    };
+    h.compute = [&](Slot& s, int p0, int np, cudaStream_t cst) -> int {
+        (void)p0;
+        // the staging holds both sides back to back: one set of 2 np frames (vLappingArea = {0, 0}, src/Frame.cc:124-125)
+        int rc2 = run_chunk(ex, s, one_set_io(s.d_in, dframe, dpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), 2 * np, 0, 0, cst);
+        if (rc2) return rc2;
+        const size_t r = (size_t)np * capacity;
+        const StereoArgs A = stereo_chunk_args(ex, s, np, s.d_kps, s.d_desc, s.d_n, s.d_kps + r, s.d_desc + r * 32, s.d_n + np, capacity, bf, maxD,
+                                               s.d_su, s.d_sd);
+        CU(launch_stereo(ex->fg, A, cst));
+        return ORBX_OK;
+    };
+    h.counts = [&](Slot& s, int p0, int np, cudaStream_t ost) -> int {
+        CU(cudaMemcpyAsync(nL + p0, s.d_n, sizeof(int) * np, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpyAsync(nR + p0, s.d_n + np, sizeof(int) * np, cudaMemcpyDeviceToHost, ost));
+        return ORBX_OK;
+    };
+    h.download = [&](Slot& s, int p0, int np, cudaStream_t ost) -> int {
         int mxL = 0, mxR = 0;
         for (int p = 0; p < np; ++p) { mxL = std::max(mxL, nL[p0 + p]); mxR = std::max(mxR, nR[p0 + p]); }
         const size_t kpitch = sizeof(orbx_keypoint) * (size_t)capacity, dpitch32 = (size_t)capacity * 32, fpitch = sizeof(float) * (size_t)capacity;
@@ -1792,45 +1913,10 @@ int orbx_extract_stereo_batch(orbx_extractor* ex, const uint8_t* const* imagesL,
             CU(cudaMemcpy2DAsync(descR + (size_t)p0 * capacity * 32, dpitch32, s.d_desc + (size_t)np * capacity * 32, dpitch32, (size_t)rowsR * 32, np,
                                  cudaMemcpyDeviceToHost, ost));
         }
-        if (serial) CU(cudaEventRecord(s.ev_out, ost));
         return ORBX_OK;
     };
-    auto upload = [&](const uint8_t* const* images, int p0, int np, uint8_t* dst, cudaStream_t ist) -> int {
-        bool contiguous = step == (size_t)cols;
-        for (int p = 1; p < np && contiguous; ++p) contiguous = images[p0 + p] == images[p0 + p - 1] + dframe;
-        if (contiguous) {
-            CU(cudaMemcpyAsync(dst, images[p0], dframe * np, cudaMemcpyHostToDevice, ist));
-        } else {
-            for (int p = 0; p < np; ++p)
-                CU(cudaMemcpy2DAsync(dst + (size_t)p * dframe, dpitch, images[p0 + p], step, cols, rows, cudaMemcpyHostToDevice, ist));
-        }
-        return ORBX_OK;
-    };
-    const int lag = 2;
-    for (int c = 0; c < nchunks; ++c) {
-        Slot& s = ex->slots[c % nslots];
-        const int p0 = sched[c].first, np = sched[c].second;
-        cudaStream_t cst = serial ? ex->compute : s.stream;
-        cudaStream_t ist = serial ? ex->copy_in : s.stream, ost = serial ? ex->copy_out : s.stream;
-        if (serial && c >= nslots) { CU(cudaStreamWaitEvent(ist, s.ev_done, 0)); CU(cudaStreamWaitEvent(cst, s.ev_out, 0)); }
-        if ((rc = upload(imagesL, p0, np, s.d_in, ist)) || (rc = upload(imagesR, p0, np, s.d_in + (size_t)np * dframe, ist))) return rc;
-        if (serial) { CU(cudaEventRecord(s.ev_in, ist)); CU(cudaStreamWaitEvent(cst, s.ev_in, 0)); }
-        // the staging holds both sides back to back: one set of 2 np frames (vLappingArea = {0, 0}, src/Frame.cc:124-125)
-        if ((rc = run_chunk(ex, s, one_set_io(s.d_in, dframe, dpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), 2 * np, 0, 0, cst))) return rc;
-        const size_t r = (size_t)np * capacity;
-        const StereoArgs A = stereo_chunk_args(ex, s, np, s.d_kps, s.d_desc, s.d_n, s.d_kps + r, s.d_desc + r * 32, s.d_n + np, capacity, bf, maxD,
-                                               s.d_su, s.d_sd);
-        CU(launch_stereo(ex->fg, A, cst));
-        if (serial) { CU(cudaEventRecord(s.ev_done, cst)); CU(cudaStreamWaitEvent(ost, s.ev_done, 0)); }
-        CU(cudaMemcpyAsync(nL + p0, s.d_n, sizeof(int) * np, cudaMemcpyDeviceToHost, ost));
-        CU(cudaMemcpyAsync(nR + p0, s.d_n + np, sizeof(int) * np, cudaMemcpyDeviceToHost, ost));
-        CU(cudaEventRecord(s.ev_cnt, ost));
-        if (c >= lag && (rc = finish(c - lag))) return rc;
-    }
-    for (int c = std::max(nchunks - lag, 0); c < nchunks; ++c)
-        if ((rc = finish(c))) return rc;
-    if (serial) { CU(cudaStreamSynchronize(ex->copy_out)); CU(cudaStreamSynchronize(ex->compute)); CU(cudaStreamSynchronize(ex->copy_in)); }
-    for (int i = 0; i < nslots; ++i) CU(cudaStreamSynchronize(ex->slots[i].stream));
+    // the two pipelines of orbx_extract_batch, chosen by the chunk's frame count
+    if ((rc = run_host_pipeline(ex, sched, nslots, 2 * chunk >= 128, h))) return rc;
     for (int p = 0; p < n_pairs; ++p)
         if (nL[p] > capacity || nR[p] > capacity)
             return fail(ORBX_ERR_CAPACITY, "pair %d has %d / %d keypoints, capacity %d", p, nL[p], nR[p], capacity);
@@ -1876,6 +1962,206 @@ int orbx_extract_stereo_batch_device(orbx_extractor* ex, const uint8_t* d_images
         const StereoArgs A = stereo_chunk_args(ex, s, np, d_kpL + r, d_descL + r * 32, d_nL + p0, d_kpR + r, d_descR + r * 32, d_nR + p0,
                                                capacity, bf, maxD, d_uRight + r, d_depth + r);
         CU(launch_stereo(ex->fg, A, st));
+    }
+    if (st != s.stream) { CU(cudaEventRecord(ex->ev_user, st)); ex->user_pending = true; }
+    return ORBX_OK;
+}
+
+// ---- RGB-D frames -------------------------------------------------------------------------------------------------------
+// ExtractORB(0, imGray, 0, 0) (src/Frame.cc:224) as for any frame, then one launch of rgbd_frame_kernel reads each keypoint where
+// the extraction left it and writes mvKeysUn, mvuRight and mvDepth.  The depth map is never converted as a whole.
+
+// Checks of the depth-map description and the calibration; fills everything of `a` but the buffers.
+static int rgbd_args(const orbx_rgbd_calib* calib, int depth_type, size_t depth_step, int cols, RgbdArgs& a)
+{
+    if (!calib) return fail(ORBX_ERR_INVALID_ARG, "calib is NULL");
+    if (depth_type != 0 && depth_type != 1) return fail(ORBX_ERR_INVALID_ARG, "depth_type %d: 0 (CV_16U) or 1 (CV_32F)", depth_type);
+    if (depth_step < (size_t)cols * (depth_type == 0 ? 2 : 4)) return fail(ORBX_ERR_INVALID_ARG, "depth step %zu < cols * element size", depth_step);
+    const int nd = calib->n_dist;
+    if ((nd != 0 && nd != 4 && nd != 5 && nd != 8 && nd != 12) || (nd > 0 && !calib->dist))
+        return fail(ORBX_ERR_INVALID_ARG, "n_dist %d: 0, 4, 5, 8 or 12 coefficients", nd);
+    a = RgbdArgs{};
+    a.depth_type = depth_type;
+    // Tracking::GrabImageRGBD: if ((fabs(mDepthMapFactor - 1.0f) > 1e-5) || imDepth.type() != CV_32F) imDepth.convertTo(imDepth,
+    // CV_32F, mDepthMapFactor) — the difference in float, the comparison with the double 1e-5
+    a.convert = (std::fabs(calib->depth_factor - 1.0f) > 1e-5 || depth_type != 1) ? 1 : 0;
+    a.factor = calib->depth_factor;
+    a.bf = calib->bf;
+    a.undistort = nd > 0 && calib->dist[0] != 0.0f;          // src/Frame.cc:779-783: mDistCoef[0] == 0 copies the keypoints
+    UndistortParams& p = a.p;
+    p.fx = p.nfx = calib->K[0]; p.fy = p.nfy = calib->K[1]; p.cx = p.ncx = calib->K[2]; p.cy = p.ncy = calib->K[3];
+    for (int i = 0; i < nd; ++i) p.k[i] = calib->dist[i];
+    p.n_dist = nd;
+    return ORBX_OK;
+}
+
+int orbx_extract_rgbd(orbx_extractor* ex, const uint8_t* image, int rows, int cols, size_t step, int channels, int rgb,
+                      const void* depth, int depth_type, size_t depth_step, const orbx_rgbd_calib* calib, orbx_keypoint* kp,
+                      orbx_keypoint* kp_un, uint8_t* desc, int capacity, int* n_out, float* uRight, float* depth_out)
+{
+    if (!ex) return fail(ORBX_ERR_INVALID_ARG, "extractor is NULL");
+    if (!image || rows <= 0 || cols <= 0) return fail(ORBX_ERR_EMPTY_IMAGE, "empty image");
+    if ((channels != 1 && channels != 3 && channels != 4) || step < (size_t)cols * channels)
+        return fail(ORBX_ERR_INVALID_ARG, "channels must be 1, 3 or 4 and step >= cols * channels");
+    if (!kp || !kp_un || !desc || !n_out || !uRight || !depth_out || capacity <= 0 || !depth)
+        return fail(ORBX_ERR_INVALID_ARG, "bad depth map / output buffers");
+    RgbdArgs A;
+    int rc = rgbd_args(calib, depth_type, depth_step, cols, A);
+    if (rc) return rc;
+    rc = channels == 1 ? enqueue_single(ex, image, rows, cols, step, 0, 0, capacity)
+                       : enqueue_color(ex, image, rows, cols, step, channels, rgb, 0, 0, capacity);
+    if (rc) return rc;
+    Slot& s = ex->slots[0];
+    const size_t zpitch = (size_t)cols * (depth_type == 0 ? 2 : 4), zbytes = zpitch * rows;
+    if (!rgbd_staging_fits(s, zbytes, (size_t)capacity) || !stereo_staging_fits(s, 1, capacity)) {   // grow-only: replaced while idle
+        CU(cudaStreamSynchronize(s.stream));
+        if ((rc = ensure_rgbd_staging(s, zbytes, (size_t)capacity)) || (rc = ensure_stereo_staging(s, 1, capacity))) return rc;
+    }
+    // the depth map goes up beside the extraction; an event joins it in front of the RGB-D kernel
+    if (!ex->depth_stream) CU(cudaStreamCreateWithFlags(&ex->depth_stream, cudaStreamNonBlocking));
+    if (!ex->ev_depth) CU(cudaEventCreateWithFlags(&ex->ev_depth, cudaEventDisableTiming));
+    CU(cudaMemcpy2DAsync(s.d_depth, zpitch, depth, depth_step, zpitch, rows, cudaMemcpyHostToDevice, ex->depth_stream));
+    CU(cudaEventRecord(ex->ev_depth, ex->depth_stream));
+    CU(cudaStreamWaitEvent(s.stream, ex->ev_depth, 0));
+    A.kp = s.d_kps; A.n = s.d_n; A.capacity = capacity;
+    A.kp_un = s.d_kpun; A.uRight = s.d_su; A.depth_out = s.d_sd;
+    A.depth = s.d_depth; A.depth_pitch = zpitch; A.depth_frame_stride = zbytes;
+    CU(launch_rgbd_frame(A, 1, s.stream));
+    const size_t kb = sizeof(orbx_keypoint) * (size_t)capacity, fb = sizeof(float) * (size_t)capacity;
+    CU(cudaMemcpyAsync(kp, s.d_kps, kb, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(desc, s.d_desc, (size_t)capacity * 32, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(kp_un, s.d_kpun, kb, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(uRight, s.d_su, fb, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(depth_out, s.d_sd, fb, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(n_out, s.d_n, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaStreamSynchronize(s.stream));
+    if (*n_out > capacity) return fail(ORBX_ERR_CAPACITY, "frame has %d keypoints, capacity %d", *n_out, capacity);
+    return ORBX_OK;
+}
+
+int orbx_extract_rgbd_batch(orbx_extractor* ex, const uint8_t* const* images, const void* const* depths, int n_frames, int rows,
+                            int cols, size_t step, int depth_type, size_t depth_step, const orbx_rgbd_calib* calib, orbx_keypoint* kp,
+                            orbx_keypoint* kp_un, uint8_t* desc, int capacity, int* n_out, float* uRight, float* depth_out)
+{
+    if (!ex) return fail(ORBX_ERR_INVALID_ARG, "extractor is NULL");
+    if (n_frames < 0) return fail(ORBX_ERR_INVALID_ARG, "n_frames %d < 0", n_frames);
+    if (n_frames == 0) return ORBX_OK;
+    if (!images || rows <= 0 || cols <= 0) return fail(ORBX_ERR_EMPTY_IMAGE, "empty image");
+    for (int i = 0; i < n_frames; ++i)
+        if (!images[i]) return fail(ORBX_ERR_EMPTY_IMAGE, "image %d is NULL", i);
+    if (!depths) return fail(ORBX_ERR_INVALID_ARG, "depths is NULL");
+    for (int i = 0; i < n_frames; ++i)
+        if (!depths[i]) return fail(ORBX_ERR_INVALID_ARG, "depth map %d is NULL", i);
+    if (!kp || !kp_un || !desc || !n_out || !uRight || !depth_out || capacity <= 0 || step < (size_t)cols)
+        return fail(ORBX_ERR_INVALID_ARG, "bad output buffers / step");
+    RgbdArgs A;
+    int rc = rgbd_args(calib, depth_type, depth_step, cols, A);
+    if (rc) return rc;
+    if ((rc = set_device(ex->device))) return rc;
+    if ((rc = configure(ex, rows, cols))) return rc;
+    wait_user_work(ex);
+    ex->last_frames = 0;
+    // orbx_extract_batch's chunking and ramp schedule
+    const int chunk = ex->max_batch > 0 ? std::min(ex->max_batch, n_frames) : std::min(n_frames, 64);
+    const std::vector<std::pair<int, int>> sched = chunk_schedule(n_frames, chunk);   // (first frame, frames)
+    const int nslots = std::min((int)sched.size(), (int)orbx_extractor::kSlots);
+    if ((rc = ensure_capacity(ex, chunk, nslots))) return rc;
+    const size_t dpitch = (size_t)cols, dframe = dpitch * rows;
+    const size_t zpitch = (size_t)cols * (depth_type == 0 ? 2 : 4), zframe = zpitch * rows;
+    const size_t rows_out = (size_t)chunk * capacity;
+    for (int i = 0; i < nslots; ++i) {
+        Slot& s = ex->slots[i];
+        if (s.d_in_bytes < dframe * chunk || s.out_cap < rows_out || s.out_frames < chunk || !rgbd_staging_fits(s, zframe * chunk, rows_out) ||
+            !stereo_staging_fits(s, chunk, capacity))
+            CU(cudaStreamSynchronize(s.stream));
+        if ((rc = ensure_host_staging(s, dframe * chunk, chunk, capacity))) return rc;
+        if ((rc = ensure_rgbd_staging(s, zframe * chunk, rows_out))) return rc;
+        if ((rc = ensure_stereo_staging(s, chunk, capacity))) return rc;
+    }
+    HostPipeline h;
+    h.upload = [&](Slot& s, int f0, int nf, cudaStream_t ist) -> int {
+        int rc2 = upload_frames(images, f0, nf, s.d_in, dpitch, rows, step, ist);
+        return rc2 ? rc2 : upload_frames(depths, f0, nf, s.d_depth, zpitch, rows, depth_step, ist);
+    };
+    h.compute = [&](Slot& s, int f0, int nf, cudaStream_t cst) -> int {
+        (void)f0;
+        int rc2 = run_chunk(ex, s, one_set_io(s.d_in, dframe, dpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), nf, 0, 0, cst);
+        if (rc2) return rc2;
+        RgbdArgs a = A;
+        a.kp = s.d_kps; a.n = s.d_n; a.capacity = capacity;
+        a.kp_un = s.d_kpun; a.uRight = s.d_su; a.depth_out = s.d_sd;
+        a.depth = s.d_depth; a.depth_pitch = zpitch; a.depth_frame_stride = zframe;
+        CU(launch_rgbd_frame(a, nf, cst));
+        return ORBX_OK;
+    };
+    h.counts = [&](Slot& s, int f0, int nf, cudaStream_t ost) -> int {
+        CU(cudaMemcpyAsync(n_out + f0, s.d_n, sizeof(int) * nf, cudaMemcpyDeviceToHost, ost));
+        return ORBX_OK;
+    };
+    h.download = [&](Slot& s, int f0, int nf, cudaStream_t ost) -> int {
+        int mx = 0;
+        for (int f = 0; f < nf; ++f) mx = std::max(mx, n_out[f0 + f]);
+        const size_t r = std::min(mx, capacity);      // a frame over capacity fails the call below
+        if (r == 0) return ORBX_OK;
+        const size_t kpitch = sizeof(orbx_keypoint) * (size_t)capacity, dpitch32 = (size_t)capacity * 32, fpitch = sizeof(float) * (size_t)capacity;
+        const size_t o = (size_t)f0 * capacity;
+        CU(cudaMemcpy2DAsync(kp + o, kpitch, s.d_kps, kpitch, sizeof(orbx_keypoint) * r, nf, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpy2DAsync(desc + o * 32, dpitch32, s.d_desc, dpitch32, r * 32, nf, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpy2DAsync(kp_un + o, kpitch, s.d_kpun, kpitch, sizeof(orbx_keypoint) * r, nf, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpy2DAsync(uRight + o, fpitch, s.d_su, fpitch, sizeof(float) * r, nf, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpy2DAsync(depth_out + o, fpitch, s.d_sd, fpitch, sizeof(float) * r, nf, cudaMemcpyDeviceToHost, ost));
+        return ORBX_OK;
+    };
+    if ((rc = run_host_pipeline(ex, sched, nslots, chunk >= 128, h))) return rc;
+    for (int f = 0; f < n_frames; ++f)
+        if (n_out[f] > capacity) return fail(ORBX_ERR_CAPACITY, "frame %d has %d keypoints, capacity %d", f, n_out[f], capacity);
+    return ORBX_OK;
+}
+
+int orbx_extract_rgbd_batch_device(orbx_extractor* ex, const uint8_t* d_images, size_t frame_stride, size_t pitch, const void* d_depths,
+                                   size_t depth_frame_stride, size_t depth_pitch, int depth_type, int n_frames, int rows, int cols,
+                                   const orbx_rgbd_calib* calib, orbx_keypoint* d_kp, orbx_keypoint* d_kp_un, uint8_t* d_desc,
+                                   int capacity, int* d_n_out, float* d_uRight, float* d_depth, void* stream)
+{
+    if (!ex) return fail(ORBX_ERR_INVALID_ARG, "extractor is NULL");
+    if (n_frames < 0) return fail(ORBX_ERR_INVALID_ARG, "n_frames %d < 0", n_frames);
+    if (n_frames == 0) return ORBX_OK;
+    if (!d_images || rows <= 0 || cols <= 0) return fail(ORBX_ERR_EMPTY_IMAGE, "empty image");
+    if (!d_kp || !d_kp_un || !d_desc || !d_n_out || !d_uRight || !d_depth || capacity <= 0 || pitch < (size_t)cols || !d_depths)
+        return fail(ORBX_ERR_INVALID_ARG, "bad depth maps / output buffers / pitch");
+    RgbdArgs A;
+    int rc = rgbd_args(calib, depth_type, depth_pitch, cols, A);
+    if (rc) return rc;
+    const size_t elem = depth_type == 0 ? 2 : 4;
+    if (((size_t)d_depths | depth_pitch | depth_frame_stride) % elem)
+        return fail(ORBX_ERR_INVALID_ARG, "depth maps: base, pitch and frame stride must be multiples of %zu bytes", elem);
+    if ((rc = set_device(ex->device))) return rc;
+    if ((rc = configure(ex, rows, cols))) return rc;
+    ex->last_frames = 0;
+    const int chunk = ex->max_batch > 0 ? std::min(ex->max_batch, n_frames) : std::min(n_frames, 256);
+    if ((rc = ensure_capacity(ex, chunk, 1))) return rc;
+    Slot& s = ex->slots[0];
+    // the extraction's monoIndex goes to the stereo staging's d_snm (2 * pairs counts; RGB-D outputs have no n_mono)
+    if (!stereo_staging_fits(s, chunk, 0)) {          // replaced below: earlier work on any stream must be done with it
+        wait_user_work(ex);
+        CU(cudaStreamSynchronize(s.stream));
+        if ((rc = ensure_stereo_staging(s, chunk, 0))) return rc;
+    }
+    cudaStream_t st = stream ? (cudaStream_t)stream : s.stream;
+    if (!ex->ev_user) CU(cudaEventCreateWithFlags(&ex->ev_user, cudaEventDisableTiming));
+    if (ex->user_pending) CU(cudaStreamWaitEvent(st, ex->ev_user, 0));
+    if (st != s.stream) { CU(cudaEventRecord(s.ev_done, s.stream)); CU(cudaStreamWaitEvent(st, s.ev_done, 0)); }
+    for (int f0 = 0; f0 < n_frames; f0 += chunk) {
+        const int nf = std::min(chunk, n_frames - f0);
+        const size_t r = (size_t)f0 * capacity;
+        if ((rc = run_chunk(ex, s, one_set_io(d_images + (size_t)f0 * frame_stride, frame_stride, pitch, d_kp + r, d_desc + r * 32, capacity,
+                                              d_n_out + f0, s.d_snm), nf, 0, 0, st)))
+            return rc;
+        RgbdArgs a = A;
+        a.kp = d_kp + r; a.n = d_n_out + f0; a.capacity = capacity;
+        a.kp_un = d_kp_un + r; a.uRight = d_uRight + r; a.depth_out = d_depth + r;
+        a.depth = (const uint8_t*)d_depths + (size_t)f0 * depth_frame_stride; a.depth_pitch = depth_pitch; a.depth_frame_stride = depth_frame_stride;
+        CU(launch_rgbd_frame(a, nf, st));
     }
     if (st != s.stream) { CU(cudaEventRecord(ex->ev_user, st)); ex->user_pending = true; }
     return ORBX_OK;

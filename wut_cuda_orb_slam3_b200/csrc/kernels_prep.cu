@@ -3,6 +3,8 @@
 //   * Frame::UndistortKeyPoints (src/Frame.cc:777-810) = cv::undistortPoints(pts, K, mDistCoef, R = I, P = mK): normalise,
 //     5 fixed-point iterations of the inverse radial-tangential distortion, re-project; double arithmetic, float results.
 //     One thread per key point; --fmad=false keeps every multiply and add separately rounded like the x86-64 build of OpenCV.
+//   * The RGB-D Frame constructor's tail (src/Frame.cc:202-260): the same undistortion plus ComputeStereoFromRGBD, one depth
+//     sample per key point (rgbd_frame_kernel).
 //   * System::TrackStereo rectification (src/System.cc:253-260) = cv::remap(im, out, M1, M2, INTER_LINEAR) with CV_32FC1 maps:
 //     the map is quantised ONCE to OpenCV's 1/32-pixel fixed point (remap_quantise_kernel), every frame then costs four
 //     gathers and one 15-bit fixed-point blend per pixel.  The packed map (8 bytes per pixel) stays L2-resident across a
@@ -13,12 +15,8 @@
 
 namespace orbx {
 
-__global__ void __launch_bounds__(128) undistort_kernel(const orbx_keypoint* __restrict__ in, int n, UndistortParams p,
-                                                        orbx_keypoint* __restrict__ out)
+__device__ __forceinline__ orbx_keypoint undistort_point(orbx_keypoint kp, const UndistortParams& p)
 {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    orbx_keypoint kp = in[i];
     const double* k = p.k;
     const double ifx = 1. / p.fx, ify = 1. / p.fy;
     const double u = kp.x, v = kp.y;
@@ -40,7 +38,40 @@ __global__ void __launch_bounds__(128) undistort_kernel(const orbx_keypoint* __r
     const double ww = 1. / (0.0 * x + 0.0 * y + 1.0);
     kp.x = (float)(xx * ww);
     kp.y = (float)(yy * ww);
-    out[i] = kp;
+    return kp;
+}
+
+__global__ void __launch_bounds__(128) undistort_kernel(const orbx_keypoint* __restrict__ in, int n, UndistortParams p,
+                                                        orbx_keypoint* __restrict__ out)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    out[i] = undistort_point(in[i], p);
+}
+
+// The tail of the RGB-D Frame constructor (src/Frame.cc:202-260) per keypoint, grid (ceil(capacity / 128), frames): mvKeysUn
+// (UndistortKeyPoints, :777-810), then ComputeStereoFromRGBD (:1014-1035) on ONE depth sample at the truncated coordinates of
+// the DISTORTED keypoint.  Tracking::GrabImageRGBD's convertTo(CV_32F, mDepthMapFactor) is element-wise, so converting only the
+// sampled pixel gives the same float as converting the whole map: fl32((float)v * factor), one rounding (OpenCV's + 0 only turns
+// a -0 product into +0, which `d > 0` does not tell apart).  The index is in
+// bounds by construction (keypoints keep EDGE_THRESHOLD - 3 pixels from every level's edge).  A frame whose count exceeds the
+// capacity has no keypoint rows: nothing is read or written for it.
+__global__ void __launch_bounds__(128) rgbd_frame_kernel(RgbdArgs a)
+{
+    const int f = blockIdx.y, i = blockIdx.x * blockDim.x + threadIdx.x;
+    const int n = a.n[f];
+    if (n > a.capacity || i >= n) return;
+    const size_t r = (size_t)f * a.capacity + i;
+    const orbx_keypoint kp = a.kp[r];
+    const orbx_keypoint un = a.undistort ? undistort_point(kp, a.p) : kp;
+    a.kp_un[r] = un;
+    const uint8_t* row = a.depth + (size_t)f * a.depth_frame_stride + (size_t)(int)kp.y * a.depth_pitch;
+    float d = a.depth_type == 0 ? (float)reinterpret_cast<const uint16_t*>(row)[(int)kp.x] : reinterpret_cast<const float*>(row)[(int)kp.x];
+    if (a.convert) d = __fmul_rn(d, a.factor);
+    float u = -1.f, z = -1.f;
+    if (d > 0) { z = d; u = __fsub_rn(un.x, __fdiv_rn(a.bf, d)); }
+    a.uRight[r] = u;
+    a.depth_out[r] = z;
 }
 
 // cvRound(map * 32) -> (sx | sy << 16, fx | fy << 5); sx, sy saturate to int16 like OpenCV's XY buffer.
@@ -361,6 +392,14 @@ cudaError_t launch_undistort(const orbx_keypoint* d_in, int n, const UndistortPa
 {
     if (n <= 0) return cudaSuccess;
     undistort_kernel<<<(n + 127) / 128, 128, 0, st>>>(d_in, n, p, d_out);
+    count_launch();
+    return cudaGetLastError();
+}
+
+cudaError_t launch_rgbd_frame(const RgbdArgs& a, int n_frames, cudaStream_t st)
+{
+    if (n_frames <= 0) return cudaSuccess;
+    rgbd_frame_kernel<<<dim3((a.capacity + 127) / 128, n_frames), 128, 0, st>>>(a);
     count_launch();
     return cudaGetLastError();
 }

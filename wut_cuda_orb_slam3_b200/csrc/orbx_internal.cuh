@@ -327,6 +327,19 @@ struct UndistortParams {
     int n_dist;
 };
 cudaError_t launch_undistort(const orbx_keypoint* d_in, int n, const UndistortParams& p, orbx_keypoint* d_out, cudaStream_t st);
+// mvKeysUn + ComputeStereoFromRGBD of n_frames frames.  Frame f: counts n[f], keypoint rows f * capacity of kp / kp_un / uRight /
+// depth_out, depth map at depth + f * depth_frame_stride (depth_pitch bytes per row, u16 or f32 elements).
+struct RgbdArgs {
+    const orbx_keypoint* kp; const int* n; int capacity;
+    orbx_keypoint* kp_un; float* uRight; float* depth_out;
+    const uint8_t* depth; size_t depth_pitch, depth_frame_stride;
+    int depth_type;              // 0: CV_16U, 1: CV_32F
+    int convert;                 // GrabImageRGBD's predicate, evaluated on the host: multiply the sample by `factor`
+    float factor, bf;
+    int undistort;               // 0: mvKeysUn = mvKeys (mDistCoef[0] == 0, src/Frame.cc:779-783)
+    UndistortParams p;
+};
+cudaError_t launch_rgbd_frame(const RgbdArgs& a, int n_frames, cudaStream_t st);
 cudaError_t launch_remap_quantise(const float* d_mapx, const float* d_mapy, size_t map_step, int dw, int dh, uint2* d_packed, cudaStream_t st);
 cudaError_t launch_remap(const uint8_t* d_src, int sw, int sh, size_t spitch, size_t sframe, const uint2* d_packed, uint8_t* d_dst, int dw,
                          int dh, size_t dpitch, size_t dframe, int n_frames, cudaStream_t st);

@@ -163,6 +163,39 @@ class ORBextractor:
                                                      ptr(d_nR), capacity, ptr(d_uRight), ptr(d_depth), ptr(stream) if stream else None))
         self._shape = (rows, cols)
 
+    def extract_rgbd_batch(self, images, depths, K, dist, bf, depth_factor):
+        """The RGB-D Frame constructor (src/Frame.cc:202-260) over N frames on this handle: images [N,H,W] uint8 grey, depths the
+        RAW [N,H,W] uint16 or float32 maps (host, ideally page-locked), depth_factor = mDepthMapFactor.  Returns (n[N], kp[N,cap],
+        kp_un[N,cap], desc[N,cap,32], uRight[N,cap], depth[N,cap]); rows of frame i past n[i] are undefined."""
+        from .prep import _depth_type, rgbd_calib
+        assert images.dtype == np.uint8 and images.ndim == 3 and images.strides[2] == 1
+        assert depths.ndim == 3 and depths.shape == images.shape and depths.strides[2] == depths.itemsize
+        N, rows, cols = images.shape
+        calib, _keep = rgbd_calib(K, dist, bf, depth_factor)
+        cap = self.max_keypoints(rows, cols)
+        kp = np.zeros((N, cap), KP_DTYPE); kp_un = np.zeros((N, cap), KP_DTYPE); desc = np.zeros((N, cap, 32), np.uint8)
+        u = np.full((N, cap), -1.0, np.float32); z = np.full((N, cap), -1.0, np.float32)
+        n = np.zeros(N, np.int32)
+        pi = (C.c_void_p * max(N, 1))(*[images.ctypes.data + i * images.strides[0] for i in range(N)])
+        pd = (C.c_void_p * max(N, 1))(*[depths.ctypes.data + i * depths.strides[0] for i in range(N)])
+        check(lib().orbx_extract_rgbd_batch(self._h, pi, pd, N, rows, cols, images.strides[1], _depth_type(depths), depths.strides[1],
+                                            C.byref(calib), ptr(kp), ptr(kp_un), ptr(desc), cap, ptr(n), ptr(u), ptr(z)))
+        self._shape = (rows, cols)
+        return n, kp, kp_un, desc, u, z
+
+    def extract_rgbd_batch_device(self, d_images, d_depths, n_frames, rows, cols, pitch, frame_stride, depth_type, depth_pitch,
+                                  depth_frame_stride, K, dist, bf, depth_factor, d_kp, d_kp_un, d_desc, capacity, d_n, d_uRight, d_depth,
+                                  stream=None):
+        """Device-resident RGB-D batch: every argument named d_* is a device pointer (int) or a torch CUDA tensor; depth_type 0 =
+        uint16, 1 = float32; the outputs are [n_frames][capacity] slabs (counts [n_frames])."""
+        from .prep import rgbd_calib
+        calib, _keep = rgbd_calib(K, dist, bf, depth_factor)
+        check(lib().orbx_extract_rgbd_batch_device(self._h, ptr(d_images), frame_stride, pitch, ptr(d_depths), depth_frame_stride,
+                                                   depth_pitch, int(depth_type), n_frames, rows, cols, C.byref(calib), ptr(d_kp),
+                                                   ptr(d_kp_un), ptr(d_desc), capacity, ptr(d_n), ptr(d_uRight), ptr(d_depth),
+                                                   ptr(stream) if stream else None))
+        self._shape = (rows, cols)
+
     def sync(self):
         check(lib().orbx_sync(self._h))
 

@@ -1,11 +1,13 @@
 """Host mirror of the preparation steps either side of the extractor (SURVEY.md §8(f)3) over the C ABI:
-Frame::UndistortKeyPoints (src/Frame.cc:777-810) and the stereo rectification of System::TrackStereo (src/System.cc:253-260).
-GPU only; no CPU fallback."""
+Frame::UndistortKeyPoints (src/Frame.cc:777-810), the stereo rectification of System::TrackStereo (src/System.cc:253-260) and
+the RGB-D Frame constructor (src/Frame.cc:202-260, with Tracking::GrabImageRGBD's conversions).  GPU only; no CPU fallback."""
 import ctypes as C
 
 import numpy as np
 
-from .capi import KP_DTYPE, check, lib, ptr
+from .capi import KP_DTYPE, RgbdCalibC, check, lib, ptr
+
+DEPTH_TYPES = {np.dtype(np.uint16): 0, np.dtype(np.float32): 1}      # CV_16U, CV_32F
 
 
 def undistort_keypoints(keypoints, K, dist, new_K=None, device=0):
@@ -17,6 +19,52 @@ def undistort_keypoints(keypoints, K, dist, new_K=None, device=0):
     out = np.zeros_like(kps)
     check(lib().orbx_undistort_keypoints(device, ptr(kps), len(kps), ptr(K), ptr(d), len(d), ptr(P), ptr(out)))
     return out
+
+
+def rgbd_calib(K, dist, bf, depth_factor):
+    """orbx_rgbd_calib from K = (fx, fy, cx, cy), dist = mDistCoef (0, 4, 5, 8 or 12 floats), mbf and mDepthMapFactor.  Returns
+    (struct, coefficient array); keep the array alive while the struct is in use."""
+    d = np.ascontiguousarray(dist if dist is not None else [], np.float32)
+    c = RgbdCalibC()
+    c.K[:] = [float(v) for v in np.asarray(K, np.float32)]
+    c.dist = d.ctypes.data if len(d) else None
+    c.n_dist = len(d)
+    c.bf = float(bf)
+    c.depth_factor = float(depth_factor)
+    return c, d
+
+
+def _depth_type(depth):
+    if depth.dtype not in DEPTH_TYPES:
+        raise TypeError("depth map must be uint16 (CV_16U) or float32 (CV_32F), got %s" % depth.dtype)
+    return DEPTH_TYPES[depth.dtype]
+
+
+def extract_rgbd(ex, image, depth, K, dist, bf, depth_factor, rgb=True):
+    """The RGB-D Frame constructor in one call (src/Frame.cc:202-260): image HxW grey or HxWx3 / HxWx4 colour (rgb = mbRGB),
+    depth the RAW HxW map (uint16 or float32) and depth_factor = mDepthMapFactor, applied as Tracking::GrabImageRGBD does.
+    Returns (mvKeys, mvKeysUn, descriptors, mvuRight, mvDepth)."""
+    image = np.asarray(image, np.uint8)
+    if image.ndim == 3 and (image.strides[2] != 1 or image.strides[1] != image.shape[2]):
+        image = np.ascontiguousarray(image)
+    if image.ndim == 2 and image.strides[1] != 1:
+        image = np.ascontiguousarray(image)
+    rows, cols = image.shape[:2]
+    ch = image.shape[2] if image.ndim == 3 else 1
+    depth = np.asarray(depth)
+    if depth.strides[1] != depth.itemsize:
+        depth = np.ascontiguousarray(depth)
+    assert depth.shape == (rows, cols), (depth.shape, image.shape)
+    calib, _keep = rgbd_calib(K, dist, bf, depth_factor)
+    cap = ex.max_keypoints(rows, cols)
+    kp = np.zeros(cap, KP_DTYPE); kp_un = np.zeros(cap, KP_DTYPE); desc = np.zeros((cap, 32), np.uint8)
+    u = np.full(cap, -1.0, np.float32); z = np.full(cap, -1.0, np.float32)
+    n = C.c_int(0)
+    check(lib().orbx_extract_rgbd(ex._h, ptr(image), rows, cols, image.strides[0], ch, int(bool(rgb)), ptr(depth), _depth_type(depth),
+                                  depth.strides[0], C.byref(calib), ptr(kp), ptr(kp_un), ptr(desc), cap, C.byref(n), ptr(u), ptr(z)))
+    ex._shape = (rows, cols)
+    k = n.value
+    return kp[:k].copy(), kp_un[:k].copy(), desc[:k].copy(), u[:k].copy(), z[:k].copy()
 
 
 class Rectifier:
