@@ -393,11 +393,38 @@ typedef struct orbx_feature_vector {
  * Outputs: mode 0: match_b[nB] = index of the A feature whose map point was assigned to B's feature j (vpMapPointMatches),
  *          mode 1: match_a[nA] = index of the B feature matched to A's feature i (vpMatches12), -1 = none; the other array
  *          (may be NULL) receives the inverse map.  *n_matches = the reference's return value (after the rotation filter).
- * Mode 0 uses the tracking thread's device scratch, mode 1 the loop-closing thread's. */
+ * Mode 0 uses the tracking thread's device scratch, mode 1 the loop-closing thread's.
+ * orbx_search_by_bow_batch with one key frame (pKF in mode 0, pKF2 in mode 1): the same checks, results and device scratch. */
 int orbx_search_by_bow(int device, int mode, const uint8_t* desc_a, const float* angle_a, const uint8_t* valid_a, int n_a,
                        const orbx_feature_vector* fv_a, const uint8_t* desc_b, const float* angle_b, const uint8_t* valid_b,
                        int n_b, const orbx_feature_vector* fv_b, int nleft_b, float nn_ratio, int check_orientation,
                        int32_t* match_a, int32_t* match_b, int* n_matches);
+
+/* One key frame of orbx_search_by_bow_batch: the side that changes from search to search (HOST pointers). */
+typedef struct orbx_bow_view {
+    int n;                       /* N of the key frame */
+    const uint8_t* desc;         /* mDescriptors, n x 32 */
+    const float* angle;          /* mvKeysUn[i].angle; may be NULL without check_orientation */
+    const uint8_t* valid;        /* [n] != 0 <=> the feature's map point is non-NULL and !isBad() */
+    orbx_feature_vector fv;      /* mFeatVec */
+} orbx_bow_view;
+/* orbx_search_by_bow of one fixed side against n_kf key frames in one call.  The two place-recognition loops of ORB-SLAM3:
+ *   mode 0, Tracking::Relocalization (src/Tracking5.cc:63-83): SearchByBoW(vpCandidateKFs[i], mCurrentFrame, ...) per candidate.
+ *           The fixed side is B, the Frame (valid is not read, may be NULL; nleft = F.Nleft as nleft_b); kfs[k] is an A side.
+ *           match[k * n + j] = index in kfs[k] whose map point the Frame's feature j received (match_b of the single call).
+ *   mode 1, LoopClosing::DetectCommonRegionsFromBoW (src/LoopClosing1.cc:591-662): SearchByBoW(mpCurrentKF, vpCovKFi[j], ...)
+ *           per covisible.  The fixed side is A, KF1 (nleft must be -1); kfs[k] is a B side, KF2.
+ *           match[k * n + i] = index in kfs[k] matched to KF1's feature i (match_a of the single call).
+ * n_matches[k] = the return value for key frame k.  Row k is bit-identical to orbx_search_by_bow on that key frame with the same
+ * nn_ratio and check_orientation (rotation filter included): neither loop changes map state between its searches, so the
+ * searches are independent.  The fixed side is uploaded once and every key frame's arrays in one packed copy; the common
+ * vocabulary nodes are found on the GPU and one launch searches every key frame (DESIGN.md §5f).
+ * n_kf == 0 does nothing; n_kf > 65535 is ORBX_ERR_UNSUPPORTED.  ORBX_ERR_INVALID_ARG, before any work is queued, for the single
+ * call's argument errors on the fixed side or on any view (null arrays, a malformed feature vector, an index out of range,
+ * angles missing under check_orientation).  Mode 0 uses the tracking thread's device scratch, mode 1 the loop-closing thread's. */
+int orbx_search_by_bow_batch(int device, int mode, const uint8_t* desc, const float* angle, const uint8_t* valid, int n,
+                             const orbx_feature_vector* fv, int nleft, int n_kf, const orbx_bow_view* kfs, float nn_ratio,
+                             int check_orientation, int32_t* match, int* n_matches);
 
 /* int ORBmatcher::SearchForTriangulation(pKF1, pKF2, vMatchedPairs, bOnlyStereo, bCoarse) — src/ORBmatcher2.cc:173-471, the
  * single-camera (pinhole, !mpCamera2) path.  Per feature of KF1 without a map point: scan the features of KF2 in the same

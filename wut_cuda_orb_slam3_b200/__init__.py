@@ -6,7 +6,7 @@ the built library raises (no CPU fallback).
 """
 from . import capi, synth  # noqa: F401
 from .capi import KP_DTYPE, OrbxError, lib  # noqa: F401
-from .bow import (FeatureVector, ORBVocabulary, search_by_bow, search_for_triangulation,  # noqa: F401
+from .bow import (FeatureVector, ORBVocabulary, search_by_bow, search_by_bow_batch, search_for_triangulation,  # noqa: F401
                   search_for_triangulation_batch)
 from .extractor import ORBextractor, compute_tables, distribute_octree  # noqa: F401
 from .prep import Rectifier, extract_rgbd, undistort_keypoints  # noqa: F401

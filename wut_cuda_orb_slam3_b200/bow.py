@@ -5,7 +5,7 @@ import ctypes as C
 
 import numpy as np
 
-from .capi import FeatureVectorC, KP_DTYPE, TriangulationViewC, check, lib, ptr
+from .capi import BowViewC, FeatureVectorC, KP_DTYPE, TriangulationViewC, check, lib, ptr
 
 TF_IDF, TF, IDF, BINARY = 0, 1, 2, 3
 L1_NORM, L2_NORM, CHI_SQUARE, KL, BHATTACHARYYA, DOT_PRODUCT = 0, 1, 2, 3, 4, 5
@@ -109,6 +109,34 @@ def search_by_bow(desc_a, angle_a, valid_a, fv_a, desc_b, angle_b, fv_b, valid_b
                                    ptr(vb), len(db), C.addressof(fb), nleft_b, float(nnratio), int(check_orientation), ptr(ma), ptr(mb),
                                    C.byref(nm)))
     return mb, ma, nm.value
+
+
+def search_by_bow_batch(desc, angle, valid, fv, kfs, kf_kf=False, nleft=-1, nnratio=0.6, check_orientation=True, device=0):
+    """ORBmatcher::SearchByBoW of one fixed side against many key frames in one call (orbx_search_by_bow_batch).  `kfs` is a
+    sequence of dicts with desc, angle, valid and fv.  kf_kf False (Tracking::Relocalization): the fixed side is the Frame
+    (`valid` may be None) and each entry a candidate key frame; match[k, j] = feature of kfs[k] whose map point the Frame's
+    feature j received.  kf_kf True (LoopClosing::DetectCommonRegionsFromBoW): the fixed side is KF1 and each entry a KF2;
+    match[k, i] = feature of kfs[k] matched to KF1's feature i.  Returns (match [n_kf, n], nmatches [n_kf]); row k equals
+    search_by_bow on kfs[k]."""
+    d = np.ascontiguousarray(desc, np.uint8).reshape(-1, 32)
+    a = np.ascontiguousarray(angle, np.float32)
+    v = np.ascontiguousarray(valid, np.uint8) if valid is not None else None
+    n_kf = len(kfs)
+    keep = []                                  # the arrays the views point into stay alive for the call
+    views = (BowViewC * max(n_kf, 1))()
+    for k, kf in enumerate(kfs):
+        dk = np.ascontiguousarray(kf["desc"], np.uint8).reshape(-1, 32)
+        ak = np.ascontiguousarray(kf["angle"], np.float32) if kf["angle"] is not None else None
+        vk = np.ascontiguousarray(kf["valid"], np.uint8)
+        keep += [dk, ak, vk, kf["fv"]]
+        w = views[k]
+        w.n = len(dk); w.desc = ptr(dk); w.angle = ptr(ak); w.valid = ptr(vk); w.fv = kf["fv"].c_struct()
+    match = np.full((n_kf, len(d)), -1, np.int32)
+    nm = np.zeros(n_kf, np.int32)
+    f = fv.c_struct()
+    check(lib().orbx_search_by_bow_batch(device, 1 if kf_kf else 0, ptr(d), ptr(a), ptr(v), len(d), C.addressof(f), nleft, n_kf,
+                                         C.addressof(views), float(nnratio), int(check_orientation), ptr(match), ptr(nm)))
+    return match, nm
 
 
 def search_for_triangulation(kp_a, desc_a, free_a, stereo_a, fv_a, kp_b, desc_b, free_b, stereo_b, fv_b, F12, ep, scale_b, sigma2_b,

@@ -89,6 +89,7 @@ SIGNATURES = {
     "orbx_compute_bow": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "orbx_bow_score": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _i, C.POINTER(C.c_double)]),
     "orbx_search_by_bow": (_i, [_i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _vp, _i, _f, _i, _vp, _vp, _vp]),
+    "orbx_search_by_bow_batch": (_i, [_i, _i, _vp, _vp, _vp, _i, _vp, _i, _i, _vp, _f, _i, _vp, _vp]),
     "orbx_search_for_triangulation": (_i, [_i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _i,
                                            _i, _i, _vp, _vp]),
     "orbx_search_for_triangulation_batch": (_i, [_i, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _i, _i, _vp, _vp]),
@@ -122,6 +123,11 @@ SIGNATURES = {
 class FeatureVectorC(C.Structure):
     """orbx_feature_vector (include/orbx.h): a DBoW2::FeatureVector in CSR form."""
     _fields_ = [("n_nodes", C.c_int), ("node_ids", _vp), ("offsets", _vp), ("indices", _vp)]
+
+
+class BowViewC(C.Structure):
+    """orbx_bow_view (include/orbx.h): one key frame of orbx_search_by_bow_batch."""
+    _fields_ = [("n", C.c_int), ("desc", _vp), ("angle", _vp), ("valid", _vp), ("fv", FeatureVectorC)]
 
 
 class TriangulationViewC(C.Structure):

@@ -11,6 +11,10 @@
 //   int SearchByProjection(Frame& Current, const Frame& Last, th, bMono)             src/ORBmatcher3.cc:256-467
 //   int SearchByBoW(KeyFrame*, Frame&, vector<MapPoint*>& vpMapPointMatches)         src/ORBmatcher1.cc:225-427
 //   int SearchByBoW(KeyFrame*, KeyFrame*, vector<MapPoint*>& vpMatches12)            src/ORBmatcher2.cc:36-171
+//   int SearchByBoW(const vector<KeyFrame*>&, Frame&, vector<vector<MapPoint*>>&, vector<int>&)
+//                                     (added: the candidate loop of Tracking::Relocalization in one call)
+//   int SearchByBoW(KeyFrame*, const vector<KeyFrame*>&, vector<vector<MapPoint*>>&, vector<int>&)
+//                                     (added: the covisible loop of LoopClosing::DetectCommonRegionsFromBoW in one call)
 //   int SearchForInitialization(Frame&, Frame&, vector<cv::Point2f>&, vector<int>&, windowSize)   src/ORBmatcher1.cc:650-765
 //   int Fuse(KeyFrame*, const vector<MapPoint*>&, th, bRight)                        src/ORBmatcher2.cc:420-610
 //   int Fuse(const vector<KeyFrame*>&, const vector<MapPoint*>&, th)  (added: the forward loop of SearchInNeighbors in one call)
@@ -361,6 +365,120 @@ public:
         for (int i = 0; i < nA; ++i)
             if (matchA[i] >= 0) vpMatches12[i] = vpMapPoints2[matchA[i]];
         return n;
+    }
+
+    // The candidate loop of Tracking::Relocalization: for every i, vnMatches[i] = SearchByBoW(vpKFs[i], F, vvpMapPointMatches[i]),
+    // except that a NULL or isBad() candidate is not searched (vnMatches[i] = 0, vvpMapPointMatches[i] empty), as the loop
+    // discards it.  One orbx_search_by_bow_batch call.  Every key frame's GetMapPointMatches() is read at entry: the loop changes
+    // no map state between its searches, and a change made by another thread between two of the reference's searches is a race
+    // the reference has too.  Returns the sum of vnMatches.  (Member templates like Fuse.)
+    template <class KF = KeyFrame, class FrameT = Frame, class MP = MapPoint>
+    int SearchByBoW(const std::vector<KF*>& vpKFs, FrameT& F, std::vector<std::vector<MP*>>& vvpMapPointMatches, std::vector<int>& vnMatches)
+    {
+        const int nK = (int)vpKFs.size();
+        vvpMapPointMatches.assign(nK, std::vector<MP*>());
+        vnMatches.assign(nK, 0);
+        std::vector<int> live;                                          // positions in vpKFs that are searched
+        std::vector<std::vector<MP*>> vpMPs;
+        std::vector<std::vector<uint8_t>> valid;
+        std::vector<std::vector<float>> ang;
+        std::vector<Csr> fv;
+        for (int i = 0; i < nK; ++i) {
+            KF* pKF = vpKFs[i];
+            if (!pKF || pKF->isBad()) continue;
+            live.push_back(i);
+            vpMPs.push_back(pKF->GetMapPointMatches());
+            const std::vector<MP*>& mp = vpMPs.back();
+            const int nA = (int)mp.size();
+            valid.emplace_back(nA); ang.emplace_back(nA);
+            for (int a = 0; a < nA; ++a) { valid.back()[a] = mp[a] && !mp[a]->isBad(); ang.back()[a] = pKF->mvKeysUn[a].angle; }   // :252-258, :335
+            fv.emplace_back(pKF->mFeatVec);
+        }
+        const int nL = (int)live.size();
+        if (nL == 0) return 0;
+        std::vector<orbx_bow_view> views(nL);
+        for (int k = 0; k < nL; ++k) {
+            KF* pKF = vpKFs[live[k]];
+            views[k] = orbx_bow_view{(int)vpMPs[k].size(), pKF->mDescriptors.ptr(0), ang[k].data(), valid[k].data(), fv[k].view()};
+        }
+        std::vector<float> angB(F.N);
+        for (int j = 0; j < F.N; ++j) angB[j] = F.mvKeys[j].angle;                                                               // :343
+        Csr fb(F.mFeatVec);
+        const orbx_feature_vector vb = fb.view();
+        std::vector<int32_t> match((size_t)nL * F.N, -1);
+        std::vector<int> nm(nL, 0);
+        orbx_adapter::check(orbx_search_by_bow_batch(device, 0, F.mDescriptors.ptr(0), angB.data(), nullptr, F.N, &vb, -1, nL, views.data(), mfNNratio,
+                                                     mbCheckOrientation, match.data(), nm.data()),
+                            "SearchByBoW");
+        int total = 0;
+        for (int k = 0; k < nL; ++k) {
+            std::vector<MP*>& out = vvpMapPointMatches[live[k]];
+            out.assign(F.N, static_cast<MP*>(NULL));
+            const int32_t* m = &match[(size_t)k * F.N];
+            for (int j = 0; j < F.N; ++j)
+                if (m[j] >= 0) out[j] = vpMPs[k][m[j]];
+            vnMatches[live[k]] = nm[k];
+            total += nm[k];
+        }
+        return total;
+    }
+
+    // The covisible loop of LoopClosing::DetectCommonRegionsFromBoW: for every j, vnMatches[j] = SearchByBoW(pKF1, vpKF2[j],
+    // vvpMatches12[j]), except that a NULL or isBad() entry is not searched (vnMatches[j] = 0, vvpMatches12[j] empty), as the
+    // loop skips it.  One orbx_search_by_bow_batch call; map points are read at entry, as in the overload above.  Returns the sum
+    // of vnMatches.
+    template <class KF = KeyFrame, class MP = MapPoint>
+    int SearchByBoW(KF* pKF1, const std::vector<KF*>& vpKF2, std::vector<std::vector<MP*>>& vvpMatches12, std::vector<int>& vnMatches)
+    {
+        const int nK = (int)vpKF2.size();
+        vvpMatches12.assign(nK, std::vector<MP*>());
+        vnMatches.assign(nK, 0);
+        const std::vector<MP*> vpMapPoints1 = pKF1->GetMapPointMatches();
+        const int nA = (int)vpMapPoints1.size();
+        std::vector<uint8_t> validA(nA);
+        std::vector<float> angA(nA);
+        for (int i = 0; i < nA; ++i) { validA[i] = vpMapPoints1[i] && !vpMapPoints1[i]->isBad(); angA[i] = pKF1->mvKeysUn[i].angle; }   // :73-82, :129
+        std::vector<int> live;
+        std::vector<std::vector<MP*>> vpMPs;
+        std::vector<std::vector<uint8_t>> valid;
+        std::vector<std::vector<float>> ang;
+        std::vector<Csr> fv;
+        for (int j = 0; j < nK; ++j) {
+            KF* pKF2 = vpKF2[j];
+            if (!pKF2 || pKF2->isBad()) continue;
+            live.push_back(j);
+            vpMPs.push_back(pKF2->GetMapPointMatches());
+            const std::vector<MP*>& mp = vpMPs.back();
+            const int nB = (int)mp.size();
+            valid.emplace_back(nB); ang.emplace_back(nB);
+            for (int b = 0; b < nB; ++b) { valid.back()[b] = mp[b] && !mp[b]->isBad(); ang.back()[b] = pKF2->mvKeysUn[b].angle; }   // :95-103
+            fv.emplace_back(pKF2->mFeatVec);
+        }
+        const int nL = (int)live.size();
+        if (nL == 0) return 0;
+        std::vector<orbx_bow_view> views(nL);
+        for (int k = 0; k < nL; ++k) {
+            KF* pKF2 = vpKF2[live[k]];
+            views[k] = orbx_bow_view{(int)vpMPs[k].size(), pKF2->mDescriptors.ptr(0), ang[k].data(), valid[k].data(), fv[k].view()};
+        }
+        Csr fa(pKF1->mFeatVec);
+        const orbx_feature_vector va = fa.view();
+        std::vector<int32_t> match((size_t)nL * nA, -1);
+        std::vector<int> nm(nL, 0);
+        orbx_adapter::check(orbx_search_by_bow_batch(device, 1, pKF1->mDescriptors.ptr(0), angA.data(), validA.data(), nA, &va, -1, nL, views.data(),
+                                                     mfNNratio, mbCheckOrientation, match.data(), nm.data()),
+                            "SearchByBoW");
+        int total = 0;
+        for (int k = 0; k < nL; ++k) {
+            std::vector<MP*>& out = vvpMatches12[live[k]];
+            out.assign(nA, static_cast<MP*>(NULL));
+            const int32_t* m = &match[(size_t)k * nA];
+            for (int i = 0; i < nA; ++i)
+                if (m[i] >= 0) out[i] = vpMPs[k][m[i]];
+            vnMatches[live[k]] = nm[k];
+            total += nm[k];
+        }
+        return total;
     }
 
 public:

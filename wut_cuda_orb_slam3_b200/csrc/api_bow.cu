@@ -52,17 +52,6 @@ int check_fv(const orbx_feature_vector* fv, int n_features, const char* name)
     return ORBX_OK;
 }
 
-// the lock-step walk over two ascending node lists (src/ORBmatcher1.cc:247-251, 397-404): pairs of positions with equal node id
-void common_nodes(const orbx_feature_vector* a, const orbx_feature_vector* b, std::vector<std::pair<int, int>>& out)
-{
-    int i = 0, j = 0;
-    while (i < a->n_nodes && j < b->n_nodes) {
-        if (a->node_ids[i] == b->node_ids[j]) { out.emplace_back(i, j); ++i; ++j; }
-        else if (a->node_ids[i] < b->node_ids[j]) ++i;      // lower_bound on an ascending list == advance
-        else ++j;
-    }
-}
-
 // SearchForTriangulation's rotation filter over vMatches12 (src/ORBmatcher2.cc:429-447); one histogram entry per match, so the
 // filter depends on bin sizes only.  *nm is decremented per dropped match.
 int tri_rotation_filter(const orbx_keypoint* kp_a, const orbx_keypoint* kp_b, int n_a, int32_t* mA, int* nm)
@@ -80,6 +69,144 @@ int tri_rotation_filter(const orbx_keypoint* kp_a, const orbx_keypoint* kp_b, in
     three_maxima(count, H, i1, i2, i3);
     for (int i = 0; i < n_a; ++i)
         if (bin[i] >= 0 && bin[i] != i1 && bin[i] != i2 && bin[i] != i3) { mA[i] = -1; --*nm; }
+    return ORBX_OK;
+}
+
+// SearchByBoW's rotation histogram + ComputeThreeMaxima over one key frame's row (src/ORBmatcher1.cc:344-356, 406-427;
+// src/ORBmatcher2.cc:127-139, 152-169).  One histogram entry per accepted match; the filter depends on bin sizes only, so the
+// entry order is irrelevant.  Mode 0: row[j] = A (key frame) index of the fixed Frame's feature j; mode 1: row[i] = B (key
+// frame) index of the fixed KF1's feature i.  inv / inv_right (may be NULL) are the key frame's inverse maps, kept consistent.
+// *nm is decremented per dropped match.
+int bow_rotation_filter(int mode, int n, int32_t* row, const float* angle_fixed, const float* angle_kf, int32_t* inv, int32_t* inv_right,
+                        int* nm)
+{
+    const int H = 30;
+    int count[H] = {0};
+    std::vector<int> bin(n, -1);
+    for (int t = 0; t < n; ++t) {
+        if (row[t] < 0) continue;
+        const int b = mode == 0 ? rotation_bin(angle_kf[row[t]], angle_fixed[t]) : rotation_bin(angle_fixed[t], angle_kf[row[t]]);
+        if (b < 0) return fail(ORBX_ERR_INVALID_ARG, "keypoint angles out of range (the reference asserts)");
+        bin[t] = b; count[b]++;
+    }
+    int i1, i2, i3;
+    three_maxima(count, H, i1, i2, i3);
+    for (int t = 0; t < n; ++t) {
+        if (bin[t] < 0 || bin[t] == i1 || bin[t] == i2 || bin[t] == i3) continue;
+        const int o = row[t];
+        row[t] = -1;
+        if (mode == 0) { if (inv && inv[o] == t) inv[o] = -1; if (inv_right && inv_right[o] == t) inv_right[o] = -1; }
+        else if (inv) inv[o] = -1;
+        --*nm;
+    }
+    return ORBX_OK;
+}
+
+// orbx_search_by_bow_batch, plus the inverse maps the single call returns: inv / inv_right (may be NULL) are HOST arrays over
+// the key frames' features, packed in order (sum of kfs[k].n): mode 0 match_a (inv_right: its right-camera twin), mode 1 match_b.
+// They are written only when n > 0 (the caller initialises them to -1).
+int search_by_bow_batch(int device, int mode, const uint8_t* desc, const float* angle, const uint8_t* valid, int n,
+                        const orbx_feature_vector* fv, int nleft, int n_kf, const orbx_bow_view* kfs, float nn_ratio, int check_orientation,
+                        int32_t* match, int* n_matches, int32_t* inv, int32_t* inv_right)
+{
+    if (n_kf < 0) return fail(ORBX_ERR_INVALID_ARG, "search_by_bow: n_kf < 0");
+    if (n_kf == 0) return ORBX_OK;
+    if (n_kf > 65535) return fail(ORBX_ERR_UNSUPPORTED, "search_by_bow: more than 65535 key frames");
+    if ((mode != 0 && mode != 1) || !kfs || !n_matches || n < 0 || (n > 0 && (!desc || !match)) || (mode == 1 && n > 0 && !valid) ||
+        (check_orientation && n > 0 && !angle))
+        return fail(ORBX_ERR_INVALID_ARG, "search_by_bow: bad arguments");
+    if (mode == 1 && nleft >= 0) return fail(ORBX_ERR_INVALID_ARG, "search_by_bow: nleft applies to mode 0 only");
+    int rc;
+    if ((rc = check_fv(fv, n, "fv"))) return rc;
+    // the single call's checks, per key frame
+    size_t n_feat = 0, n_nodes = 0, n_idx = 0;
+    for (int k = 0; k < n_kf; ++k) {
+        const orbx_bow_view& V = kfs[k];
+        if (V.n < 0 || (V.n > 0 && (!V.desc || !V.valid)) || (check_orientation && V.n > 0 && !V.angle))
+            return fail(ORBX_ERR_INVALID_ARG, "search_by_bow: kfs[%d]: bad arguments", k);
+        char name[32];
+        snprintf(name, sizeof name, "kfs[%d].fv", k);
+        if ((rc = check_fv(&V.fv, V.n, name))) return rc;
+        n_feat += (size_t)V.n; n_nodes += (size_t)V.fv.n_nodes; n_idx += V.fv.n_nodes ? (size_t)V.fv.offsets[V.fv.n_nodes] : 0;
+    }
+    const size_t rows = (size_t)n_kf * n;
+    if (n > 0) {
+        if ((rc = set_device(device))) return rc;
+        const int f_nodes = fv->n_nodes, f_idx = f_nodes ? fv->offsets[f_nodes] : 0;
+        const size_t vf = mode == 1 ? (size_t)n : 0;
+        // KF -> Frame runs on the tracking thread, KF <-> KF on loop closing
+        Lease L(device, mode == 0 ? g_arena : g_loop_arena);
+        const size_t total = lease_pad((size_t)n_kf * sizeof(BowKF)) + lease_pad((size_t)n * 32) + lease_pad(vf) + lease_pad((size_t)f_nodes * 4) +
+                             lease_pad((size_t)(f_nodes + 1) * 4) + lease_pad((size_t)f_idx * 4) + lease_pad(n_feat * 32) + lease_pad(n_feat) +
+                             lease_pad(n_nodes * 4) + lease_pad((n_nodes + n_kf) * 4) + lease_pad(n_idx * 4) +
+                             lease_pad((size_t)n_kf * f_nodes * 16) + lease_pad((size_t)n_kf * 4) + lease_pad(rows * 4) + 2 * lease_pad(n_feat * 4);
+        if ((rc = L.reserve(total))) return rc;
+        // upload range: the key-frame table, the fixed side once, then every key frame's arrays packed back to back
+        const size_t o_kf = L.take<BowKF>(n_kf), o_d = L.take<uint8_t>((size_t)n * 32), o_v = L.take<uint8_t>(vf),
+                     o_n = L.take<uint32_t>(f_nodes), o_o = L.take<int32_t>(f_nodes + 1), o_i = L.take<uint32_t>(f_idx),
+                     o_dk = L.take<uint8_t>(n_feat * 32), o_vk = L.take<uint8_t>(n_feat), o_nk = L.take<uint32_t>(n_nodes),
+                     o_ok = L.take<int32_t>(n_nodes + n_kf), o_ik = L.take<uint32_t>(n_idx);
+        L.upload_end = L.off;
+        // device-only scratch / outputs
+        const size_t o_jobs = L.take<int4>((size_t)n_kf * f_nodes), o_cnt = L.take<int>(n_kf), o_row = L.take<int>(rows),
+                     o_feat = L.take<int>(n_feat), o_right = L.take<int>(n_feat);
+        memcpy(L.host<uint8_t>(o_d), desc, (size_t)n * 32);
+        if (vf) memcpy(L.host<uint8_t>(o_v), valid, vf);
+        if (f_nodes) {
+            memcpy(L.host<uint32_t>(o_n), fv->node_ids, (size_t)f_nodes * 4);
+            memcpy(L.host<int32_t>(o_o), fv->offsets, (size_t)(f_nodes + 1) * 4);
+            if (f_idx) memcpy(L.host<uint32_t>(o_i), fv->indices, (size_t)f_idx * 4);
+        }
+        BowKF* T = L.host<BowKF>(o_kf);
+        size_t f0 = 0, n0 = 0, i0 = 0, b0 = 0;                   // running bases: features, node ids, indices, offsets
+        for (int k = 0; k < n_kf; ++k) {
+            const orbx_bow_view& V = kfs[k];
+            const int nn = V.fv.n_nodes, ni = nn ? V.fv.offsets[nn] : 0;
+            BowKF e{};
+            e.desc = L.dev<uint8_t>(o_dk) + f0 * 32; e.valid = L.dev<uint8_t>(o_vk) + f0;
+            e.node_ids = L.dev<uint32_t>(o_nk) + n0; e.offsets = L.dev<int32_t>(o_ok) + b0; e.indices = L.dev<uint32_t>(o_ik) + i0;
+            e.n = V.n; e.n_nodes = nn; e.base = f0;
+            T[k] = e;
+            if (V.n) {
+                memcpy(L.host<uint8_t>(o_dk) + f0 * 32, V.desc, (size_t)V.n * 32);
+                memcpy(L.host<uint8_t>(o_vk) + f0, V.valid, (size_t)V.n);
+            }
+            if (nn) {
+                memcpy(L.host<uint32_t>(o_nk) + n0, V.fv.node_ids, (size_t)nn * 4);
+                if (ni) memcpy(L.host<uint32_t>(o_ik) + i0, V.fv.indices, (size_t)ni * 4);
+            }
+            for (int p = 0; p <= nn; ++p) L.host<int32_t>(o_ok)[b0 + p] = nn ? V.fv.offsets[p] : 0;
+            f0 += (size_t)V.n; n0 += (size_t)nn; i0 += (size_t)ni; b0 += (size_t)nn + 1;
+        }
+        BowBatchArgs A{};
+        A.mode = mode; A.n_kf = n_kf; A.kfs = L.dev<BowKF>(o_kf);
+        A.n = n; A.desc = L.dev<uint8_t>(o_d); A.valid = vf ? L.dev<uint8_t>(o_v) : nullptr;
+        A.n_nodes = f_nodes; A.node_ids = L.dev<uint32_t>(o_n); A.offsets = L.dev<int32_t>(o_o); A.indices = L.dev<uint32_t>(o_i);
+        A.nleft = nleft; A.nn_ratio = nn_ratio;
+        A.jobs = L.dev<int4>(o_jobs); A.job_count = L.dev<int>(o_cnt); A.job_stride = f_nodes; A.row = L.dev<int>(o_row);
+        A.feat = mode == 1 || inv ? L.dev<int>(o_feat) : nullptr;
+        A.feat_right = mode == 0 && inv_right ? L.dev<int>(o_right) : nullptr;
+        cudaStream_t st = L.A.st;
+        cudaError_t e = cudaMemcpyAsync(L.A.d, L.A.h, L.upload_end, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) e = launch_search_by_bow_batch(A, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(match, A.row, rows * 4, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess && inv && n_feat) e = cudaMemcpyAsync(inv, A.feat, n_feat * 4, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess && A.feat_right && n_feat) e = cudaMemcpyAsync(inv_right, A.feat_right, n_feat * 4, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "search_by_bow: %s", cudaGetErrorString(e));
+    }
+    // the return value and the rotation filter per key frame, on the host as in the reference
+    size_t f0 = 0;
+    for (int k = 0; k < n_kf; ++k) {
+        int32_t* r = match + (size_t)k * n;
+        int nm = 0;
+        for (int t = 0; t < n; ++t) nm += r[t] >= 0;
+        if (check_orientation &&
+            (rc = bow_rotation_filter(mode, n, r, angle, kfs[k].angle, inv ? inv + f0 : nullptr, inv_right ? inv_right + f0 : nullptr, &nm)))
+            return rc;
+        n_matches[k] = nm;
+        f0 += (size_t)kfs[k].n;
+    }
     return ORBX_OK;
 }
 
@@ -291,84 +418,33 @@ int orbx_search_by_bow(int device, int mode, const uint8_t* desc_a, const float*
                        const orbx_feature_vector* fv_b, int nleft_b, float nn_ratio, int check_orientation, int32_t* match_a,
                        int32_t* match_b, int* n_matches)
 {
-    if ((mode != 0 && mode != 1) || n_a < 0 || n_b < 0 || !n_matches || (n_a > 0 && (!desc_a || !valid_a)) || (n_b > 0 && !desc_b) ||
-        (mode == 1 && n_b > 0 && !valid_b) || (check_orientation && ((n_a > 0 && !angle_a) || (n_b > 0 && !angle_b))))
-        return fail(ORBX_ERR_INVALID_ARG, "bad arguments");
-    if (mode == 1 && nleft_b >= 0) return fail(ORBX_ERR_INVALID_ARG, "nleft_b applies to mode 0 only");
-    int rc;
-    if ((rc = check_fv(fv_a, n_a, "fv_a")) || (rc = check_fv(fv_b, n_b, "fv_b"))) return rc;
+    // the one-key-frame batch; these are the arguments the view cannot carry (the batch checks the rest)
+    if ((mode != 0 && mode != 1) || n_a < 0 || n_b < 0 || !n_matches || !fv_a || !fv_b) return fail(ORBX_ERR_INVALID_ARG, "bad arguments");
+    const bool kf_frame = mode == 0;
+    orbx_bow_view V{};                                       // mode 0: A = pKF, mode 1: B = pKF2
+    if (kf_frame) { V.n = n_a; V.desc = desc_a; V.angle = angle_a; V.valid = valid_a; V.fv = *fv_a; }
+    else { V.n = n_b; V.desc = desc_b; V.angle = angle_b; V.valid = valid_b; V.fv = *fv_b; }
+    const int n = kf_frame ? n_b : n_a;
+    std::vector<int32_t> row(n, -1), inv(V.n, -1), inv_right(kf_frame && nleft_b >= 0 ? V.n : 0, -1);
     *n_matches = 0;
-    std::vector<int32_t> mA(n_a, -1), mAR(n_a, -1), mB(n_b, -1);
-    std::vector<std::pair<int, int>> common;
-    common_nodes(fv_a, fv_b, common);
-    if (!common.empty() && n_a > 0 && n_b > 0) {
-        if ((rc = set_device(device))) return rc;
-        std::vector<int4> pairs;
-        for (auto& c : common)
-            pairs.push_back(make_int4(fv_a->offsets[c.first], fv_a->offsets[c.first + 1], fv_b->offsets[c.second], fv_b->offsets[c.second + 1]));
-        // KF -> Frame runs on the tracking thread, KF <-> KF on loop closing
-        Lease L(device, mode == 0 ? g_arena : g_loop_arena);
-        const size_t ia = (size_t)fv_a->offsets[fv_a->n_nodes], ib = (size_t)fv_b->offsets[fv_b->n_nodes], vb = mode == 1 ? (size_t)n_b : 0;
-        if ((rc = L.reserve(lease_pad(pairs.size() * 16) + lease_pad(ia * 4) + lease_pad(ib * 4) + lease_pad((size_t)n_a * 32) +
-                            lease_pad((size_t)n_b * 32) + lease_pad((size_t)n_a) + lease_pad(vb) + lease_pad((size_t)n_b * 4) +
-                            2 * lease_pad((size_t)n_a * 4))))
-            return rc;
-        // upload range; the three match arrays (initialised to -1) come back in one copy
-        const size_t o_pairs = L.take<int4>(pairs.size()), o_ia = L.take<uint32_t>(ia), o_ib = L.take<uint32_t>(ib),
-                     o_da = L.take<uint8_t>((size_t)n_a * 32), o_db = L.take<uint8_t>((size_t)n_b * 32), o_va = L.take<uint8_t>(n_a),
-                     o_vb = L.take<uint8_t>(vb), o_mb = L.take<int>(n_b), o_ma = L.take<int>(n_a), o_mar = L.take<int>(n_a);
-        L.upload_end = L.off;
-        memcpy(L.host<int4>(o_pairs), pairs.data(), pairs.size() * 16);
-        memcpy(L.host<uint32_t>(o_ia), fv_a->indices, ia * 4);
-        memcpy(L.host<uint32_t>(o_ib), fv_b->indices, ib * 4);
-        memcpy(L.host<uint8_t>(o_da), desc_a, (size_t)n_a * 32);
-        memcpy(L.host<uint8_t>(o_db), desc_b, (size_t)n_b * 32);
-        memcpy(L.host<uint8_t>(o_va), valid_a, (size_t)n_a);
-        if (vb) memcpy(L.host<uint8_t>(o_vb), valid_b, vb);
-        memset(L.host<uint8_t>(o_mb), 0xff, L.upload_end - o_mb);
-        BowSearchArgs A{};
-        A.mode = mode; A.n_pairs = (int)pairs.size(); A.pairs = L.dev<int4>(o_pairs); A.idx_a = L.dev<uint32_t>(o_ia); A.idx_b = L.dev<uint32_t>(o_ib);
-        A.desc_a = L.dev<uint8_t>(o_da); A.desc_b = L.dev<uint8_t>(o_db); A.valid_a = L.dev<uint8_t>(o_va); A.valid_b = vb ? L.dev<uint8_t>(o_vb) : nullptr;
-        A.nleft_b = nleft_b; A.nn_ratio = nn_ratio; A.match_b = L.dev<int>(o_mb); A.match_a = L.dev<int>(o_ma); A.match_a_right = L.dev<int>(o_mar);
-        cudaStream_t st = L.A.st;
-        cudaError_t e = cudaMemcpyAsync(L.A.d, L.A.h, L.upload_end, cudaMemcpyHostToDevice, st);
-        if (e == cudaSuccess) e = launch_search_by_bow(A, st);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(L.host<int>(o_mb), A.match_b, L.upload_end - o_mb, cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-        if (e != cudaSuccess) return fail(ORBX_ERR_CUDA, "search_by_bow: %s", cudaGetErrorString(e));
-        memcpy(mB.data(), L.host<int>(o_mb), (size_t)n_b * 4);
-        memcpy(mA.data(), L.host<int>(o_ma), (size_t)n_a * 4);
-        memcpy(mAR.data(), L.host<int>(o_mar), (size_t)n_a * 4);
-    }
-    // rotation histogram + ComputeThreeMaxima (src/ORBmatcher1.cc:344-356, 406-427; src/ORBmatcher2.cc:127-139, 152-169).
-    // One histogram entry per accepted match; the filter depends on bin sizes only, so the entry order is irrelevant.
-    int nm = 0;
-    if (mode == 0) { for (int j = 0; j < n_b; ++j) nm += mB[j] >= 0; }
-    else { for (int i = 0; i < n_a; ++i) nm += mA[i] >= 0; }
-    if (check_orientation) {
-        const int H = 30;
-        int count[H] = {0};
-        std::vector<int> bin(mode == 0 ? n_b : n_a, -1);
-        for (int t = 0; t < (int)bin.size(); ++t) {
-            const int iA = mode == 0 ? mB[t] : t, jB = mode == 0 ? t : mA[t];
-            if (iA < 0 || jB < 0) continue;
-            const int b = rotation_bin(angle_a[iA], angle_b[jB]);
-            if (b < 0) return fail(ORBX_ERR_INVALID_ARG, "keypoint angles out of range (the reference asserts)");
-            bin[t] = b; count[b]++;
-        }
-        int i1, i2, i3;
-        three_maxima(count, H, i1, i2, i3);
-        for (int t = 0; t < (int)bin.size(); ++t) {
-            if (bin[t] < 0 || bin[t] == i1 || bin[t] == i2 || bin[t] == i3) continue;
-            if (mode == 0) { const int iA = mB[t]; mB[t] = -1; if (mA[iA] == t) mA[iA] = -1; if (mAR[iA] == t) mAR[iA] = -1; }
-            else { mB[mA[t]] = -1; mA[t] = -1; }
-            --nm;
-        }
-    }
-    if (match_a) for (int i = 0; i < n_a; ++i) match_a[i] = mA[i];
-    if (match_b) for (int j = 0; j < n_b; ++j) match_b[j] = mB[j];
-    *n_matches = nm;
+    const int rc = kf_frame ? search_by_bow_batch(device, 0, desc_b, angle_b, nullptr, n_b, fv_b, nleft_b, 1, &V, nn_ratio, check_orientation,
+                                                  row.data(), n_matches, inv.data(), inv_right.empty() ? nullptr : inv_right.data())
+                            : search_by_bow_batch(device, 1, desc_a, angle_a, valid_a, n_a, fv_a, nleft_b, 1, &V, nn_ratio, check_orientation,
+                                                  row.data(), n_matches, inv.data(), nullptr);
+    if (rc) return rc;
+    int32_t* out_row = kf_frame ? match_b : match_a;
+    int32_t* out_inv = kf_frame ? match_a : match_b;
+    if (out_row) std::copy(row.begin(), row.end(), out_row);
+    if (out_inv) std::copy(inv.begin(), inv.end(), out_inv);
     return ORBX_OK;
+}
+
+int orbx_search_by_bow_batch(int device, int mode, const uint8_t* desc, const float* angle, const uint8_t* valid, int n,
+                             const orbx_feature_vector* fv, int nleft, int n_kf, const orbx_bow_view* kfs, float nn_ratio,
+                             int check_orientation, int32_t* match, int* n_matches)
+{
+    return search_by_bow_batch(device, mode, desc, angle, valid, n, fv, nleft, n_kf, kfs, nn_ratio, check_orientation, match, n_matches,
+                               nullptr, nullptr);
 }
 
 int orbx_search_for_triangulation(int device, const orbx_keypoint* kp_a, const uint8_t* desc_a, const uint8_t* free_a,

@@ -6,7 +6,7 @@
 //   * ORBmatcher::SearchByBoW(KF, Frame) src/ORBmatcher1.cc:225-427 and SearchByBoW(KF, KF) src/ORBmatcher2.cc:36-171: per common
 //     vocabulary node, the A features are visited IN ORDER, each scans the node's B features for best / second-best distance
 //     (strict '<': the earlier candidate keeps a tie) and B features matched earlier are skipped — a sequential dependence
-//     inside a node, none across nodes (a feature belongs to exactly one node).
+//     inside a node, none across nodes (a feature belongs to exactly one node) and none across the key frames of a batch.
 //   * ORBmatcher::SearchForTriangulation src/ORBmatcher2.cc:173-471 (single pinhole camera): independent 1-NN per A feature
 //     with the epipole gate and Pinhole::epipolarConstrain (src/CameraModels/Pinhole.cpp:107-129).
 //
@@ -115,56 +115,115 @@ __device__ __forceinline__ void best2_warp_reduce(Best2& s)
 
 }  // namespace
 
-// One warp per common vocabulary node.  match_b doubles as the "already matched" state of B (mode 0: vpMapPointMatches,
-// mode 1: vbMatched2); it is read/written through L2 (ld.cg / st.cg) and ordered by __syncwarp between A features.
-__global__ void __launch_bounds__(128) search_by_bow_kernel(BowSearchArgs a)
+// Job build of key frame blockIdx.x: its row of the fixed side and its own per-feature rows = -1, then the common nodes of the
+// two ascending node lists (a node of the fixed side is looked up in the key frame's list by binary search: the node ids are
+// strictly ascending, so the equal pairs are those of the lock-step walk, src/ORBmatcher1.cc:247-251, 397-404), one job per
+// common node with features on both sides.  A node of the fixed side gives at most one job, so key frame k has at most
+// job_stride jobs; the order of the jobs is irrelevant (different nodes hold different features of both sides).
+__global__ void __launch_bounds__(256) bow_jobs_kernel(BowBatchArgs a)
+{
+    const int k = blockIdx.x;
+    const BowKF& K = a.kfs[k];
+    __shared__ int s_count;
+    if (threadIdx.x == 0) s_count = 0;
+    int* row = a.row + (size_t)k * a.n;
+    for (int i = threadIdx.x; i < a.n; i += blockDim.x) row[i] = -1;
+    for (int i = threadIdx.x; i < K.n; i += blockDim.x) {
+        if (a.feat) a.feat[K.base + i] = -1;
+        if (a.feat_right) a.feat_right[K.base + i] = -1;
+    }
+    __syncthreads();
+    const int nb = K.n_nodes;
+    int4* jobs = a.jobs + (size_t)k * a.job_stride;
+    for (int p = threadIdx.x; p < a.n_nodes; p += blockDim.x) {
+        const uint32_t id = __ldg(a.node_ids + p);
+        int lo = 0, hi = nb;                                 // first position of the key frame's list with node id >= id
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (__ldg(K.node_ids + mid) < id) lo = mid + 1;
+            else hi = mid;
+        }
+        if (lo == nb || __ldg(K.node_ids + lo) != id) continue;
+        const int f0 = __ldg(a.offsets + p), f1 = __ldg(a.offsets + p + 1), k0 = __ldg(K.offsets + lo), k1 = __ldg(K.offsets + lo + 1);
+        if (f0 == f1 || k0 == k1) continue;                  // no A feature to walk or no B feature to scan: no match either way
+        const int slot = atomicAdd(&s_count, 1);
+        jobs[slot] = a.mode == 0 ? make_int4(k0, k1, f0, f1) : make_int4(f0, f1, k0, k1);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) a.job_count[k] = s_count;
+}
+
+// One warp per job (a common vocabulary node) of key frame blockIdx.y.  match_b doubles as the "already matched" state of B
+// (mode 0: the key frame's row of vpMapPointMatches, mode 1: the key frame's vbMatched2); it is read/written through L2
+// (ld.cg / st.cg) and ordered by __syncwarp between A features.  kf_frame = mode 0.
+template <bool kf_frame>
+__global__ void __launch_bounds__(128) search_by_bow_kernel(BowBatchArgs a)
 {
     const int lane = threadIdx.x & 31;
-    const int p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (p >= a.n_pairs) return;
-    const int4 pr = __ldg(a.pairs + p);                      // (a_begin, a_end, b_begin, b_end) into the index arrays
+    const int k = blockIdx.y;
+    const int jb = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (jb >= __ldg(a.job_count + k)) return;
+    const BowKF* K = a.kfs + k;
+    const int4 pr = __ldg(a.jobs + (size_t)k * a.job_stride + jb);      // (a_begin, a_end, b_begin, b_end) into idx_a / idx_b
+    const size_t base = K->base;
+    const uint32_t* __restrict__ idx_a = kf_frame ? K->indices : a.indices;
+    const uint32_t* __restrict__ idx_b = kf_frame ? a.indices : K->indices;
+    const uint8_t* __restrict__ desc_a = kf_frame ? K->desc : a.desc;
+    const uint8_t* __restrict__ desc_b = kf_frame ? a.desc : K->desc;
+    const uint8_t* __restrict__ valid_a = kf_frame ? K->valid : a.valid;
+    const uint8_t* __restrict__ valid_b = K->valid;                         // read in mode 1 only
+    int* row = a.row + (size_t)k * a.n;
+    int* match_b = kf_frame ? row : a.feat + base;
+    int* match_a = kf_frame ? (a.feat ? a.feat + base : nullptr) : row;
+    int* match_a_right = kf_frame && a.feat_right ? a.feat_right + base : nullptr;
     const int TH_LOW = 50;                                   // src/ORBmatcher1.cc:37
     for (int ia = pr.x; ia < pr.y; ++ia) {
-        const int iA = (int)__ldg(a.idx_a + ia);
-        if (!__ldg(a.valid_a + iA)) continue;                // !pMP || pMP->isBad()   (src/ORBmatcher1.cc:259-265)
+        const int iA = (int)__ldg(idx_a + ia);
+        if (!__ldg(valid_a + iA)) continue;                  // !pMP || pMP->isBad()   (src/ORBmatcher1.cc:259-265)
         uint32_t q[8];
-        load_desc(a.desc_a, (size_t)iA, q);
+        load_desc(desc_a, (size_t)iA, q);
         Best2 L, R;
         best2_init(L); best2_init(R);
         for (int t = pr.z + lane; t < pr.w; t += 32) {
-            const int j = (int)__ldg(a.idx_b + t);
-            if (__ldcg(a.match_b + j) >= 0) continue;        // vpMapPointMatches[realIdxF] / vbMatched2[idx2]
-            if (a.mode == 1 && !__ldg(a.valid_b + j)) continue;      // !pMP2 || pMP2->isBad()   (src/ORBmatcher2.cc:95-103)
+            const int j = (int)__ldg(idx_b + t);
+            if (__ldcg(match_b + j) >= 0) continue;          // vpMapPointMatches[realIdxF] / vbMatched2[idx2]
+            if (!kf_frame && !__ldg(valid_b + j)) continue;  // !pMP2 || pMP2->isBad()   (src/ORBmatcher2.cc:95-103)
             uint32_t d[8];
-            load_desc(a.desc_b, (size_t)j, d);
+            load_desc(desc_b, (size_t)j, d);
             const int dist = hamming256(q, d);
-            if (a.nleft_b < 0 || j < a.nleft_b) best2_push(L, dist, t);
+            if (a.nleft < 0 || j < a.nleft) best2_push(L, dist, t);
             else best2_push(R, dist, t);                     // src/ORBmatcher1.cc:323-330
         }
         best2_warp_reduce(L);
-        if (a.nleft_b >= 0) best2_warp_reduce(R);
+        if (a.nleft >= 0) best2_warp_reduce(R);
         // acceptance (identical on all lanes); lane 0 writes
         int jL = -1, jR = -1;
-        if (a.mode == 0) {
+        if (kf_frame) {
             if (L.b1 <= TH_LOW) {                                                            // src/ORBmatcher1.cc:336
-                if ((float)L.b1 < __fmul_rn(a.nn_ratio, (float)L.b2)) jL = (int)__ldg(a.idx_b + L.t1);          // :338
-                if (a.nleft_b >= 0 && R.b1 <= TH_LOW) jR = (int)__ldg(a.idx_b + R.t1);       // :366-368 ('|| true')
+                if ((float)L.b1 < __fmul_rn(a.nn_ratio, (float)L.b2)) jL = (int)__ldg(idx_b + L.t1);            // :338
+                if (a.nleft >= 0 && R.b1 <= TH_LOW) jR = (int)__ldg(idx_b + R.t1);           // :366-368 ('|| true')
             }
         } else {
-            if (L.b1 < TH_LOW && (float)L.b1 < __fmul_rn(a.nn_ratio, (float)L.b2)) jL = (int)__ldg(a.idx_b + L.t1);  // ORBmatcher2.cc:120-122
+            if (L.b1 < TH_LOW && (float)L.b1 < __fmul_rn(a.nn_ratio, (float)L.b2)) jL = (int)__ldg(idx_b + L.t1);    // ORBmatcher2.cc:120-122
         }
         if (lane == 0) {
-            if (jL >= 0) { __stcg(a.match_b + jL, iA); if (a.match_a) a.match_a[iA] = jL; }
-            if (jR >= 0) { __stcg(a.match_b + jR, iA); if (a.match_a_right) a.match_a_right[iA] = jR; }
+            if (jL >= 0) { __stcg(match_b + jL, iA); if (match_a) match_a[iA] = jL; }
+            if (jR >= 0) { __stcg(match_b + jR, iA); if (match_a_right) match_a_right[iA] = jR; }
         }
         __syncwarp();
     }
 }
 
-cudaError_t launch_search_by_bow(const BowSearchArgs& a, cudaStream_t st)
+cudaError_t launch_search_by_bow_batch(const BowBatchArgs& a, cudaStream_t st)
 {
-    if (a.n_pairs <= 0) return cudaSuccess;
-    search_by_bow_kernel<<<(a.n_pairs + 3) / 4, 128, 0, st>>>(a);
+    if (a.n_kf <= 0 || a.n <= 0) return cudaSuccess;
+    bow_jobs_kernel<<<a.n_kf, 256, 0, st>>>(a);
+    count_launch();
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess || a.job_stride <= 0) return e;
+    const dim3 grid((a.job_stride + 3) / 4, a.n_kf);
+    if (a.mode == 0) search_by_bow_kernel<true><<<grid, 128, 0, st>>>(a);
+    else search_by_bow_kernel<false><<<grid, 128, 0, st>>>(a);
     count_launch();
     return cudaGetLastError();
 }

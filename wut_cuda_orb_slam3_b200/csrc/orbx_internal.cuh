@@ -224,20 +224,33 @@ struct VocabDev {
 cudaError_t launch_bow_descend(const VocabDev& v, const uint8_t* d_desc, int n, int nid_level, uint32_t* d_word, double* d_weight,
                                uint32_t* d_node, cudaStream_t st);
 
-struct BowSearchArgs {
-    int mode;                    // 0: KF -> Frame (src/ORBmatcher1.cc:225-427), 1: KF -> KF (src/ORBmatcher2.cc:36-171)
-    int n_pairs;
-    const int4* pairs;           // per common node: (a_begin, a_end, b_begin, b_end) into idx_a / idx_b
-    const uint32_t* idx_a; const uint32_t* idx_b;
-    const uint8_t* desc_a; const uint8_t* desc_b;
-    const uint8_t* valid_a; const uint8_t* valid_b;
-    int nleft_b;
-    float nn_ratio;
-    int* match_b;                // [nB] init -1: A index matched to B's feature (also the "already matched" state)
-    int* match_a;                // [nA] init -1 (may be null)
-    int* match_a_right;          // [nA] init -1 (mode 0 with nleft_b >= 0; may be null)
+// SearchByBoW of one fixed side against many key frames.  Mode 0 (KF -> Frame, src/ORBmatcher1.cc:225-427): the fixed side is B
+// and each key frame an A side; mode 1 (KF -> KF, src/ORBmatcher2.cc:36-171): the fixed side is A and each key frame a B side.
+// A job-build kernel (one CTA per key frame) sets key frame k's rows to -1 and writes its common nodes as jobs into
+// jobs[k * job_stride, k * job_stride + job_count[k]); the search kernel takes the key frame as blockIdx.y.  Feature indices
+// inside a key frame are its own (0 .. n - 1); its arrays point into the packed upload, its per-feature rows start at `base`.
+struct BowKF {
+    const uint8_t* desc; const uint8_t* valid;
+    const uint32_t* node_ids; const int32_t* offsets; const uint32_t* indices;   // mFeatVec in CSR form
+    int n, n_nodes;
+    size_t base;                 // first feature of this key frame in the packed per-feature arrays
 };
-cudaError_t launch_search_by_bow(const BowSearchArgs& a, cudaStream_t st);
+struct BowBatchArgs {
+    int mode;
+    int n_kf; const BowKF* kfs;
+    int n; const uint8_t* desc; const uint8_t* valid;                          // the fixed side (valid: mode 1 only)
+    int n_nodes; const uint32_t* node_ids; const int32_t* offsets; const uint32_t* indices;
+    int nleft;                   // mode 0: F.Nleft (separate left / right best for j < nleft and j >= nleft), else -1
+    float nn_ratio;
+    int4* jobs;                  // [n_kf][job_stride] (a_begin, a_end, b_begin, b_end) into the A / B index arrays
+    int* job_count;              // [n_kf]
+    int job_stride;              // n_nodes of the fixed side: a key frame has at most that many common nodes
+    int* row;                    // [n_kf][n] per feature of the fixed side: mode 0 match_b (also the "already matched" state),
+                                 //           mode 1 match_a
+    int* feat;                   // [sum n] per key-frame feature: mode 1 match_b (vbMatched2), mode 0 match_a (may be null)
+    int* feat_right;             // [sum n] mode 0 with nleft >= 0: match_a of the right camera (may be null)
+};
+cudaError_t launch_search_by_bow_batch(const BowBatchArgs& a, cudaStream_t st);
 
 // SearchForTriangulation of one KF1 against many neighbours: a job-build kernel (one CTA per neighbour) writes the jobs of
 // neighbour k into jobs[k * n_a, k * n_a + job_count[k]) and sets match row k to -1; the scan kernel takes the neighbour as
