@@ -105,26 +105,32 @@ static EncodeTiledFn get_encode_tiled()
     return fn;
 }
 
+// A grow-only staging buffer of a slot: `n` elements at `p` (see grow()).
+template <typename T>
+struct SlotBuf {
+    T* p = nullptr;
+    size_t n = 0;
+};
+
 struct Slot {
     Workspace ws{};
     cudaStream_t stream = nullptr;
     cudaEvent_t ev_in = nullptr, ev_done = nullptr, ev_out = nullptr;   // H2D complete / compute complete / D2H complete (serial-compute pipeline)
     cudaEvent_t ev_cnt = nullptr;                                       // the chunk's per-frame counts have reached the host
     int cap_frames = 0;
-    // staging for the host-buffer API
-    uint8_t* d_in = nullptr; size_t d_in_bytes = 0;
-    uint8_t* d_color = nullptr; size_t d_color_bytes = 0;      // colour input of orbx_extract_color
-    orbx_keypoint* d_kps = nullptr; uint8_t* d_desc = nullptr; int* d_n = nullptr; int* d_nm = nullptr;
-    size_t out_cap = 0;            // keypoint rows the output staging holds
-    int out_frames = 0;            // frames the per-frame counters hold
-    // stereo batches: mvuRight / mvDepth staging of the host-buffer call and the matcher's SAD scratch, [pairs][capacity]
-    float* d_su = nullptr; float* d_sd = nullptr; int* d_sad = nullptr;
-    int* d_snm = nullptr;          // [2 * pairs] monoIndex scratch of the device call (stereo outputs have no n_mono)
-    size_t stereo_rows = 0; int stereo_pairs = 0;
-    // RGB-D frames: the raw depth maps of the host-buffer calls and the mvKeysUn slab (mvuRight / mvDepth use d_su / d_sd)
-    uint8_t* d_depth = nullptr; size_t d_depth_bytes = 0;
-    orbx_keypoint* d_kpun = nullptr; size_t kpun_rows = 0;
-    std::vector<void*> allocs;
+    std::vector<void*> allocs;     // the workspace
+    // staging of the host-buffer calls: grey frames, colour input of a single frame, [frame][capacity] keypoints and descriptors,
+    // per-frame counts
+    SlotBuf<uint8_t> in, color, desc;
+    SlotBuf<orbx_keypoint> kps;
+    SlotBuf<int> n, nm;
+    // stereo: mvuRight / mvDepth and the matcher's SAD scratch, [pair][capacity]; the monoIndex scratch of the device batches,
+    // whose outputs have no n_mono
+    SlotBuf<float> su, sd;
+    SlotBuf<int> sad, snm;
+    // RGB-D: the raw depth maps of the host-buffer calls and the mvKeysUn slab (mvuRight / mvDepth use su / sd)
+    SlotBuf<uint8_t> depth;
+    SlotBuf<orbx_keypoint> kpun;
 };
 
 int rotation_bin(float angle_a, float angle_b)
@@ -168,10 +174,10 @@ struct orbx_extractor {
     int max_batch = 0;
     static const int kSlots = 6;
     Slot slots[kSlots];
-    cudaStream_t compute = nullptr, copy_in = nullptr, copy_out = nullptr;   // serial-compute pipeline of orbx_extract_batch (3 streams)
+    cudaStream_t compute = nullptr, copy_in = nullptr, copy_out = nullptr;   // serial-compute pipeline of run_host_pipeline (3 streams)
     int last_frames = 0;           // frames of the last call that are probe-able (slot 0)
-    // orbx_extract_batch_device on a caller's stream: an event recorded behind its last launch.  orbx_sync, the probes,
-    // stereo matching, re-configuration and the next extraction on the extractor's own streams wait for it.
+    // a device batch on a caller's stream: an event recorded behind its last launch.  orbx_sync, the probes, stereo matching,
+    // re-configuration, staging growth and the next extraction on the extractor's own streams wait for it.
     cudaEvent_t ev_user = nullptr;
     bool user_pending = false;
     int max_kp = 0;
@@ -179,12 +185,13 @@ struct orbx_extractor {
     // launch gaps, not kernels, dominate it).  The graph is keyed by everything the captured launches bake in.
     struct GraphKey {
         int rows = 0, cols = 0, lap0 = 0, lap1 = 0, capacity = 0, cap_frames = 0;
-        const void* pyr = nullptr; const void* d_in = nullptr; const void* d_kps = nullptr; const void* cand = nullptr;
-        const void* d_n = nullptr; const void* tables = nullptr; const void* mirror = nullptr;
+        const void* pyr = nullptr; const void* d_in = nullptr; const void* d_kps = nullptr; const void* d_desc = nullptr; const void* cand = nullptr;
+        const void* d_n = nullptr; const void* d_nm = nullptr; const void* tables = nullptr; const void* mirror = nullptr;
         bool operator==(const GraphKey& o) const
         {
             return mirror == o.mirror && rows == o.rows && cols == o.cols && lap0 == o.lap0 && lap1 == o.lap1 && capacity == o.capacity && cap_frames == o.cap_frames &&
-                   pyr == o.pyr && d_in == o.d_in && d_kps == o.d_kps && cand == o.cand && d_n == o.d_n && tables == o.tables;
+                   pyr == o.pyr && d_in == o.d_in && d_kps == o.d_kps && d_desc == o.d_desc && cand == o.cand && d_n == o.d_n && d_nm == o.d_nm &&
+                   tables == o.tables;
         }
     } graph_key;
     cudaGraphExec_t graph_exec = nullptr;
@@ -274,27 +281,35 @@ int Lease::reserve(size_t bytes, size_t staged)
     return ORBX_OK;
 }
 
+template <typename T>
+static void release(SlotBuf<T>& b)
+{
+    if (b.p) cudaFree(b.p);
+    b = SlotBuf<T>{};
+}
+
 static void free_slot(Slot& s)
 {
     for (void* p : s.allocs) cudaFree(p);
     s.allocs.clear();
     s.ws = Workspace{};
     s.cap_frames = 0;
-    s.d_in = nullptr; s.d_in_bytes = 0; s.d_color = nullptr; s.d_color_bytes = 0; s.d_kps = nullptr; s.d_desc = nullptr; s.d_n = nullptr; s.d_nm = nullptr;
-    s.out_cap = 0; s.out_frames = 0;
-    s.d_su = nullptr; s.d_sd = nullptr; s.d_sad = nullptr; s.d_snm = nullptr; s.stereo_rows = 0; s.stereo_pairs = 0;
-    s.d_depth = nullptr; s.d_depth_bytes = 0; s.d_kpun = nullptr; s.kpun_rows = 0;
+    release(s.in); release(s.color); release(s.desc); release(s.kps); release(s.n); release(s.nm);
+    release(s.su); release(s.sd); release(s.sad); release(s.snm); release(s.depth); release(s.kpun);
 }
 
-// release one buffer of a slot early (a staging buffer that is being replaced by a larger one)
+// Make `b` hold at least n elements.  A buffer is replaced only after everything queued before may have used it has finished:
+// a device batch on a caller's stream and the slot's own stream (the host batches' three-stream pipeline is idle between calls).
 template <typename T>
-static void dev_release(Slot& s, T*& p)
+static int grow(orbx_extractor* ex, Slot& s, SlotBuf<T>& b, size_t n)
 {
-    if (!p) return;
-    for (size_t i = 0; i < s.allocs.size(); ++i)
-        if (s.allocs[i] == (void*)p) { s.allocs[i] = s.allocs.back(); s.allocs.pop_back(); break; }
-    cudaFree((void*)p);
-    p = nullptr;
+    if (b.n >= n) return ORBX_OK;
+    wait_user_work(ex);
+    CU(cudaStreamSynchronize(s.stream));
+    release(b);
+    CU(cudaMalloc((void**)&b.p, std::max<size_t>(n * sizeof(T), 16)));
+    b.n = n;
+    return ORBX_OK;
 }
 
 template <typename T>
@@ -656,74 +671,22 @@ static int ensure_capacity(orbx_extractor* ex, int frames, int nslots)
     return ORBX_OK;
 }
 
-// Staging of the host-buffer API.  The caller has made sure no work is in flight on the slot when a buffer is replaced.
-static int ensure_host_staging(Slot& s, size_t in_bytes, int frames, int capacity)
+// The staging of every extraction from host buffers: `frames` grey frames of frame_bytes each and their results.
+static int grow_extract_staging(orbx_extractor* ex, Slot& s, int frames, size_t frame_bytes, int capacity)
 {
-    int rc;
-    if (s.d_in_bytes < in_bytes) {
-        dev_release(s, s.d_in);
-        s.d_in_bytes = 0;
-        if ((rc = dev_alloc(s, &s.d_in, in_bytes))) return rc;
-        s.d_in_bytes = in_bytes;
-    }
     const size_t rows = (size_t)frames * capacity;
-    if (s.out_cap < rows || !s.d_kps) {
-        dev_release(s, s.d_kps); dev_release(s, s.d_desc);
-        s.out_cap = 0;
-        if ((rc = dev_alloc(s, &s.d_kps, rows))) return rc;
-        if ((rc = dev_alloc(s, &s.d_desc, rows * 32))) return rc;
-        s.out_cap = rows;
-    }
-    if (s.out_frames < frames || !s.d_n) {          // the per-frame counters follow the FRAME count, not rows
-        dev_release(s, s.d_n); dev_release(s, s.d_nm);
-        s.out_frames = 0;
-        if ((rc = dev_alloc(s, &s.d_n, (size_t)frames))) return rc;
-        if ((rc = dev_alloc(s, &s.d_nm, (size_t)frames))) return rc;
-        s.out_frames = frames;
-    }
-    return ORBX_OK;
-}
-
-// Matcher staging of a stereo chunk of `pairs` pairs.  As above: nothing may be in flight on the slot.
-static bool stereo_staging_fits(const Slot& s, int pairs, int capacity)
-{
-    return s.stereo_pairs >= pairs && s.stereo_rows >= (size_t)pairs * capacity;
-}
-static int ensure_stereo_staging(Slot& s, int pairs, int capacity)
-{
-    if (stereo_staging_fits(s, pairs, capacity)) return ORBX_OK;
-    dev_release(s, s.d_su); dev_release(s, s.d_sd); dev_release(s, s.d_sad); dev_release(s, s.d_snm);
-    s.stereo_rows = 0; s.stereo_pairs = 0;
-    const size_t rows = (size_t)pairs * capacity;
     int rc;
-    if ((rc = dev_alloc(s, &s.d_su, rows)) || (rc = dev_alloc(s, &s.d_sd, rows)) || (rc = dev_alloc(s, &s.d_sad, rows)) ||
-        (rc = dev_alloc(s, &s.d_snm, 2 * (size_t)pairs)))
+    if ((rc = grow(ex, s, s.in, frame_bytes * frames)) || (rc = grow(ex, s, s.kps, rows)) || (rc = grow(ex, s, s.desc, rows * 32)) ||
+        (rc = grow(ex, s, s.n, (size_t)frames)) || (rc = grow(ex, s, s.nm, (size_t)frames)))
         return rc;
-    s.stereo_rows = rows; s.stereo_pairs = pairs;
     return ORBX_OK;
 }
 
-// RGB-D staging of the host-buffer calls: raw depth maps and mvKeysUn rows.  As above: nothing may be in flight on the slot.
-static bool rgbd_staging_fits(const Slot& s, size_t depth_bytes, size_t rows)
+// Frames per chunk of a call over n frames: `max_batch` when the handle was created with one, else 64 for the host-buffer
+// batches (small chunks overlap each other on the slot streams, see run_host_pipeline) and 256 for the device-resident batches.
+static int chunk_frames(const orbx_extractor* ex, int n, bool host)
 {
-    return s.d_depth_bytes >= depth_bytes && s.kpun_rows >= rows;
-}
-static int ensure_rgbd_staging(Slot& s, size_t depth_bytes, size_t rows)
-{
-    int rc;
-    if (s.d_depth_bytes < depth_bytes) {
-        dev_release(s, s.d_depth);
-        s.d_depth_bytes = 0;
-        if ((rc = dev_alloc(s, &s.d_depth, depth_bytes))) return rc;
-        s.d_depth_bytes = depth_bytes;
-    }
-    if (s.kpun_rows < rows) {
-        dev_release(s, s.d_kpun);
-        s.kpun_rows = 0;
-        if ((rc = dev_alloc(s, &s.d_kpun, rows))) return rc;
-        s.kpun_rows = rows;
-    }
-    return ORBX_OK;
+    return ex->max_batch > 0 ? std::min(ex->max_batch, n) : std::min(n, host ? 64 : 256);
 }
 
 // Chunk schedule of the host-buffer batches: the first host->device copy cannot overlap any compute, so the pipeline ramps
@@ -760,33 +723,54 @@ static int upload_frames(const T* const* src, int i0, int n, uint8_t* dst, size_
     return ORBX_OK;
 }
 
-// The driver loop of the host-buffer batches of stereo pairs and RGB-D frames.  Chunk c of `sched` (first item, items) runs on
-// slot c % nslots, whose staging the caller has sized.  serial = false: each chunk runs whole on its slot's stream; serial = true:
-// orbx_extract_batch's three-stream pipeline (there: why), tied by the slot's events.  Results go home trimmed, as in
-// orbx_extract_batch: `counts` queues the copy of a chunk's per-item counts, and the host reads them after it has queued chunk
-// c + 2, then `download` asks for the rows the chunk's items actually have.
+// The driver loop of the host-buffer batches (orbx_extract_batch, orbx_extract_stereo_batch, orbx_extract_rgbd_batch).  Chunk c
+// of `sched` (first item, items; at most `chunk` items) runs on slot c % nslots, whose staging the caller has sized.
+//
+// Two pipelines, chosen by the chunk's frame count.  Small chunks (< 128 frames) run whole on their slot's stream, so that chunks
+// overlap each other (a small chunk under-fills the GPU: its octree is one partial wave).  Large chunks compute on ONE stream in
+// order: interleaving the kernels of two big chunks costs ~20 % (measured: 80 k vs 98 k frames/s at 256-frame chunks).  The
+// serial pipeline uses exactly three streams — H2D, compute, D2H — tied by per-slot events: with one copy stream per slot (seven
+// streams) two of them regularly landed on the same hardware connection (8 by default) and a chunk's D2H or the next H2D queued
+// behind an unrelated copy (90.5 k frames/s; 97.9 k with CUDA_DEVICE_MAX_CONNECTIONS=32; 98 k with three streams at any setting).
+//
+// Results go home trimmed: `counts` queues the copy of a chunk's per-item counts (a few hundred bytes), the host reads them and
+// then `download` asks for the rows every item of the chunk actually has — one strided copy per array, row count = the chunk's
+// largest count — instead of `capacity` rows per item.  The host looks at the counts of chunk c - 2 after it has queued chunk c,
+// so two chunks of compute are always queued behind the one it waits for and the next upload never starts late.
+//
+// ORBX_TRACE_BATCH=1: per-chunk timeline (H2D start / end, compute end, D2H end; ms since the first H2D) on stderr.
 struct HostPipeline {
     // (slot, first item, items, stream): upload on the H2D stream, compute on the compute stream, counts and download on the D2H
     // stream (all three are the slot's stream when not serial)
     std::function<int(Slot&, int, int, cudaStream_t)> upload, compute, counts, download;
+    int item_frames = 1;           // frames per item of the schedule (2: a stereo pair)
 };
-static int run_host_pipeline(orbx_extractor* ex, const std::vector<std::pair<int, int>>& sched, int nslots, bool serial, const HostPipeline& h)
+static int run_host_pipeline(orbx_extractor* ex, const std::vector<std::pair<int, int>>& sched, int nslots, int chunk, const HostPipeline& h)
 {
     const int nchunks = (int)sched.size();
+    const bool serial = chunk * h.item_frames >= 128;
     int rc;
     if (serial && !ex->compute) {
         CU(cudaStreamCreateWithFlags(&ex->compute, cudaStreamNonBlocking));
         CU(cudaStreamCreateWithFlags(&ex->copy_in, cudaStreamNonBlocking));
         CU(cudaStreamCreateWithFlags(&ex->copy_out, cudaStreamNonBlocking));
     }
-    if (serial)      // earlier work of this extractor on the slot streams must be complete
+    if (serial)      // earlier work of this extractor on the slot streams (single-frame calls, small batches) must be complete
         for (int i = 0; i < nslots; ++i) CU(cudaStreamSynchronize(ex->slots[i].stream));
+    static const bool trace = getenv("ORBX_TRACE_BATCH") != nullptr;
+    std::vector<cudaEvent_t> tev;                    // [chunk][4]: H2D start / end, compute end (= D2H may start), D2H end
+    auto mark = [&](cudaStream_t st, int c, int k) {
+        if (!trace) return;
+        if (tev.empty()) tev.assign((size_t)4 * nchunks, nullptr);
+        cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, st); tev[(size_t)4 * c + k] = e;
+    };
     auto finish = [&](int c) -> int {
         Slot& s = ex->slots[c % nslots];
         cudaStream_t ost = serial ? ex->copy_out : s.stream;
         CU(cudaEventSynchronize(s.ev_cnt));
         int rc2 = h.download(s, sched[c].first, sched[c].second, ost);
         if (rc2) return rc2;
+        mark(ost, c, 3);
         if (serial) CU(cudaEventRecord(s.ev_out, ost));
         return ORBX_OK;
     };
@@ -797,12 +781,16 @@ static int run_host_pipeline(orbx_extractor* ex, const std::vector<std::pair<int
         cudaStream_t cst = serial ? ex->compute : s.stream;
         cudaStream_t ist = serial ? ex->copy_in : s.stream, ost = serial ? ex->copy_out : s.stream;
         // reuse of a slot: its input staging is free once the chunk that used it has been computed, its output staging once that
-        // chunk's D2H has completed (queued when chunk c - nslots + lag was; nslots > lag whenever a slot is reused)
+        // chunk's D2H has completed (one slot stream orders all of this by itself in the other pipeline).  The D2H of chunk
+        // c - nslots was queued when chunk c - nslots + lag was (nslots > lag whenever a slot is reused).
         if (serial && c >= nslots) { CU(cudaStreamWaitEvent(ist, s.ev_done, 0)); CU(cudaStreamWaitEvent(cst, s.ev_out, 0)); }
+        mark(ist, c, 0);
         if ((rc = h.upload(s, i0, ni, ist))) return rc;
+        mark(ist, c, 1);
         if (serial) { CU(cudaEventRecord(s.ev_in, ist)); CU(cudaStreamWaitEvent(cst, s.ev_in, 0)); }
         if ((rc = h.compute(s, i0, ni, cst))) return rc;
         if (serial) { CU(cudaEventRecord(s.ev_done, cst)); CU(cudaStreamWaitEvent(ost, s.ev_done, 0)); }
+        mark(ost, c, 2);
         if ((rc = h.counts(s, i0, ni, ost))) return rc;
         CU(cudaEventRecord(s.ev_cnt, ost));
         if (c >= lag && (rc = finish(c - lag))) return rc;
@@ -811,6 +799,15 @@ static int run_host_pipeline(orbx_extractor* ex, const std::vector<std::pair<int
         if ((rc = finish(c))) return rc;
     if (serial) { CU(cudaStreamSynchronize(ex->copy_out)); CU(cudaStreamSynchronize(ex->compute)); CU(cudaStreamSynchronize(ex->copy_in)); }
     for (int i = 0; i < nslots; ++i) CU(cudaStreamSynchronize(ex->slots[i].stream));
+    if (trace) {
+        for (int c = 0; c < nchunks; ++c) {
+            float t[4];
+            for (int k = 0; k < 4; ++k) cudaEventElapsedTime(&t[k], tev[0], tev[4 * c + k]);      // (all four marks of every chunk exist)
+            fprintf(stderr, "[orbx] chunk %2d frames %3d: h2d %.3f-%.3f compute-end %.3f d2h-end %.3f ms\n", c, sched[c].second * h.item_frames,
+                    t[0], t[1], t[2], t[3]);
+        }
+        for (cudaEvent_t e : tev) if (e) cudaEventDestroy(e);
+    }
     return ORBX_OK;
 }
 
@@ -935,9 +932,12 @@ static int ensure_mirror(orbx_extractor* ex, cudaStream_t st)
     return ORBX_OK;
 }
 
-// Upload one host image into slot 0 and queue its extraction on the slot's stream (captured graph after the first call).
-// Results stay on the device (s.d_kps / s.d_desc / s.d_n / s.d_nm); nothing is copied back and nothing is waited for.
-static int enqueue_single(orbx_extractor* ex, const uint8_t* image, int rows, int cols, size_t step, int lap0, int lap1, int capacity)
+// Upload one host image into slot 0 and queue its extraction on the slot's stream.  A grey image (channels 1) is uploaded into
+// the input staging and replays a captured graph after the first call; a colour image (channels 3 or 4) goes to the colour
+// staging, is converted to grey into the input staging and runs eagerly (the colour staging is not part of the captured graph).
+// Results stay on the device (s.kps / s.desc / s.n / s.nm); nothing is copied back and nothing is waited for.
+static int enqueue_single(orbx_extractor* ex, const uint8_t* image, int rows, int cols, size_t step, int channels, int rgb, int lap0,
+                          int lap1, int capacity)
 {
     int rc = set_device(ex->device);
     if (rc) return rc;
@@ -945,22 +945,28 @@ static int enqueue_single(orbx_extractor* ex, const uint8_t* image, int rows, in
     wait_user_work(ex);
     if ((rc = ensure_capacity(ex, 1, 1))) return rc;
     Slot& s = ex->slots[0];
-    const size_t dpitch = (size_t)cols, dframe = dpitch * rows;
-    if (s.d_in_bytes < dframe || s.out_cap < (size_t)capacity || s.out_frames < 1) CU(cudaStreamSynchronize(s.stream));
-    if ((rc = ensure_host_staging(s, dframe, 1, capacity))) return rc;
+    const size_t dpitch = (size_t)cols, dframe = dpitch * rows, cpitch = align_up((size_t)cols * channels, 16);
+    if ((rc = grow_extract_staging(ex, s, 1, dframe, capacity))) return rc;
+    if (channels != 1 && (rc = grow(ex, s, s.color, cpitch * rows))) return rc;
     cudaStream_t st = s.stream;
     if ((rc = ensure_mirror(ex, st))) return rc;
-    if (step == (size_t)cols) CU(cudaMemcpyAsync(s.d_in, image, dframe, cudaMemcpyHostToDevice, st));
-    else CU(cudaMemcpy2DAsync(s.d_in, dpitch, image, step, cols, rows, cudaMemcpyHostToDevice, st));
+    if (channels != 1) {
+        CU(cudaMemcpy2DAsync(s.color.p, cpitch, image, step, (size_t)cols * channels, rows, cudaMemcpyHostToDevice, st));
+        CU(launch_cvt_gray(s.color.p, cpitch, 0, channels, rgb, 1, rows, cols, s.in.p, dpitch, 0, st));
+    } else if (step == (size_t)cols) {
+        CU(cudaMemcpyAsync(s.in.p, image, dframe, cudaMemcpyHostToDevice, st));
+    } else {
+        CU(cudaMemcpy2DAsync(s.in.p, dpitch, image, step, cols, rows, cudaMemcpyHostToDevice, st));
+    }
     auto body = [&](cudaStream_t cs) -> int {
-        if (!ex->profiling || ex->mirror) return run_single_forked(ex, s, s.d_in, dpitch, lap0, lap1, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm, cs);
-        return run_chunk(ex, s, one_set_io(s.d_in, dframe, dpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), 1, lap0, lap1, cs);
+        if (!ex->profiling || ex->mirror) return run_single_forked(ex, s, s.in.p, dpitch, lap0, lap1, s.kps.p, s.desc.p, capacity, s.n.p, s.nm.p, cs);
+        return run_chunk(ex, s, one_set_io(s.in.p, dframe, dpitch, s.kps.p, s.desc.p, capacity, s.n.p, s.nm.p), 1, lap0, lap1, cs);
     };
-    if (!ex->profiling && !ex->force_eager && ex->single_calls++ > 0) {
+    if (channels == 1 && !ex->profiling && !ex->force_eager && ex->single_calls++ > 0) {
         orbx_extractor::GraphKey key;
         key.rows = rows; key.cols = cols; key.lap0 = lap0; key.lap1 = lap1; key.capacity = capacity;
-        key.pyr = s.ws.pyr; key.d_in = s.d_in; key.d_kps = s.d_kps; key.cand = s.ws.cand;
-        key.cap_frames = s.cap_frames; key.d_n = s.d_n; key.tables = ex->d_tables; key.mirror = ex->mirror ? ex->h_mirror : nullptr;
+        key.pyr = s.ws.pyr; key.d_in = s.in.p; key.d_kps = s.kps.p; key.d_desc = s.desc.p; key.cand = s.ws.cand;
+        key.cap_frames = s.cap_frames; key.d_n = s.n.p; key.d_nm = s.nm.p; key.tables = ex->d_tables; key.mirror = ex->mirror ? ex->h_mirror : nullptr;
         if (!ex->graph_exec || !(key == ex->graph_key)) {
             if (ex->graph_exec) { cudaGraphExecDestroy(ex->graph_exec); ex->graph_exec = nullptr; }
             cudaGraph_t g = nullptr;
@@ -985,30 +991,34 @@ static int enqueue_single(orbx_extractor* ex, const uint8_t* image, int rows, in
     return ORBX_OK;
 }
 
-// The same for a host colour image (channels 3 or 4): upload into the slot's colour staging, convert to grey into its input
-// staging, and the per-level fork / join of orbx_extract launched eagerly (the colour staging is not part of the captured graph).
-static int enqueue_color(orbx_extractor* ex, const uint8_t* image, int rows, int cols, size_t step, int channels, int rgb, int lap0,
-                         int lap1, int capacity)
+// The results of enqueue_single into the caller's buffers (orbx_extract, orbx_extract_color).
+static int download_single(orbx_extractor* ex, orbx_keypoint* keypoints, uint8_t* descriptors, int capacity, int* n_out, int* n_mono)
 {
-    int rc = set_device(ex->device);
-    if (rc) return rc;
-    if ((rc = configure(ex, rows, cols))) return rc;
-    wait_user_work(ex);
-    if ((rc = ensure_capacity(ex, 1, 1))) return rc;
     Slot& s = ex->slots[0];
-    const size_t gpitch = (size_t)cols, cpitch = align_up((size_t)cols * channels, 16);
-    if ((rc = ensure_host_staging(s, gpitch * rows, 1, capacity))) return rc;
-    if (s.d_color_bytes < cpitch * rows) {
-        if ((rc = dev_alloc(s, &s.d_color, cpitch * rows))) return rc;
-        s.d_color_bytes = cpitch * rows;
-    }
-    CU(cudaMemcpy2DAsync(s.d_color, cpitch, image, step, (size_t)cols * channels, rows, cudaMemcpyHostToDevice, s.stream));
-    CU(launch_cvt_gray(s.d_color, cpitch, 0, channels, rgb, 1, rows, cols, s.d_in, gpitch, 0, s.stream));
-    if ((rc = ensure_mirror(ex, s.stream))) return rc;
-    if (ex->profiling) rc = run_chunk(ex, s, one_set_io(s.d_in, gpitch * rows, gpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), 1, lap0, lap1, s.stream);
-    else rc = run_single_forked(ex, s, s.d_in, gpitch, lap0, lap1, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm, s.stream);
-    if (rc) return rc;
-    ex->last_frames = 1;
+    CU(cudaMemcpyAsync(keypoints, s.kps.p, sizeof(orbx_keypoint) * (size_t)capacity, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(descriptors, s.desc.p, (size_t)capacity * 32, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(n_out, s.n.p, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(n_mono, s.nm.p, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaStreamSynchronize(s.stream));
+    if (*n_out > capacity) return fail(ORBX_ERR_CAPACITY, "frame has %d keypoints, capacity %d", *n_out, capacity);
+    return ORBX_OK;
+}
+
+// The device batches queue their work on the caller's stream (slot 0's when the caller passes none), with slot 0's workspace.
+// begin_caller_stream puts the extractor's earlier work in front of that stream: the last device batch on another caller stream
+// and everything queued on the slot's stream.  end_caller_stream makes the extractor's later work wait for this call's.
+static int begin_caller_stream(orbx_extractor* ex, void* stream, cudaStream_t* st)
+{
+    Slot& s = ex->slots[0];
+    *st = stream ? (cudaStream_t)stream : s.stream;
+    if (!ex->ev_user) CU(cudaEventCreateWithFlags(&ex->ev_user, cudaEventDisableTiming));
+    if (ex->user_pending) CU(cudaStreamWaitEvent(*st, ex->ev_user, 0));
+    if (*st != s.stream) { CU(cudaEventRecord(s.ev_done, s.stream)); CU(cudaStreamWaitEvent(*st, s.ev_done, 0)); }
+    return ORBX_OK;
+}
+static int end_caller_stream(orbx_extractor* ex, cudaStream_t st)
+{
+    if (st != ex->slots[0].stream) { CU(cudaEventRecord(ex->ev_user, st)); ex->user_pending = true; }
     return ORBX_OK;
 }
 
@@ -1170,14 +1180,11 @@ int orbx_extract_batch_device(orbx_extractor* ex, const uint8_t* d_images, size_
     int rc = set_device(ex->device);
     if (rc) return rc;
     if ((rc = configure(ex, rows, cols))) return rc;
-    const int chunk = ex->max_batch > 0 ? std::min(ex->max_batch, n_frames) : std::min(n_frames, 256);
+    const int chunk = chunk_frames(ex, n_frames, false);
     if ((rc = ensure_capacity(ex, chunk, 1))) return rc;
     Slot& s = ex->slots[0];
-    cudaStream_t st = stream ? (cudaStream_t)stream : s.stream;
-    if (!ex->ev_user) CU(cudaEventCreateWithFlags(&ex->ev_user, cudaEventDisableTiming));
-    // the workspace is shared with whatever ran before: earlier work on another stream must be complete first
-    if (ex->user_pending) CU(cudaStreamWaitEvent(st, ex->ev_user, 0));
-    if (st != s.stream) { CU(cudaEventRecord(s.ev_done, s.stream)); CU(cudaStreamWaitEvent(st, s.ev_done, 0)); }
+    cudaStream_t st;
+    if ((rc = begin_caller_stream(ex, stream, &st))) return rc;
     for (int f0 = 0; f0 < n_frames; f0 += chunk) {
         const int nf = std::min(chunk, n_frames - f0);
         rc = run_chunk(ex, s, one_set_io(d_images + (size_t)f0 * frame_stride, frame_stride, pitch, d_keypoints + (size_t)f0 * capacity,
@@ -1186,8 +1193,7 @@ int orbx_extract_batch_device(orbx_extractor* ex, const uint8_t* d_images, size_
         if (rc) return rc;
         ex->last_frames = nf;
     }
-    if (st != s.stream) { CU(cudaEventRecord(ex->ev_user, st)); ex->user_pending = true; }
-    return ORBX_OK;
+    return end_caller_stream(ex, st);
 }
 
 int orbx_extract_batch(orbx_extractor* ex, const uint8_t* const* images, int n_frames, int rows, int cols, size_t step,
@@ -1205,102 +1211,37 @@ int orbx_extract_batch(orbx_extractor* ex, const uint8_t* const* images, int n_f
     if (rc) return rc;
     if ((rc = configure(ex, rows, cols))) return rc;
     wait_user_work(ex);
-    const int chunk = ex->max_batch > 0 ? std::min(ex->max_batch, n_frames) : std::min(n_frames, 64);
+    const int chunk = chunk_frames(ex, n_frames, true);
     const std::vector<std::pair<int, int>> sched = chunk_schedule(n_frames, chunk);   // (first frame, frames)
-    const int nchunks = (int)sched.size();
-    const int nslots = std::min(nchunks, (int)orbx_extractor::kSlots);
+    const int nslots = std::min((int)sched.size(), (int)orbx_extractor::kSlots);
     if ((rc = ensure_capacity(ex, chunk, nslots))) return rc;
-    const size_t dpitch = (size_t)cols;
-    const size_t dframe = dpitch * rows;
+    const size_t dpitch = (size_t)cols, dframe = dpitch * rows;
     for (int i = 0; i < nslots; ++i)
-        if ((rc = ensure_host_staging(ex->slots[i], dframe * chunk, chunk, capacity))) return rc;
-    // ORBX_TRACE_BATCH=1: per-chunk timeline (H2D start/end, compute end, D2H end; ms since the first H2D) on stderr
-    static const bool trace = getenv("ORBX_TRACE_BATCH") != nullptr;
-    std::vector<cudaEvent_t> tev;                    // [chunk][4]: H2D start / end, compute end (= D2H may start), D2H end
-    auto mark = [&](cudaStream_t st, int chunk, int k) {
-        if (!trace) return;
-        if (tev.empty()) tev.assign((size_t)4 * sched.size(), nullptr);
-        cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, st); tev[(size_t)4 * chunk + k] = e;
+        if ((rc = grow_extract_staging(ex, ex->slots[i], chunk, dframe, capacity))) return rc;
+    HostPipeline h;
+    h.upload = [&](Slot& s, int f0, int nf, cudaStream_t ist) { return upload_frames(images, f0, nf, s.in.p, dpitch, rows, step, ist); };
+    h.compute = [&](Slot& s, int f0, int nf, cudaStream_t cst) -> int {
+        (void)f0;
+        const int rc2 = run_chunk(ex, s, one_set_io(s.in.p, dframe, dpitch, s.kps.p, s.desc.p, capacity, s.n.p, s.nm.p), nf, lap0, lap1, cst);
+        if (!rc2 && &s == &ex->slots[0]) ex->last_frames = nf;     // slot 0's last chunk stays inspectable
+        return rc2;
     };
-    // Two pipelines.  Small chunks (< 128 frames) run whole on their slot's stream, so that chunks overlap each other (a small
-    // chunk under-fills the GPU: its octree is one partial wave).  Large chunks compute on ONE stream in order: interleaving the
-    // kernels of two big chunks costs ~20 % (measured: 80 k vs 98 k frames/s at 256-frame chunks).  The serial pipeline uses
-    // exactly three streams — H2D, compute, D2H — tied by per-slot events: with one copy stream per slot (seven streams) two of
-    // them regularly landed on the same hardware connection (8 by default) and a chunk's D2H or the next H2D queued behind an
-    // unrelated copy (90.5 k frames/s; 97.9 k with CUDA_DEVICE_MAX_CONNECTIONS=32; 98 k with three streams at any setting).
-    const bool serial = chunk >= 128;
-    if (serial && !ex->compute) {
-        CU(cudaStreamCreateWithFlags(&ex->compute, cudaStreamNonBlocking));
-        CU(cudaStreamCreateWithFlags(&ex->copy_in, cudaStreamNonBlocking));
-        CU(cudaStreamCreateWithFlags(&ex->copy_out, cudaStreamNonBlocking));
-    }
-    if (serial)      // earlier work of this extractor on the slot streams (single-frame calls, small batches) must be complete
-        for (int i = 0; i < nslots; ++i) CU(cudaStreamSynchronize(ex->slots[i].stream));
-    // Results go home trimmed: a chunk's per-frame counts are copied first (a few hundred bytes), the host reads them and
-    // then asks for the keypoint / descriptor rows every frame of the chunk actually has — one strided copy per array, row
-    // count = the chunk's largest n_out — instead of `capacity` rows per frame.  The host looks at the counts of chunk c - 2
-    // after it has queued chunk c, so two chunks of compute are always queued behind the one it waits for and the next
-    // upload never starts late.
-    auto finish = [&](int c) -> int {
-        Slot& s = ex->slots[c % nslots];
-        const int f0 = sched[c].first, nf = sched[c].second;
-        cudaStream_t ost = serial ? ex->copy_out : s.stream;
-        CU(cudaEventSynchronize(s.ev_cnt));
-        int mx = 0;
-        for (int f = 0; f < nf; ++f) mx = std::max(mx, n_out[f0 + f]);
-        const int rows_out = std::min(mx, capacity);   // a frame over capacity wrote nothing: the call fails below
-        if (rows_out > 0) {
-            CU(cudaMemcpy2DAsync(keypoints + (size_t)f0 * capacity, sizeof(orbx_keypoint) * (size_t)capacity, s.d_kps,
-                                 sizeof(orbx_keypoint) * (size_t)capacity, sizeof(orbx_keypoint) * (size_t)rows_out, nf, cudaMemcpyDeviceToHost, ost));
-            CU(cudaMemcpy2DAsync(descriptors + (size_t)f0 * capacity * 32, (size_t)capacity * 32, s.d_desc, (size_t)capacity * 32,
-                                 (size_t)rows_out * 32, nf, cudaMemcpyDeviceToHost, ost));
-        }
-        mark(ost, c, 3);
-        if (serial) CU(cudaEventRecord(s.ev_out, ost));
+    h.counts = [&](Slot& s, int f0, int nf, cudaStream_t ost) -> int {
+        CU(cudaMemcpyAsync(n_out + f0, s.n.p, sizeof(int) * nf, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpyAsync(n_mono + f0, s.nm.p, sizeof(int) * nf, cudaMemcpyDeviceToHost, ost));
         return ORBX_OK;
     };
-    const int lag = 2;
-    for (int c = 0; c < nchunks; ++c) {
-        Slot& s = ex->slots[c % nslots];
-        const int f0 = sched[c].first, nf = sched[c].second;
-        cudaStream_t cst = serial ? ex->compute : s.stream;
-        cudaStream_t ist = serial ? ex->copy_in : s.stream, ost = serial ? ex->copy_out : s.stream;
-        // reuse of a slot: its input staging is free once the chunk that used it has been computed, its output staging once
-        // that chunk's D2H has completed (one slot stream orders all of this by itself in the other pipeline).  The D2H of
-        // chunk c - nslots was queued when chunk c - nslots + lag was (nslots > lag whenever a slot is reused).
-        if (serial && c >= nslots) { CU(cudaStreamWaitEvent(ist, s.ev_done, 0)); CU(cudaStreamWaitEvent(cst, s.ev_out, 0)); }
-        mark(ist, c, 0);
-        bool contiguous = step == (size_t)cols;
-        for (int f = 1; f < nf && contiguous; ++f) contiguous = images[f0 + f] == images[f0 + f - 1] + dframe;
-        if (contiguous) {
-            CU(cudaMemcpyAsync(s.d_in, images[f0], dframe * nf, cudaMemcpyHostToDevice, ist));
-        } else {
-            for (int f = 0; f < nf; ++f)
-                CU(cudaMemcpy2DAsync(s.d_in + (size_t)f * dframe, dpitch, images[f0 + f], step, cols, rows, cudaMemcpyHostToDevice, ist));
-        }
-        mark(ist, c, 1);
-        if (serial) { CU(cudaEventRecord(s.ev_in, ist)); CU(cudaStreamWaitEvent(cst, s.ev_in, 0)); }
-        if ((rc = run_chunk(ex, s, one_set_io(s.d_in, dframe, dpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), nf, lap0, lap1, cst))) return rc;
-        if (serial) { CU(cudaEventRecord(s.ev_done, cst)); CU(cudaStreamWaitEvent(ost, s.ev_done, 0)); }
-        mark(ost, c, 2);
-        CU(cudaMemcpyAsync(n_out + f0, s.d_n, sizeof(int) * nf, cudaMemcpyDeviceToHost, ost));
-        CU(cudaMemcpyAsync(n_mono + f0, s.d_nm, sizeof(int) * nf, cudaMemcpyDeviceToHost, ost));
-        CU(cudaEventRecord(s.ev_cnt, ost));
-        if (c % nslots == 0) ex->last_frames = nf;
-        if (c >= lag && (rc = finish(c - lag))) return rc;
-    }
-    for (int c = std::max(nchunks - lag, 0); c < nchunks; ++c)
-        if ((rc = finish(c))) return rc;
-    if (serial) { CU(cudaStreamSynchronize(ex->copy_out)); CU(cudaStreamSynchronize(ex->compute)); CU(cudaStreamSynchronize(ex->copy_in)); }
-    for (int i = 0; i < nslots; ++i) CU(cudaStreamSynchronize(ex->slots[i].stream));
-    if (trace) {
-        for (int c = 0; c < nchunks; ++c) {
-            float t[4];
-            for (int k = 0; k < 4; ++k) cudaEventElapsedTime(&t[k], tev[0], tev[4 * c + k]);      // (all four marks of every chunk exist)
-            fprintf(stderr, "[orbx] chunk %2d frames %3d: h2d %.3f-%.3f compute-end %.3f d2h-end %.3f ms\n", c, sched[c].second, t[0], t[1], t[2], t[3]);
-        }
-        for (cudaEvent_t e : tev) if (e) cudaEventDestroy(e);
-    }
+    h.download = [&](Slot& s, int f0, int nf, cudaStream_t ost) -> int {
+        int mx = 0;
+        for (int f = 0; f < nf; ++f) mx = std::max(mx, n_out[f0 + f]);
+        const int r = std::min(mx, capacity);         // a frame over capacity wrote nothing: the call fails below
+        if (r <= 0) return ORBX_OK;
+        const size_t kpitch = sizeof(orbx_keypoint) * (size_t)capacity, dpitch32 = (size_t)capacity * 32;
+        CU(cudaMemcpy2DAsync(keypoints + (size_t)f0 * capacity, kpitch, s.kps.p, kpitch, sizeof(orbx_keypoint) * (size_t)r, nf, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpy2DAsync(descriptors + (size_t)f0 * capacity * 32, dpitch32, s.desc.p, dpitch32, (size_t)r * 32, nf, cudaMemcpyDeviceToHost, ost));
+        return ORBX_OK;
+    };
+    if ((rc = run_host_pipeline(ex, sched, nslots, chunk, h))) return rc;
     for (int f = 0; f < n_frames; ++f)
         if (n_out[f] > capacity) return fail(ORBX_ERR_CAPACITY, "frame %d has %d keypoints, capacity %d", f, n_out[f], capacity);
     return ORBX_OK;
@@ -1313,16 +1254,8 @@ int orbx_extract(orbx_extractor* ex, const uint8_t* image, int rows, int cols, s
     if (!image || rows <= 0 || cols <= 0) return fail(ORBX_ERR_EMPTY_IMAGE, "empty image");
     if (!keypoints || !descriptors || !n_out || !n_mono || capacity <= 0 || step < (size_t)cols)
         return fail(ORBX_ERR_INVALID_ARG, "bad output buffers / step");
-    int rc = enqueue_single(ex, image, rows, cols, step, lap0, lap1, capacity);
-    if (rc) return rc;
-    Slot& s = ex->slots[0];
-    CU(cudaMemcpyAsync(keypoints, s.d_kps, sizeof(orbx_keypoint) * (size_t)capacity, cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(descriptors, s.d_desc, (size_t)capacity * 32, cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(n_out, s.d_n, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(n_mono, s.d_nm, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaStreamSynchronize(s.stream));
-    if (*n_out > capacity) return fail(ORBX_ERR_CAPACITY, "frame has %d keypoints, capacity %d", *n_out, capacity);
-    return ORBX_OK;
+    int rc = enqueue_single(ex, image, rows, cols, step, 1, 0, lap0, lap1, capacity);
+    return rc ? rc : download_single(ex, keypoints, descriptors, capacity, n_out, n_mono);
 }
 
 int orbx_set_pyramid_mirror(orbx_extractor* ex, int enable)
@@ -1366,16 +1299,8 @@ int orbx_extract_color(orbx_extractor* ex, const uint8_t* image, int rows, int c
     if (channels == 1) return orbx_extract(ex, image, rows, cols, step, lap0, lap1, keypoints, descriptors, capacity, n_out, n_mono);
     if ((channels != 3 && channels != 4) || step < (size_t)cols * channels) return fail(ORBX_ERR_INVALID_ARG, "channels must be 1, 3 or 4");
     if (!keypoints || !descriptors || !n_out || !n_mono || capacity <= 0) return fail(ORBX_ERR_INVALID_ARG, "bad output buffers");
-    int rc = enqueue_color(ex, image, rows, cols, step, channels, rgb, lap0, lap1, capacity);
-    if (rc) return rc;
-    Slot& s = ex->slots[0];
-    CU(cudaMemcpyAsync(keypoints, s.d_kps, sizeof(orbx_keypoint) * (size_t)capacity, cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(descriptors, s.d_desc, (size_t)capacity * 32, cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(n_out, s.d_n, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(n_mono, s.d_nm, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaStreamSynchronize(s.stream));
-    if (*n_out > capacity) return fail(ORBX_ERR_CAPACITY, "%d keypoints, capacity %d", *n_out, capacity);
-    return ORBX_OK;
+    int rc = enqueue_single(ex, image, rows, cols, step, channels, rgb, lap0, lap1, capacity);
+    return rc ? rc : download_single(ex, keypoints, descriptors, capacity, n_out, n_mono);
 }
 
 // ---- per-stage timing with CUDA events on the launching stream ---------------------------------------------------------
@@ -1779,34 +1704,30 @@ int orbx_extract_stereo(orbx_extractor* exL, orbx_extractor* exR, const uint8_t*
     if (capacity >= (1 << 20)) return fail(ORBX_ERR_UNSUPPORTED, "capacity %d: the stereo kernels index at most 2^20 - 1 rows", capacity);
     // vLappingArea = {0, 0} for both cameras of a rectified pair (src/Frame.cc:124-125)
     int rc;
-    if ((rc = enqueue_single(exL, imageL, rows, cols, step, 0, 0, capacity))) return rc;
-    if ((rc = enqueue_single(exR, imageR, rows, cols, step, 0, 0, capacity))) return rc;
+    if ((rc = enqueue_single(exL, imageL, rows, cols, step, 1, 0, 0, 0, capacity))) return rc;
+    if ((rc = enqueue_single(exR, imageR, rows, cols, step, 1, 0, 0, 0, capacity))) return rc;
     Slot& sL = exL->slots[0];
     Slot& sR = exR->slots[0];
-    // the matcher's outputs and scratch: slot 0's stereo staging (that of orbx_extract_stereo_batch), replaced only while the
-    // slot's stream is idle
-    if (!stereo_staging_fits(sL, 1, capacity)) {
-        CU(cudaStreamSynchronize(sL.stream));
-        if ((rc = ensure_stereo_staging(sL, 1, capacity))) return rc;
-    }
+    // the matcher's outputs and scratch: slot 0's stereo staging (that of orbx_extract_stereo_batch)
+    if ((rc = grow(exL, sL, sL.su, capacity)) || (rc = grow(exL, sL, sL.sd, capacity)) || (rc = grow(exL, sL, sL.sad, capacity))) return rc;
     StereoArgs A{};
     if ((rc = stereo_prepare(exL, 0, exR, 0, A))) return rc;          // (cannot fail after the checks above)
     // right side: its results go home on its own stream while the matcher runs
     CU(cudaEventRecord(sR.ev_done, sR.stream));
-    CU(cudaMemcpyAsync(kpR, sR.d_kps, sizeof(orbx_keypoint) * (size_t)capacity, cudaMemcpyDeviceToHost, sR.stream));
-    CU(cudaMemcpyAsync(descR, sR.d_desc, (size_t)capacity * 32, cudaMemcpyDeviceToHost, sR.stream));
-    CU(cudaMemcpyAsync(nR, sR.d_n, sizeof(int), cudaMemcpyDeviceToHost, sR.stream));
+    CU(cudaMemcpyAsync(kpR, sR.kps.p, sizeof(orbx_keypoint) * (size_t)capacity, cudaMemcpyDeviceToHost, sR.stream));
+    CU(cudaMemcpyAsync(descR, sR.desc.p, (size_t)capacity * 32, cudaMemcpyDeviceToHost, sR.stream));
+    CU(cudaMemcpyAsync(nR, sR.n.p, sizeof(int), cudaMemcpyDeviceToHost, sR.stream));
     // left side: wait for the right extraction, match on the device, then copy everything back
     CU(cudaStreamWaitEvent(sL.stream, sR.ev_done, 0));
-    A.kpL = sL.d_kps; A.descL = sL.d_desc; A.nL = capacity; A.d_nL = sL.d_n;
-    A.kpR = sR.d_kps; A.descR = sR.d_desc; A.nR = capacity; A.d_nR = sR.d_n;
-    A.bf = bf; A.maxD = maxD; A.uRight = sL.d_su; A.depth = sL.d_sd; A.sad = sL.d_sad;
+    A.kpL = sL.kps.p; A.descL = sL.desc.p; A.nL = capacity; A.d_nL = sL.n.p;
+    A.kpR = sR.kps.p; A.descR = sR.desc.p; A.nR = capacity; A.d_nR = sR.n.p;
+    A.bf = bf; A.maxD = maxD; A.uRight = sL.su.p; A.depth = sL.sd.p; A.sad = sL.sad.p;
     CU(launch_stereo(exL->fg, A, sL.stream));
-    CU(cudaMemcpyAsync(kpL, sL.d_kps, sizeof(orbx_keypoint) * (size_t)capacity, cudaMemcpyDeviceToHost, sL.stream));
-    CU(cudaMemcpyAsync(descL, sL.d_desc, (size_t)capacity * 32, cudaMemcpyDeviceToHost, sL.stream));
-    CU(cudaMemcpyAsync(nL, sL.d_n, sizeof(int), cudaMemcpyDeviceToHost, sL.stream));
-    CU(cudaMemcpyAsync(uRight, sL.d_su, sizeof(float) * (size_t)capacity, cudaMemcpyDeviceToHost, sL.stream));
-    CU(cudaMemcpyAsync(depth, sL.d_sd, sizeof(float) * (size_t)capacity, cudaMemcpyDeviceToHost, sL.stream));
+    CU(cudaMemcpyAsync(kpL, sL.kps.p, sizeof(orbx_keypoint) * (size_t)capacity, cudaMemcpyDeviceToHost, sL.stream));
+    CU(cudaMemcpyAsync(descL, sL.desc.p, (size_t)capacity * 32, cudaMemcpyDeviceToHost, sL.stream));
+    CU(cudaMemcpyAsync(nL, sL.n.p, sizeof(int), cudaMemcpyDeviceToHost, sL.stream));
+    CU(cudaMemcpyAsync(uRight, sL.su.p, sizeof(float) * (size_t)capacity, cudaMemcpyDeviceToHost, sL.stream));
+    CU(cudaMemcpyAsync(depth, sL.sd.p, sizeof(float) * (size_t)capacity, cudaMemcpyDeviceToHost, sL.stream));
     CU(cudaStreamSynchronize(sL.stream));
     CU(cudaStreamSynchronize(sR.stream));
     if (*nL > capacity || *nR > capacity) return fail(ORBX_ERR_CAPACITY, "%d / %d keypoints, capacity %d", *nL, *nR, capacity);
@@ -1842,7 +1763,7 @@ static StereoArgs stereo_chunk_args(const orbx_extractor* ex, const Slot& s, int
     A.frameL = 0; A.frameR = np; A.n_pairs = np;
     A.kpL = kpL; A.descL = descL; A.nL = capacity; A.d_nL = d_nL;
     A.kpR = kpR; A.descR = descR; A.nR = capacity; A.d_nR = d_nR;
-    A.bf = bf; A.maxD = maxD; A.uRight = uRight; A.depth = depth; A.sad = s.d_sad;
+    A.bf = bf; A.maxD = maxD; A.uRight = uRight; A.depth = depth; A.sad = s.sad.p;
     return A;
 }
 
@@ -1859,41 +1780,38 @@ int orbx_extract_stereo_batch(orbx_extractor* ex, const uint8_t* const* imagesL,
     if ((rc = configure(ex, rows, cols))) return rc;
     wait_user_work(ex);
     ex->last_frames = 0;
-    // orbx_extract_batch's chunking and ramp schedule, in whole pairs
-    const int chunk_frames = ex->max_batch > 0 ? std::min(ex->max_batch, 2 * n_pairs) : std::min(2 * n_pairs, 64);
-    const int chunk = std::max(chunk_frames / 2, 1);
+    // the chunking and ramp schedule of orbx_extract_batch, in whole pairs
+    const int chunk = std::max(chunk_frames(ex, 2 * n_pairs, true) / 2, 1);
     const std::vector<std::pair<int, int>> sched = chunk_schedule(n_pairs, chunk);   // (first pair, pairs)
-    const int nchunks = (int)sched.size();
-    const int nslots = std::min(nchunks, (int)orbx_extractor::kSlots);
+    const int nslots = std::min((int)sched.size(), (int)orbx_extractor::kSlots);
     if ((rc = ensure_capacity(ex, 2 * chunk, nslots))) return rc;
-    const size_t dpitch = (size_t)cols, dframe = dpitch * rows;
+    const size_t dpitch = (size_t)cols, dframe = dpitch * rows, rows_out = (size_t)chunk * capacity;
     for (int i = 0; i < nslots; ++i) {
         Slot& s = ex->slots[i];
-        if (s.d_in_bytes < dframe * 2 * chunk || s.out_cap < (size_t)2 * chunk * capacity || s.out_frames < 2 * chunk ||
-            !stereo_staging_fits(s, chunk, capacity))
-            CU(cudaStreamSynchronize(s.stream));
-        if ((rc = ensure_host_staging(s, dframe * 2 * chunk, 2 * chunk, capacity))) return rc;
-        if ((rc = ensure_stereo_staging(s, chunk, capacity))) return rc;
+        if ((rc = grow_extract_staging(ex, s, 2 * chunk, dframe, capacity)) || (rc = grow(ex, s, s.su, rows_out)) ||
+            (rc = grow(ex, s, s.sd, rows_out)) || (rc = grow(ex, s, s.sad, rows_out)))
+            return rc;
     }
     HostPipeline h;
+    h.item_frames = 2;
     h.upload = [&](Slot& s, int p0, int np, cudaStream_t ist) -> int {
-        int rc2 = upload_frames(imagesL, p0, np, s.d_in, dpitch, rows, step, ist);
-        return rc2 ? rc2 : upload_frames(imagesR, p0, np, s.d_in + (size_t)np * dframe, dpitch, rows, step, ist);
+        int rc2 = upload_frames(imagesL, p0, np, s.in.p, dpitch, rows, step, ist);
+        return rc2 ? rc2 : upload_frames(imagesR, p0, np, s.in.p + (size_t)np * dframe, dpitch, rows, step, ist);
     };
     h.compute = [&](Slot& s, int p0, int np, cudaStream_t cst) -> int {
         (void)p0;
         // the staging holds both sides back to back: one set of 2 np frames (vLappingArea = {0, 0}, src/Frame.cc:124-125)
-        int rc2 = run_chunk(ex, s, one_set_io(s.d_in, dframe, dpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), 2 * np, 0, 0, cst);
+        int rc2 = run_chunk(ex, s, one_set_io(s.in.p, dframe, dpitch, s.kps.p, s.desc.p, capacity, s.n.p, s.nm.p), 2 * np, 0, 0, cst);
         if (rc2) return rc2;
         const size_t r = (size_t)np * capacity;
-        const StereoArgs A = stereo_chunk_args(ex, s, np, s.d_kps, s.d_desc, s.d_n, s.d_kps + r, s.d_desc + r * 32, s.d_n + np, capacity, bf, maxD,
-                                               s.d_su, s.d_sd);
+        const StereoArgs A = stereo_chunk_args(ex, s, np, s.kps.p, s.desc.p, s.n.p, s.kps.p + r, s.desc.p + r * 32, s.n.p + np, capacity, bf, maxD,
+                                               s.su.p, s.sd.p);
         CU(launch_stereo(ex->fg, A, cst));
         return ORBX_OK;
     };
     h.counts = [&](Slot& s, int p0, int np, cudaStream_t ost) -> int {
-        CU(cudaMemcpyAsync(nL + p0, s.d_n, sizeof(int) * np, cudaMemcpyDeviceToHost, ost));
-        CU(cudaMemcpyAsync(nR + p0, s.d_n + np, sizeof(int) * np, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpyAsync(nL + p0, s.n.p, sizeof(int) * np, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpyAsync(nR + p0, s.n.p + np, sizeof(int) * np, cudaMemcpyDeviceToHost, ost));
         return ORBX_OK;
     };
     h.download = [&](Slot& s, int p0, int np, cudaStream_t ost) -> int {
@@ -1902,21 +1820,20 @@ int orbx_extract_stereo_batch(orbx_extractor* ex, const uint8_t* const* imagesL,
         const size_t kpitch = sizeof(orbx_keypoint) * (size_t)capacity, dpitch32 = (size_t)capacity * 32, fpitch = sizeof(float) * (size_t)capacity;
         const int rowsL = std::min(mxL, capacity), rowsR = std::min(mxR, capacity);   // a pair over capacity fails the call below
         if (rowsL > 0) {
-            CU(cudaMemcpy2DAsync(kpL + (size_t)p0 * capacity, kpitch, s.d_kps, kpitch, sizeof(orbx_keypoint) * (size_t)rowsL, np, cudaMemcpyDeviceToHost, ost));
-            CU(cudaMemcpy2DAsync(descL + (size_t)p0 * capacity * 32, dpitch32, s.d_desc, dpitch32, (size_t)rowsL * 32, np, cudaMemcpyDeviceToHost, ost));
-            CU(cudaMemcpy2DAsync(uRight + (size_t)p0 * capacity, fpitch, s.d_su, fpitch, sizeof(float) * (size_t)rowsL, np, cudaMemcpyDeviceToHost, ost));
-            CU(cudaMemcpy2DAsync(depth + (size_t)p0 * capacity, fpitch, s.d_sd, fpitch, sizeof(float) * (size_t)rowsL, np, cudaMemcpyDeviceToHost, ost));
+            CU(cudaMemcpy2DAsync(kpL + (size_t)p0 * capacity, kpitch, s.kps.p, kpitch, sizeof(orbx_keypoint) * (size_t)rowsL, np, cudaMemcpyDeviceToHost, ost));
+            CU(cudaMemcpy2DAsync(descL + (size_t)p0 * capacity * 32, dpitch32, s.desc.p, dpitch32, (size_t)rowsL * 32, np, cudaMemcpyDeviceToHost, ost));
+            CU(cudaMemcpy2DAsync(uRight + (size_t)p0 * capacity, fpitch, s.su.p, fpitch, sizeof(float) * (size_t)rowsL, np, cudaMemcpyDeviceToHost, ost));
+            CU(cudaMemcpy2DAsync(depth + (size_t)p0 * capacity, fpitch, s.sd.p, fpitch, sizeof(float) * (size_t)rowsL, np, cudaMemcpyDeviceToHost, ost));
         }
         if (rowsR > 0) {
-            CU(cudaMemcpy2DAsync(kpR + (size_t)p0 * capacity, kpitch, s.d_kps + (size_t)np * capacity, kpitch, sizeof(orbx_keypoint) * (size_t)rowsR, np,
+            CU(cudaMemcpy2DAsync(kpR + (size_t)p0 * capacity, kpitch, s.kps.p + (size_t)np * capacity, kpitch, sizeof(orbx_keypoint) * (size_t)rowsR, np,
                                  cudaMemcpyDeviceToHost, ost));
-            CU(cudaMemcpy2DAsync(descR + (size_t)p0 * capacity * 32, dpitch32, s.d_desc + (size_t)np * capacity * 32, dpitch32, (size_t)rowsR * 32, np,
+            CU(cudaMemcpy2DAsync(descR + (size_t)p0 * capacity * 32, dpitch32, s.desc.p + (size_t)np * capacity * 32, dpitch32, (size_t)rowsR * 32, np,
                                  cudaMemcpyDeviceToHost, ost));
         }
         return ORBX_OK;
     };
-    // the two pipelines of orbx_extract_batch, chosen by the chunk's frame count
-    if ((rc = run_host_pipeline(ex, sched, nslots, 2 * chunk >= 128, h))) return rc;
+    if ((rc = run_host_pipeline(ex, sched, nslots, chunk, h))) return rc;
     for (int p = 0; p < n_pairs; ++p)
         if (nL[p] > capacity || nR[p] > capacity)
             return fail(ORBX_ERR_CAPACITY, "pair %d has %d / %d keypoints, capacity %d", p, nL[p], nR[p], capacity);
@@ -1934,19 +1851,13 @@ int orbx_extract_stereo_batch_device(orbx_extractor* ex, const uint8_t* d_images
     if ((rc = set_device(ex->device))) return rc;
     if ((rc = configure(ex, rows, cols))) return rc;
     ex->last_frames = 0;
-    const int chunk_frames = ex->max_batch > 0 ? std::min(ex->max_batch, 2 * n_pairs) : std::min(2 * n_pairs, 256);
-    const int chunk = std::max(chunk_frames / 2, 1);
+    const int chunk = std::max(chunk_frames(ex, 2 * n_pairs, false) / 2, 1);
     if ((rc = ensure_capacity(ex, 2 * chunk, 1))) return rc;
     Slot& s = ex->slots[0];
-    if (!stereo_staging_fits(s, chunk, capacity)) {          // replaced below: earlier work on any stream must be done with it
-        wait_user_work(ex);
-        CU(cudaStreamSynchronize(s.stream));
-        if ((rc = ensure_stereo_staging(s, chunk, capacity))) return rc;
-    }
-    cudaStream_t st = stream ? (cudaStream_t)stream : s.stream;
-    if (!ex->ev_user) CU(cudaEventCreateWithFlags(&ex->ev_user, cudaEventDisableTiming));
-    if (ex->user_pending) CU(cudaStreamWaitEvent(st, ex->ev_user, 0));
-    if (st != s.stream) { CU(cudaEventRecord(s.ev_done, s.stream)); CU(cudaStreamWaitEvent(st, s.ev_done, 0)); }
+    // the matcher's SAD scratch and the extraction's monoIndex (stereo outputs have no n_mono)
+    if ((rc = grow(ex, s, s.sad, (size_t)chunk * capacity)) || (rc = grow(ex, s, s.snm, 2 * (size_t)chunk))) return rc;
+    cudaStream_t st;
+    if ((rc = begin_caller_stream(ex, stream, &st))) return rc;
     for (int p0 = 0; p0 < n_pairs; p0 += chunk) {
         const int np = std::min(chunk, n_pairs - p0);
         const size_t r = (size_t)p0 * capacity;
@@ -1956,15 +1867,14 @@ int orbx_extract_stereo_batch_device(orbx_extractor* ex, const uint8_t* d_images
         io.img0 = d_imagesL + (size_t)p0 * frame_stride; io.img1 = d_imagesR + (size_t)p0 * frame_stride;
         io.frame_stride = frame_stride; io.pitch = pitch;
         io.kps0 = d_kpL + r; io.kps1 = d_kpR + r; io.desc0 = d_descL + r * 32; io.desc1 = d_descR + r * 32;
-        io.n_out0 = d_nL + p0; io.n_out1 = d_nR + p0; io.n_mono0 = s.d_snm; io.n_mono1 = s.d_snm + np;
+        io.n_out0 = d_nL + p0; io.n_out1 = d_nR + p0; io.n_mono0 = s.snm.p; io.n_mono1 = s.snm.p + np;
         io.capacity = capacity; io.split = np;
         if ((rc = run_chunk(ex, s, io, 2 * np, 0, 0, st))) return rc;
         const StereoArgs A = stereo_chunk_args(ex, s, np, d_kpL + r, d_descL + r * 32, d_nL + p0, d_kpR + r, d_descR + r * 32, d_nR + p0,
                                                capacity, bf, maxD, d_uRight + r, d_depth + r);
         CU(launch_stereo(ex->fg, A, st));
     }
-    if (st != s.stream) { CU(cudaEventRecord(ex->ev_user, st)); ex->user_pending = true; }
-    return ORBX_OK;
+    return end_caller_stream(ex, st);
 }
 
 // ---- RGB-D frames -------------------------------------------------------------------------------------------------------
@@ -2008,32 +1918,29 @@ int orbx_extract_rgbd(orbx_extractor* ex, const uint8_t* image, int rows, int co
     RgbdArgs A;
     int rc = rgbd_args(calib, depth_type, depth_step, cols, A);
     if (rc) return rc;
-    rc = channels == 1 ? enqueue_single(ex, image, rows, cols, step, 0, 0, capacity)
-                       : enqueue_color(ex, image, rows, cols, step, channels, rgb, 0, 0, capacity);
-    if (rc) return rc;
+    if ((rc = enqueue_single(ex, image, rows, cols, step, channels, rgb, 0, 0, capacity))) return rc;
     Slot& s = ex->slots[0];
     const size_t zpitch = (size_t)cols * (depth_type == 0 ? 2 : 4), zbytes = zpitch * rows;
-    if (!rgbd_staging_fits(s, zbytes, (size_t)capacity) || !stereo_staging_fits(s, 1, capacity)) {   // grow-only: replaced while idle
-        CU(cudaStreamSynchronize(s.stream));
-        if ((rc = ensure_rgbd_staging(s, zbytes, (size_t)capacity)) || (rc = ensure_stereo_staging(s, 1, capacity))) return rc;
-    }
+    if ((rc = grow(ex, s, s.depth, zbytes)) || (rc = grow(ex, s, s.kpun, capacity)) || (rc = grow(ex, s, s.su, capacity)) ||
+        (rc = grow(ex, s, s.sd, capacity)))
+        return rc;
     // the depth map goes up beside the extraction; an event joins it in front of the RGB-D kernel
     if (!ex->depth_stream) CU(cudaStreamCreateWithFlags(&ex->depth_stream, cudaStreamNonBlocking));
     if (!ex->ev_depth) CU(cudaEventCreateWithFlags(&ex->ev_depth, cudaEventDisableTiming));
-    CU(cudaMemcpy2DAsync(s.d_depth, zpitch, depth, depth_step, zpitch, rows, cudaMemcpyHostToDevice, ex->depth_stream));
+    CU(cudaMemcpy2DAsync(s.depth.p, zpitch, depth, depth_step, zpitch, rows, cudaMemcpyHostToDevice, ex->depth_stream));
     CU(cudaEventRecord(ex->ev_depth, ex->depth_stream));
     CU(cudaStreamWaitEvent(s.stream, ex->ev_depth, 0));
-    A.kp = s.d_kps; A.n = s.d_n; A.capacity = capacity;
-    A.kp_un = s.d_kpun; A.uRight = s.d_su; A.depth_out = s.d_sd;
-    A.depth = s.d_depth; A.depth_pitch = zpitch; A.depth_frame_stride = zbytes;
+    A.kp = s.kps.p; A.n = s.n.p; A.capacity = capacity;
+    A.kp_un = s.kpun.p; A.uRight = s.su.p; A.depth_out = s.sd.p;
+    A.depth = s.depth.p; A.depth_pitch = zpitch; A.depth_frame_stride = zbytes;
     CU(launch_rgbd_frame(A, 1, s.stream));
     const size_t kb = sizeof(orbx_keypoint) * (size_t)capacity, fb = sizeof(float) * (size_t)capacity;
-    CU(cudaMemcpyAsync(kp, s.d_kps, kb, cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(desc, s.d_desc, (size_t)capacity * 32, cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(kp_un, s.d_kpun, kb, cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(uRight, s.d_su, fb, cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(depth_out, s.d_sd, fb, cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(n_out, s.d_n, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(kp, s.kps.p, kb, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(desc, s.desc.p, (size_t)capacity * 32, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(kp_un, s.kpun.p, kb, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(uRight, s.su.p, fb, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(depth_out, s.sd.p, fb, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(n_out, s.n.p, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
     CU(cudaStreamSynchronize(s.stream));
     if (*n_out > capacity) return fail(ORBX_ERR_CAPACITY, "frame has %d keypoints, capacity %d", *n_out, capacity);
     return ORBX_OK;
@@ -2061,8 +1968,8 @@ int orbx_extract_rgbd_batch(orbx_extractor* ex, const uint8_t* const* images, co
     if ((rc = configure(ex, rows, cols))) return rc;
     wait_user_work(ex);
     ex->last_frames = 0;
-    // orbx_extract_batch's chunking and ramp schedule
-    const int chunk = ex->max_batch > 0 ? std::min(ex->max_batch, n_frames) : std::min(n_frames, 64);
+    // the chunking and ramp schedule of orbx_extract_batch
+    const int chunk = chunk_frames(ex, n_frames, true);
     const std::vector<std::pair<int, int>> sched = chunk_schedule(n_frames, chunk);   // (first frame, frames)
     const int nslots = std::min((int)sched.size(), (int)orbx_extractor::kSlots);
     if ((rc = ensure_capacity(ex, chunk, nslots))) return rc;
@@ -2071,31 +1978,28 @@ int orbx_extract_rgbd_batch(orbx_extractor* ex, const uint8_t* const* images, co
     const size_t rows_out = (size_t)chunk * capacity;
     for (int i = 0; i < nslots; ++i) {
         Slot& s = ex->slots[i];
-        if (s.d_in_bytes < dframe * chunk || s.out_cap < rows_out || s.out_frames < chunk || !rgbd_staging_fits(s, zframe * chunk, rows_out) ||
-            !stereo_staging_fits(s, chunk, capacity))
-            CU(cudaStreamSynchronize(s.stream));
-        if ((rc = ensure_host_staging(s, dframe * chunk, chunk, capacity))) return rc;
-        if ((rc = ensure_rgbd_staging(s, zframe * chunk, rows_out))) return rc;
-        if ((rc = ensure_stereo_staging(s, chunk, capacity))) return rc;
+        if ((rc = grow_extract_staging(ex, s, chunk, dframe, capacity)) || (rc = grow(ex, s, s.depth, zframe * chunk)) ||
+            (rc = grow(ex, s, s.kpun, rows_out)) || (rc = grow(ex, s, s.su, rows_out)) || (rc = grow(ex, s, s.sd, rows_out)))
+            return rc;
     }
     HostPipeline h;
     h.upload = [&](Slot& s, int f0, int nf, cudaStream_t ist) -> int {
-        int rc2 = upload_frames(images, f0, nf, s.d_in, dpitch, rows, step, ist);
-        return rc2 ? rc2 : upload_frames(depths, f0, nf, s.d_depth, zpitch, rows, depth_step, ist);
+        int rc2 = upload_frames(images, f0, nf, s.in.p, dpitch, rows, step, ist);
+        return rc2 ? rc2 : upload_frames(depths, f0, nf, s.depth.p, zpitch, rows, depth_step, ist);
     };
     h.compute = [&](Slot& s, int f0, int nf, cudaStream_t cst) -> int {
         (void)f0;
-        int rc2 = run_chunk(ex, s, one_set_io(s.d_in, dframe, dpitch, s.d_kps, s.d_desc, capacity, s.d_n, s.d_nm), nf, 0, 0, cst);
+        int rc2 = run_chunk(ex, s, one_set_io(s.in.p, dframe, dpitch, s.kps.p, s.desc.p, capacity, s.n.p, s.nm.p), nf, 0, 0, cst);
         if (rc2) return rc2;
         RgbdArgs a = A;
-        a.kp = s.d_kps; a.n = s.d_n; a.capacity = capacity;
-        a.kp_un = s.d_kpun; a.uRight = s.d_su; a.depth_out = s.d_sd;
-        a.depth = s.d_depth; a.depth_pitch = zpitch; a.depth_frame_stride = zframe;
+        a.kp = s.kps.p; a.n = s.n.p; a.capacity = capacity;
+        a.kp_un = s.kpun.p; a.uRight = s.su.p; a.depth_out = s.sd.p;
+        a.depth = s.depth.p; a.depth_pitch = zpitch; a.depth_frame_stride = zframe;
         CU(launch_rgbd_frame(a, nf, cst));
         return ORBX_OK;
     };
     h.counts = [&](Slot& s, int f0, int nf, cudaStream_t ost) -> int {
-        CU(cudaMemcpyAsync(n_out + f0, s.d_n, sizeof(int) * nf, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpyAsync(n_out + f0, s.n.p, sizeof(int) * nf, cudaMemcpyDeviceToHost, ost));
         return ORBX_OK;
     };
     h.download = [&](Slot& s, int f0, int nf, cudaStream_t ost) -> int {
@@ -2105,14 +2009,14 @@ int orbx_extract_rgbd_batch(orbx_extractor* ex, const uint8_t* const* images, co
         if (r == 0) return ORBX_OK;
         const size_t kpitch = sizeof(orbx_keypoint) * (size_t)capacity, dpitch32 = (size_t)capacity * 32, fpitch = sizeof(float) * (size_t)capacity;
         const size_t o = (size_t)f0 * capacity;
-        CU(cudaMemcpy2DAsync(kp + o, kpitch, s.d_kps, kpitch, sizeof(orbx_keypoint) * r, nf, cudaMemcpyDeviceToHost, ost));
-        CU(cudaMemcpy2DAsync(desc + o * 32, dpitch32, s.d_desc, dpitch32, r * 32, nf, cudaMemcpyDeviceToHost, ost));
-        CU(cudaMemcpy2DAsync(kp_un + o, kpitch, s.d_kpun, kpitch, sizeof(orbx_keypoint) * r, nf, cudaMemcpyDeviceToHost, ost));
-        CU(cudaMemcpy2DAsync(uRight + o, fpitch, s.d_su, fpitch, sizeof(float) * r, nf, cudaMemcpyDeviceToHost, ost));
-        CU(cudaMemcpy2DAsync(depth_out + o, fpitch, s.d_sd, fpitch, sizeof(float) * r, nf, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpy2DAsync(kp + o, kpitch, s.kps.p, kpitch, sizeof(orbx_keypoint) * r, nf, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpy2DAsync(desc + o * 32, dpitch32, s.desc.p, dpitch32, r * 32, nf, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpy2DAsync(kp_un + o, kpitch, s.kpun.p, kpitch, sizeof(orbx_keypoint) * r, nf, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpy2DAsync(uRight + o, fpitch, s.su.p, fpitch, sizeof(float) * r, nf, cudaMemcpyDeviceToHost, ost));
+        CU(cudaMemcpy2DAsync(depth_out + o, fpitch, s.sd.p, fpitch, sizeof(float) * r, nf, cudaMemcpyDeviceToHost, ost));
         return ORBX_OK;
     };
-    if ((rc = run_host_pipeline(ex, sched, nslots, chunk >= 128, h))) return rc;
+    if ((rc = run_host_pipeline(ex, sched, nslots, chunk, h))) return rc;
     for (int f = 0; f < n_frames; ++f)
         if (n_out[f] > capacity) return fail(ORBX_ERR_CAPACITY, "frame %d has %d keypoints, capacity %d", f, n_out[f], capacity);
     return ORBX_OK;
@@ -2138,24 +2042,17 @@ int orbx_extract_rgbd_batch_device(orbx_extractor* ex, const uint8_t* d_images, 
     if ((rc = set_device(ex->device))) return rc;
     if ((rc = configure(ex, rows, cols))) return rc;
     ex->last_frames = 0;
-    const int chunk = ex->max_batch > 0 ? std::min(ex->max_batch, n_frames) : std::min(n_frames, 256);
+    const int chunk = chunk_frames(ex, n_frames, false);
     if ((rc = ensure_capacity(ex, chunk, 1))) return rc;
     Slot& s = ex->slots[0];
-    // the extraction's monoIndex goes to the stereo staging's d_snm (2 * pairs counts; RGB-D outputs have no n_mono)
-    if (!stereo_staging_fits(s, chunk, 0)) {          // replaced below: earlier work on any stream must be done with it
-        wait_user_work(ex);
-        CU(cudaStreamSynchronize(s.stream));
-        if ((rc = ensure_stereo_staging(s, chunk, 0))) return rc;
-    }
-    cudaStream_t st = stream ? (cudaStream_t)stream : s.stream;
-    if (!ex->ev_user) CU(cudaEventCreateWithFlags(&ex->ev_user, cudaEventDisableTiming));
-    if (ex->user_pending) CU(cudaStreamWaitEvent(st, ex->ev_user, 0));
-    if (st != s.stream) { CU(cudaEventRecord(s.ev_done, s.stream)); CU(cudaStreamWaitEvent(st, s.ev_done, 0)); }
+    if ((rc = grow(ex, s, s.snm, (size_t)chunk))) return rc;     // the extraction's monoIndex (RGB-D outputs have no n_mono)
+    cudaStream_t st;
+    if ((rc = begin_caller_stream(ex, stream, &st))) return rc;
     for (int f0 = 0; f0 < n_frames; f0 += chunk) {
         const int nf = std::min(chunk, n_frames - f0);
         const size_t r = (size_t)f0 * capacity;
         if ((rc = run_chunk(ex, s, one_set_io(d_images + (size_t)f0 * frame_stride, frame_stride, pitch, d_kp + r, d_desc + r * 32, capacity,
-                                              d_n_out + f0, s.d_snm), nf, 0, 0, st)))
+                                              d_n_out + f0, s.snm.p), nf, 0, 0, st)))
             return rc;
         RgbdArgs a = A;
         a.kp = d_kp + r; a.n = d_n_out + f0; a.capacity = capacity;
@@ -2163,8 +2060,7 @@ int orbx_extract_rgbd_batch_device(orbx_extractor* ex, const uint8_t* d_images, 
         a.depth = (const uint8_t*)d_depths + (size_t)f0 * depth_frame_stride; a.depth_pitch = depth_pitch; a.depth_frame_stride = depth_frame_stride;
         CU(launch_rgbd_frame(a, nf, st));
     }
-    if (st != s.stream) { CU(cudaEventRecord(ex->ev_user, st)); ex->user_pending = true; }
-    return ORBX_OK;
+    return end_caller_stream(ex, st);
 }
 
 // ---- measurement ------------------------------------------------------------------------------------------------------
